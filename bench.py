@@ -12,6 +12,9 @@ BGZF inflate -> CRC -> record scan -> record facets + coverage scatter (per wave
   parity  the TIMED runs' own result buffers (last resident step and last e2e step, after the NCCL merge at N>1)
           are compared with the committed full-size golden of the workload (tests/golden/fullsize_*.npz: the
           oracle's integers over exactly these shard files); a difference fails the run.
+  --dump-outputs DIR   the last timed resident step's results (every integer array the C ABI returns, as float64)
+          go to DIR/<name>.npy.  The synthetic inputs are seeded, so two builds run with the same arguments can be
+          compared file for file.
   --impl reference   the CPU oracle (restatement of the reference's single-threaded algorithm;
           the Rust reference cannot be built in this image) on a bounded sample, rank 0 only.
 
@@ -50,7 +53,12 @@ def parse_args():
     p.add_argument("--no-crc", action="store_true", help="skip the per-block CRC32 check (reference verifies it)")
     p.add_argument("--no-e2e", action="store_true")
     p.add_argument("--no-cpu", action="store_true")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write the results of the last timed device-resident step to DIR/<name>.npy (float64)")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    return args
 
 
 def measured_peak():
@@ -163,6 +171,35 @@ def lpt_partition(weights, n_parts):
         parts[k].append(c)
         loads[k] += weights[c]
     return parts, loads
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(res, out_dir):
+    """Writes the integer results a caller of the engine receives (helpers.collect) as float64 .npy files, so that two
+    builds can be compared output for output.  Every count is below 2**53, so float64 holds it exactly."""
+    arrays = {}
+    if "general" in res:
+        arrays.update(general=res["general"], tlen_hist=res["tlen_hist"], tlen_counts=[res["tlen_processed"], res["tlen_ignored"]],
+                      gc_hist=res["gc_hist"], gc_nuc=res["gc_nuc"], gc_rec=res["gc_rec"], quality=res["quality"])
+    if "coverage" in res:
+        contigs = sorted(res["coverage"])
+        cov = [res["coverage"][c] for c in contigs]
+        arrays.update(coverage_contigs=contigs, coverage_hist=np.array([v["hist"] for v in cov], dtype=np.uint64).reshape(len(cov), 2049),
+                      coverage_too_large=[v["too_large"] for v in cov], coverage_n_bins=[len(v["bin_sums"]) for v in cov],
+                      coverage_bin_sums=np.concatenate([v["bin_sums"] for v in cov]) if cov else [],
+                      nonsensical=[res["nonsensical"]])
+    arrays = {k: np.asarray(v, dtype=np.uint64) for k, v in arrays.items()}
+    for k, a in arrays.items():
+        if a.size and int(a.max()) >= 1 << 53:
+            raise SystemExit(f"--dump-outputs: {k} holds a count that float64 cannot represent exactly")
+    total = sum(8 * a.size for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of results exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a.astype(np.float64))
 
 
 def cpu_sample(args, wl):
@@ -407,6 +444,8 @@ def main():
     clocks = sampler.stop()
     dev_step_ms = float(np.mean(dev_ms))
     res_resident = collect(eng, lens, enabled, wl["records"], wl["coverage"])  # the last TIMED step's own results
+    if args.dump_outputs and rank == 0:  # after the NCCL merge, rank 0 holds the results of the whole logical BAM
+        dump_outputs(res_resident, args.dump_outputs)
 
     # ---- timed: end to end from pinned host memory ----
     log(f"resident steps done: {dev_step_ms:.1f} ms/step")
