@@ -8,10 +8,9 @@
 // (cov_scan_tiles) and one streaming pass (cov_resolve: per tile a local scan fused with the run-length
 // aggregated, shared-memory privatised histogram and the bin sums).  HBM-bound: 4 B/position.
 //
-// cov_resolve_kernel<kBulk>: the tile reaches the CTA either by per-thread 128-bit loads (kBulk = false) or by
-// one cp.async.bulk (TMA 1-D bulk copy, SASS UBLKCP) per 16 KB tile into a double-buffered shared-memory
-// stage, completion on an mbarrier (kBulk = true).  Which one ships is decided by the ncu A/B in
-// profiles/ (DESIGN.md section 4).
+// cov_resolve_kernel: each 16 KB tile reaches the CTA by one cp.async.bulk (TMA 1-D bulk copy, SASS UBLKCP)
+// into a double-buffered shared-memory stage, completion on an mbarrier.  Against per-thread 128-bit loads
+// it removes the long-scoreboard stall and is 2.6 % faster on a B200 (profiles/round2_coverage_bulk_ab.md).
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>
@@ -90,7 +89,6 @@ __device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, u
 }
 
 // Persistent CTAs loop over tiles; slot = this contig's [touched, too_large, hist[2049], bins[]].
-template <bool kBulk>
 __global__ void __launch_bounds__(kCovThreads)
 cov_resolve_kernel(const int32_t* __restrict__ diff, uint32_t n, const int64_t* __restrict__ tile_base, uint32_t n_tiles,
                    uint64_t* __restrict__ slot) {
@@ -98,10 +96,10 @@ cov_resolve_kernel(const int32_t* __restrict__ diff, uint32_t n, const int64_t* 
   __shared__ uint32_t hist[2050];  // [2049] = deeper than 2048
   __shared__ int64_t ws[kCovThreads / 32];
   __shared__ unsigned long long bsum[2];
-  __shared__ __align__(128) int32_t stage[kBulk ? 2 : 1][kBulk ? kCovTile : 4];
+  __shared__ __align__(128) int32_t stage[2][kCovTile];
   __shared__ __align__(8) uint64_t bar[2];
   for (uint32_t i = threadIdx.x; i < 2050; i += blockDim.x) hist[i] = 0;
-  if (kBulk && threadIdx.x == 0) {
+  if (threadIdx.x == 0) {
     mbar_init(&bar[0], 1);
     mbar_init(&bar[1], 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -110,7 +108,7 @@ cov_resolve_kernel(const int32_t* __restrict__ diff, uint32_t n, const int64_t* 
   const uint32_t lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   // bytes of tile t in the array, rounded up to the 16 bytes a bulk copy moves (the array is padded: engine.cu)
   auto tile_bytes = [&](uint32_t t) { const uint32_t left = n - t * kCovTile; return ((left < (uint32_t)kCovTile ? left : (uint32_t)kCovTile) * 4u + 15u) & ~15u; };
-  if (kBulk && threadIdx.x == 0 && blockIdx.x < n_tiles) {
+  if (threadIdx.x == 0 && blockIdx.x < n_tiles) {
     mbar_expect_tx(&bar[0], tile_bytes(blockIdx.x));
     bulk_g2s(stage[0], diff + (size_t)blockIdx.x * kCovTile, tile_bytes(blockIdx.x), &bar[0]);
   }
@@ -118,35 +116,21 @@ cov_resolve_kernel(const int32_t* __restrict__ diff, uint32_t n, const int64_t* 
   for (uint32_t t = blockIdx.x; t < n_tiles; t += gridDim.x, ++it) {
     const uint32_t p0 = t * kCovTile + threadIdx.x * kCovPerThread;  // first position of this thread
     int32_t v[kCovPerThread];
-    if (kBulk) {
-      const uint32_t buf = it & 1;
-      // the next tile streams into the other stage while this one is consumed (every thread left that stage at the
-      // __syncthreads() that closed the previous iteration)
-      const uint32_t tn = t + gridDim.x;
-      if (threadIdx.x == 0 && tn < n_tiles) {
-        mbar_expect_tx(&bar[buf ^ 1], tile_bytes(tn));
-        bulk_g2s(stage[buf ^ 1], diff + (size_t)tn * kCovTile, tile_bytes(tn), &bar[buf ^ 1]);
-      }
-      mbar_wait(&bar[buf], (it >> 1) & 1);
-      const int4* sp = reinterpret_cast<const int4*>(&stage[buf][threadIdx.x * kCovPerThread]);
+    const uint32_t buf = it & 1;
+    // the next tile streams into the other stage while this one is consumed (every thread left that stage at the
+    // __syncthreads() that closed the previous iteration)
+    const uint32_t tn = t + gridDim.x;
+    if (threadIdx.x == 0 && tn < n_tiles) {
+      mbar_expect_tx(&bar[buf ^ 1], tile_bytes(tn));
+      bulk_g2s(stage[buf ^ 1], diff + (size_t)tn * kCovTile, tile_bytes(tn), &bar[buf ^ 1]);
+    }
+    mbar_wait(&bar[buf], (it >> 1) & 1);
+    const int4* sp = reinterpret_cast<const int4*>(&stage[buf][threadIdx.x * kCovPerThread]);
 #pragma unroll
-      for (int k = 0; k < kCovPerThread; k += 4) {
-        const int4 q = sp[k / 4];
-        const uint32_t i = p0 + k;
-        v[k] = i < n ? q.x : 0; v[k + 1] = i + 1 < n ? q.y : 0; v[k + 2] = i + 2 < n ? q.z : 0; v[k + 3] = i + 3 < n ? q.w : 0;
-      }
-    } else {
-#pragma unroll
-      for (int k = 0; k < kCovPerThread; k += 4) {
-        uint32_t i = p0 + k;
-        if (i + 3 < n) {
-          int4 q = *reinterpret_cast<const int4*>(diff + i);
-          v[k] = q.x; v[k + 1] = q.y; v[k + 2] = q.z; v[k + 3] = q.w;
-        } else {
-#pragma unroll
-          for (int j = 0; j < 4; ++j) v[k + j] = (i + j < n) ? diff[i + j] : 0;
-        }
-      }
+    for (int k = 0; k < kCovPerThread; k += 4) {
+      const int4 q = sp[k / 4];
+      const uint32_t i = p0 + k;
+      v[k] = i < n ? q.x : 0; v[k + 1] = i + 1 < n ? q.y : 0; v[k + 2] = i + 2 < n ? q.z : 0; v[k + 3] = i + 3 < n ? q.w : 0;
     }
     int64_t tsum = 0;
 #pragma unroll

@@ -105,7 +105,6 @@ struct ngsq_engine {
   bool trace = false;                // NGSQ_TRACE=1: per-wave and per-chunk timeline on stderr at ngsq_finish
   std::vector<double> host_ms;       // host clock at every wave launch (trace)
   double host_t0 = 0;
-  bool cov_bulk = true;              // cov_resolve_kernel<true>: cp.async.bulk staging (NGSQ_COV_BULK=0 selects the direct loads)
 
   // results: [fixed | per-contig coverage slots | quality table, qpos_cap rows]
   uint64_t* d_res = nullptr;
@@ -783,7 +782,6 @@ int ngsq_create(int device, const ngsq_config* cfg, ngsq_engine** out) {
   if (cfg) memcpy(&ne->cfg, cfg, std::min<size_t>(cfg->struct_size ? cfg->struct_size : sizeof(ngsq_config), sizeof(ngsq_config)));
   if (!ne->cfg.flags) ne->cfg.flags = NGSQ_F_RECORD_FACETS | NGSQ_F_COVERAGE;
   if (const char* v = getenv("NGSQ_TRACE")) ne->trace = atoi(v) != 0;
-  if (const char* v = getenv("NGSQ_COV_BULK")) ne->cov_bulk = atoi(v) != 0;  // A/B switch for profiles/ (default: the measured winner)
   ne->headroom = ne->cfg.carry_bytes ? ((ne->cfg.carry_bytes + 63u) & ~63u) : kDefaultHeadroom;
   e = ne;
   auto bail = [&](int code) { std::string m = e->err; ngsq_destroy(e); g_create_err = m; return code; };
@@ -1233,8 +1231,7 @@ int ngsq_finish(ngsq_engine* e) {
       uint64_t* slot = e->d_res + e->cov_slot[c];
       cov_scan_tiles_kernel<<<1, 1024, 0, s>>>(e->d_tile_sum + e->tile_off[c], e->d_tile, n_tiles, slot + COV_TOUCHED);
       const uint32_t grid = std::min<uint32_t>(n_tiles, e->n_sm * 4);
-      if (e->cov_bulk) cov_resolve_kernel<true><<<grid, kCovThreads, 0, s>>>(df, n, e->d_tile, n_tiles, slot);
-      else cov_resolve_kernel<false><<<grid, kCovThreads, 0, s>>>(df, n, e->d_tile, n_tiles, slot);
+      cov_resolve_kernel<<<grid, kCovThreads, 0, s>>>(df, n, e->d_tile, n_tiles, slot);
       e->other_launches += 2;
     }
     CU(cudaGetLastError());

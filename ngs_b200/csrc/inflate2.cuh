@@ -21,11 +21,7 @@
 namespace ngsq {
 
 constexpr int kDecBatch = 32;  // symbols per lane between header / overrun checks
-#if NGSQ_DEC_VARIANT & 8
-constexpr int kDecWarps = 18;  // 18 x 32 x 396 B of slabs (+ 256 B of static shared memory with variant 1)
-#else
-constexpr int kDecWarps = (227 * 1024 / kSlabBytes) / 32 > 17 ? 17 : (227 * 1024 / kSlabBytes) / 32;  // 17 x 32 x 420 B of slabs; 120 registers per thread
-#endif
+constexpr int kDecWarps = 18;  // 18 x 32 x 396 B of slabs + 256 B of static shared memory (s_base_lut)
 constexpr int kDecThreads = kDecWarps * 32;
 constexpr size_t kDecSmem = (size_t)kDecThreads * kSlabBytes;
 
@@ -37,12 +33,10 @@ inflate_decode_kernel(uint8_t* __restrict__ out, const BlockDesc* __restrict__ b
   Lane L;
   L.slab = smem_raw + (size_t)threadIdx.x * kSlabBytes;
   L.state = LS_IDLE;
-#if NGSQ_DEC_VARIANT & 1
   __shared__ uint32_t s_base_lut[64];
   if (threadIdx.x < 64) s_base_lut[threadIdx.x] = base_lut_entry(threadIdx.x);
   __syncthreads();
   L.lut = s_base_lut;
-#endif
   // First batch of every warp: static and interleaved over the CTAs (warp w of CTA c takes batch w * grid + c), so that a
   // partial wave — the tail of a run — spreads over all SMs with few warps each instead of filling a few SMs with 18: a
   // lane decodes its block serially, and a warp that shares its scheduler with four others runs at a fraction of the
@@ -77,18 +71,10 @@ inflate_decode_kernel(uint8_t* __restrict__ out, const BlockDesc* __restrict__ b
   }
 }
 
-// Resolve variants (bit mask, -DNGSQ_RES_VARIANT=n; measured on a B200, 30 M records: 0 -> 29.3 ms, 1 -> 25.7 ms; default 1):
-//   1  dependency masks from the bitmap's ranks (two popcounts over the super-window's bitmap words + one look at the
-//      preceding token) instead of two 6-step binary searches by shuffle: 2 shared-memory loads + 1 shuffle instead of 12 shuffles, the same masks
-//      (tools/inflate_model.cpp checks the equality on every batch)
-//   2  the 1024-byte super-window is staged in shared memory: coalesced 128-bit loads in, tokens / near sources / match bytes
-//      read and written on chip, coalesced 128-bit stores out.  The kernel's L1/L2 transactions are its byte-granular
-//      stores (one per output byte); sources before the window come from global memory (final bytes of earlier windows),
-//      bytes of a match that runs past the window go to global memory directly
-#ifndef NGSQ_RES_VARIANT
-#define NGSQ_RES_VARIANT 1
-#endif
-
+// The resolve kernel's dependency masks come from the bitmap's ranks (two popcounts over the super-window's bitmap words +
+// one look at the preceding token): 2 shared-memory loads + 1 shuffle instead of the 12 shuffles of two binary searches
+// over the lanes' destinations, which give the same masks (tools/inflate_model.cpp checks the equality on every batch).
+// Measured on a B200, 30 M records: 29.3 -> 25.7 ms (profiles/round2_ab_inflate_variants.md).
 constexpr int kResThreads = 256;
 constexpr int kResWarps = kResThreads / 32;
 constexpr int kResList = 352;  // matches that can start inside 1024 bytes (every match is >= 3 bytes)
@@ -131,47 +117,11 @@ __device__ __forceinline__ void resolve_copy(uint8_t* dst, uint32_t mlen, uint32
   }
 }
 
-// the same copy with the window [w0, w1) of the block staged at wptr (shared memory); ob = the block in global memory
-__device__ __forceinline__ void resolve_copy_win(uint8_t* ob, uint8_t* wptr, uint32_t w0, uint32_t w1, uint32_t pos, uint32_t mlen, uint32_t dist) {
-  uint32_t D = dist;
-  for (uint32_t done = 0; done < mlen;) {
-    const uint32_t n = min(min(8u, D), mlen - done);
-    const uint32_t d0 = pos + done, s0 = d0 - D;  // block-relative
-    uint2 v;
-    if (s0 >= w0 && s0 + n <= w1) v = load8_unaligned(wptr + (s0 - w0), n);
-    else if (s0 + n <= w0 || s0 >= w1) v = load8_unaligned(ob + s0, n);  // before the window, or the tail of a match that ran past it
-    else {  // the source straddles an end of the window
-      v = make_uint2(0, 0);
-      for (uint32_t k = 0; k < n; ++k) {
-        const uint32_t byte = (s0 + k >= w0 && s0 + k < w1) ? wptr[s0 + k - w0] : ob[s0 + k];
-        if (k < 4) v.x |= byte << (8 * k); else v.y |= byte << (8 * (k - 4));
-      }
-    }
-    if (d0 + n <= w1) store_bytes(wptr + (d0 - w0), v, n);
-    else {  // the match runs past the window: those bytes are read back when the next window is staged
-      for (uint32_t k = 0; k < n; ++k) {
-        const uint8_t byte = (uint8_t)(k < 4 ? v.x >> (8 * k) : v.y >> (8 * (k - 4)));
-        if (d0 + k < w1) wptr[d0 + k - w0] = byte; else ob[d0 + k] = byte;
-      }
-    }
-    done += n;
-    if (D < 8) D <<= 1;
-  }
-}
-
-constexpr int kResWin = 1024;
-constexpr int kResStage = kResWin + 32;  // the window at any 16-byte phase
-
 __global__ void __launch_bounds__(kResThreads)
 inflate_resolve_kernel(uint8_t* __restrict__ out, const BlockDesc* __restrict__ blocks, uint32_t n_blocks,
                        const uint32_t* __restrict__ bitmap, const uint32_t* __restrict__ status) {
   __shared__ uint16_t s_pos[kResWarps][kResList];
-#if NGSQ_RES_VARIANT & 1
   __shared__ uint2 s_rank[kResWarps][32];
-#endif
-#if NGSQ_RES_VARIANT & 2
-  __shared__ __align__(16) uint8_t s_win[kResWarps][kResStage];
-#endif
   const uint32_t lane = threadIdx.x & 31, wic = threadIdx.x >> 5;
   const uint32_t n_warps = gridDim.x * kResWarps;
   uint16_t* list = s_pos[wic];
@@ -193,40 +143,22 @@ inflate_resolve_kernel(uint8_t* __restrict__ out, const BlockDesc* __restrict__ 
       const uint32_t total = __shfl_sync(0xFFFFFFFFu, incl, 31);
       if (!total) continue;
       uint32_t o = incl - cnt;
-#if NGSQ_RES_VARIANT & 1
       // entry w: bitmap word w of this super-window and the number of matches that start before it (shared memory
       // rather than shuffles: the kernel runs at 32 registers per thread for full occupancy)
       s_rank[wic][lane] = make_uint2(word, o);
-#endif
       const uint32_t pbase = (sw << 10) + (lane << 5);
       while (word) {
         const uint32_t bit = __ffs(word) - 1;
         word &= word - 1;
         list[o++] = (uint16_t)(pbase + bit);
       }
-#if NGSQ_RES_VARIANT & 2
-      // stage the window: block bytes [w0, w1) -> win + mis, through aligned 16-byte chunks (the few bytes around the block
-      // that ride along belong to its neighbours: never used, never written back)
-      const uint32_t w0 = sw << 10, w1 = min(w0 + (uint32_t)kResWin, d.isize);
-      uint8_t* const gbase = ob + w0;
-      const uint32_t mis = (uint32_t)(reinterpret_cast<uintptr_t>(gbase) & 15);
-      uint8_t* const abase = gbase - mis;
-      uint8_t* const win = s_win[wic];
-      uint8_t* const wptr = win + mis;
-      const uint32_t n_chunks = (mis + (w1 - w0) + 2 + 15) >> 4;  // + 2: the 3-byte token of a match that starts on the window's last bytes
-      for (uint32_t c = lane; c < n_chunks; c += 32) *reinterpret_cast<uint4*>(win + 16 * c) = *reinterpret_cast<const uint4*>(abase + 16 * c);
-#endif
       __syncwarp();
       // token of the first batch; later batches are fetched one batch ahead (their bytes sit in
       // their own destinations, which no earlier copy touches)
       uint32_t pos_n = 0xFFFFu, tok_n = 0;
       if (lane < total) {
         pos_n = list[lane];
-#if NGSQ_RES_VARIANT & 2
-        const uint8_t* t = wptr + (pos_n - w0);
-#else
         const uint8_t* t = ob + pos_n;
-#endif
         tok_n = (uint32_t)t[0] | ((uint32_t)t[1] << 8) | ((uint32_t)t[2] << 16);
       }
       for (uint32_t base = 0; base < total; base += 32) {
@@ -235,20 +167,15 @@ inflate_resolve_kernel(uint8_t* __restrict__ out, const BlockDesc* __restrict__ 
         const uint32_t jn = base + 32 + lane;
         if (jn < total) {
           pos_n = list[jn];
-#if NGSQ_RES_VARIANT & 2
-          const uint8_t* t = wptr + (pos_n - w0);
-#else
           const uint8_t* t = ob + pos_n;
-#endif
           tok_n = (uint32_t)t[0] | ((uint32_t)t[1] << 8) | ((uint32_t)t[2] << 16);
         }
         const uint32_t mlen = (tok & 255u) + 3u, dist = (tok >> 8) + 1u;
         // destinations [pos, dend) are ascending and disjoint across lanes (inactive lanes: empty at the top)
-        const uint32_t dpos = active ? pos : 0x20000u, dend = active ? pos + mlen : 0x20000u;
+        const uint32_t dend = active ? pos + mlen : 0x20000u;
         const uint32_t s_lo = pos - dist, s_hi = s_lo + min(mlen, dist);  // source bytes [s_lo, s_hi)
         // earlier lanes whose destination overlaps my source: lanes [lo, hi) with
-        //   lo = first lane with dend > s_lo,  hi = first lane with dpos >= s_hi
-#if NGSQ_RES_VARIANT & 1
+        //   lo = first lane with dend > s_lo,  hi = first lane with pos >= s_hi
         // rank(x) = matches of this super-window that start before window-relative byte x: the matches that start inside
         // my source are the list entries [rank(s_lo), rank(s_hi)); the one before them counts if it reaches past s_lo.
         // Matches of earlier batches and earlier super-windows are resolved already.
@@ -262,41 +189,15 @@ inflate_resolve_kernel(uint8_t* __restrict__ out, const BlockDesc* __restrict__ 
         const int lo = max((int)r_lo - (int)base - ((pl >= 0 && prev_end > s_lo) ? 1 : 0), 0), hi = (int)r_hi - (int)base;
         uint32_t dep = 0;
         if (active && hi > lo) dep = ((1u << hi) - 1u) & ~((1u << lo) - 1u) & ((1u << lane) - 1u);  // hi <= lane
-#else
-        uint32_t lo = 0, hi = 0;
-#pragma unroll
-        for (int step = 32; step; step >>= 1) {
-          const uint32_t il = lo + step - 1, ih = hi + step - 1;
-          const uint32_t e = __shfl_sync(0xFFFFFFFFu, dend, il & 31);
-          const uint32_t p2 = __shfl_sync(0xFFFFFFFFu, dpos, ih & 31);
-          if (il < 32 && e <= s_lo) lo += step;
-          if (ih < 32 && p2 < s_hi) hi += step;
-        }
-        uint32_t dep = 0;
-        if (active && hi > lo) dep = (hi >= 32 ? 0xFFFFFFFFu : ((1u << hi) - 1u)) & ~((1u << lo) - 1u) & ((1u << lane) - 1u);
-#endif
         uint32_t done = __ballot_sync(0xFFFFFFFFu, !active);
         while (done != 0xFFFFFFFFu) {
           const bool ready = !((done >> lane) & 1u) && (dep & ~done) == 0;
-#if NGSQ_RES_VARIANT & 2
-          if (ready) resolve_copy_win(ob, wptr, w0, w1, pos, mlen, dist);
-#else
           if (ready) resolve_copy(ob + pos, mlen, dist);
-#endif
           __syncwarp();
           done |= __ballot_sync(0xFFFFFFFFu, ready);
         }
       }
       __syncwarp();
-#if NGSQ_RES_VARIANT & 2
-      // write the window back: whole chunks as 128-bit stores, the (at most two) chunks shared with a neighbouring block bytewise
-      for (uint32_t c = lane; c < n_chunks; c += 32) {
-        const uint32_t lo = 16 * c, hi = lo + 16, end = mis + (w1 - w0);
-        if (lo >= mis && hi <= end) *reinterpret_cast<uint4*>(abase + lo) = *reinterpret_cast<const uint4*>(win + lo);
-        else for (uint32_t k = max(lo, mis); k < min(hi, end); ++k) abase[k] = win[k];
-      }
-      __syncwarp();
-#endif
     }
   }
 }

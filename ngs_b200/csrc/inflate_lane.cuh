@@ -23,12 +23,12 @@
 //
 // Per-lane shared-memory slab (kSlabBytes, odd number of words so that equal indices of
 // neighbouring lanes fall into different banks):
+//   SL_LLBT  u32 ll_bt[15]       per code length: (index of first symbol - first code) & 0xFFFF
+//                                | (index of the first symbol >= 256 of that length) << 16
 //   SL_LLS   u8  ll_sorted[288]  literal/length symbols (& 255) in canonical order
 //                                (while a dynamic header is parsed: the code-length-code LUT)
-//   SL_LLBT  u32 ll_bt[16]       per code length: (index of first symbol - first code) & 0xFFFF
-//                                | (index of the first symbol >= 256 of that length) << 16
+//   SL_DB    u8  d_base[15]      per code length: (index of first symbol - first code) mod 32
 //   SL_DS    u8  d_sorted[32]    distance symbols in canonical order
-//   SL_DB    i16 d_base[16]
 // The 4-bit code lengths of a dynamic header and the build counters live in per-thread local
 // memory (header() only; lanes of a warp parse their headers in lock step, so those accesses
 // coalesce): shared memory is spent on what the symbol loop reads.
@@ -46,33 +46,14 @@
 
 namespace ngsq {
 
-// Symbol-loop variants (bit mask; build with -DNGSQ_DEC_VARIANT=n).  Every variant decodes bit-identically in the host
-// model (tests/test_inflate_model.py) and on the GPU (tools/ab_decode.sh runs the parity tests per variant).  Measured on
-// a B200, 30 M records (profiles/round2_ab_inflate_variants.md): 0 -> 36.6 ms, 7 -> 32.5, 15 -> 32.1, 31 -> 33.1; the
-// default is 15.
-//   1  length / distance bases and extra-bit counts from a 64-word table (per-CTA shared memory) instead of arithmetic
-//   2  match bitmap word flushed by a predicated store instead of a branch
-//   4  emit(): chunk stores predicated, accumulator updates by selects (no divergent flush paths, no phi copies)
-//   8  396-byte slab (u8 distance bases, exact-size symbol arrays): 18 decoder warps per SM instead of 17
-//  16  code length = 1 - (signed byte dot product of the sign-replicated flag bytes): 4 PRMT + 4 IDP.4A instead of
-//      4 PRMT + 7 logic ops + POPC, twice per match
-#ifndef NGSQ_DEC_VARIANT
-#define NGSQ_DEC_VARIANT 15
-#endif
+// The symbol loop takes its length / distance bases from a 64-word table, stores under predicates instead of branching,
+// and uses the 396-byte slab, which fits 18 decoder warps per SM instead of 17: the fastest of the forms measured on a
+// B200 (profiles/round2_ab_inflate_variants.md: 36.6 -> 32.1 ms per 30 M records).
 
-#if NGSQ_DEC_VARIANT & 8
 // ll_bt[15] and d_base[15] are indexed by length - 1 (length 16 = invalid code reads the neighbouring bytes of the
 // slab; the block is failed anyway), distance bases are kept mod 32 in bytes: 60 + 288 + 15 + 32 = 395 -> 99 words
 constexpr int SL_LLBT = 0, SL_LLS = 60, SL_DB = 348, SL_DS = 363;
 constexpr int kSlabBytes = 396;
-constexpr int kLenIndexBias = 1;
-typedef uint8_t dbase_t;
-#else
-constexpr int SL_LLS = 0, SL_LLBT = 288, SL_DS = 352, SL_DB = 384;
-constexpr int kSlabBytes = 416 + 4;
-constexpr int kLenIndexBias = 0;
-typedef int16_t dbase_t;
-#endif
 constexpr uint32_t kBitmapWords = 2048;  // per BGZF block: one bit per inflated byte (<= 65536)
 
 enum : uint32_t { kBlkOk = 0, kBlkBadStream = 1, kBlkIsize = 2, kBlkOverrun = 3 };
@@ -98,7 +79,7 @@ NGSQ_HD uint32_t brev32(uint32_t x) {
 #endif
 }
 
-// variant 1: entry i < 32: length symbol 257 + i -> (match length - 3 base) | extra bits << 8;
+// entry i < 32: length symbol 257 + i -> (match length - 3 base) | extra bits << 8;
 // entry 32 + i: distance symbol i -> (distance - 1 base) | extra bits << 16
 NGSQ_HD uint32_t base_lut_entry(uint32_t i) {
   if (i < 32) {
@@ -111,32 +92,6 @@ NGSQ_HD uint32_t base_lut_entry(uint32_t i) {
   const uint32_t deb = ds < 4 ? 0 : (ds >> 1) - 1;
   const uint32_t b = ds < 4 ? ds : (2 + (ds & 1)) << deb;
   return b | (deb << 16);
-}
-
-NGSQ_HD uint32_t byte_perm(uint32_t a, uint32_t b, uint32_t sel) {  // PRMT, default mode (selector bit 3: replicate the sign)
-#if defined(__CUDA_ARCH__)
-  uint32_t r;  // not __byte_perm(): the intrinsic masks each selector nibble to 3 bits and drops the sign mode
-  asm("prmt.b32 %0, %1, %2, %3;" : "=r"(r) : "r"(a), "r"(b), "r"(sel));
-  return r;
-#else
-  const uint64_t v = (uint64_t)a | ((uint64_t)b << 32);
-  uint32_t r = 0;
-  for (int i = 0; i < 4; ++i) {
-    const uint32_t n = (sel >> (4 * i)) & 15;
-    uint32_t byte = (uint32_t)(v >> (8 * (n & 7))) & 255;
-    if (n & 8) byte = (byte & 128) ? 255 : 0;
-    r |= byte << (8 * i);
-  }
-  return r;
-#endif
-}
-NGSQ_HD int dp4a_s8(uint32_t a, uint32_t b, int c) {  // IDP.4A, signed bytes
-#if defined(__CUDA_ARCH__)
-  return __dp4a((int)a, (int)b, c);
-#else
-  for (int i = 0; i < 4; ++i) c += (int)(int8_t)(a >> (8 * i)) * (int)(int8_t)(b >> (8 * i));
-  return c;
-#endif
 }
 
 struct Quad { uint32_t x, y, z, w; };
@@ -182,9 +137,7 @@ struct Lane {
   // canonical-code limits: llim[i] = lim[2i] | lim[2i+1] << 16, lim[0] = 0x8000 (never reached)
   uint32_t llim[8], dlim[8];
   uint8_t* slab;            // shared memory (host model: heap)
-#if NGSQ_DEC_VARIANT & 1
   const uint32_t* lut;      // base_lut_entry(0..63)
-#endif
   uint32_t err;
   int state;
   bool bfinal;
@@ -193,9 +146,9 @@ struct Lane {
 #endif
 
   NGSQ_HD uint8_t* ll_sorted() const { return slab + SL_LLS; }
-  NGSQ_HD uint32_t* ll_bt() const { return reinterpret_cast<uint32_t*>(slab + SL_LLBT) - kLenIndexBias; }  // index: code length
+  NGSQ_HD uint32_t* ll_bt() const { return reinterpret_cast<uint32_t*>(slab + SL_LLBT) - 1; }  // index: code length
   NGSQ_HD uint8_t* d_sorted() const { return slab + SL_DS; }
-  NGSQ_HD dbase_t* d_base() const { return reinterpret_cast<dbase_t*>(slab + SL_DB) - kLenIndexBias; }
+  NGSQ_HD uint8_t* d_base() const { return slab + SL_DB - 1; }  // index: code length
 
   // ---------------- bit reader ----------------
   static NGSQ_HD void ld64(const uint8_t* p, uint32_t& lo, uint32_t& hi) {  // p is 8-byte aligned
@@ -321,16 +274,7 @@ struct Lane {
       q = sq;
     }
   }
-  NGSQ_HD void mark_match(uint32_t p) {  // p: block-relative position of the match start
-    uint32_t w = p >> 5;
-    if (w != bm_w) {
-      if (bm) bitmap[bm_w] = bm;
-      bm_w = w;
-      bm = 0;
-    }
-    bm |= 1u << (p & 31);
-  }
-  // ---- variants 2 / 4: stores under a predicate instead of a branch (device: one @p ST; host: an if) ----
+  // stores under a predicate instead of a branch (device: one @p ST; host: an if)
   static NGSQ_HD void store16_if(bool c, uint8_t* p, uint64_t lo, uint64_t hi) {
 #if defined(__CUDA_ARCH__)
     asm volatile("{\n\t.reg .pred p;\n\t.reg .u64 a;\n\tsetp.ne.u32 p, %0, 0;\n\tcvta.to.global.u64 a, %1;\n\t@p st.global.v4.u32 [a], {%2, %3, %4, %5};\n\t}"
@@ -423,9 +367,9 @@ struct Lane {
   // ---------------- canonical tables ----------------
   // lens(k): code length of symbol k in [0, n).  Fills sorted[], the per-length bases and the
   // packed limits.  Literal/length table: bt32 != nullptr and `split` = 256 (the index of the first
-  // symbol >= split of each length goes into the high half of bt32[]); distance table: base16.
+  // symbol >= split of each length goes into the high half of bt32[]); distance table: base8.
   template <class LenFn>
-  NGSQ_HD bool build(LenFn lens, uint32_t n, uint8_t* sorted, uint32_t* lim_packed, uint32_t* bt32, dbase_t* base16, uint32_t split,
+  NGSQ_HD bool build(LenFn lens, uint32_t n, uint8_t* sorted, uint32_t* lim_packed, uint32_t* bt32, uint8_t* base8, uint32_t split,
                      uint16_t* nx /* scratch[16] */) {
     for (int i = 0; i < 16; ++i) nx[i] = 0;
     for (uint32_t k = 0; k < n; ++k) nx[lens(k)]++;
@@ -442,7 +386,7 @@ struct Lane {
       const uint32_t lim = (code + c) << (15 - l);  // <= 0x8000
       if (l & 1) lim_packed[l >> 1] = lim_lo | (lim << 16); else lim_lo = lim;
       const int b = (int)off - (int)code;
-      if (bt32) bt32[l] = ((uint32_t)b & 0xFFFFu) | (off << 16); else base16[l] = (dbase_t)b;  // used mod 32
+      if (bt32) bt32[l] = ((uint32_t)b & 0xFFFFu) | (off << 16); else base8[l] = (uint8_t)b;  // used mod 32
       nx[l] = (uint16_t)off;  // running index of the next symbol of this length
       off += c;
     }
@@ -460,17 +404,7 @@ struct Lane {
   // code length of the next symbol: 1 + number of limits the next 15 bits (MSB first) reach
   static NGSQ_HD uint32_t code_len(uint32_t x, const uint32_t* lim_packed) {
     const uint32_t x2 = (x * 0x10001u) | 0x80008000u;
-#if NGSQ_DEC_VARIANT & 16
-    // bytes 1 and 3 of (x2 - lim) carry the "x >= lim" flags in their top bits: replicate them to 0x00 / 0xFF
-    // (= 0 / -1 as signed bytes) and add the sixteen of them up with four dot products
-    const uint32_t h0 = byte_perm(x2 - lim_packed[0], x2 - lim_packed[1], 0xFDB9);
-    const uint32_t h1 = byte_perm(x2 - lim_packed[2], x2 - lim_packed[3], 0xFDB9);
-    const uint32_t h2 = byte_perm(x2 - lim_packed[4], x2 - lim_packed[5], 0xFDB9);
-    const uint32_t h3 = byte_perm(x2 - lim_packed[6], x2 - lim_packed[7], 0xFDB9);
-    const int c01 = dp4a_s8(h1, 0x01010101u, dp4a_s8(h0, 0x01010101u, -1));  // -1 - (limits 0..7 reached)
-    const int c23 = dp4a_s8(h3, 0x01010101u, dp4a_s8(h2, 0x01010101u, 0));   // -(limits 8..15 reached)
-    return (uint32_t)(0 - c01 - c23);
-#elif defined(__CUDA_ARCH__)
+#if defined(__CUDA_ARCH__)
     // bit 15 of each half of (x2 - lim) says x >= lim: gather the 16 flag bytes with four byte
     // permutes, interleave their top bits into one word, popcount
     const uint32_t g0 = __byte_perm(x2 - lim_packed[0], x2 - lim_packed[1], 0x7531);
@@ -611,18 +545,14 @@ struct Lane {
   // Straight-line on purpose: every warp step runs the union of the paths its lanes take and waits
   // out every branch (ncu: each warp is bound by its own dependency / branch-resolve latency, not by
   // issue slots), so range checks only accumulate flags that are tested once at the end, and the
-  // length / distance bases are computed without branches.  Out-of-range values are clamped where
+  // length / distance bases are looked up without branches.  Out-of-range values are clamped where
   // they index memory; a flagged block is failed and never reaches the resolve kernel.
   NGSQ_HD void step() {
     refill();
     const uint32_t x = brev32(peek()) >> 17;
     const uint32_t len = code_len(x, llim);             // 1..15, 16 = bits beyond an incomplete code
     uint32_t bad_stream = len >> 4, overrun = 0;
-#if NGSQ_DEC_VARIANT & 8
     const uint32_t bt = ll_bt()[len];  // 1..16
-#else
-    const uint32_t bt = ll_bt()[len & 15];
-#endif
     const uint32_t idx = ((x >> ((15 - len) & 31)) + bt) & 0xFFFFu;  // index into sorted (the base is kept mod 2^16)
     const uint32_t s8 = ll_sorted()[idx < 288 ? idx : 0];
     const bool upper = idx >= (bt >> 16);  // symbol >= 256
@@ -640,26 +570,12 @@ struct Lane {
       // length symbol 257 + li: li < 8: 3 + li;  li = 28: 258;  else 3 + ((4 + (li & 3)) << eb) + extra, eb = (li - 4) >> 2
       const uint32_t li = s8 - 1;
       bad_stream |= li > 28;
-#if NGSQ_DEC_VARIANT & 1
       const uint32_t le = lut[li & 31];
       const uint32_t mlen = 3 + (le & 255) + take(le >> 8);
-#else
-      const uint32_t lc = li > 28 ? 28 : li;
-      uint32_t eb = ((lc < 4 ? 4 : lc) - 4) >> 2;
-      uint32_t lbase = (4 + (lc & 3)) << eb;
-      lbase = lc < 4 ? lc : lbase;
-      lbase = lc == 28 ? 255 : lbase;
-      eb = lc == 28 ? 0 : eb;
-      const uint32_t mlen = 3 + lbase + take(eb);
-#endif
       const uint32_t dx = brev32(peek()) >> 17;
       const uint32_t dl = code_len(dx, dlim);
       bad_stream |= dl >> 4;
-#if NGSQ_DEC_VARIANT & 8
       const uint32_t di = ((dx >> ((15 - dl) & 31)) + (uint32_t)d_base()[dl]) & 31u;
-#else
-      const uint32_t di = ((dx >> ((15 - dl) & 31)) + (uint32_t)(int)d_base()[dl & 15]) & 31u;
-#endif
       const uint32_t ds = d_sorted()[di];
       bad_stream |= ds > 29;
       drop(dl);
@@ -667,23 +583,11 @@ struct Lane {
       if (ctr) ctr->d_len_hist[dl]++;
 #endif
       // distance symbol ds: ds < 4: 1 + ds;  else 1 + ((2 + (ds & 1)) << deb) + extra, deb = (ds >> 1) - 1
-#if NGSQ_DEC_VARIANT & 1
       const uint32_t de = lut[32 + (ds & 31)];
       const uint32_t dist = 1 + (de & 0xFFFFu) + take(de >> 16);
-#else
-      const uint32_t dc = ds > 29 ? 29 : ds;
-      const uint32_t deb = ((dc >> 1) < 1 ? 1 : (dc >> 1)) - 1;
-      uint32_t dbase = 1 + ((2 + (dc & 1)) << deb);
-      dbase = dc < 2 ? dc + 1 : dbase;
-      const uint32_t dist = dbase + take(deb);
-#endif
       const uint32_t p = q - q0;
       overrun |= (dist > p) | (q + mlen > qend);
-#if NGSQ_DEC_VARIANT & 2
       mark_match_if(!(bad_stream | overrun), p);
-#else
-      if (!(bad_stream | overrun)) mark_match(p);
-#endif
       v = (mlen - 3) | ((dist - 1) << 8);
       n = 3;
       sk = mlen - 3;
@@ -697,11 +601,7 @@ struct Lane {
 #endif
     }
     if (bad_stream | overrun) { end_block(bad_stream ? kBlkBadStream : kBlkOverrun); return; }
-#if NGSQ_DEC_VARIANT & 4
     emit_sel(v, n, sk);
-#else
-    emit(v, n, sk);
-#endif
   }
 };
 

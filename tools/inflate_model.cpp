@@ -69,7 +69,7 @@ static void resolve_block_model(uint8_t* ob, uint32_t isize, const uint32_t* bit
         }
         dep[l] = 0;
         if (active[l] && hi > lo) dep[l] = (hi >= 32 ? 0xFFFFFFFFu : ((1u << hi) - 1u)) & ~((1u << lo) - 1u) & ((1u << l) - 1u);
-        // the rank formulation of NGSQ_RES_VARIANT 1 (inflate2.cuh) must give the same mask
+        // the rank masks of inflate2.cuh must give the same mask
         {
           const uint32_t W = sw << 10;
           const uint32_t x_lo = std::min(std::max(s_lo[l], W) - W, 1023u), x_hi = std::min(std::max(s_hi[l], W) - W, 1023u);
@@ -120,10 +120,8 @@ int main(int argc, char** argv) {
   uint64_t fuzz_runs = 0, fuzz_failed = 0, fuzz_ok = 0, rng = 0x9E3779B97F4A7C15ull;
 
   InflateCounters ctr;
-#if NGSQ_DEC_VARIANT & 1
   static uint32_t base_lut[64];
   for (uint32_t i = 0; i < 64; ++i) base_lut[i] = base_lut_entry(i);
-#endif
   std::vector<uint8_t> slab(kSlabBytes);
 
   std::vector<uint32_t> bitmap(kBitmapWords);
@@ -161,9 +159,7 @@ int main(int argc, char** argv) {
       memset(bitmap.data(), 0, kBitmapWords * 4);
       Lane L;
       L.slab = slab.data();
-#if NGSQ_DEC_VARIANT & 1
       L.lut = base_lut;
-#endif
       L.ctr = nullptr;
       L.begin_block(d, out.data(), bitmap.data());
       uint64_t steps = 0;
@@ -205,10 +201,7 @@ int main(int argc, char** argv) {
         memset(bitmap.data(), 0, kBitmapWords * 4);
         Lane L;
         L.slab = slab.data();
-#if NGSQ_DEC_VARIANT & 1
-      L.lut = base_lut;
-#endif
-
+        L.lut = base_lut;
         L.ctr = mis == 0 ? &ctr : nullptr;
         L.begin_block(d, out.data(), bitmap.data());
         while (L.state != LS_IDLE) {

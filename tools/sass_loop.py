@@ -1,7 +1,7 @@
 """Static size of a kernel's hot loop: disassembles <lib.so>, finds in kernel <symbol-substring> the smallest loop
 (backward branch) that contains all of the given marker mnemonics, and prints its instruction count by mnemonic
 plus the count outside side exits (blocks that end in CALL / EXIT / a jump out of the loop are listed separately).
-No GPU needed: used to compare symbol-loop variants before spending GPU time (DESIGN.md section 7).
+No GPU needed: used to compare symbol-loop versions before spending GPU time (DESIGN.md section 7).
 usage: sass_loop.py <lib.so> <kernel-substring> [marker ...]      (default markers: BREV POPC)"""
 import re
 import subprocess
