@@ -54,7 +54,8 @@ enum {
   NGSQ_E_NOMEM = -10,
   NGSQ_E_EDITS = -11,     /* the Edits facet met a record / reference the reference program aborts on */
   NGSQ_E_FEATURES = -12,  /* likewise for the Genomic Features facet */
-  NGSQ_E_QUAL_CAP = -13   /* a read is longer than the quality table: raise quality_positions and run again */
+  NGSQ_E_QUAL_CAP = -13,  /* a read is longer than the quality table: raise quality_positions and run again */
+  NGSQ_E_UNSORTED = -14   /* NGSQ_F_INDEX: the records are not coordinate-sorted (the message names the first offender) */
 };
 
 /* ngsq_config.flags */
@@ -65,6 +66,10 @@ enum {
 #define NGSQ_F_FEATURES 16u     /* Genomic Features (needs ngsq_set_feature_model + ngsq_set_features) */
 #define NGSQ_F_SERIAL_STAGES 32u /* measurement aid: every kernel of a wave on ONE stream (no overlap with the next wave's
                                     inflate), so that per-stage event times are the kernels' own; results are identical */
+#define NGSQ_F_INDEX 64u        /* build the file's BAI in the same pass (`ngs index`, src/index/bam.rs:39-109); combines with every
+                                   other flag.  The range must start at the first record and reach to the end (end_voffset 0),
+                                   max_records must be 0, references must be shorter than 2^29 (longer ones need CSI) and the
+                                   records coordinate-sorted (NGSQ_E_UNSORTED otherwise).  Read the bytes with ngsq_get_bai. */
 
 typedef struct ngsq_engine ngsq_engine;
 
@@ -107,7 +112,8 @@ typedef struct ngsq_stats {
   float ms_inflate;          /* device time of the inflate launches (bitmap clear + decode + resolve; CUDA events) */
   float ms_crc;
   float ms_scan;             /* record-boundary discovery + offset table */
-  float ms_facets;           /* fused record-facet + coverage-scatter kernel */
+  float ms_facets;           /* fused record-facet + coverage-scatter kernel, and the other per-wave record kernels (Edits,
+                                Genomic Features, the NGSQ_F_INDEX key / run kernel) */
   float ms_coverage;         /* difference-array resolve */
   float ms_total;            /* first submit -> end of finish on the engine's stream */
   uint32_t inflate_launches, other_launches;
@@ -222,6 +228,10 @@ int ngsq_get_edits(ngsq_engine* e, uint64_t read_one[513], uint64_t read_two[513
  * of its own shard (contig-exclusive shards: the owner's are the sequence's). */
 int ngsq_get_edit_positions(ngsq_engine* e, uint32_t ref, uint32_t* refs, uint32_t* alts, uint64_t n);
 int ngsq_get_stats(ngsq_engine* e, ngsq_stats* out);
+/* NGSQ_F_INDEX: the complete .bai file (magic, every reference's bins, chunks, metadata pseudo-bin 37450 and linear index,
+ * n_no_coor) of the records submitted since ngsq_set_range.  After ngsq_finish.  *n_out = its size; out = NULL with cap = 0
+ * asks for the size only.  DESIGN.md section 4 (K13) lists where its bytes may differ from samtools' index of the same file. */
+int ngsq_get_bai(ngsq_engine* e, uint8_t* out, size_t cap, size_t* n_out);
 
 /* ---- multi-GPU merge: one sum-reduce of the packed u64 result buffer ---- */
 int ngsq_nccl_unique_id(char out[128]);

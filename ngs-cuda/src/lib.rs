@@ -8,7 +8,9 @@
 //!     and `:350-397` (pass 2), including the BGZF read + inflate + CRC check that `bam::Reader` performs under them
 //!     (`src/utils/formats/bam.rs:41-44`);
 //!   * `Engine::general()` .. `Engine::coverage_contig()`   the integer state the facets hold when their
-//!     `summarize()` / `teardown()` / `aggregate()` run.  Every float stays where it is: in the facets.
+//!     `summarize()` / `teardown()` / `aggregate()` run.  Every float stays where it is: in the facets;
+//!   * `Engine::create_indexer` + `Engine::build_bai`   the record loop of `ngs index` for a BAM (`src/index/bam.rs:66-100`):
+//!     the bytes of the `.bai` from one streamed pass.
 //! One `Engine` per GPU, driven by one thread (the qc path is single-threaded: `src/qc.rs:49` uses `Rc`).
 
 use std::ffi::CStr;
@@ -94,6 +96,8 @@ pub mod sys {
     /// measurement aid: every kernel of a wave on one stream (no overlap with the next wave's inflate); results identical
     pub const NGSQ_F_SERIAL_STAGES: u32 = 32;
     pub const NGSQ_E_QUAL_CAP: c_int = -13;
+    pub const NGSQ_F_INDEX: u32 = 64;
+    pub const NGSQ_E_UNSORTED: c_int = -14;
 
     extern "C" {
         pub fn ngsq_version() -> c_int;
@@ -133,6 +137,7 @@ pub mod sys {
         pub fn ngsq_host_free(p: *mut c_void);
         pub fn ngsq_host_register(p: *mut c_void, nbytes: usize) -> c_int;
         pub fn ngsq_host_unregister(p: *mut c_void) -> c_int;
+        pub fn ngsq_get_bai(e: *mut NgsqEngine, out: *mut u8, cap: usize, n_out: *mut usize) -> c_int;
         pub fn ngsq_inflate_to_host(e: *mut NgsqEngine, bgzf: *const u8, nbytes: usize, out: *mut u8, cap: usize, n_out: *mut usize) -> c_int;
     }
 }
@@ -283,6 +288,38 @@ impl Engine {
         let mut st = sys::NgsqStats::default();
         self.check(unsafe { sys::ngsq_get_stats(self.raw, &mut st) })?;
         Ok(st)
+    }
+
+    /// An engine that builds the BAI of a whole coordinate-sorted BAM (NGSQ_F_INDEX, CRC checked like noodles-bgzf does).
+    pub fn create_indexer(device: i32) -> anyhow::Result<Self> {
+        let cfg = sys::NgsqConfig {
+            struct_size: std::mem::size_of::<sys::NgsqConfig>() as u32,
+            flags: sys::NGSQ_F_INDEX | sys::NGSQ_F_VERIFY_CRC,
+            ..Default::default()
+        };
+        let mut raw = std::ptr::null_mut();
+        let rc = unsafe { sys::ngsq_create(device as c_int, &cfg, &mut raw) };
+        if rc != 0 {
+            let msg = unsafe { CStr::from_ptr(sys::ngsq_last_error(std::ptr::null_mut())) }.to_string_lossy().into_owned();
+            bail!("ngs-cuda: {}", msg);
+        }
+        Ok(Self { raw, submits: 0 })
+    }
+
+    /// The `.bai` bytes of the BAM at `path` (`src/index/bam.rs:66-100`): `lengths` are the header's reference lengths and
+    /// `first_record` the reader's virtual position after the header.  Unsorted records fail (NGSQ_E_UNSORTED), like the
+    /// reference's indexer; references of 2^29 bases or more need CSI and are refused.
+    pub fn build_bai(&mut self, path: &Path, lengths: &[u32], first_record: u64, chunk_bytes: usize, on_progress: impl FnMut(u64)) -> anyhow::Result<Vec<u8>> {
+        self.set_references(lengths, &vec![false; lengths.len()])?;
+        self.set_range(first_record, 0)?;
+        let size = std::fs::metadata(path)?.len();
+        self.stream_file(path, first_record >> 16, size, chunk_bytes, on_progress)?;
+        self.finish()?;
+        let mut n = 0usize;
+        self.check(unsafe { sys::ngsq_get_bai(self.raw, std::ptr::null_mut(), 0, &mut n) })?;
+        let mut out = vec![0u8; n];
+        self.check(unsafe { sys::ngsq_get_bai(self.raw, out.as_mut_ptr(), out.len(), &mut n) })?;
+        Ok(out)
     }
 
     /// A read longer than the quality table: raise it and run the file again (include/ngs_cuda.h, NGSQ_E_QUAL_CAP).

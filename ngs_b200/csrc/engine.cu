@@ -30,6 +30,7 @@
 #include "edits.cuh"
 #include "facets.cuh"
 #include "features.cuh"
+#include "index.cuh"
 #include "inflate2.cuh"
 #include "recscan.cuh"
 
@@ -189,6 +190,27 @@ struct ngsq_engine {
   unsigned long long* d_ft_res = nullptr;
   std::vector<uint64_t> h_ft_res;
 
+  // BAI build (NGSQ_F_INDEX): per-reference linear-index tables and counters for the whole run; per indexed wave a run table
+  // (two, by parity), drained to pinned host memory when the wave two later is launched
+  IndexState* d_ix = nullptr;
+  IndexRun* d_ix_runs[2] = {nullptr, nullptr};
+  uint64_t ix_runs_cap = 0;
+  IndexRun* d_ix_ovf = nullptr;
+  uint64_t* d_ix_win_base = nullptr;
+  uint32_t* d_ix_win_n = nullptr;
+  unsigned long long* d_ix_win = nullptr;
+  unsigned int* d_ix_maxw = nullptr;
+  unsigned long long* d_ix_counts = nullptr;
+  std::vector<uint64_t> ix_win_base;
+  std::vector<uint32_t> ix_win_n;
+  uint64_t ix_win_total = 0;
+  uint64_t* h_ix_probe = nullptr;    // pinned: run count of the wave in slot 0 / 1
+  struct IxWave { cudaEvent_t done; bool drained; };
+  std::vector<IxWave> ix_waves;
+  std::vector<std::pair<const IndexRun*, uint64_t>> ix_drained;  // pinned copies of drained run tables
+  uint64_t data_end_coff = 0;        // end of the last non-empty block submitted (the offset after the last record)
+  std::vector<uint8_t> bai;
+
   // nccl
   void* comm = nullptr;
   int n_ranks = 1, rank = 0;
@@ -201,6 +223,7 @@ constexpr uint32_t kDefaultHeadroom = 16u << 20;       // longest record that ma
 constexpr uint32_t kDefaultQualPositions = 1u << 17;   // rows of the global quality table (98 MB)
 constexpr uint32_t kProgSlots = 1024;
 constexpr size_t kDefaultCompRing = (size_t)8 << 30;   // compressed staging kept on the device when the caller reserves nothing
+constexpr uint64_t kIndexOverflowCap = 1u << 20;       // records that reach past their reference's linear-index table
 
 int fail(ngsq_engine* e, int code, const char* fmt, ...) {
   char buf[512];
@@ -303,6 +326,18 @@ int start_run(ngsq_engine* e) {
   e->h_state->next_carry = kNoCarry;
   CU(cudaMemcpyAsync(e->d_state, e->h_state, sizeof(RunState), cudaMemcpyHostToDevice, e->s_comp));
   if ((e->cfg.flags & NGSQ_F_FEATURES) && e->d_ft_res) CU(cudaMemsetAsync(e->d_ft_res, 0, F_WORDS * 8, e->s_comp));
+  if (e->cfg.flags & NGSQ_F_INDEX) {
+    if (!e->d_ix) return fail(e, NGSQ_E_ARG, "NGSQ_F_INDEX needs ngsq_set_references before the first submit");
+    IndexState z{};
+    z.carry[0].run_key = kIxNoRun;
+    z.unsorted_voff = ~0ull;
+    CU(cudaMemcpyAsync(e->d_ix, &z, sizeof z, cudaMemcpyHostToDevice, e->s_comp));
+    if (e->ix_win_total) CU(cudaMemsetAsync(e->d_ix_win, 0xFF, e->ix_win_total * 8, e->s_comp));
+    if (e->n_ref) {
+      CU(cudaMemsetAsync(e->d_ix_maxw, 0, (size_t)e->n_ref * 4, e->s_comp));
+      CU(cudaMemsetAsync(e->d_ix_counts, 0, (size_t)e->n_ref * 16, e->s_comp));
+    }
+  }
   if ((e->cfg.flags & NGSQ_F_EDITS) && e->d_ed_res) {
     CU(cudaMemsetAsync(e->d_ed_res, 0, E_WORDS * 8, e->s_comp));
     if (e->ed_pos_total) {
@@ -331,6 +366,7 @@ int append_blocks(ngsq_engine* e, const ngsq_block* blk, uint32_t n, uint64_t de
     e->h_blocks.push_back(d);
     e->h_crc.push_back(b.crc32);
     e->out_used += b.isize;
+    e->data_end_coff = b.coffset + b.csize;
   }
   return NGSQ_OK;
 }
@@ -441,6 +477,23 @@ int launch_inflate(ngsq_engine* e, const BlockDesc* blocks, uint32_t n, uint8_t*
   return NGSQ_OK;
 }
 
+// NGSQ_F_INDEX: copies the run table of indexed wave j to pinned host memory once its kernel is done, on stream `s` (ahead of
+// the kernel of wave j + 2, which reuses the table).  Waits for wave j's index kernel, which by then runs beside the
+// inflate of the wave after it.
+int ix_drain(ngsq_engine* e, uint32_t j, cudaStream_t s) {
+  auto& w = e->ix_waves[j];
+  if (w.drained) return NGSQ_OK;
+  CU(cudaEventSynchronize(w.done));
+  w.drained = true;
+  const uint64_t n = std::min<uint64_t>(e->h_ix_probe[j & 1], e->ix_runs_cap);  // more tickets than room: the kernel flagged it
+  if (!n) return NGSQ_OK;
+  IndexRun* h = (IndexRun*)pin_alloc(e, n * sizeof(IndexRun));
+  if (!h) return fail(e, NGSQ_E_NOMEM, "cudaHostAlloc index runs (%llu)", (unsigned long long)n);
+  CU(cudaMemcpyAsync(h, e->d_ix_runs[j & 1], n * sizeof(IndexRun), cudaMemcpyDeviceToHost, s));
+  e->ix_drained.push_back({h, n});
+  return NGSQ_OK;
+}
+
 // Device buffers of one wave of n blocks / `bytes` inflated bytes in slot `s`.  Growing a buffer waits for the work in
 // flight (only the first waves of a run ever grow anything; reserve_* avoids even that).
 int ensure_wave_buffers(ngsq_engine* e, int s, uint32_t n, uint64_t bytes) {
@@ -485,6 +538,16 @@ int ensure_wave_buffers(ngsq_engine* e, int s, uint32_t n, uint64_t bytes) {
     if ((rc = quiesce())) return rc;
     if ((rc = fresh(e, e->d_rec, need_rec, "record table"))) return rc;
     e->rec_cap = need_rec;
+  }
+  // a run starts at a record: the run tables are sized like the record table (the runs of earlier waves are drained first)
+  if ((e->cfg.flags & NGSQ_F_INDEX) && need_rec > e->ix_runs_cap) {
+    if ((rc = quiesce())) return rc;
+    for (uint32_t j = 0; j < e->ix_waves.size(); ++j)
+      if ((rc = ix_drain(e, j, e->s_scan))) return rc;
+    CU(cudaStreamSynchronize(e->s_scan));
+    if ((rc = fresh(e, e->d_ix_runs[0], need_rec, "index run table"))) return rc;
+    if ((rc = fresh(e, e->d_ix_runs[1], need_rec, "index run table"))) return rc;
+    e->ix_runs_cap = need_rec;
   }
   // a read with more than kQualSmemPositions bases takes more than 260 bytes
   const uint64_t need_long = (e->headroom + std::max<uint64_t>(e->slot_cap[0], e->slot_cap[1])) / 260 + 2;
@@ -693,6 +756,27 @@ int launch_wave(ngsq_engine* e, uint32_t b0, uint32_t b1, bool final_wave) {
     CU(cudaGetLastError());
     e->other_launches++;
   }
+  if (e->cfg.flags & NGSQ_F_INDEX) {
+    // K13: keys, runs, order check, counters and linear index of the wave's records
+    const uint32_t j = (uint32_t)e->ix_waves.size(), par = j & 1;
+    if (j >= 2 && (rc = ix_drain(e, j - 2, st))) return rc;
+    CU(cudaMemsetAsync(&e->d_ix->n_runs[par], 0, 8, st));
+    IndexParams X{};
+    X.d = slot; X.rec = e->d_rec; X.st = e->d_state; X.blocks = wblocks; X.headroom = e->headroom; X.par = par; X.out0 = out0;
+    X.n_ref = (int32_t)e->n_ref; X.S = e->d_ix; X.runs = e->d_ix_runs[par]; X.runs_cap = e->ix_runs_cap;
+    X.ovf = e->d_ix_ovf; X.ovf_cap = kIndexOverflowCap;
+    X.win_base = e->d_ix_win_base; X.win_n = e->d_ix_win_n; X.win = e->d_ix_win; X.max_win = e->d_ix_maxw; X.counts = e->d_ix_counts;
+    const uint32_t per_cta = 31 * (kIndexThreads / 32);
+    const uint32_t xgrid = (uint32_t)std::min<uint64_t>((bytes / 36 + 2 + per_cta - 1) / per_cta, (uint64_t)e->n_sm * 8);
+    index_kernel<<<xgrid, kIndexThreads, 0, st>>>(X);
+    CU(cudaGetLastError());
+    e->other_launches++;
+    CU(cudaMemcpyAsync(e->h_ix_probe + par, &e->d_ix->n_runs[par], 8, cudaMemcpyDeviceToHost, st));
+    ngsq_engine::IxWave xw{nullptr, false};
+    CU(cudaEventCreateWithFlags(&xw.done, cudaEventDisableTiming));
+    e->ix_waves.push_back(xw);
+    CU(cudaEventRecord(xw.done, st));
+  }
   CU(cudaEventRecord(w.facets_end, st));
   e->waves.push_back(w);
   e->stats.inflate_launches++;
@@ -760,6 +844,103 @@ int acquire_comp(ngsq_engine* e, size_t nbytes, uint8_t** dst) {
   return NGSQ_OK;
 }
 
+// K13 on the host, at ngsq_finish: runs -> chunks per (reference, bin), the linear index, the .bai bytes.
+int finish_index(ngsq_engine* e) {
+  for (uint32_t j = 0; j < e->ix_waves.size(); ++j) {
+    int rc = ix_drain(e, j, e->s_comp);
+    if (rc) return rc;
+  }
+  CU(cudaStreamSynchronize(e->s_comp));
+  IndexState S;
+  CU(cudaMemcpy(&S, e->d_ix, sizeof S, cudaMemcpyDeviceToHost));
+  if (S.err & kIxBadRecord) return fail(e, NGSQ_E_BAD_RECORD, "malformed BAM record (field overrun, CIGAR op > 8 or reference id out of range)");
+  if (S.err & kIxTooLong) return fail(e, NGSQ_E_BAD_RECORD, "a record ends beyond position 2^29, which a BAI cannot address (CSI can)");
+  if (S.err & kIxRunTable) return fail(e, NGSQ_E_CHAIN, "index run table overflow");
+  if (S.err & kIxOverflowList)
+    return fail(e, NGSQ_E_NOMEM, "more than %llu records reach past the end of their reference sequence", (unsigned long long)kIndexOverflowCap);
+  if (S.unsorted_voff != ~0ull)
+    return fail(e, NGSQ_E_UNSORTED, "the records are not coordinate-sorted: the record at virtual offset %llu (block at file offset %llu, offset %llu) "
+                "comes after a record with a larger (reference, position) or an unplaced one; sort the file before indexing it",
+                (unsigned long long)S.unsorted_voff, (unsigned long long)(S.unsorted_voff >> 16), (unsigned long long)(S.unsorted_voff & 0xFFFF));
+  const uint32_t nr = e->n_ref;
+  std::vector<uint64_t> win(e->ix_win_total), counts((size_t)nr * 2);
+  std::vector<uint32_t> maxw(nr);
+  if (e->ix_win_total) CU(cudaMemcpy(win.data(), e->d_ix_win, e->ix_win_total * 8, cudaMemcpyDeviceToHost));
+  if (nr) {
+    CU(cudaMemcpy(counts.data(), e->d_ix_counts, (size_t)nr * 16, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(maxw.data(), e->d_ix_maxw, (size_t)nr * 4, cudaMemcpyDeviceToHost));
+  }
+  std::vector<IndexRun> ovf(std::min<uint64_t>(S.n_ovf, kIndexOverflowCap));
+  if (!ovf.empty()) CU(cudaMemcpy(ovf.data(), e->d_ix_ovf, ovf.size() * sizeof(IndexRun), cudaMemcpyDeviceToHost));
+  std::vector<IndexRun> runs;
+  for (auto& d : e->ix_drained) runs.insert(runs.end(), d.first, d.first + d.second);
+  // runs were ticketed in any order; each starts at a distinct record, and run r ends where run r + 1 starts
+  std::sort(runs.begin(), runs.end(), [](const IndexRun& a, const IndexRun& b) { return a.voff < b.voff; });
+  struct Ref {
+    std::vector<std::pair<uint32_t, std::vector<std::pair<uint64_t, uint64_t>>>> bins;  // in order of first use
+    uint64_t beg = 0, end = 0;
+    bool any = false;
+  };
+  std::vector<Ref> refs(nr);
+  const uint64_t data_end = e->data_end_coff << 16;
+  // the runs of one reference are consecutive (sorted input): one bin -> slot table, cleared when the reference changes
+  std::vector<int32_t> slot_of(kIxMetaBin, -1);
+  uint32_t cur = kIxUnplacedRef;
+  size_t chunks = 0;
+  for (size_t i = 0; i < runs.size(); ++i) {
+    const IndexRun& u = runs[i];
+    if (u.ref == kIxUnplacedRef) continue;
+    const uint64_t end = i + 1 < runs.size() ? runs[i + 1].voff : data_end;
+    Ref& R = refs[u.ref];
+    if (u.ref != cur) {
+      if (cur != kIxUnplacedRef) for (auto& bn : refs[cur].bins) slot_of[bn.first] = -1;
+      cur = u.ref;
+    }
+    if (!R.any) { R.any = true; R.beg = u.voff; }
+    R.end = end;
+    int32_t& sl = slot_of[u.bin];
+    if (sl < 0) { sl = (int32_t)R.bins.size(); R.bins.push_back({u.bin, {}}); }
+    auto& ch = R.bins[sl].second;
+    if (!ch.empty() && ch.back().second == u.voff) ch.back().second = end;  // contiguous with the bin's last chunk
+    else { ch.push_back({u.voff, end}); ++chunks; }
+  }
+  std::vector<uint8_t>& b = e->bai;
+  b.clear();
+  b.reserve(16 + (size_t)nr * 64 + chunks * 16 + ((e->ix_win_total + ovf.size()) * 8));
+  auto p32 = [&](uint32_t v) { uint8_t t[4]; memcpy(t, &v, 4); b.insert(b.end(), t, t + 4); };
+  auto p64 = [&](uint64_t v) { uint8_t t[8]; memcpy(t, &v, 8); b.insert(b.end(), t, t + 8); };
+  b.insert(b.end(), {'B', 'A', 'I', 1});
+  p32(nr);
+  std::vector<uint64_t> lin;
+  for (uint32_t c = 0; c < nr; ++c) {
+    const Ref& R = refs[c];
+    if (!R.any) { p32(0); p32(0); continue; }
+    p32((uint32_t)R.bins.size() + 1);
+    for (auto& bn : R.bins) {
+      p32(bn.first);
+      p32((uint32_t)bn.second.size());
+      for (auto& ck : bn.second) { p64(ck.first); p64(ck.second); }
+    }
+    p32(kIxMetaBin); p32(2); p64(R.beg); p64(R.end); p64(counts[2 * c]); p64(counts[2 * c + 1]);
+    // windows nobody touched take the previous window's value (0 before the first touched one)
+    const uint32_t n_intv = maxw[c] + 1;
+    lin.assign(n_intv, ~0ull);
+    const uint32_t in_table = std::min(n_intv, e->ix_win_n[c]);
+    for (uint32_t w = 0; w < in_table; ++w) lin[w] = win[e->ix_win_base[c] + w];
+    for (const IndexRun& o : ovf)
+      if (o.ref == c)
+        for (uint32_t w = o.bin & 0xFFFF; w <= (o.bin >> 16) && w < n_intv; ++w) lin[w] = std::min(lin[w], o.voff);
+    uint64_t last = 0;
+    for (uint32_t w = 0; w < n_intv; ++w) {
+      if (lin[w] == ~0ull) lin[w] = last; else last = lin[w];
+    }
+    p32(n_intv);
+    for (uint64_t v : lin) p64(v);
+  }
+  p64(S.n_no_coor);
+  return NGSQ_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -777,6 +958,8 @@ int ngsq_create(int device, const ngsq_config* cfg, ngsq_engine** out) {
   if (rc != cudaSuccess || n_dev == 0)
     return fail(e, NGSQ_E_CUDA, "no CUDA device available (%s); the ngs-cuda engine has no CPU fallback", cudaGetErrorString(rc));
   if (device < 0 || device >= n_dev) return fail(e, NGSQ_E_ARG, "device %d out of range (%d devices)", device, n_dev);
+  if (cfg && (cfg->flags & NGSQ_F_INDEX) && cfg->max_records)
+    return fail(e, NGSQ_E_ARG, "NGSQ_F_INDEX cannot be combined with max_records: an index covers every record of the file");
   ngsq_engine* ne = new ngsq_engine();
   ne->device = device;
   if (cfg) memcpy(&ne->cfg, cfg, std::min<size_t>(cfg->struct_size ? cfg->struct_size : sizeof(ngsq_config), sizeof(ngsq_config)));
@@ -806,6 +989,11 @@ int ngsq_create(int device, const ngsq_config* cfg, ngsq_engine** out) {
   CUC(cudaMalloc(&e->d_state, sizeof(RunState)));
   CUC(cudaHostAlloc((void**)&e->h_state, sizeof(RunState), cudaHostAllocDefault));
   CUC(cudaHostAlloc((void**)&e->h_prog, kProgSlots * 16, cudaHostAllocDefault));
+  if (e->cfg.flags & NGSQ_F_INDEX) {
+    CUC(cudaMalloc(&e->d_ix, sizeof(IndexState)));
+    CUC(cudaMalloc(&e->d_ix_ovf, kIndexOverflowCap * sizeof(IndexRun)));
+    CUC(cudaHostAlloc((void**)&e->h_ix_probe, 16, cudaHostAllocDefault));
+  }
   CUC(cudaMalloc(&e->d_crc_tables, sizeof(CrcTables)));
   // opt-in shared memory sizes are per device: set them for this engine's device (several engines of
   // one process may sit on different GPUs)
@@ -853,6 +1041,10 @@ void ngsq_destroy(ngsq_engine* e) {
   for (void* p : {(void*)e->d_ed_contigs, (void*)e->d_ed_refs, (void*)e->d_ed_alts, (void*)e->d_ed_res}) if (p) cudaFree(p);
   for (void* p : e->ft_allocs) cudaFree(p);
   for (void* p : {(void*)e->d_ft_contigs, (void*)e->d_ft_res}) if (p) cudaFree(p);
+  for (auto& w : e->ix_waves) cudaEventDestroy(w.done);
+  for (void* p : {(void*)e->d_ix, (void*)e->d_ix_runs[0], (void*)e->d_ix_runs[1], (void*)e->d_ix_ovf, (void*)e->d_ix_win_base, (void*)e->d_ix_win_n,
+                  (void*)e->d_ix_win, (void*)e->d_ix_maxw, (void*)e->d_ix_counts}) if (p) cudaFree(p);
+  if (e->h_ix_probe) cudaFreeHost(e->h_ix_probe);
   for (auto& sg : e->comp_segs) cudaFree(sg.ptr);
   if (e->s_copy) cudaStreamDestroy(e->s_copy);
   if (e->s_comp) cudaStreamDestroy(e->s_comp);
@@ -886,6 +1078,11 @@ int ngsq_reset(ngsq_engine* e) {
   e->h_res.clear(); e->h_qpos = 0;
   e->h_ed_res.clear();
   e->h_ft_res.clear();
+  for (auto& w : e->ix_waves) cudaEventDestroy(w.done);
+  e->ix_waves.clear();
+  e->ix_drained.clear();  // pinned memory of the pin slabs, released above
+  e->data_end_coff = 0;
+  e->bai.clear();
   memset(&e->stats, 0, sizeof e->stats);
   return NGSQ_OK;
 }
@@ -893,6 +1090,10 @@ int ngsq_reset(ngsq_engine* e) {
 int ngsq_set_references(ngsq_engine* e, uint32_t n_ref, const uint32_t* ref_len, const uint8_t* coverage_enabled) {
   if (!e || (n_ref && (!ref_len || !coverage_enabled))) return fail(e, NGSQ_E_ARG, "bad references");
   if (e->run_started) return fail(e, NGSQ_E_ARG, "ngsq_set_references must precede the first submit");
+  if (e->cfg.flags & NGSQ_F_INDEX)
+    for (uint32_t c = 0; c < n_ref; ++c)
+      if (ref_len[c] >= kIxMaxEnd)
+        return fail(e, NGSQ_E_ARG, "reference %u is %u bases long: a BAI addresses fewer than 2^29 bases (index this file as CSI)", c, ref_len[c]);
   CU(cudaSetDevice(e->device));
   e->n_ref = n_ref;
   e->ref_len.assign(ref_len, ref_len + n_ref);
@@ -979,6 +1180,28 @@ int ngsq_set_references(ngsq_engine* e, uint32_t n_ref, const uint32_t* ref_len,
     if (n_ref) CU(cudaMemcpy(e->d_ft_contigs, e->ft_contigs.data(), n_ref * sizeof(FeatureContig), cudaMemcpyHostToDevice));
     if (!e->d_ft_res) CU(cudaMalloc(&e->d_ft_res, F_WORDS * 8));
   }
+  if (e->cfg.flags & NGSQ_F_INDEX) {
+    // linear-index table per reference: windows 0 ..= L >> 14 (reads overhanging the end go to the overflow list)
+    e->ix_win_base.assign(n_ref, 0);
+    e->ix_win_n.assign(n_ref, 0);
+    uint64_t total = 0;
+    for (uint32_t c = 0; c < n_ref; ++c) {
+      e->ix_win_base[c] = total;
+      e->ix_win_n[c] = (ref_len[c] >> kIxWindowShift) + 1;
+      total += e->ix_win_n[c];
+    }
+    e->ix_win_total = total;
+    for (void* p : {(void*)e->d_ix_win_base, (void*)e->d_ix_win_n, (void*)e->d_ix_win, (void*)e->d_ix_maxw, (void*)e->d_ix_counts}) if (p) cudaFree(p);
+    CU(cudaMalloc(&e->d_ix_win_base, nr * 8));
+    CU(cudaMalloc(&e->d_ix_win_n, nr * 4));
+    CU(cudaMalloc(&e->d_ix_win, std::max<uint64_t>(total, 1) * 8));
+    CU(cudaMalloc(&e->d_ix_maxw, nr * 4));
+    CU(cudaMalloc(&e->d_ix_counts, nr * 16));
+    if (n_ref) {
+      CU(cudaMemcpy(e->d_ix_win_base, e->ix_win_base.data(), n_ref * 8, cudaMemcpyHostToDevice));
+      CU(cudaMemcpy(e->d_ix_win_n, e->ix_win_n.data(), n_ref * 4, cudaMemcpyHostToDevice));
+    }
+  }
   return NGSQ_OK;
 }
 
@@ -1060,6 +1283,8 @@ int ngsq_set_reference_bases(ngsq_engine* e, uint32_t ref, const uint8_t* letter
 int ngsq_set_range(ngsq_engine* e, uint64_t first_rec_voffset, uint64_t end_voffset) {
   if (!e) return NGSQ_E_ARG;
   if (e->launched) return fail(e, NGSQ_E_ARG, "ngsq_set_range must precede the first submit of a run");
+  if ((e->cfg.flags & NGSQ_F_INDEX) && end_voffset)
+    return fail(e, NGSQ_E_ARG, "NGSQ_F_INDEX needs end_voffset 0: an index covers the whole file from its first record");
   e->first_voff = first_rec_voffset;
   e->end_voff = end_voffset;
   e->range_set = true;
@@ -1338,6 +1563,18 @@ int ngsq_finish(ngsq_engine* e) {
     const uint64_t k = e->h_ft_res[F_ERR];
     return fail(e, NGSQ_E_FEATURES, "Genomic Features: %s (the reference aborts the run here)", k < sizeof kinds / sizeof *kinds ? kinds[k] : "unknown failure");
   }
+  if (e->cfg.flags & NGSQ_F_INDEX) return finish_index(e);
+  return NGSQ_OK;
+}
+
+int ngsq_get_bai(ngsq_engine* e, uint8_t* out, size_t cap, size_t* n_out) {
+  if (!e) return NGSQ_E_ARG;
+  if (!(e->cfg.flags & NGSQ_F_INDEX)) return fail(e, NGSQ_E_ARG, "ngsq_get_bai: the engine was created without NGSQ_F_INDEX");
+  if (!e->finished || e->bai.empty()) return fail(e, NGSQ_E_ARG, "ngsq_get_bai: no index before a successful ngsq_finish");
+  if (n_out) *n_out = e->bai.size();
+  if (!out && !cap) return NGSQ_OK;
+  if (!out || cap < e->bai.size()) return fail(e, NGSQ_E_ARG, "ngsq_get_bai: buffer holds %zu bytes, %zu needed", cap, e->bai.size());
+  memcpy(out, e->bai.data(), e->bai.size());
   return NGSQ_OK;
 }
 
@@ -1506,6 +1743,7 @@ int ngsq_refresh_results(ngsq_engine* e) {
 // first reduce of an engine agrees on the layout beforehand (a mismatch would mean mismatched counts inside NCCL).
 int ngsq_reduce(ngsq_engine* e, int root) {
   if (!e || !e->finished) return fail(e, NGSQ_E_ARG, "reduce before finish");
+  if (e->cfg.flags & NGSQ_F_INDEX) return fail(e, NGSQ_E_ARG, "ngsq_reduce: an index is built by one engine over the whole file (NGSQ_F_INDEX)");
   if (!e->comm) return fail(e, NGSQ_E_NCCL, "ngsq_comm_init was not called");
   if (e->n_ranks > (int)kMaxRanks) return fail(e, NGSQ_E_ARG, "at most %u ranks", kMaxRanks);
   CU(cudaSetDevice(e->device));

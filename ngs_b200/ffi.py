@@ -22,11 +22,13 @@ NGSQ_F_VERIFY_CRC = 4
 NGSQ_F_EDITS = 8
 NGSQ_F_FEATURES = 16
 NGSQ_F_SERIAL_STAGES = 32  # measurement aid: no overlap between the stages of consecutive waves
+NGSQ_F_INDEX = 64  # build the file's BAI in the same pass (Engine.bai())
 
 ERROR_NAMES = {
     0: "NGSQ_OK", -1: "NGSQ_E_ARG", -2: "NGSQ_E_CUDA", -3: "NGSQ_E_TRUNCATED", -4: "NGSQ_E_BAD_BLOCK",
     -5: "NGSQ_E_CRC", -6: "NGSQ_E_BAD_RECORD", -7: "NGSQ_E_QUAL_RANGE", -8: "NGSQ_E_CHAIN",
     -9: "NGSQ_E_NCCL", -10: "NGSQ_E_NOMEM", -11: "NGSQ_E_EDITS", -12: "NGSQ_E_FEATURES", -13: "NGSQ_E_QUAL_CAP",
+    -14: "NGSQ_E_UNSORTED",
 }
 
 # every symbol include/ngs_cuda.h declares (tests check the library exports all of them)
@@ -38,6 +40,7 @@ EXPORTED = [
     "ngsq_result_buffer", "ngsq_refresh_results", "ngsq_host_alloc", "ngsq_host_free", "ngsq_inflate_to_host",
     "ngsq_set_reference_bases", "ngsq_get_edits", "ngsq_get_edit_positions", "ngsq_set_feature_model", "ngsq_set_features", "ngsq_get_features",
     "ngsq_wait_copied", "ngsq_host_register", "ngsq_host_unregister", "ngsq_flush", "ngsq_progress",
+    "ngsq_get_bai",
 ]
 
 
@@ -132,6 +135,7 @@ def load_library() -> C.CDLL:
     lib.ngsq_progress.argtypes = [P, u64p]
     lib.ngsq_host_register.argtypes = [P, C.c_size_t]
     lib.ngsq_host_unregister.argtypes = [P]
+    lib.ngsq_get_bai.argtypes = [P, P, C.c_size_t, C.POINTER(C.c_size_t)]
     _lib = lib
     return lib
 
@@ -319,6 +323,15 @@ class Engine:
         out = np.zeros(9, dtype=np.uint64)
         self._check(self.lib.ngsq_get_features(self.h, out.ctypes.data_as(C.POINTER(C.c_uint64))))
         return out
+
+    # ---- BAI (NGSQ_F_INDEX) ----
+    def bai(self) -> bytes:
+        """The .bai file of the records submitted since set_range (after finish)."""
+        n = C.c_size_t(0)
+        self._check(self.lib.ngsq_get_bai(self.h, None, 0, C.byref(n)))
+        buf = np.empty(max(n.value, 1), dtype=np.uint8)
+        self._check(self.lib.ngsq_get_bai(self.h, buf.ctypes.data, n.value, C.byref(n)))
+        return buf[: n.value].tobytes()
 
     def stats(self) -> dict:
         st = Stats()

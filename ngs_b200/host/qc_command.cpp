@@ -1,10 +1,13 @@
 // ngs-cuda-qc — host driver of the CUDA `ngs qc` path.  Mirrors the reference's subcommand
 // (src/qc/command.rs): QcArgs (36-102), qc() (109-218), app() (226-421).  Same positional
 // arguments and flags, same checks in the same order, same output file; the two hot loops of
-// app() (305-316 and 350-397) are replaced by one pass of the CUDA engine per GPU.
+// app() (305-316 and 350-397) are replaced by one pass of the CUDA engine per GPU.  `index` builds the
+// BAI that `qc` needs (src/index/bam.rs:39-109) in one pass of the engine on one GPU.
 //
 //   ngs-cuda-qc qc <BAM> <REFERENCE_GENOME> [-n N] [-o DIR] [-p PREFIX] [--only FACET]
 //               [--cuda-devices 0,1,..] [--cuda-gc-seed S] [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io] [--cuda-perf]
+//   ngs-cuda-qc index <BAM> [--cuda-device N] [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io]
+#include <cerrno>
 #include <cstdio>
 #include <cstdlib>
 #include <filesystem>
@@ -349,9 +352,86 @@ int qc(const QcArgs& args) {
   return app(args, *genome, prefix, outdir);
 }
 
+// `ngs index` for a BAM (src/index/bam.rs:39-109): the header, then every record through the engine's NGSQ_F_INDEX pass, and
+// the .bai next to the file (utils/pathbuf.rs:59-75: x.bam -> x.bam.bai).  Like the reference (bam.rs:52-58) it never
+// overwrites an existing index.
+struct IndexArgs {
+  std::string src;
+  int device = 0;
+  bool verify_crc = true;
+  size_t chunk_mb = 64;
+  bool direct_io = true;
+};
+
+int index_bam(const IndexArgs& a) {
+  info("Starting index command...");
+  const std::string dst = a.src + ".bai";
+  if (std::filesystem::exists(dst)) throw std::runtime_error("index file already exists: " + dst);
+  MappedFile file(a.src);
+  ngsq_config cfg{};
+  cfg.struct_size = sizeof cfg;
+  cfg.flags = NGSQ_F_INDEX | (a.verify_crc ? NGSQ_F_VERIFY_CRC : 0u);
+  ngsq_engine* e = nullptr;
+  if (ngsq_create(a.device, &cfg, &e)) throw std::runtime_error(std::string("CUDA engine: ") + ngsq_last_error(nullptr));
+  struct Cleanup { ngsq_engine* e; ~Cleanup() { ngsq_destroy(e); } } cleanup{e};
+  BamHeader header = read_bam_header(e, file.data(), file.size());
+  std::vector<uint32_t> ref_len;
+  for (auto& rs : header.reference_sequences) ref_len.push_back(rs.length);
+  std::vector<uint8_t> no_coverage(ref_len.size(), 0);
+  check(e, ngsq_set_references(e, (uint32_t)ref_len.size(), ref_len.data(), no_coverage.data()));
+  check(e, ngsq_set_range(e, header.first_record_voffset, 0));
+  info("Indexing BAM file.");
+  {
+    ChunkReader reader(a.src, a.chunk_mb << 20, a.direct_io);
+    Progress progress;
+    reader.run(e, std::min<uint64_t>(header.first_record_voffset >> 16, file.size()), file.size(), &progress);
+    check(e, ngsq_finish(e));
+    progress.report(e);
+  }
+  ngsq_stats st;
+  check(e, ngsq_get_stats(e, &st));
+  info("Processed " + std::to_string(st.records) + " records.");
+  size_t n = 0;
+  check(e, ngsq_get_bai(e, nullptr, 0, &n));
+  std::vector<uint8_t> bai(n);
+  check(e, ngsq_get_bai(e, bai.data(), bai.size(), &n));
+  info("Writing index to " + dst + ".");
+  // O_EXCL: an index that appeared while the file was read is not replaced either
+  const int fd = open(dst.c_str(), O_WRONLY | O_CREAT | O_EXCL, 0644);
+  if (fd < 0) throw std::runtime_error("cannot create " + dst + (errno == EEXIST ? ": index file already exists" : ""));
+  size_t done = 0;
+  while (done < bai.size()) {
+    const ssize_t w = write(fd, bai.data() + done, bai.size() - done);
+    if (w <= 0) { close(fd); std::filesystem::remove(dst); throw std::runtime_error("write error on " + dst); }
+    done += (size_t)w;
+  }
+  if (close(fd)) { std::filesystem::remove(dst); throw std::runtime_error("write error on " + dst); }
+  return 0;
+}
+
+int index_main(int argc, char** argv, int i) {
+  IndexArgs a;
+  std::vector<std::string> pos;
+  for (; i < argc; ++i) {
+    std::string s = argv[i];
+    auto val = [&]() -> std::string { if (i + 1 >= argc) throw std::runtime_error("missing value for " + s); return argv[++i]; };
+    if (s == "--cuda-device") a.device = std::stoi(val());
+    else if (s == "--cuda-no-crc") a.verify_crc = false;
+    else if (s == "--cuda-chunk-mb") a.chunk_mb = std::stoull(val());
+    else if (s == "--cuda-buffered-io") a.direct_io = false;
+    else if (!s.empty() && s[0] == '-' && s != "-") throw std::runtime_error("unknown flag " + s);
+    else pos.push_back(s);
+  }
+  if (pos.size() != 1 || !a.chunk_mb) return -1;
+  a.src = pos[0];
+  return index_bam(a);
+}
+
 void usage() {
   std::cerr << "usage: ngs-cuda-qc qc <BAM> <REFERENCE_GENOME> [-n N] [-o DIR] [-p PREFIX] [--only FACET]\n"
-               "                  [--cuda-devices 0,1,..] [--cuda-gc-seed S] [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io] [--cuda-perf]\n";
+               "                  [--cuda-devices 0,1,..] [--cuda-gc-seed S] [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io] [--cuda-perf]\n"
+               "       ngs-cuda-qc index <BAM> [--cuda-device N] [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io]\n"
+               "                  (writes <BAM>.bai; an existing index is never overwritten)\n";
 }
 
 }  // namespace
@@ -361,6 +441,11 @@ extern "C" int ngs_cuda_qc_main(int argc, char** argv) {
     QcArgs a;
     std::vector<std::string> pos;
     int i = 1;
+    if (i < argc && std::string(argv[i]) == "index") {
+      const int rc = index_main(argc, argv, i + 1);
+      if (rc < 0) { usage(); return 2; }
+      return rc;
+    }
     if (i < argc && std::string(argv[i]) == "qc") ++i;
     for (; i < argc; ++i) {
       std::string s = argv[i];
