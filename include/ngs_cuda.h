@@ -119,7 +119,8 @@ typedef struct ngsq_stats {
   uint32_t inflate_launches, other_launches;
   float ms_inflate_decode;   /* of ms_inflate: the lane-per-block Huffman decode kernel */
   float ms_inflate_resolve;  /* of ms_inflate: the warp-per-block LZ77 resolve kernel */
-  float ms_reduce;           /* ngsq_reduce: agreement all-reduce + sum-reduce + refresh (0 without it) */
+  float ms_reduce;           /* ngsq_reduce: agreement all-reduce + split-reference reduce and resolve + sum-reduce + refresh
+                                (0 without it) */
   float ms_edits;            /* VAF histogram of the Edits facet (its per-record kernel runs inside ms_facets) */
   float ms_tail;             /* start of the LAST wave -> end of finish: what is left once the last chunk has arrived */
   uint32_t waves;            /* inflate waves of the run (= inflate_launches) */
@@ -225,7 +226,8 @@ int ngsq_get_edits(ngsq_engine* e, uint64_t read_one[513], uint64_t read_two[513
 /* The VAF file of edits.rs:317-340 (`--vaf-file`): refs_per_position / alts_per_position of header sequence `ref` when its
  * teardown runs, n = sequence length + 1 entries each, index = 1-based reference position (alignment_start + reference_ptr,
  * edits.rs:279-281; entry 0 stays 0).  After ngsq_finish; with several engines every engine holds the counts of the records
- * of its own shard (contig-exclusive shards: the owner's are the sequence's). */
+ * of its own shard (contig-exclusive shards: the owner's are the sequence's; a split reference's counts are the root's once
+ * merged, the other engines' are zero). */
 int ngsq_get_edit_positions(ngsq_engine* e, uint32_t ref, uint32_t* refs, uint32_t* alts, uint64_t n);
 int ngsq_get_stats(ngsq_engine* e, ngsq_stats* out);
 /* NGSQ_F_INDEX: the complete .bai file (magic, every reference's bins, chunks, metadata pseudo-bin 37450 and linear index,
@@ -244,6 +246,29 @@ int ngsq_set_quality_positions(ngsq_engine* e, uint32_t n_positions);
 int ngsq_result_buffer(ngsq_engine* e, void** dev_ptr, size_t* n_words);
 /* After an external reduction of that buffer: refresh the host copy the ngsq_get_* getters read. */
 int ngsq_refresh_results(ngsq_engine* e);
+
+/* ---- shards cut inside a contig (DESIGN.md section 5) ----
+ * Reference `ref` is split between shards: this engine scatters into its arrays as usual, but ngsq_finish does not resolve
+ * it (K9, and the Edits VAF pass); ngsq_reduce sums every rank's partial arrays of ref onto `root` and resolves it there.
+ * Same set on every rank; after ngsq_set_references, before the first submit; kept across ngsq_reset.  Change the set only
+ * together with ngsq_set_references on every rank: a rank that adds a reference on its own re-runs the layout agreement of its
+ * next ngsq_reduce alone, and the ranks' collectives no longer match.
+ * NGSQ_E_ARG with NGSQ_F_INDEX or max_records != 0.  Until the merge, ngsq_get_coverage_contig and ngsq_get_edit_positions
+ * of a split reference, and ngsq_get_edits whenever one is declared, fail with NGSQ_E_ARG instead of partial numbers. */
+int ngsq_split_reference(ngsq_engine* e, uint32_t ref);
+
+/* Callers that bring their own collective (the pattern of ngsq_result_buffer): the device arrays of a split reference.
+ * Valid until the next ngsq_set_references or ngsq_set_quality_positions. */
+struct ngsq_split_arrays {
+  int32_t*  diff;       uint64_t n_diff;       /* coverage difference array, L + 2 (NULL without NGSQ_F_COVERAGE / mask) */
+  int32_t*  tile_sums;  uint64_t n_tiles;      /* its 4096-position tile sums */
+  uint64_t* touched;                           /* the contig's touched word */
+  uint32_t* edit_refs;  uint32_t* edit_alts;  uint64_t n_positions;  /* L + 1 each (NULL without NGSQ_F_EDITS) */
+};
+int ngsq_split_arrays(ngsq_engine* e, uint32_t ref, struct ngsq_split_arrays* out);
+/* After the caller summed every engine's split arrays element-wise into the root's: the root resolves its split references
+ * into its result buffer; every other engine zeroes its split partials (so per-position reads and later sums count once). */
+int ngsq_resolve_split(ngsq_engine* e, int is_root);
 
 /* ---- utilities ---- */
 void* ngsq_host_alloc(size_t nbytes); /* pinned host memory for ngsq_submit */

@@ -99,6 +99,20 @@ pub mod sys {
     pub const NGSQ_F_INDEX: u32 = 64;
     pub const NGSQ_E_UNSORTED: c_int = -14;
 
+    /// Device arrays of a reference split between shards (`struct ngsq_split_arrays`); null pointers for facets that are off.
+    #[repr(C)]
+    #[derive(Clone, Copy, Debug)]
+    pub struct NgsqSplitArrays {
+        pub diff: *mut i32,
+        pub n_diff: u64,
+        pub tile_sums: *mut i32,
+        pub n_tiles: u64,
+        pub touched: *mut u64,
+        pub edit_refs: *mut u32,
+        pub edit_alts: *mut u32,
+        pub n_positions: u64,
+    }
+
     extern "C" {
         pub fn ngsq_version() -> c_int;
         pub fn ngsq_last_error(e: *mut NgsqEngine) -> *const c_char;
@@ -139,6 +153,9 @@ pub mod sys {
         pub fn ngsq_host_unregister(p: *mut c_void) -> c_int;
         pub fn ngsq_get_bai(e: *mut NgsqEngine, out: *mut u8, cap: usize, n_out: *mut usize) -> c_int;
         pub fn ngsq_inflate_to_host(e: *mut NgsqEngine, bgzf: *const u8, nbytes: usize, out: *mut u8, cap: usize, n_out: *mut usize) -> c_int;
+        pub fn ngsq_split_reference(e: *mut NgsqEngine, r: u32) -> c_int;
+        pub fn ngsq_split_arrays(e: *mut NgsqEngine, r: u32, out: *mut NgsqSplitArrays) -> c_int;
+        pub fn ngsq_resolve_split(e: *mut NgsqEngine, is_root: c_int) -> c_int;
     }
 }
 
@@ -431,9 +448,36 @@ impl Engine {
     pub fn comm_init(&mut self, n_ranks: i32, rank: i32, id: &[c_char; 128]) -> anyhow::Result<()> {
         self.check(unsafe { sys::ngsq_comm_init(self.raw, n_ranks, rank, id.as_ptr()) })
     }
-    /// ONE sum all-reduce of the packed integer results (after every engine's `finish`).
+    /// ONE sum all-reduce of the packed integer results (after every engine's `finish`); references declared with
+    /// `split_reference` are summed onto `root` and resolved there first.
     pub fn reduce(&mut self, root: i32) -> anyhow::Result<()> {
         self.check(unsafe { sys::ngsq_reduce(self.raw, root) })
+    }
+
+    // ---- shards cut inside a contig (DESIGN.md section 5) ----
+    /// Declares reference `r` split between shards: the same set on every engine, after `set_references`, before the first
+    /// submit.  Its coverage and VAF counters are resolved by `reduce` (or `resolve_split`), not by `finish`.
+    pub fn split_reference(&mut self, r: u32) -> anyhow::Result<()> {
+        self.check(unsafe { sys::ngsq_split_reference(self.raw, r) })
+    }
+    /// The device arrays of a split reference, for a caller that sums them with its own collective.
+    pub fn split_arrays(&mut self, r: u32) -> anyhow::Result<sys::NgsqSplitArrays> {
+        let mut out = sys::NgsqSplitArrays {
+            diff: std::ptr::null_mut(),
+            n_diff: 0,
+            tile_sums: std::ptr::null_mut(),
+            n_tiles: 0,
+            touched: std::ptr::null_mut(),
+            edit_refs: std::ptr::null_mut(),
+            edit_alts: std::ptr::null_mut(),
+            n_positions: 0,
+        };
+        self.check(unsafe { sys::ngsq_split_arrays(self.raw, r, &mut out) })?;
+        Ok(out)
+    }
+    /// After the split arrays of every engine were summed into the root's: resolve them on the root, zero them elsewhere.
+    pub fn resolve_split(&mut self, is_root: bool) -> anyhow::Result<()> {
+        self.check(unsafe { sys::ngsq_resolve_split(self.raw, is_root as c_int) })
     }
 }
 

@@ -211,6 +211,11 @@ struct ngsq_engine {
   uint64_t data_end_coff = 0;        // end of the last non-empty block submitted (the offset after the last record)
   std::vector<uint8_t> bai;
 
+  // references split between shards (ngsq_split_reference): scattered as usual, resolved only by the merge
+  std::vector<uint8_t> split_ref;
+  uint32_t n_split = 0;
+  bool split_merged = false;         // the split references of this run have been merged (reduce / resolve_split)
+
   // nccl
   void* comm = nullptr;
   int n_ranks = 1, rank = 0;
@@ -941,6 +946,69 @@ int finish_index(ngsq_engine* e) {
   return NGSQ_OK;
 }
 
+// K9 for contig c: scan of its tile sums, then the streaming resolve into its result slot (both skip an untouched contig)
+void launch_cov_resolve(ngsq_engine* e, uint32_t c, cudaStream_t s) {
+  uint32_t n = e->ref_len[c] + 1;
+  uint32_t n_tiles = (n + kCovTile - 1) / kCovTile;
+  const int32_t* df = e->d_diff + e->diff_base[c];
+  uint64_t* slot = e->d_res + e->cov_slot[c];
+  cov_scan_tiles_kernel<<<1, 1024, 0, s>>>(e->d_tile_sum + e->tile_off[c], e->d_tile, n_tiles, slot + COV_TOUCHED);
+  const uint32_t grid = std::min<uint32_t>(n_tiles, e->n_sm * 4);
+  cov_resolve_kernel<<<grid, kCovThreads, 0, s>>>(df, n, e->d_tile, n_tiles, slot);
+  e->other_launches += 2;
+}
+
+// K11 teardown over the per-position counters [off, off + n)
+void launch_vaf(ngsq_engine* e, uint64_t off, uint64_t n, cudaStream_t s) {
+  const uint32_t vgrid = (uint32_t)std::min<uint64_t>((n + 255) / 256, (uint64_t)e->n_sm * 8);
+  edits_vaf_kernel<<<vgrid, 256, 0, s>>>(e->d_ed_refs + off, e->d_ed_alts + off, n, e->d_ed_res);
+  e->other_launches += 1;
+}
+
+uint32_t cov_tiles(const ngsq_engine* e, uint32_t c) { return (uint32_t)(((uint64_t)e->ref_len[c] + 1 + kCovTile - 1) / kCovTile); }
+bool is_split(const ngsq_engine* e, uint32_t c) { return c < e->split_ref.size() && e->split_ref[c]; }
+bool edits_loaded(const ngsq_engine* e) { return (e->cfg.flags & NGSQ_F_EDITS) && e->d_ed_res && e->ed_contigs.size() == e->n_ref; }
+
+// Folded into the layout word the ranks agree on: 0 without split references, so that layout stays what it was.
+uint64_t split_signature(const ngsq_engine* e) {
+  uint64_t h = 0;
+  for (uint32_t c = 0; c < e->n_ref; ++c) {
+    if (!e->split_ref[c]) continue;
+    uint64_t z = h ^ (0x9E3779B97F4A7C15ull * (c + 1ull));
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    h = z ^ (z >> 31);
+  }
+  return e->n_split ? (h | 1) : 0;
+}
+
+// Once every rank's split arrays have been summed into the root's: the root resolves its split references (K9 and the VAF
+// pass over their counters; a contig is resolved iff some rank touched it); every other rank zeroes its partials, so that
+// per-position reads and later sums of result buffers count each position once.  Enqueued on s.
+int merge_split_local(ngsq_engine* e, bool is_root, cudaStream_t s) {
+  const bool edits = edits_loaded(e) && e->ed_pos_total;
+  for (uint32_t c = 0; c < e->n_ref; ++c) {
+    if (!e->split_ref[c]) continue;
+    if (is_root) {
+      if (e->cov_enabled[c]) launch_cov_resolve(e, c, s);
+      if (edits) launch_vaf(e, e->ed_contigs[c].pos_off, (uint64_t)e->ed_contigs[c].hdr_len + 1, s);
+    } else {
+      if (e->cov_enabled[c]) {
+        CU(cudaMemsetAsync(e->d_diff + e->diff_base[c], 0, ((uint64_t)e->ref_len[c] + 2) * 4, s));
+        CU(cudaMemsetAsync(e->d_tile_sum + e->tile_off[c], 0, (size_t)cov_tiles(e, c) * 4, s));
+        CU(cudaMemsetAsync(e->d_res + e->cov_slot[c] + COV_TOUCHED, 0, 8, s));
+      }
+      if (edits) {
+        const EditsContig& ec = e->ed_contigs[c];
+        CU(cudaMemsetAsync(e->d_ed_refs + ec.pos_off, 0, ((uint64_t)ec.hdr_len + 1) * 4, s));
+        CU(cudaMemsetAsync(e->d_ed_alts + ec.pos_off, 0, ((uint64_t)ec.hdr_len + 1) * 4, s));
+      }
+    }
+  }
+  CU(cudaGetLastError());
+  return NGSQ_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1083,6 +1151,7 @@ int ngsq_reset(ngsq_engine* e) {
   e->ix_drained.clear();  // pinned memory of the pin slabs, released above
   e->data_end_coff = 0;
   e->bai.clear();
+  e->split_merged = false;  // the split set itself is kept
   memset(&e->stats, 0, sizeof e->stats);
   return NGSQ_OK;
 }
@@ -1101,6 +1170,9 @@ int ngsq_set_references(ngsq_engine* e, uint32_t n_ref, const uint32_t* ref_len,
   if (!(e->cfg.flags & NGSQ_F_COVERAGE)) std::fill(e->cov_enabled.begin(), e->cov_enabled.end(), 0);
   e->diff_base.assign(n_ref, 0);
   e->tile_off.assign(n_ref, 0);
+  e->split_ref.assign(n_ref, 0);
+  e->n_split = 0;
+  e->split_merged = false;
   e->layout_agreed = false;
   uint64_t elems = 0, tiles = 0;
   uint32_t max_tiles = 1;
@@ -1446,29 +1518,28 @@ int ngsq_finish(ngsq_engine* e) {
     CU(cudaStreamWaitEvent(s, e->waves.back().facets_end, 0));  // the scan stream's last kernel
   }
   CU(cudaEventRecord(e->ev_d, s));
-  // K9
+  // K9 (split references wait for the merge: their arrays hold this shard's part only)
   if (e->cfg.flags & NGSQ_F_COVERAGE) {
-    for (uint32_t c = 0; c < e->n_ref; ++c) {
-      if (!e->cov_enabled[c]) continue;
-      uint32_t n = e->ref_len[c] + 1;
-      uint32_t n_tiles = (n + kCovTile - 1) / kCovTile;
-      const int32_t* df = e->d_diff + e->diff_base[c];
-      uint64_t* slot = e->d_res + e->cov_slot[c];
-      cov_scan_tiles_kernel<<<1, 1024, 0, s>>>(e->d_tile_sum + e->tile_off[c], e->d_tile, n_tiles, slot + COV_TOUCHED);
-      const uint32_t grid = std::min<uint32_t>(n_tiles, e->n_sm * 4);
-      cov_resolve_kernel<<<grid, kCovThreads, 0, s>>>(df, n, e->d_tile, n_tiles, slot);
-      e->other_launches += 2;
-    }
+    for (uint32_t c = 0; c < e->n_ref; ++c)
+      if (e->cov_enabled[c] && !e->split_ref[c]) launch_cov_resolve(e, c, s);
     CU(cudaGetLastError());
   }
   CU(cudaEventRecord(e->ev_e, s));
-  // K11 teardown (edits.rs:318-334): the VAF histogram over the per-position counters of every wave
-  const bool do_edits = (e->cfg.flags & NGSQ_F_EDITS) && e->d_ed_res && e->ed_contigs.size() == e->n_ref;
+  // K11 teardown (edits.rs:318-334): the VAF histogram over the per-position counters of every wave; with split references,
+  // one launch per run of contiguous non-split contigs (the counters are laid out contig after contig)
+  const bool do_edits = edits_loaded(e);
   if (do_edits && e->ed_pos_total && !e->waves.empty()) {
-    const uint32_t vgrid = (uint32_t)std::min<uint64_t>((e->ed_pos_total + 255) / 256, (uint64_t)e->n_sm * 8);
-    edits_vaf_kernel<<<vgrid, 256, 0, s>>>(e->d_ed_refs, e->d_ed_alts, e->ed_pos_total, e->d_ed_res);
+    if (!e->n_split) {
+      launch_vaf(e, 0, e->ed_pos_total, s);
+    } else {
+      uint64_t run_beg = 0, run_end = 0;
+      for (uint32_t c = 0; c <= e->n_ref; ++c) {
+        if (c < e->n_ref && !e->split_ref[c]) { run_end = e->ed_contigs[c].pos_off + e->ed_contigs[c].hdr_len + 1; continue; }
+        if (run_end > run_beg) launch_vaf(e, run_beg, run_end - run_beg, s);
+        if (c < e->n_ref) run_beg = run_end = e->ed_contigs[c].pos_off + e->ed_contigs[c].hdr_len + 1;
+      }
+    }
     CU(cudaGetLastError());
-    e->other_launches += 1;
   }
   if (do_edits) {
     e->h_ed_res.resize(E_WORDS);
@@ -1590,6 +1661,8 @@ int ngsq_get_edits(ngsq_engine* e, uint64_t read_one[513], uint64_t read_two[513
   if (!e) return NGSQ_E_ARG;
   if (!e->finished || e->h_ed_res.size() != E_WORDS) return fail(e, NGSQ_E_ARG, "Edits results requested before ngsq_finish or without NGSQ_F_EDITS");
   if (e->h_ed_res[E_ERR]) return fail(e, NGSQ_E_EDITS, "the Edits facet failed; no results");
+  if (e->n_split && !e->split_merged)
+    return fail(e, NGSQ_E_ARG, "Edits results requested before the split references were merged (ngsq_reduce or ngsq_resolve_split): the VAF histogram is incomplete");
   if (read_one) memcpy(read_one, &e->h_ed_res[E_READ_ONE], 513 * 8);
   if (read_two) memcpy(read_two, &e->h_ed_res[E_READ_TWO], 513 * 8);
   if (vaf) memcpy(vaf, &e->h_ed_res[E_VAF], 101 * 8);
@@ -1604,6 +1677,8 @@ int ngsq_get_edit_positions(ngsq_engine* e, uint32_t ref, uint32_t* refs, uint32
   if (!e->finished || e->h_ed_res.size() != E_WORDS) return fail(e, NGSQ_E_ARG, "Edits results requested before ngsq_finish or without NGSQ_F_EDITS");
   if (e->h_ed_res[E_ERR]) return fail(e, NGSQ_E_EDITS, "the Edits facet failed; no results");
   if (ref >= e->n_ref || ref >= e->ed_contigs.size() || !refs || !alts) return fail(e, NGSQ_E_ARG, "ngsq_get_edit_positions: bad reference id or null output");
+  if (is_split(e, ref) && !e->split_merged)
+    return fail(e, NGSQ_E_ARG, "ngsq_get_edit_positions: reference %u is split between shards and not merged yet (ngsq_reduce or ngsq_resolve_split)", ref);
   const EditsContig& c = e->ed_contigs[ref];
   if (n != (uint64_t)c.hdr_len + 1) return fail(e, NGSQ_E_ARG, "ngsq_get_edit_positions: reference %u has %u + 1 positions, %llu requested", ref, c.hdr_len, (unsigned long long)n);
   CU(cudaSetDevice(e->device));
@@ -1651,6 +1726,8 @@ int ngsq_get_quality(ngsq_engine* e, uint64_t* out, size_t cap_positions, uint32
 int ngsq_get_coverage_contig(ngsq_engine* e, uint32_t ref, ngsq_cov_ints* out, uint64_t* bin_sums, size_t cap) {
   NEED_RESULTS();
   if (ref >= e->n_ref || !out) return fail(e, NGSQ_E_ARG, "bad reference index");
+  if (is_split(e, ref) && !e->split_merged)
+    return fail(e, NGSQ_E_ARG, "reference %u is split between shards and not merged yet (ngsq_reduce or ngsq_resolve_split)", ref);
   memset(out, 0, sizeof *out);
   if (!e->cov_enabled[ref]) return NGSQ_OK;
   const uint64_t* slot = &e->h_res[e->cov_slot[ref]];
@@ -1749,9 +1826,10 @@ int ngsq_reduce(ngsq_engine* e, int root) {
   CU(cudaSetDevice(e->device));
   cudaStream_t s = e->s_comp;
   CU(cudaEventRecord(e->ev_a, s));
-  const int ncclUint64 = 5, ncclSum = 0, ncclMax = 2;
+  const int ncclInt32 = 2, ncclUint32 = 3, ncclUint64 = 5, ncclSum = 0, ncclMax = 2;
   auto nccl_err = [&](const char* what, int rc) { return fail(e, NGSQ_E_NCCL, "%s: %s", what, g_nccl.GetErrorString ? g_nccl.GetErrorString(rc) : "?"); };
-  const uint64_t layout = (uint64_t)e->qual_off | ((uint64_t)e->qpos_cap << 32);
+  // the split set is part of the agreed layout: ranks that disagree on it would issue different collectives below
+  const uint64_t layout = ((uint64_t)e->qual_off | ((uint64_t)e->qpos_cap << 32)) ^ split_signature(e);
   int rc;
   if (!e->layout_agreed) {
     uint64_t agree[2] = {layout, ~layout};
@@ -1762,9 +1840,35 @@ int ngsq_reduce(ngsq_engine* e, int root) {
     CU(cudaMemcpyAsync(agree, d_agree, sizeof agree, cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
     if (agree[0] != layout || ~agree[1] != layout)
-      return fail(e, NGSQ_E_ARG, "result layouts differ across ranks: ngsq_set_references must get the same lengths and coverage mask, and ngsq_config.quality_positions the same value, on every rank");
+      return fail(e, NGSQ_E_ARG, "result layouts differ across ranks: ngsq_set_references must get the same lengths and coverage mask, ngsq_split_reference the same references, and ngsq_config.quality_positions the same value, on every rank");
     e->layout_agreed = true;
     e->other_launches += 1;
+  }
+  // split references first: every rank's partial arrays summed onto the root, which resolves them before the result buffer
+  // (its slots of those contigs included) is summed below
+  if (e->n_split && !e->split_merged) {
+    const bool edits = edits_loaded(e) && e->ed_pos_total;
+    for (uint32_t c = 0; c < e->n_ref; ++c) {
+      if (!e->split_ref[c]) continue;
+      if (e->cov_enabled[c]) {
+        int32_t* df = e->d_diff + e->diff_base[c];
+        int32_t* ts = e->d_tile_sum + e->tile_off[c];
+        uint64_t* touched = e->d_res + e->cov_slot[c] + COV_TOUCHED;
+        if ((rc = g_nccl.Reduce(df, df, (size_t)e->ref_len[c] + 2, ncclInt32, ncclSum, root, e->comm, s))) return nccl_err("ncclReduce (split coverage)", rc);
+        if ((rc = g_nccl.Reduce(ts, ts, cov_tiles(e, c), ncclInt32, ncclSum, root, e->comm, s))) return nccl_err("ncclReduce (split tile sums)", rc);
+        if ((rc = g_nccl.Reduce(touched, touched, 1, ncclUint64, ncclSum, root, e->comm, s))) return nccl_err("ncclReduce (split touched)", rc);
+        e->other_launches += 3;
+      }
+      if (edits) {
+        const EditsContig& ec = e->ed_contigs[c];
+        const size_t n = (size_t)ec.hdr_len + 1;
+        if ((rc = g_nccl.Reduce(e->d_ed_refs + ec.pos_off, e->d_ed_refs + ec.pos_off, n, ncclUint32, ncclSum, root, e->comm, s))) return nccl_err("ncclReduce (split edits)", rc);
+        if ((rc = g_nccl.Reduce(e->d_ed_alts + ec.pos_off, e->d_ed_alts + ec.pos_off, n, ncclUint32, ncclSum, root, e->comm, s))) return nccl_err("ncclReduce (split edits)", rc);
+        e->other_launches += 2;
+      }
+    }
+    rc = merge_split_local(e, e->rank == root, s);
+    if (rc) return rc;
   }
   std::vector<uint64_t> slots(2 * kMaxRanks + 0, 0);
   slots[e->rank] = e->h_qpos;
@@ -1809,16 +1913,67 @@ int ngsq_reduce(ngsq_engine* e, int root) {
   }
   rc = ngsq_refresh_results(e);
   if (rc) return rc;
+  e->split_merged = true;
   // the `touched` flags were summed: a contig two ranks scattered into would get a depth histogram that is the sum of two
-  // partial resolves, not the histogram of the summed depth (shards must be contig-exclusive, SURVEY 8(e))
+  // partial resolves, not the histogram of the summed depth (shards must be contig-exclusive unless the contig was declared
+  // with ngsq_split_reference, SURVEY 8(e))
   for (uint32_t c = 0; c < e->n_ref; ++c)
-    if (e->cov_enabled[c] && e->h_res[e->cov_slot[c] + COV_TOUCHED] > 1)
+    if (e->cov_enabled[c] && !e->split_ref[c] && e->h_res[e->cov_slot[c] + COV_TOUCHED] > 1)
       return fail(e, NGSQ_E_ARG, "reference %u holds coverage from %llu ranks: every contig must lie in one shard", c, (unsigned long long)e->h_res[e->cov_slot[c] + COV_TOUCHED]);
   CU(cudaEventRecord(e->ev_b, s));
   CU(cudaEventSynchronize(e->ev_b));
   cudaEventElapsedTime(&e->stats.ms_reduce, e->ev_a, e->ev_b);
   e->stats.other_launches = e->other_launches;
   // touched flags were summed: any non-zero means touched (getters test != 0)
+  return NGSQ_OK;
+}
+
+int ngsq_split_reference(ngsq_engine* e, uint32_t ref) {
+  if (!e) return NGSQ_E_ARG;
+  if (e->cfg.flags & NGSQ_F_INDEX) return fail(e, NGSQ_E_ARG, "ngsq_split_reference: an index is built by one engine over the whole file (NGSQ_F_INDEX)");
+  if (e->cfg.max_records) return fail(e, NGSQ_E_ARG, "ngsq_split_reference: max_records counts records in file order on one engine");
+  if (ref >= e->n_ref || e->split_ref.size() != e->n_ref) return fail(e, NGSQ_E_ARG, "ngsq_split_reference: reference %u is not in the header given to ngsq_set_references", ref);
+  if (e->run_started) return fail(e, NGSQ_E_ARG, "ngsq_split_reference must precede the first submit");
+  if (!e->split_ref[ref]) {
+    e->split_ref[ref] = 1;
+    ++e->n_split;
+    e->layout_agreed = false;
+  }
+  return NGSQ_OK;
+}
+
+int ngsq_split_arrays(ngsq_engine* e, uint32_t ref, struct ngsq_split_arrays* out) {
+  if (!e || !out) return NGSQ_E_ARG;
+  if (!is_split(e, ref)) return fail(e, NGSQ_E_ARG, "ngsq_split_arrays: reference %u was not declared with ngsq_split_reference", ref);
+  memset(out, 0, sizeof *out);
+  if (e->cov_enabled[ref]) {
+    out->diff = e->d_diff + e->diff_base[ref];
+    out->n_diff = (uint64_t)e->ref_len[ref] + 2;
+    out->tile_sums = e->d_tile_sum + e->tile_off[ref];
+    out->n_tiles = cov_tiles(e, ref);
+    out->touched = e->d_res + e->cov_slot[ref] + COV_TOUCHED;
+  }
+  if (edits_loaded(e) && e->ed_pos_total) {
+    const EditsContig& ec = e->ed_contigs[ref];
+    out->edit_refs = e->d_ed_refs + ec.pos_off;
+    out->edit_alts = e->d_ed_alts + ec.pos_off;
+    out->n_positions = (uint64_t)ec.hdr_len + 1;
+  }
+  return NGSQ_OK;
+}
+
+int ngsq_resolve_split(ngsq_engine* e, int is_root) {
+  if (!e || !e->finished) return fail(e, NGSQ_E_ARG, "ngsq_resolve_split before finish");
+  if (e->split_merged) return fail(e, NGSQ_E_ARG, "ngsq_resolve_split: the split references of this run are merged already");
+  CU(cudaSetDevice(e->device));
+  cudaStream_t s = e->s_comp;
+  int rc = merge_split_local(e, is_root != 0, s);
+  if (rc) return rc;
+  if (edits_loaded(e) && e->h_ed_res.size() == E_WORDS) CU(cudaMemcpyAsync(e->h_ed_res.data(), e->d_ed_res, E_WORDS * 8, cudaMemcpyDeviceToHost, s));
+  rc = ngsq_refresh_results(e);  // synchronises s
+  if (rc) return rc;
+  e->split_merged = true;
+  e->stats.other_launches = e->other_launches;
   return NGSQ_OK;
 }
 

@@ -40,7 +40,7 @@ EXPORTED = [
     "ngsq_result_buffer", "ngsq_refresh_results", "ngsq_host_alloc", "ngsq_host_free", "ngsq_inflate_to_host",
     "ngsq_set_reference_bases", "ngsq_get_edits", "ngsq_get_edit_positions", "ngsq_set_feature_model", "ngsq_set_features", "ngsq_get_features",
     "ngsq_wait_copied", "ngsq_host_register", "ngsq_host_unregister", "ngsq_flush", "ngsq_progress",
-    "ngsq_get_bai",
+    "ngsq_get_bai", "ngsq_split_reference", "ngsq_split_arrays", "ngsq_resolve_split",
 ]
 
 
@@ -71,6 +71,14 @@ class Stats(C.Structure):
         ("other_launches", C.c_uint32), ("ms_inflate_decode", C.c_float), ("ms_inflate_resolve", C.c_float), ("ms_reduce", C.c_float),
         ("ms_edits", C.c_float), ("ms_tail", C.c_float), ("waves", C.c_uint32),
     ]
+
+    def as_dict(self):
+        return {n: getattr(self, n) for n, _ in self._fields_}
+
+
+class SplitArrays(C.Structure):
+    _fields_ = [("diff", C.c_void_p), ("n_diff", C.c_uint64), ("tile_sums", C.c_void_p), ("n_tiles", C.c_uint64),
+                ("touched", C.c_void_p), ("edit_refs", C.c_void_p), ("edit_alts", C.c_void_p), ("n_positions", C.c_uint64)]
 
     def as_dict(self):
         return {n: getattr(self, n) for n, _ in self._fields_}
@@ -136,6 +144,9 @@ def load_library() -> C.CDLL:
     lib.ngsq_host_register.argtypes = [P, C.c_size_t]
     lib.ngsq_host_unregister.argtypes = [P]
     lib.ngsq_get_bai.argtypes = [P, P, C.c_size_t, C.POINTER(C.c_size_t)]
+    lib.ngsq_split_reference.argtypes = [P, C.c_uint32]
+    lib.ngsq_split_arrays.argtypes = [P, C.c_uint32, C.POINTER(SplitArrays)]
+    lib.ngsq_resolve_split.argtypes = [P, C.c_int]
     _lib = lib
     return lib
 
@@ -356,6 +367,23 @@ class Engine:
 
     def reduce(self, root: int = 0):
         self._check(self.lib.ngsq_reduce(self.h, root))
+
+    # ---- shards cut inside a contig ----
+    def split_reference(self, ref: int):
+        """Declares reference `ref` split between shards (same set on every engine; before the first submit)."""
+        self._check(self.lib.ngsq_split_reference(self.h, ref))
+
+    def split_arrays(self, ref: int) -> dict:
+        """Device pointers and lengths of a split reference's partial arrays (for a caller's own collective):
+        diff / n_diff (int32), tile_sums / n_tiles (int32), touched (one u64), edit_refs / edit_alts / n_positions (u32);
+        a pointer is None when its facet is off."""
+        out = SplitArrays()
+        self._check(self.lib.ngsq_split_arrays(self.h, ref, C.byref(out)))
+        return out.as_dict()
+
+    def resolve_split(self, is_root: bool):
+        """After the split arrays were summed into the root's: resolve them there, zero them elsewhere."""
+        self._check(self.lib.ngsq_resolve_split(self.h, int(bool(is_root))))
 
 
 def nccl_unique_id() -> bytes:

@@ -6,6 +6,7 @@ driver (ngs_b200/host) holds the same logic for the product path.
 """
 from __future__ import annotations
 
+import bisect
 import os
 import re
 import struct
@@ -201,6 +202,51 @@ def plan_shards(header: BamHeader, bai: Bai, n_shards: int, file_size: int) -> l
     while len(shards) < n_shards:
         shards.append(Shard(0, 0, []))  # empty shard (more GPUs than contigs)
     return shards
+
+
+def bai_anchors(bai: Bai) -> list:
+    """Record starts a shard may be cut at: every contig's first record (pseudo-bin 37450) and its linear-index ioffsets,
+    ascending and distinct (zeros, entries below the contig's first record and repeats dropped)."""
+    out = set()
+    for r in bai.refs:
+        if r.ref_beg is None or r.ref_end is None or r.ref_end <= r.ref_beg:
+            continue
+        out.add(r.ref_beg)
+        out.update(v for v in r.linear if v and r.ref_beg <= v < r.ref_end)
+    return sorted(out)
+
+
+def plan_shards_split(header: BamHeader, bai: Bai, n_shards: int, file_size: int):
+    """Shards cut inside contigs at BAI anchors, balanced by compressed bytes (mirror of plan_shards_split in
+    ngs_b200/host/bam.hpp).  Returns (shards, split): `split` lists the contigs with records on both sides of a cut, in
+    ascending order; a shard's `contigs` are the references it holds records of.  Shards past the anchors are empty."""
+    first = header.first_voffset
+    cand = [v for v in bai_anchors(bai) if v > first]
+    base = first >> 16
+    total = float(max(file_size - base, 0))
+    m = len(cand)
+    n_cuts = min(max(n_shards - 1, 0), m)
+    key = [(v >> 16) - base for v in cand]
+    cuts, lo = [], 0
+    for k in range(1, n_cuts + 1):
+        target = total * k / n_shards
+        hi = m - (n_cuts - k)
+        j = bisect.bisect_left(key, target, lo, hi)  # the nearest candidate in [lo, hi), ties: the earlier one
+        if j == hi or (j > lo and target - key[j - 1] <= key[j] - target):
+            j -= 1
+        cuts.append(cand[j])
+        lo = j + 1
+    bounds = [first] + cuts
+    extents = [(c, r.ref_beg, r.ref_end) for c, r in enumerate(bai.refs)
+               if r.ref_beg is not None and r.ref_end is not None and r.ref_end > r.ref_beg]
+    shards = []
+    for i, b in enumerate(bounds):
+        end = bounds[i + 1] if i + 1 < len(bounds) else 0
+        shards.append(Shard(b, end, [c for c, beg, e in extents if e > b and (end == 0 or beg < end)]))
+    split = [c for c, beg, e in extents if any(beg < v < e for v in cuts)]
+    while len(shards) < n_shards:
+        shards.append(Shard(0, 0, []))
+    return shards, split
 
 
 def shard_byte_range(shard: Shard, blocks, n_blocks: int, file_size: int):

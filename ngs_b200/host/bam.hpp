@@ -101,8 +101,14 @@ inline BamHeader read_bam_header(ngsq_engine* e, const uint8_t* bam, size_t size
   }
 }
 
-// BAI (SAM spec 5.2): only what sharding needs — per-reference file extents from pseudo-bin 37450.
-struct BaiReference { bool has_extent = false; uint64_t ref_beg = 0, ref_end = 0, n_mapped = 0, n_unmapped = 0; uint32_t n_bins = 0, n_intv = 0; };
+// BAI (SAM spec 5.2): only what sharding needs — per-reference file extents from pseudo-bin 37450 and the linear index
+// (ioffset of every 16 kb window: the first record overlapping it, a record start the shard planner may cut at).
+struct BaiReference {
+  bool has_extent = false;
+  uint64_t ref_beg = 0, ref_end = 0, n_mapped = 0, n_unmapped = 0;
+  uint32_t n_bins = 0, n_intv = 0;
+  std::vector<uint64_t> ioffset;
+};
 struct BaiIndex { std::vector<BaiReference> refs; bool has_n_no_coor = false; uint64_t n_no_coor = 0; };
 
 // IndexCheck::Full (utils/formats/bam.rs:86-96): the index must exist next to the BAM and parse.
@@ -141,6 +147,8 @@ inline BaiIndex read_bai(const std::string& path) {
     memcpy(&R.n_intv, &b[o], 4);
     o += 4;
     need(8ull * R.n_intv);
+    R.ioffset.resize(R.n_intv);
+    if (R.n_intv) memcpy(R.ioffset.data(), &b[o], 8ull * R.n_intv);
     o += 8ull * R.n_intv;
     idx.refs.push_back(R);
   }
@@ -193,6 +201,121 @@ inline std::vector<Shard> plan_shards(const BamHeader& h, const BaiIndex& bai, u
   }
   while (out.size() < n_shards) { Shard s; s.empty = true; out.push_back(s); }
   return out;
+}
+
+// Cuts inside contigs (SURVEY 8(e), DESIGN 5): shards balanced by compressed bytes, cut at record starts the BAI names.
+// The anchors are every contig's first record (pseudo-bin 37450) and its linear-index ioffsets; the linear index is
+// non-decreasing in file order, so each anchor is the start of a record.  A contig with records on both sides of a cut is
+// a split reference: every engine must declare it (ngsq_split_reference) and the merge resolves it once, on the root.
+struct ShardPlan {
+  std::vector<Shard> shards;
+  std::vector<uint32_t> split;  // split references, ascending
+  bool split_plan = false;      // plan_shards_split's plan (choose_shards)
+};
+
+// Record starts the planner may cut at, ascending and distinct: zeros, entries below their contig's first record and
+// repeats (long reads make consecutive windows share an offset) are dropped.
+inline std::vector<uint64_t> bai_anchors(const BaiIndex& bai) {
+  std::vector<uint64_t> a;
+  for (const BaiReference& r : bai.refs) {
+    if (!r.has_extent) continue;
+    a.push_back(r.ref_beg);
+    for (uint64_t v : r.ioffset)
+      if (v && v >= r.ref_beg && v < r.ref_end) a.push_back(v);
+  }
+  std::sort(a.begin(), a.end());
+  a.erase(std::unique(a.begin(), a.end()), a.end());
+  return a;
+}
+
+inline ShardPlan plan_shards_split(const BamHeader& h, const BaiIndex& bai, uint32_t n_shards, uint64_t file_size) {
+  ShardPlan plan;
+  const uint64_t first = h.first_record_voffset;
+  std::vector<uint64_t> cand;  // possible cuts: anchors after the first record
+  for (uint64_t v : bai_anchors(bai)) if (v > first) cand.push_back(v);
+  const uint64_t base = first >> 16;
+  const double total = (double)(file_size > base ? file_size - base : 0);
+  std::vector<uint64_t> cuts;
+  const size_t m = cand.size();
+  const size_t n_cuts = std::min<size_t>(n_shards ? n_shards - 1 : 0, m);
+  size_t lo = 0;  // first candidate the next cut may take
+  for (size_t k = 1; k <= n_cuts; ++k) {
+    const double target = total * (double)k / (double)n_shards;
+    const size_t hi = m - (n_cuts - k);  // leave one candidate for every later cut
+    // the candidate nearest the target (ties: the earlier one) within [lo, hi)
+    size_t j = (size_t)(std::lower_bound(cand.begin() + lo, cand.begin() + hi, target,
+                                         [&](uint64_t v, double t) { return (double)((v >> 16) - base) < t; }) - cand.begin());
+    if (j == hi || (j > lo && target - (double)((cand[j - 1] >> 16) - base) <= (double)((cand[j] >> 16) - base) - target)) --j;
+    cuts.push_back(cand[j]);
+    lo = j + 1;
+  }
+  std::vector<uint64_t> bounds{first};
+  bounds.insert(bounds.end(), cuts.begin(), cuts.end());
+  for (size_t i = 0; i < bounds.size(); ++i) {
+    Shard s;
+    s.first_voffset = bounds[i];
+    s.end_voffset = i + 1 < bounds.size() ? bounds[i + 1] : 0;  // the last shard runs to EOF: the unplaced tail
+    for (uint32_t c = 0; c < bai.refs.size(); ++c) {
+      const BaiReference& r = bai.refs[c];
+      if (r.has_extent && r.ref_end > s.first_voffset && (s.end_voffset == 0 || r.ref_beg < s.end_voffset)) s.contigs.push_back(c);
+    }
+    plan.shards.push_back(s);
+  }
+  for (uint32_t c = 0; c < bai.refs.size(); ++c) {
+    const BaiReference& r = bai.refs[c];
+    for (uint64_t v : cuts)
+      if (r.has_extent && r.ref_beg < v && v < r.ref_end) { plan.split.push_back(c); break; }
+  }
+  while (plan.shards.size() < n_shards) { Shard s; s.empty = true; plan.shards.push_back(s); }
+  plan.split_plan = true;
+  return plan;
+}
+
+// Compressed bytes a shard covers, for balancing: from its first record's block to the block of its end (or EOF).
+inline uint64_t shard_compressed_bytes(const Shard& s, uint64_t file_size) {
+  if (s.empty) return 0;
+  const uint64_t lo = s.first_voffset >> 16, hi = s.end_voffset ? s.end_voffset >> 16 : file_size;
+  return hi > lo ? hi - lo : 0;
+}
+
+// Bytes the merge moves per rank for a split plan: every split contig's int32 difference array (L + 2) and tile sums, and
+// its touched word (Edits adds two u32 counters per position; not counted).
+inline uint64_t split_reduce_bytes(const BamHeader& h, const std::vector<uint32_t>& split) {
+  uint64_t b = 0;
+  for (uint32_t c : split) {
+    const uint64_t L = c < h.reference_sequences.size() ? h.reference_sequences[c].length : 0;
+    b += (L + 2) * 4 + (L + 4096) / 4096 * 4 + 8;
+  }
+  return b;
+}
+
+// The plan `ngs qc` runs.  The split plan is taken when the contig-aligned one leaves a device without a shard.  When every
+// device has one, it is taken for balance only if the largest contig-aligned shard holds more than 25 % above the mean
+// compressed bytes AND the split plan's merge moves at most twice a balanced shard's compressed bytes per rank
+// (split_reduce_bytes).  Measured on one B200 with every shard run alone (DESIGN 6, profiles/split_bench_1gpu.json): where
+// the second condition fails, on the 25-contig WGS shape at 8 shards (26 % imbalance, 7 split contigs, 4.2 GB of difference
+// arrays per rank), the split plan saves 0.5 ms of the slowest shard's 27 ms including the root's 2.5 ms resolve, before the
+// reduce itself; where it holds (shape 2 at 2 and 4 shards, shape 0 at 2) the split plan is 18-36 % faster.  The ncclReduce
+// of the split arrays has not been timed on several GPUs.
+constexpr double kSplitImbalance = 1.25;
+constexpr double kSplitReduceShards = 2.0;
+inline ShardPlan choose_shards(const BamHeader& h, const BaiIndex& bai, uint32_t n_shards, uint64_t file_size) {
+  ShardPlan plan;
+  plan.shards = plan_shards(h, bai, n_shards, file_size);
+  if (n_shards <= 1) return plan;
+  uint64_t total = 0, most = 0;
+  bool all_live = true;
+  for (const Shard& s : plan.shards) {
+    const uint64_t b = shard_compressed_bytes(s, file_size);
+    total += b;
+    most = std::max(most, b);
+    all_live = all_live && !s.empty;
+  }
+  const double mean = (double)total / (double)n_shards;
+  if (all_live && (double)most <= kSplitImbalance * mean) return plan;
+  ShardPlan split = plan_shards_split(h, bai, n_shards, file_size);
+  if (all_live && (double)split_reduce_bytes(h, split.split) > kSplitReduceShards * mean) return plan;
+  return split;
 }
 
 // Compressed byte range [lo, hi) a shard submits: through the block that holds end_voffset.

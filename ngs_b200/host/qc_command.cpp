@@ -248,8 +248,15 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   for (auto& f : facets.record_based) info(std::string("  [*] ") + f->name() + ", " + to_string(f->computational_load()));
   for (auto& f : facets.sequence_based) info(std::string("  [*] ") + f->name() + ", " + to_string(f->computational_load()));
 
-  // shards: contig-aligned file ranges from the BAI
-  std::vector<Shard> shards = plan_shards(header, bai, n_dev, file.size());
+  // shards: contig-aligned file ranges from the BAI, or ranges cut inside contigs when those leave a device idle or
+  // unbalanced (choose_shards); a contig cut between shards is declared on every engine and merged by ngsq_reduce
+  const ShardPlan plan = choose_shards(header, bai, n_dev, file.size());
+  const std::vector<Shard>& shards = plan.shards;
+  if (plan.split_plan) {
+    std::string names;
+    for (uint32_t c : plan.split) names += (names.empty() ? "" : ", ") + header.reference_sequences[c].name;
+    info("  [*] Sharding inside contigs: " + std::to_string(n_dev) + " shards" + (names.empty() ? std::string() : ", split: " + names) + ".");
+  }
   std::vector<uint32_t> ref_len;
   for (auto& rs : header.reference_sequences) ref_len.push_back(rs.length);
   for (uint32_t i = 0; i < n_dev; ++i) {
@@ -262,6 +269,7 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
     check(engines[i], ngsq_set_references(engines[i], (uint32_t)ref_len.size(), ref_len.data(), enabled.data()));
     if (features) features->upload(engines[i], header.reference_sequences);
     if (edits) edits->upload(engines[i], header.reference_sequences);
+    for (uint32_t c : plan.split) check(engines[i], ngsq_split_reference(engines[i], c));
   }
   if (n_dev > 1) {
     char id[128];
