@@ -390,6 +390,7 @@ struct Lane {
       nx[l] = (uint16_t)off;  // running index of the next symbol of this length
       off += c;
     }
+    if (left > 0 && off > 1) return false;  // incomplete with two or more codes (zero or one used symbol is accepted)
     for (uint32_t k = 0; k < n; ++k) {
       const uint32_t l = lens(k);
       if (!l) continue;
@@ -482,7 +483,7 @@ struct Lane {
           for (int t = 1; t < 8; ++t) c[t] += (l == (uint32_t)t);
         }
         uint32_t nx[8];
-        uint32_t code = 0, prev = 0;
+        uint32_t code = 0, prev = 0, used = 0;
         int left = 1;
         nx[0] = 0;
 #pragma unroll
@@ -491,8 +492,10 @@ struct Lane {
           code = (code + prev) << 1;
           prev = c[l];
           nx[l] = code;
+          used += c[l];
         }
-        if (left < 0) { end_block(kBlkBadStream); return; }
+        // over-subscribed, or incomplete with two or more codes
+        if (left < 0 || (left > 0 && used > 1)) { end_block(kBlkBadStream); return; }
         uint32_t* lw = reinterpret_cast<uint32_t*>(cl_lut);
         for (int i = 0; i < 32; ++i) lw[i] = 0;
         for (int k = 0; k < 19; ++k) {

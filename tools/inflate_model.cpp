@@ -6,6 +6,10 @@
 //   /tmp/inflate_model file.bam [max_blocks]
 //   /tmp/inflate_model file.bam --fuzz N     N corrupted copies of every block: the decoder must fail
 //                                            or finish, never write outside its block, never run away
+//   /tmp/inflate_model file.bam --all-alignments   decode and resolve every block at all 16 output alignments
+//                                            (the first with the scalar resolve pass, the others with the warp one)
+//   /tmp/inflate_model file.bam --expect-reject    every block is invalid: the decoder must fail it (at every
+//                                            output alignment), write nothing outside it, and zlib must reject it
 #include <zlib.h>
 
 #include <cstdio>
@@ -114,9 +118,20 @@ int main(int argc, char** argv) {
   std::vector<uint8_t> buf(n + 1024, 0);
   if (fread(buf.data(), 1, n, f) != n) { perror("read"); return 2; }
   fclose(f);
-  size_t max_blocks = argc > 2 ? strtoull(argv[2], nullptr, 10) : ~size_t(0);
+  size_t max_blocks = ~size_t(0);
   int fuzz = 0;
-  if (argc > 3 && !strcmp(argv[2], "--fuzz")) { fuzz = atoi(argv[3]); max_blocks = ~size_t(0); }
+  bool all_alignments = false, expect_reject = false;
+  for (int a = 2; a < argc; ++a) {
+    if (!strcmp(argv[a], "--fuzz") && a + 1 < argc) fuzz = atoi(argv[++a]);
+    else if (!strcmp(argv[a], "--all-alignments")) all_alignments = true;
+    else if (!strcmp(argv[a], "--expect-reject")) expect_reject = true;
+    else max_blocks = strtoull(argv[a], nullptr, 10);
+  }
+  if (fuzz || expect_reject) max_blocks = ~size_t(0);
+  uint64_t rejected = 0;
+  // output alignments (offset of the block's first byte mod 16): the first one uses the scalar resolve pass
+  std::vector<uint32_t> aligns = {0, 9};
+  if (all_alignments) { aligns.clear(); for (uint32_t a = 0; a < 16; ++a) aligns.push_back(a); }
   uint64_t fuzz_runs = 0, fuzz_failed = 0, fuzz_ok = 0, rng = 0x9E3779B97F4A7C15ull;
 
   InflateCounters ctr;
@@ -190,11 +205,60 @@ int main(int argc, char** argv) {
       } else fuzz_failed++;
       fuzz_runs++;
     }
-    if (isize && !fuzz) {
-      for (int mis = 0; mis < 4; mis += 3) {  // two output alignments
+    if (expect_reject) {
+      if (isize > 65536) { fprintf(stderr, "block at %zu: ISIZE %u > 65536\n", o, isize); return 1; }
+      bool failed_everywhere = true;
+      for (uint32_t a = 0; a < 16; ++a) {
         BlockDesc d;
         d.in_off = (uint64_t)(uintptr_t)(h + hdr);
-        d.out_off = 16 + mis * 3;
+        d.out_off = 16 + a;
+        d.clen = clen;
+        d.isize = isize;
+        memset(out.data(), 0xAA, out.size());
+        memset(bitmap.data(), 0, kBitmapWords * 4);
+        Lane L;
+        L.slab = slab.data();
+        L.lut = base_lut;
+        L.ctr = nullptr;
+        L.begin_block(d, out.data(), bitmap.data());
+        uint64_t steps = 0;
+        while (L.state != LS_IDLE && steps < 4000000) {
+          if (L.state == LS_HEADER) L.header();
+          else {
+            L.step();
+            L.settle();
+            if (L.state == LS_DECODE && L.overran()) L.end_block(kBlkBadStream);
+          }
+          ++steps;
+        }
+        if (L.state != LS_IDLE) { fprintf(stderr, "block at %zu: did not terminate\n", o); bad++; }
+        if (!L.err) { fprintf(stderr, "block at %zu: decoded without error (output alignment %u)\n", o, a); failed_everywhere = false; }
+        uint8_t* ob = out.data() + d.out_off;
+        for (int g = 1; g <= 16; ++g)
+          if (ob[-g] != 0xAA || ob[isize + g - 1] != 0xAA) { fprintf(stderr, "block at %zu: wrote outside its range\n", o); bad++; break; }
+        for (uint32_t w = (isize + 31) / 32 + 1; w < kBitmapWords; ++w)
+          if (bitmap[w]) { fprintf(stderr, "block at %zu: marked a match beyond its size\n", o); bad++; break; }
+      }
+      if (failed_everywhere) rejected++; else bad++;
+      z_stream zs;
+      memset(&zs, 0, sizeof zs);
+      inflateInit2(&zs, -15);
+      zs.next_in = const_cast<uint8_t*>(h + hdr);
+      zs.avail_in = clen;
+      zs.next_out = ref.data();
+      zs.avail_out = 65536;
+      const int rc = inflate(&zs, Z_FINISH);
+      inflateEnd(&zs);
+      if (rc == Z_STREAM_END && zs.total_out == isize) { fprintf(stderr, "block at %zu: zlib accepts it\n", o); bad++; }
+      n_blocks++;
+      o += total;
+      continue;
+    }
+    if (isize && !fuzz) {
+      for (uint32_t mis = 0; mis < aligns.size(); ++mis) {
+        BlockDesc d;
+        d.in_off = (uint64_t)(uintptr_t)(h + hdr);
+        d.out_off = 16 + aligns[mis];
         d.clen = clen;
         d.isize = isize;
         memset(out.data(), 0xAA, out.size());
@@ -216,7 +280,7 @@ int main(int argc, char** argv) {
         // guard bytes
         uint8_t* ob = out.data() + d.out_off;
         for (int g = 1; g <= 4; ++g)
-          if (ob[-g] != 0xAA || ob[isize + g - 1] != 0xAA) { fprintf(stderr, "block at %zu: wrote outside (mis %d)\n", o, mis); bad++; }
+          if (ob[-g] != 0xAA || ob[isize + g - 1] != 0xAA) { fprintf(stderr, "block at %zu: wrote outside (alignment %u)\n", o, aligns[mis]); bad++; }
         // dependency depth of the resolve kernel's 32-token batches (per 1024-byte super-window)
         if (mis == 0) {
           for (uint32_t sw = 0; sw < kBitmapWords / 32; ++sw) {
@@ -275,7 +339,7 @@ int main(int argc, char** argv) {
         if (memcmp(ref.data(), ob, isize) != 0) {
           uint32_t k = 0;
           while (ref[k] == ob[k]) ++k;
-          fprintf(stderr, "block at %zu (mis %d): MISMATCH at byte %u of %u\n", o, mis, k, isize);
+          fprintf(stderr, "block at %zu (alignment %u): MISMATCH at byte %u of %u\n", o, aligns[mis], k, isize);
           bad++;
         }
         if (crc32(0, ref.data(), isize) != crc) { fprintf(stderr, "crc mismatch at %zu\n", o); bad++; }
@@ -285,6 +349,10 @@ int main(int argc, char** argv) {
       total_in += clen;
     }
     o += total;
+  }
+  if (expect_reject) {
+    printf("reject: %llu blocks, %llu rejected, bad %llu\n", (unsigned long long)n_blocks, (unsigned long long)rejected, (unsigned long long)bad);
+    return bad ? 1 : 0;
   }
   if (fuzz) {
     printf("fuzz: %llu corrupted blocks, %llu rejected, %llu decoded, bad %llu\n", (unsigned long long)fuzz_runs,
