@@ -70,6 +70,12 @@ enum {
                                    other flag.  The range must start at the first record and reach to the end (end_voffset 0),
                                    max_records must be 0, references must be shorter than 2^29 (longer ones need CSI) and the
                                    records coordinate-sorted (NGSQ_E_UNSORTED otherwise).  Read the bytes with ngsq_get_bai. */
+#define NGSQ_F_INDEX_PART 128u  /* index ONE contiguous range of a file cut between engines; set instead of NGSQ_F_INDEX (both:
+                                   NGSQ_E_ARG), combines with every other flag.  The range is [first, end) of ngsq_set_range (end 0 =
+                                   to the end of the data); max_records must be 0; ngsq_reduce and the split-reference calls are
+                                   allowed.  ngsq_finish keeps the part's index state on the host without assembling it, and does not
+                                   check the order (it is checked across the parts by the join); ngsq_get_bai is refused: join the
+                                   finished parts with ngsq_join_bai. */
 
 typedef struct ngsq_engine ngsq_engine;
 
@@ -234,6 +240,23 @@ int ngsq_get_stats(ngsq_engine* e, ngsq_stats* out);
  * n_no_coor) of the records submitted since ngsq_set_range.  After ngsq_finish.  *n_out = its size; out = NULL with cap = 0
  * asks for the size only.  DESIGN.md section 4 (K13) lists where its bytes may differ from samtools' index of the same file. */
 int ngsq_get_bai(ngsq_engine* e, uint8_t* out, size_t cap, size_t* n_out);
+
+/* ---- a BAM without an index cut between engines (DESIGN.md sections 4 K13 and 5) ----
+ * Record anchor finder: `bgzf` holds whole BGZF blocks starting at file offset `file_off`.  They are inflated on the device
+ * and every offset is tested in parallel for the start of a chain of plausible records (recscan.cuh: plausible()) that runs
+ * to the end of the inflated window (its last record may run past it).  *voffset = the smallest such offset as a virtual
+ * offset and *ref_id = that record's reference id; *voffset = 0 (and *ref_id = -1) when the window holds none, e.g. when
+ * every block lies inside one long read: offer a larger window.  The result is SPECULATIVE: bytes inside a record may look
+ * like records.  It is proven only by the closure check of the range that ends there (a range whose end is not a record
+ * start fails with NGSQ_E_CHAIN or NGSQ_E_TRUNCATED).  After ngsq_set_references (the test needs n_ref), outside a run. */
+int ngsq_find_record(ngsq_engine* e, const uint8_t* bgzf, size_t nbytes, uint64_t file_off, uint64_t* voffset, int32_t* ref_id);
+/* Joins the index parts of NGSQ_F_INDEX_PART engines into the file's .bai, on the host (no device work): the same bytes one
+ * NGSQ_F_INDEX engine gives for the whole file.  parts[0..n) in file order, each finished without error, all with the same
+ * references; part k's end offset equals part k+1's first offset and the last part runs to the end of the data
+ * (NGSQ_E_ARG otherwise).  Unsorted records fail with NGSQ_E_UNSORTED and the offset and message one engine gives.  *n_out =
+ * the size; out = NULL with cap = 0 asks for the size only.  The message of a failure is ngsq_last_error(parts[0]) (of NULL
+ * when parts is NULL or n is 0). */
+int ngsq_join_bai(ngsq_engine* const* parts, uint32_t n, uint8_t* out, size_t cap, size_t* n_out);
 
 /* ---- multi-GPU merge: one sum-reduce of the packed u64 result buffer ---- */
 int ngsq_nccl_unique_id(char out[128]);

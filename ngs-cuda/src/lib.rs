@@ -97,6 +97,8 @@ pub mod sys {
     pub const NGSQ_F_SERIAL_STAGES: u32 = 32;
     pub const NGSQ_E_QUAL_CAP: c_int = -13;
     pub const NGSQ_F_INDEX: u32 = 64;
+    /// index one range of a file cut between engines (set instead of NGSQ_F_INDEX); join the parts with ngsq_join_bai
+    pub const NGSQ_F_INDEX_PART: u32 = 128;
     pub const NGSQ_E_UNSORTED: c_int = -14;
 
     /// Device arrays of a reference split between shards (`struct ngsq_split_arrays`); null pointers for facets that are off.
@@ -156,6 +158,8 @@ pub mod sys {
         pub fn ngsq_split_reference(e: *mut NgsqEngine, r: u32) -> c_int;
         pub fn ngsq_split_arrays(e: *mut NgsqEngine, r: u32, out: *mut NgsqSplitArrays) -> c_int;
         pub fn ngsq_resolve_split(e: *mut NgsqEngine, is_root: c_int) -> c_int;
+        pub fn ngsq_find_record(e: *mut NgsqEngine, bgzf: *const u8, nbytes: usize, file_off: u64, voffset: *mut u64, ref_id: *mut i32) -> c_int;
+        pub fn ngsq_join_bai(parts: *const *mut NgsqEngine, n: u32, out: *mut u8, cap: usize, n_out: *mut usize) -> c_int;
     }
 }
 
@@ -339,6 +343,31 @@ impl Engine {
         Ok(out)
     }
 
+    /// An engine that indexes one range of a file cut between engines (NGSQ_F_INDEX_PART beside `flags`, e.g. the qc flags);
+    /// its part is joined with the others by `join_bai` after `finish`.
+    pub fn create_index_part(device: i32, flags: u32) -> anyhow::Result<Self> {
+        let cfg = sys::NgsqConfig {
+            struct_size: std::mem::size_of::<sys::NgsqConfig>() as u32,
+            flags: flags | sys::NGSQ_F_INDEX_PART,
+            ..Default::default()
+        };
+        let mut raw = std::ptr::null_mut();
+        let rc = unsafe { sys::ngsq_create(device as c_int, &cfg, &mut raw) };
+        if rc != 0 {
+            let msg = unsafe { CStr::from_ptr(sys::ngsq_last_error(std::ptr::null_mut())) }.to_string_lossy().into_owned();
+            bail!("ngs-cuda: {}", msg);
+        }
+        Ok(Self { raw, submits: 0 })
+    }
+
+    /// The first record start in whole BGZF blocks `bgzf` that begin at file offset `file_off`, as (virtual offset, reference
+    /// id); None when the window holds none (offer a larger one).  Speculative: the range that ends there proves it.
+    pub fn find_record(&mut self, bgzf: &[u8], file_off: u64) -> anyhow::Result<Option<(u64, i32)>> {
+        let (mut v, mut r) = (0u64, -1i32);
+        self.check(unsafe { sys::ngsq_find_record(self.raw, bgzf.as_ptr(), bgzf.len(), file_off, &mut v, &mut r) })?;
+        Ok(if v == 0 { None } else { Some((v, r)) })
+    }
+
     /// A read longer than the quality table: raise it and run the file again (include/ngs_cuda.h, NGSQ_E_QUAL_CAP).
     pub fn set_quality_positions(&mut self, n: u32) -> anyhow::Result<()> {
         self.check(unsafe { sys::ngsq_set_quality_positions(self.raw, n) })
@@ -479,6 +508,19 @@ impl Engine {
     pub fn resolve_split(&mut self, is_root: bool) -> anyhow::Result<()> {
         self.check(unsafe { sys::ngsq_resolve_split(self.raw, is_root as c_int) })
     }
+}
+
+/// The `.bai` of a file from its finished NGSQ_F_INDEX_PART engines, in file order (ngsq_join_bai, on the host).
+pub fn join_bai(parts: &[&Engine]) -> anyhow::Result<Vec<u8>> {
+    if parts.is_empty() {
+        bail!("ngs-cuda: join_bai needs at least one part");
+    }
+    let raws: Vec<*mut sys::NgsqEngine> = parts.iter().map(|e| e.raw).collect();
+    let mut n = 0usize;
+    parts[0].check(unsafe { sys::ngsq_join_bai(raws.as_ptr(), raws.len() as u32, std::ptr::null_mut(), 0, &mut n) })?;
+    let mut out = vec![0u8; n];
+    parts[0].check(unsafe { sys::ngsq_join_bai(raws.as_ptr(), raws.len() as u32, out.as_mut_ptr(), out.len(), &mut n) })?;
+    Ok(out)
 }
 
 impl Drop for Engine {

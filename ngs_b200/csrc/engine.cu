@@ -76,6 +76,18 @@ bool load_nccl(std::string& err) {
 
 }  // namespace
 
+// NGSQ_F_INDEX / NGSQ_F_INDEX_PART: an engine's index state on the host once its last wave is done.  Every part is linear or
+// order-free, so the state of parts cut from one file joins exactly (ngsq_join_bai): runs and overflow lists concatenate,
+// windows take the minimum, maxw the maximum, counts and n_no_coor add up.
+struct IxHost {
+  IndexState S{};
+  std::vector<IndexRun> runs, ovf;  // runs in any order (assemble_bai sorts them)
+  std::vector<uint64_t> win, counts;
+  std::vector<uint32_t> maxw;
+  uint64_t last_order_key = 0;      // of the part's last record that constrains the order (0 = none)
+  uint64_t data_end = 0;            // virtual offset behind the last record submitted
+};
+
 struct ngsq_engine {
   int device = 0;
   int n_sm = 0;
@@ -210,6 +222,8 @@ struct ngsq_engine {
   std::vector<std::pair<const IndexRun*, uint64_t>> ix_drained;  // pinned copies of drained run tables
   uint64_t data_end_coff = 0;        // end of the last non-empty block submitted (the offset after the last record)
   std::vector<uint8_t> bai;
+  IxHost ix;                         // NGSQ_F_INDEX_PART: the part's state for ngsq_join_bai
+  bool ix_part_ok = false;           // ... valid: ngsq_finish succeeded
 
   // references split between shards (ngsq_split_reference): scattered as usual, resolved only by the merge
   std::vector<uint8_t> split_ref;
@@ -257,6 +271,9 @@ int fresh(ngsq_engine* e, T*& ptr, size_t n, const char* what) {
 }
 
 uint32_t wave_blocks(const ngsq_engine* e) { return (uint32_t)e->n_sm * kDecThreads; }
+
+// the K13 index pass runs: a whole file (NGSQ_F_INDEX) or one part of it (NGSQ_F_INDEX_PART)
+bool ix_on(const ngsq_engine* e) { return e->cfg.flags & (NGSQ_F_INDEX | NGSQ_F_INDEX_PART); }
 
 uint32_t launch_quantum(const ngsq_engine* e) {
   // One wave = one block per decoder lane: a launch takes about one block-decode latency whatever its size (every
@@ -331,11 +348,12 @@ int start_run(ngsq_engine* e) {
   e->h_state->next_carry = kNoCarry;
   CU(cudaMemcpyAsync(e->d_state, e->h_state, sizeof(RunState), cudaMemcpyHostToDevice, e->s_comp));
   if ((e->cfg.flags & NGSQ_F_FEATURES) && e->d_ft_res) CU(cudaMemsetAsync(e->d_ft_res, 0, F_WORDS * 8, e->s_comp));
-  if (e->cfg.flags & NGSQ_F_INDEX) {
+  if (ix_on(e)) {
     if (!e->d_ix) return fail(e, NGSQ_E_ARG, "NGSQ_F_INDEX needs ngsq_set_references before the first submit");
     IndexState z{};
     z.carry[0].run_key = kIxNoRun;
     z.unsorted_voff = ~0ull;
+    z.first_key = z.first_voff = ~0ull;
     CU(cudaMemcpyAsync(e->d_ix, &z, sizeof z, cudaMemcpyHostToDevice, e->s_comp));
     if (e->ix_win_total) CU(cudaMemsetAsync(e->d_ix_win, 0xFF, e->ix_win_total * 8, e->s_comp));
     if (e->n_ref) {
@@ -545,7 +563,7 @@ int ensure_wave_buffers(ngsq_engine* e, int s, uint32_t n, uint64_t bytes) {
     e->rec_cap = need_rec;
   }
   // a run starts at a record: the run tables are sized like the record table (the runs of earlier waves are drained first)
-  if ((e->cfg.flags & NGSQ_F_INDEX) && need_rec > e->ix_runs_cap) {
+  if (ix_on(e) && need_rec > e->ix_runs_cap) {
     if ((rc = quiesce())) return rc;
     for (uint32_t j = 0; j < e->ix_waves.size(); ++j)
       if ((rc = ix_drain(e, j, e->s_scan))) return rc;
@@ -761,7 +779,7 @@ int launch_wave(ngsq_engine* e, uint32_t b0, uint32_t b1, bool final_wave) {
     CU(cudaGetLastError());
     e->other_launches++;
   }
-  if (e->cfg.flags & NGSQ_F_INDEX) {
+  if (ix_on(e)) {
     // K13: keys, runs, order check, counters and linear index of the wave's records
     const uint32_t j = (uint32_t)e->ix_waves.size(), par = j & 1;
     if (j >= 2 && (rc = ix_drain(e, j - 2, st))) return rc;
@@ -771,6 +789,7 @@ int launch_wave(ngsq_engine* e, uint32_t b0, uint32_t b1, bool final_wave) {
     X.n_ref = (int32_t)e->n_ref; X.S = e->d_ix; X.runs = e->d_ix_runs[par]; X.runs_cap = e->ix_runs_cap;
     X.ovf = e->d_ix_ovf; X.ovf_cap = kIndexOverflowCap;
     X.win_base = e->d_ix_win_base; X.win_n = e->d_ix_win_n; X.win = e->d_ix_win; X.max_win = e->d_ix_maxw; X.counts = e->d_ix_counts;
+    X.part = (e->cfg.flags & NGSQ_F_INDEX_PART) ? 1u : 0u;
     const uint32_t per_cta = 31 * (kIndexThreads / 32);
     const uint32_t xgrid = (uint32_t)std::min<uint64_t>((bytes / 36 + 2 + per_cta - 1) / per_cta, (uint64_t)e->n_sm * 8);
     index_kernel<<<xgrid, kIndexThreads, 0, st>>>(X);
@@ -849,36 +868,10 @@ int acquire_comp(ngsq_engine* e, size_t nbytes, uint8_t** dst) {
   return NGSQ_OK;
 }
 
-// K13 on the host, at ngsq_finish: runs -> chunks per (reference, bin), the linear index, the .bai bytes.
-int finish_index(ngsq_engine* e) {
-  for (uint32_t j = 0; j < e->ix_waves.size(); ++j) {
-    int rc = ix_drain(e, j, e->s_comp);
-    if (rc) return rc;
-  }
-  CU(cudaStreamSynchronize(e->s_comp));
-  IndexState S;
-  CU(cudaMemcpy(&S, e->d_ix, sizeof S, cudaMemcpyDeviceToHost));
-  if (S.err & kIxBadRecord) return fail(e, NGSQ_E_BAD_RECORD, "malformed BAM record (field overrun, CIGAR op > 8 or reference id out of range)");
-  if (S.err & kIxTooLong) return fail(e, NGSQ_E_BAD_RECORD, "a record ends beyond position 2^29, which a BAI cannot address (CSI can)");
-  if (S.err & kIxRunTable) return fail(e, NGSQ_E_CHAIN, "index run table overflow");
-  if (S.err & kIxOverflowList)
-    return fail(e, NGSQ_E_NOMEM, "more than %llu records reach past the end of their reference sequence", (unsigned long long)kIndexOverflowCap);
-  if (S.unsorted_voff != ~0ull)
-    return fail(e, NGSQ_E_UNSORTED, "the records are not coordinate-sorted: the record at virtual offset %llu (block at file offset %llu, offset %llu) "
-                "comes after a record with a larger (reference, position) or an unplaced one; sort the file before indexing it",
-                (unsigned long long)S.unsorted_voff, (unsigned long long)(S.unsorted_voff >> 16), (unsigned long long)(S.unsorted_voff & 0xFFFF));
-  const uint32_t nr = e->n_ref;
-  std::vector<uint64_t> win(e->ix_win_total), counts((size_t)nr * 2);
-  std::vector<uint32_t> maxw(nr);
-  if (e->ix_win_total) CU(cudaMemcpy(win.data(), e->d_ix_win, e->ix_win_total * 8, cudaMemcpyDeviceToHost));
-  if (nr) {
-    CU(cudaMemcpy(counts.data(), e->d_ix_counts, (size_t)nr * 16, cudaMemcpyDeviceToHost));
-    CU(cudaMemcpy(maxw.data(), e->d_ix_maxw, (size_t)nr * 4, cudaMemcpyDeviceToHost));
-  }
-  std::vector<IndexRun> ovf(std::min<uint64_t>(S.n_ovf, kIndexOverflowCap));
-  if (!ovf.empty()) CU(cudaMemcpy(ovf.data(), e->d_ix_ovf, ovf.size() * sizeof(IndexRun), cudaMemcpyDeviceToHost));
-  std::vector<IndexRun> runs;
-  for (auto& d : e->ix_drained) runs.insert(runs.end(), d.first, d.first + d.second);
+// K13 on the host: runs -> chunks per (reference, bin), the linear index, the .bai bytes of the state H (one engine's, or the
+// join of several parts').  Sorts H.runs.
+void assemble_bai(IxHost& H, uint32_t nr, const std::vector<uint64_t>& win_base, const std::vector<uint32_t>& win_n, std::vector<uint8_t>& b) {
+  std::vector<IndexRun>& runs = H.runs;
   // runs were ticketed in any order; each starts at a distinct record, and run r ends where run r + 1 starts
   std::sort(runs.begin(), runs.end(), [](const IndexRun& a, const IndexRun& b) { return a.voff < b.voff; });
   struct Ref {
@@ -887,7 +880,7 @@ int finish_index(ngsq_engine* e) {
     bool any = false;
   };
   std::vector<Ref> refs(nr);
-  const uint64_t data_end = e->data_end_coff << 16;
+  const uint64_t data_end = H.data_end;
   // the runs of one reference are consecutive (sorted input): one bin -> slot table, cleared when the reference changes
   std::vector<int32_t> slot_of(kIxMetaBin, -1);
   uint32_t cur = kIxUnplacedRef;
@@ -906,12 +899,13 @@ int finish_index(ngsq_engine* e) {
     int32_t& sl = slot_of[u.bin];
     if (sl < 0) { sl = (int32_t)R.bins.size(); R.bins.push_back({u.bin, {}}); }
     auto& ch = R.bins[sl].second;
-    if (!ch.empty() && ch.back().second == u.voff) ch.back().second = end;  // contiguous with the bin's last chunk
+    // contiguous with the bin's last chunk (also a run that a cut between two parts split in two)
+    if (!ch.empty() && ch.back().second == u.voff) ch.back().second = end;
     else { ch.push_back({u.voff, end}); ++chunks; }
   }
-  std::vector<uint8_t>& b = e->bai;
+  const uint64_t win_total = H.win.size();
   b.clear();
-  b.reserve(16 + (size_t)nr * 64 + chunks * 16 + ((e->ix_win_total + ovf.size()) * 8));
+  b.reserve(16 + (size_t)nr * 64 + chunks * 16 + ((win_total + H.ovf.size()) * 8));
   auto p32 = [&](uint32_t v) { uint8_t t[4]; memcpy(t, &v, 4); b.insert(b.end(), t, t + 4); };
   auto p64 = [&](uint64_t v) { uint8_t t[8]; memcpy(t, &v, 8); b.insert(b.end(), t, t + 8); };
   b.insert(b.end(), {'B', 'A', 'I', 1});
@@ -926,13 +920,13 @@ int finish_index(ngsq_engine* e) {
       p32((uint32_t)bn.second.size());
       for (auto& ck : bn.second) { p64(ck.first); p64(ck.second); }
     }
-    p32(kIxMetaBin); p32(2); p64(R.beg); p64(R.end); p64(counts[2 * c]); p64(counts[2 * c + 1]);
+    p32(kIxMetaBin); p32(2); p64(R.beg); p64(R.end); p64(H.counts[2 * c]); p64(H.counts[2 * c + 1]);
     // windows nobody touched take the previous window's value (0 before the first touched one)
-    const uint32_t n_intv = maxw[c] + 1;
+    const uint32_t n_intv = H.maxw[c] + 1;
     lin.assign(n_intv, ~0ull);
-    const uint32_t in_table = std::min(n_intv, e->ix_win_n[c]);
-    for (uint32_t w = 0; w < in_table; ++w) lin[w] = win[e->ix_win_base[c] + w];
-    for (const IndexRun& o : ovf)
+    const uint32_t in_table = std::min(n_intv, win_n[c]);
+    for (uint32_t w = 0; w < in_table; ++w) lin[w] = H.win[win_base[c] + w];
+    for (const IndexRun& o : H.ovf)
       if (o.ref == c)
         for (uint32_t w = o.bin & 0xFFFF; w <= (o.bin >> 16) && w < n_intv; ++w) lin[w] = std::min(lin[w], o.voff);
     uint64_t last = 0;
@@ -942,7 +936,51 @@ int finish_index(ngsq_engine* e) {
     p32(n_intv);
     for (uint64_t v : lin) p64(v);
   }
-  p64(S.n_no_coor);
+  p64(H.S.n_no_coor);
+}
+
+int fail_unsorted(ngsq_engine* e, uint64_t voff) {
+  return fail(e, NGSQ_E_UNSORTED, "the records are not coordinate-sorted: the record at virtual offset %llu (block at file offset %llu, offset %llu) "
+              "comes after a record with a larger (reference, position) or an unplaced one; sort the file before indexing it",
+              (unsigned long long)voff, (unsigned long long)(voff >> 16), (unsigned long long)(voff & 0xFFFF));
+}
+
+// K13 at ngsq_finish: the index state back from the device (the run tables drained so far, the rest now), its error bits;
+// then the .bai bytes (NGSQ_F_INDEX) or the part's state for the join (NGSQ_F_INDEX_PART).
+int finish_index(ngsq_engine* e) {
+  for (uint32_t j = 0; j < e->ix_waves.size(); ++j) {
+    int rc = ix_drain(e, j, e->s_comp);
+    if (rc) return rc;
+  }
+  CU(cudaStreamSynchronize(e->s_comp));
+  IxHost& H = e->ix;
+  H = IxHost{};
+  IndexState& S = H.S;
+  CU(cudaMemcpy(&S, e->d_ix, sizeof S, cudaMemcpyDeviceToHost));
+  if (S.err & kIxBadRecord) return fail(e, NGSQ_E_BAD_RECORD, "malformed BAM record (field overrun, CIGAR op > 8 or reference id out of range)");
+  if (S.err & kIxTooLong) return fail(e, NGSQ_E_BAD_RECORD, "a record ends beyond position 2^29, which a BAI cannot address (CSI can)");
+  if (S.err & kIxRunTable) return fail(e, NGSQ_E_CHAIN, "index run table overflow");
+  if (S.err & kIxOverflowList)
+    return fail(e, NGSQ_E_NOMEM, "more than %llu records reach past the end of their reference sequence", (unsigned long long)kIndexOverflowCap);
+  const bool part = e->cfg.flags & NGSQ_F_INDEX_PART;
+  if (!part && S.unsorted_voff != ~0ull) return fail_unsorted(e, S.unsorted_voff);
+  const uint32_t nr = e->n_ref;
+  H.win.resize(e->ix_win_total);
+  H.counts.resize((size_t)nr * 2);
+  H.maxw.resize(nr);
+  if (e->ix_win_total) CU(cudaMemcpy(H.win.data(), e->d_ix_win, e->ix_win_total * 8, cudaMemcpyDeviceToHost));
+  if (nr) {
+    CU(cudaMemcpy(H.counts.data(), e->d_ix_counts, (size_t)nr * 16, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(H.maxw.data(), e->d_ix_maxw, (size_t)nr * 4, cudaMemcpyDeviceToHost));
+  }
+  H.ovf.resize(std::min<uint64_t>(S.n_ovf, kIndexOverflowCap));
+  if (!H.ovf.empty()) CU(cudaMemcpy(H.ovf.data(), e->d_ix_ovf, H.ovf.size() * sizeof(IndexRun), cudaMemcpyDeviceToHost));
+  for (auto& d : e->ix_drained) H.runs.insert(H.runs.end(), d.first, d.first + d.second);
+  H.last_order_key = S.carry[e->ix_waves.size() & 1].order_key;  // the carry the last indexed wave wrote
+  H.data_end = e->data_end_coff << 16;
+  if (part) { e->ix_part_ok = true; return NGSQ_OK; }
+  assemble_bai(H, nr, e->ix_win_base, e->ix_win_n, e->bai);
+  H = IxHost{};
   return NGSQ_OK;
 }
 
@@ -1009,6 +1047,58 @@ int merge_split_local(ngsq_engine* e, bool is_root, cudaStream_t s) {
   return NGSQ_OK;
 }
 
+// Whole BGZF blocks inflated into device memory on s_copy by the engine's inflate kernels (ngsq_inflate_to_host,
+// ngsq_find_record); freed with the object.
+struct DevInflated {
+  uint8_t *in = nullptr, *out = nullptr;
+  BlockDesc* blocks = nullptr;
+  uint32_t *status = nullptr, *bitmap = nullptr;  // status: one word per block, then the decoder's queue word and 60 spare bytes
+  std::vector<BlockDesc> hb;                      // non-empty blocks; coff absolute, out_off from the window's first byte
+  size_t used = 0;                                // bytes of whole blocks
+  uint64_t total = 0;                             // inflated bytes
+  ~DevInflated() {
+    for (void* p : {(void*)in, (void*)out, (void*)blocks, (void*)status, (void*)bitmap}) if (p) cudaFree(p);
+  }
+};
+
+// BGZF framing of `bgzf` (file bytes from `file_off`) and the compressed bytes' device buffer
+int inflate_frame(ngsq_engine* e, const uint8_t* bgzf, size_t nbytes, uint64_t file_off, DevInflated& D) {
+  uint32_t n = 0;
+  int rc = ngsq_bgzf_walk(bgzf, nbytes, file_off, nullptr, 0, &n, &D.used);
+  if (rc) return fail(e, rc, "malformed BGZF framing");
+  std::vector<ngsq_block> blk(n);
+  ngsq_bgzf_walk(bgzf, nbytes, file_off, blk.data(), n, &n, &D.used);
+  CU(cudaMalloc(&D.in, D.used + 512));
+  for (auto& b : blk) {
+    if (b.csize < b.hdr_len + 8 || b.isize > 65536) return fail(e, NGSQ_E_BAD_BLOCK, "malformed BGZF block");
+    if (!b.isize) continue;
+    D.hb.push_back({(uint64_t)(uintptr_t)D.in + (b.coffset - file_off) + b.hdr_len, D.total, b.csize - b.hdr_len - 8, b.isize, b.coffset});
+    D.total += b.isize;
+  }
+  return NGSQ_OK;
+}
+
+// K2 over the framed blocks; fails with the first block that does not inflate
+int inflate_run(ngsq_engine* e, const uint8_t* bgzf, DevInflated& D) {
+  if (D.hb.empty()) return NGSQ_OK;
+  cudaStream_t s = e->s_copy;
+  const size_t nb = D.hb.size();
+  CU(cudaMalloc(&D.out, D.total + 64));
+  CU(cudaMalloc(&D.blocks, nb * sizeof(BlockDesc)));
+  CU(cudaMalloc(&D.status, nb * 4 + 64));
+  CU(cudaMalloc(&D.bitmap, nb * kBitmapWords * 4));
+  CU(cudaMemcpyAsync(D.in, bgzf, D.used, cudaMemcpyHostToDevice, s));
+  CU(cudaMemcpyAsync(D.blocks, D.hb.data(), nb * sizeof(BlockDesc), cudaMemcpyHostToDevice, s));
+  int rc = launch_inflate(e, D.blocks, (uint32_t)nb, D.out, D.status + nb, D.status, D.bitmap, s);
+  if (rc) return rc;
+  std::vector<uint32_t> st(nb);
+  CU(cudaMemcpyAsync(st.data(), D.status, nb * 4, cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  for (size_t i = 0; i < nb; ++i)
+    if (st[i]) return fail(e, NGSQ_E_BAD_BLOCK, "block %zu failed to inflate (status %u)", i, st[i]);
+  return NGSQ_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1026,7 +1116,9 @@ int ngsq_create(int device, const ngsq_config* cfg, ngsq_engine** out) {
   if (rc != cudaSuccess || n_dev == 0)
     return fail(e, NGSQ_E_CUDA, "no CUDA device available (%s); the ngs-cuda engine has no CPU fallback", cudaGetErrorString(rc));
   if (device < 0 || device >= n_dev) return fail(e, NGSQ_E_ARG, "device %d out of range (%d devices)", device, n_dev);
-  if (cfg && (cfg->flags & NGSQ_F_INDEX) && cfg->max_records)
+  if (cfg && (cfg->flags & NGSQ_F_INDEX) && (cfg->flags & NGSQ_F_INDEX_PART))
+    return fail(e, NGSQ_E_ARG, "NGSQ_F_INDEX_PART is set instead of NGSQ_F_INDEX, not with it");
+  if (cfg && (cfg->flags & (NGSQ_F_INDEX | NGSQ_F_INDEX_PART)) && cfg->max_records)
     return fail(e, NGSQ_E_ARG, "NGSQ_F_INDEX cannot be combined with max_records: an index covers every record of the file");
   ngsq_engine* ne = new ngsq_engine();
   ne->device = device;
@@ -1057,7 +1149,7 @@ int ngsq_create(int device, const ngsq_config* cfg, ngsq_engine** out) {
   CUC(cudaMalloc(&e->d_state, sizeof(RunState)));
   CUC(cudaHostAlloc((void**)&e->h_state, sizeof(RunState), cudaHostAllocDefault));
   CUC(cudaHostAlloc((void**)&e->h_prog, kProgSlots * 16, cudaHostAllocDefault));
-  if (e->cfg.flags & NGSQ_F_INDEX) {
+  if (ix_on(e)) {
     CUC(cudaMalloc(&e->d_ix, sizeof(IndexState)));
     CUC(cudaMalloc(&e->d_ix_ovf, kIndexOverflowCap * sizeof(IndexRun)));
     CUC(cudaHostAlloc((void**)&e->h_ix_probe, 16, cudaHostAllocDefault));
@@ -1151,6 +1243,8 @@ int ngsq_reset(ngsq_engine* e) {
   e->ix_drained.clear();  // pinned memory of the pin slabs, released above
   e->data_end_coff = 0;
   e->bai.clear();
+  e->ix = IxHost{};
+  e->ix_part_ok = false;
   e->split_merged = false;  // the split set itself is kept
   memset(&e->stats, 0, sizeof e->stats);
   return NGSQ_OK;
@@ -1159,7 +1253,7 @@ int ngsq_reset(ngsq_engine* e) {
 int ngsq_set_references(ngsq_engine* e, uint32_t n_ref, const uint32_t* ref_len, const uint8_t* coverage_enabled) {
   if (!e || (n_ref && (!ref_len || !coverage_enabled))) return fail(e, NGSQ_E_ARG, "bad references");
   if (e->run_started) return fail(e, NGSQ_E_ARG, "ngsq_set_references must precede the first submit");
-  if (e->cfg.flags & NGSQ_F_INDEX)
+  if (ix_on(e))
     for (uint32_t c = 0; c < n_ref; ++c)
       if (ref_len[c] >= kIxMaxEnd)
         return fail(e, NGSQ_E_ARG, "reference %u is %u bases long: a BAI addresses fewer than 2^29 bases (index this file as CSI)", c, ref_len[c]);
@@ -1252,7 +1346,7 @@ int ngsq_set_references(ngsq_engine* e, uint32_t n_ref, const uint32_t* ref_len,
     if (n_ref) CU(cudaMemcpy(e->d_ft_contigs, e->ft_contigs.data(), n_ref * sizeof(FeatureContig), cudaMemcpyHostToDevice));
     if (!e->d_ft_res) CU(cudaMalloc(&e->d_ft_res, F_WORDS * 8));
   }
-  if (e->cfg.flags & NGSQ_F_INDEX) {
+  if (ix_on(e)) {
     // linear-index table per reference: windows 0 ..= L >> 14 (reads overhanging the end go to the overflow list)
     e->ix_win_base.assign(n_ref, 0);
     e->ix_win_n.assign(n_ref, 0);
@@ -1634,12 +1728,14 @@ int ngsq_finish(ngsq_engine* e) {
     const uint64_t k = e->h_ft_res[F_ERR];
     return fail(e, NGSQ_E_FEATURES, "Genomic Features: %s (the reference aborts the run here)", k < sizeof kinds / sizeof *kinds ? kinds[k] : "unknown failure");
   }
-  if (e->cfg.flags & NGSQ_F_INDEX) return finish_index(e);
+  if (ix_on(e)) return finish_index(e);
   return NGSQ_OK;
 }
 
 int ngsq_get_bai(ngsq_engine* e, uint8_t* out, size_t cap, size_t* n_out) {
   if (!e) return NGSQ_E_ARG;
+  if (e->cfg.flags & NGSQ_F_INDEX_PART)
+    return fail(e, NGSQ_E_ARG, "ngsq_get_bai: this engine indexed one part of a file (NGSQ_F_INDEX_PART); join the finished parts with ngsq_join_bai");
   if (!(e->cfg.flags & NGSQ_F_INDEX)) return fail(e, NGSQ_E_ARG, "ngsq_get_bai: the engine was created without NGSQ_F_INDEX");
   if (!e->finished || e->bai.empty()) return fail(e, NGSQ_E_ARG, "ngsq_get_bai: no index before a successful ngsq_finish");
   if (n_out) *n_out = e->bai.size();
@@ -1998,53 +2094,99 @@ int ngsq_host_unregister(void* p) { return cudaHostUnregister(p) == cudaSuccess 
 int ngsq_inflate_to_host(ngsq_engine* e, const uint8_t* bgzf, size_t nbytes, uint8_t* out, size_t cap, size_t* n_out) {
   if (!e || !bgzf || !out) return fail(e, NGSQ_E_ARG, "bad arguments");
   CU(cudaSetDevice(e->device));
-  uint32_t n = 0;
-  size_t used = 0;
-  int rc = ngsq_bgzf_walk(bgzf, nbytes, 0, nullptr, 0, &n, &used);
-  if (rc) return fail(e, rc, "malformed BGZF framing");
-  std::vector<ngsq_block> blk(n);
-  ngsq_bgzf_walk(bgzf, nbytes, 0, blk.data(), n, &n, &used);
-  uint8_t* d_in = nullptr;
-  uint8_t* d_o = nullptr;
-  BlockDesc* d_b = nullptr;
-  uint32_t *d_st = nullptr, *d_q = nullptr;
-  std::vector<BlockDesc> hb;
-  uint64_t total = 0;
-  CU(cudaMalloc(&d_in, used + 512));
-  for (auto& b : blk) {
-    if (b.csize < b.hdr_len + 8 || b.isize > 65536) { cudaFree(d_in); return fail(e, NGSQ_E_BAD_BLOCK, "malformed BGZF block"); }
-    if (!b.isize) continue;
-    hb.push_back({(uint64_t)(uintptr_t)d_in + b.coffset + b.hdr_len, total, b.csize - b.hdr_len - 8, b.isize, b.coffset});
-    total += b.isize;
+  DevInflated D;
+  int rc = inflate_frame(e, bgzf, nbytes, 0, D);
+  if (rc) return rc;
+  if (n_out) *n_out = (size_t)D.total;
+  if (D.total > cap) return fail(e, NGSQ_E_ARG, "output buffer too small (%llu needed)", (unsigned long long)D.total);
+  if ((rc = inflate_run(e, bgzf, D))) return rc;
+  if (D.total) {
+    CU(cudaMemcpyAsync(out, D.out, D.total, cudaMemcpyDeviceToHost, e->s_copy));
+    CU(cudaStreamSynchronize(e->s_copy));
   }
-  if (n_out) *n_out = (size_t)total;
-  if (total > cap) { cudaFree(d_in); return fail(e, NGSQ_E_ARG, "output buffer too small (%llu needed)", (unsigned long long)total); }
-  int ret = NGSQ_OK;
-  if (!hb.empty()) {
-    cudaStream_t s = e->s_copy;
-    CU(cudaMalloc(&d_o, total + 64));
-    CU(cudaMalloc(&d_b, hb.size() * sizeof(BlockDesc)));
-    CU(cudaMalloc(&d_st, hb.size() * 4 + 64));
-    d_q = d_st + hb.size();
-    CU(cudaMemcpyAsync(d_in, bgzf, used, cudaMemcpyHostToDevice, s));
-    CU(cudaMemcpyAsync(d_b, hb.data(), hb.size() * sizeof(BlockDesc), cudaMemcpyHostToDevice, s));
-    uint32_t* d_bm = nullptr;
-    CU(cudaMalloc(&d_bm, hb.size() * kBitmapWords * 4));
-    ret = launch_inflate(e, d_b, (uint32_t)hb.size(), d_o, d_q, d_st, d_bm, s);
-    std::vector<uint32_t> st(hb.size());
-    if (!ret) {
-      CU(cudaMemcpyAsync(out, d_o, total, cudaMemcpyDeviceToHost, s));
-      CU(cudaMemcpyAsync(st.data(), d_st, hb.size() * 4, cudaMemcpyDeviceToHost, s));
-      CU(cudaStreamSynchronize(s));
-      for (size_t i = 0; i < st.size(); ++i)
-        if (st[i]) { ret = fail(e, NGSQ_E_BAD_BLOCK, "block %zu failed to inflate (status %u)", i, st[i]); break; }
-    }
-    cudaStreamSynchronize(s);
-    cudaFree(d_o); cudaFree(d_b); cudaFree(d_st);
-    if (d_bm) cudaFree(d_bm);
+  return NGSQ_OK;
+}
+
+int ngsq_find_record(ngsq_engine* e, const uint8_t* bgzf, size_t nbytes, uint64_t file_off, uint64_t* voffset, int32_t* ref_id) {
+  if (!e || !bgzf || !voffset) return fail(e, NGSQ_E_ARG, "bad arguments");
+  if (!e->d_ref_len) return fail(e, NGSQ_E_ARG, "ngsq_find_record needs ngsq_set_references first (the record test needs n_ref)");
+  *voffset = 0;
+  if (ref_id) *ref_id = -1;
+  CU(cudaSetDevice(e->device));
+  DevInflated D;
+  int rc = inflate_frame(e, bgzf, nbytes, file_off, D);
+  if (rc) return rc;
+  if (D.used != nbytes)
+    return fail(e, NGSQ_E_TRUNCATED, "ngsq_find_record: the bytes at file offset %llu end inside a BGZF block", (unsigned long long)file_off);
+  if ((rc = inflate_run(e, bgzf, D))) return rc;
+  if (D.total < 36) return NGSQ_OK;
+  cudaStream_t s = e->s_copy;
+  // an 8-byte word in the spare bytes behind the decoder's queue word
+  unsigned long long* d_best = reinterpret_cast<unsigned long long*>(((uintptr_t)(D.status + D.hb.size() + 1) + 7) & ~(uintptr_t)7);
+  CU(cudaMemsetAsync(d_best, 0xFF, 8, s));
+  const uint32_t grid = (uint32_t)std::min<uint64_t>((D.total + 255) / 256, (uint64_t)e->n_sm * 16);
+  find_record_kernel<<<grid, 256, 0, s>>>(D.out, D.total, (int32_t)e->n_ref, d_best);
+  CU(cudaGetLastError());
+  unsigned long long best = 0;
+  CU(cudaMemcpyAsync(&best, d_best, 8, cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  if (best == ~0ull) return NGSQ_OK;
+  int32_t ref = -1;
+  CU(cudaMemcpy(&ref, D.out + best + 4, 4, cudaMemcpyDeviceToHost));
+  // the block that holds inflated offset `best` (empty blocks are not in the table)
+  size_t k = 0;
+  while (k + 1 < D.hb.size() && D.hb[k + 1].out_off <= best) ++k;
+  *voffset = (D.hb[k].coff << 16) | (best - D.hb[k].out_off);
+  if (ref_id) *ref_id = ref;
+  return NGSQ_OK;
+}
+
+int ngsq_join_bai(ngsq_engine* const* parts, uint32_t n, uint8_t* out, size_t cap, size_t* n_out) {
+  if (!parts || !n) return fail(nullptr, NGSQ_E_ARG, "ngsq_join_bai: no parts");
+  ngsq_engine* e = parts[0];  // carries the message
+  for (uint32_t k = 0; k < n; ++k) {
+    const ngsq_engine* p = parts[k];
+    if (!p) return fail(e, NGSQ_E_ARG, "ngsq_join_bai: part %u is NULL", k);
+    if (!(p->cfg.flags & NGSQ_F_INDEX_PART)) return fail(e, NGSQ_E_ARG, "ngsq_join_bai: part %u was created without NGSQ_F_INDEX_PART", k);
+    if (!p->finished || !p->ix_part_ok) return fail(e, NGSQ_E_ARG, "ngsq_join_bai: part %u has no index (it did not finish without error)", k);
+    if (p->ref_len != parts[0]->ref_len) return fail(e, NGSQ_E_ARG, "ngsq_join_bai: part %u has other references than part 0", k);
+    if (k + 1 < n && p->end_voff != parts[k + 1]->first_voff)
+      return fail(e, NGSQ_E_ARG, "ngsq_join_bai: part %u ends at virtual offset %llu, part %u starts at %llu: the parts must be contiguous, in file order", k,
+                  (unsigned long long)p->end_voff, k + 1, (unsigned long long)parts[k + 1]->first_voff);
   }
-  cudaFree(d_in);
-  return ret;
+  if (parts[n - 1]->end_voff) return fail(e, NGSQ_E_ARG, "ngsq_join_bai: the last part must run to the end of the data (end offset 0)");
+  // the order across every cut: a part's first placed record against the last record before the part that constrains the
+  // order (an unplaced one: ~0); every other record was checked inside its part
+  uint64_t unsorted = ~0ull, last = 0;
+  for (uint32_t k = 0; k < n; ++k) {
+    const IxHost& H = parts[k]->ix;
+    unsorted = std::min<uint64_t>(unsorted, H.S.unsorted_voff);
+    if (H.S.first_voff != ~0ull && H.S.first_key < last) unsorted = std::min<uint64_t>(unsorted, H.S.first_voff);
+    if (H.last_order_key) last = H.last_order_key;
+  }
+  if (unsorted != ~0ull) return fail_unsorted(e, unsorted);
+  const ngsq_engine* p0 = parts[0];
+  IxHost U;
+  U.win.assign(p0->ix_win_total, ~0ull);
+  U.counts.assign((size_t)p0->n_ref * 2, 0);
+  U.maxw.assign(p0->n_ref, 0);
+  for (uint32_t k = 0; k < n; ++k) {
+    const IxHost& H = parts[k]->ix;
+    U.runs.insert(U.runs.end(), H.runs.begin(), H.runs.end());
+    U.ovf.insert(U.ovf.end(), H.ovf.begin(), H.ovf.end());
+    for (size_t w = 0; w < U.win.size(); ++w) U.win[w] = std::min(U.win[w], H.win[w]);
+    for (size_t c = 0; c < U.counts.size(); ++c) U.counts[c] += H.counts[c];
+    for (size_t c = 0; c < U.maxw.size(); ++c) U.maxw[c] = std::max(U.maxw[c], H.maxw[c]);
+    U.S.n_no_coor += H.S.n_no_coor;
+  }
+  U.data_end = parts[n - 1]->ix.data_end;
+  std::vector<uint8_t> b;
+  assemble_bai(U, p0->n_ref, p0->ix_win_base, p0->ix_win_n, b);
+  if (n_out) *n_out = b.size();
+  if (!out && !cap) return NGSQ_OK;
+  if (!out || cap < b.size()) return fail(e, NGSQ_E_ARG, "ngsq_join_bai: buffer holds %zu bytes, %zu needed", cap, b.size());
+  memcpy(out, b.data(), b.size());
+  return NGSQ_OK;
 }
 
 }  // extern "C"

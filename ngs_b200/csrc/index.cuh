@@ -144,6 +144,10 @@ struct IndexCarry {
 };
 
 struct IndexState {
+  // NGSQ_F_INDEX_PART: order key and virtual offset of the part's first placed record (~0 = none), the two halves of one
+  // 128-bit word with the offset high, so that a 128-bit minimum takes the first record with its key
+  alignas(16) unsigned long long first_key;
+  unsigned long long first_voff;
   IndexCarry carry[2];
   unsigned long long n_runs[2];     // entries in the run table of slot j & 1 (zeroed before the wave's kernel)
   unsigned long long n_no_coor;     // unplaced records
@@ -171,7 +175,22 @@ struct IndexParams {
   unsigned long long* win;  // linear index: smallest start offset per window (~0 = untouched)
   unsigned int* max_win;    // per reference: largest window touched
   unsigned long long* counts;  // per reference: mapped, unmapped
+  uint32_t part;            // NGSQ_F_INDEX_PART: also record the first placed record (IndexState::first_key / first_voff)
 };
+
+// 128-bit minimum of (voff, key) into S->first_key / first_voff.  A torn read of the current value only costs a failed CAS:
+// the offset half never grows, and no two records share an offset.
+__device__ __forceinline__ void index_first_min(IndexState* S, uint64_t voff, uint64_t key) {
+  unsigned __int128* p = reinterpret_cast<unsigned __int128*>(&S->first_key);
+  const unsigned __int128 v = ((unsigned __int128)voff << 64) | key;
+  const volatile unsigned long long* h = &S->first_key;
+  unsigned __int128 o = ((unsigned __int128)h[1] << 64) | h[0];
+  while (v < o) {
+    const unsigned __int128 r = atomicCAS(p, o, v);
+    if (r == o) break;
+    o = r;
+  }
+}
 
 constexpr int kIndexThreads = 256;
 
@@ -273,6 +292,7 @@ __global__ void __launch_bounds__(kIndexThreads) index_kernel(IndexParams P) {
     const bool pl = own && k.placed;
     no_coor += __popc(__ballot_sync(0xFFFFFFFFu, own && !k.placed && !bad));
     const uint32_t pm = __ballot_sync(0xFFFFFFFFu, pl);
+    if (P.part && pm && (int)lane == __ffs(pm) - 1) index_first_min(P.S, voff, index_order_key(k));  // the warp's first in file order
     uint32_t w_lo = 0, w_hi = 0, nw = 0;
     if (pl) {
       index_windows(k, &w_lo, &w_hi);

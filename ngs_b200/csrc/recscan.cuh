@@ -25,6 +25,7 @@
 //                    positive of step 1 can never change results;
 //   4. scan_counts — exclusive scan of the counts + the wave's commit (record count, next carry, errors);
 //   5. walk<emit>  — same walk, writes rec[i] = offset in the slot | (block + 1) << 40 (0 = the carried record).
+// find_record_kernel serves ngsq_find_record (record anchors of a file without an index) with the same plausibility test.
 #pragma once
 #include <cstdint>
 #include <cuda_runtime.h>
@@ -229,6 +230,24 @@ __global__ void find_first_kernel(WaveParams W) {
     }
   }
   if (lane == 0) W.first[warp] = res;
+}
+
+// ngsq_find_record: one thread per offset of an inflated window [0, n) (grid-stride, so a thread's offsets only grow).  An
+// offset passes when a chain of plausible records starts there and runs to the end of the window (the last record may run
+// past it; a tail too short for a header is not judged).  *best = the smallest passing offset (~0 = none).
+__global__ void find_record_kernel(const uint8_t* __restrict__ d, uint64_t n, int32_t n_ref, unsigned long long* best) {
+  const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+  for (uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; c + 36 <= n; c += stride) {
+    if (c >= *(volatile unsigned long long*)best) return;
+    uint64_t off = c;
+    bool ok = true;
+    while (off + 36 <= n) {
+      const uint64_t nx = plausible(d, off, n, n_ref, true);
+      if (!nx) { ok = false; break; }
+      off = nx;
+    }
+    if (ok) { atomicMin(best, (unsigned long long)c); return; }
+  }
 }
 
 // the walk that reaches the end of the wave names the next carry; two different claims = two chains = closure failure

@@ -23,6 +23,7 @@ NGSQ_F_EDITS = 8
 NGSQ_F_FEATURES = 16
 NGSQ_F_SERIAL_STAGES = 32  # measurement aid: no overlap between the stages of consecutive waves
 NGSQ_F_INDEX = 64  # build the file's BAI in the same pass (Engine.bai())
+NGSQ_F_INDEX_PART = 128  # index one range of a file cut between engines (join the parts with join_bai())
 
 ERROR_NAMES = {
     0: "NGSQ_OK", -1: "NGSQ_E_ARG", -2: "NGSQ_E_CUDA", -3: "NGSQ_E_TRUNCATED", -4: "NGSQ_E_BAD_BLOCK",
@@ -40,7 +41,7 @@ EXPORTED = [
     "ngsq_result_buffer", "ngsq_refresh_results", "ngsq_host_alloc", "ngsq_host_free", "ngsq_inflate_to_host",
     "ngsq_set_reference_bases", "ngsq_get_edits", "ngsq_get_edit_positions", "ngsq_set_feature_model", "ngsq_set_features", "ngsq_get_features",
     "ngsq_wait_copied", "ngsq_host_register", "ngsq_host_unregister", "ngsq_flush", "ngsq_progress",
-    "ngsq_get_bai", "ngsq_split_reference", "ngsq_split_arrays", "ngsq_resolve_split",
+    "ngsq_get_bai", "ngsq_split_reference", "ngsq_split_arrays", "ngsq_resolve_split", "ngsq_find_record", "ngsq_join_bai",
 ]
 
 
@@ -147,6 +148,8 @@ def load_library() -> C.CDLL:
     lib.ngsq_split_reference.argtypes = [P, C.c_uint32]
     lib.ngsq_split_arrays.argtypes = [P, C.c_uint32, C.POINTER(SplitArrays)]
     lib.ngsq_resolve_split.argtypes = [P, C.c_int]
+    lib.ngsq_find_record.argtypes = [P, P, C.c_size_t, C.c_uint64, u64p, C.POINTER(C.c_int32)]
+    lib.ngsq_join_bai.argtypes = [C.POINTER(P), C.c_uint32, P, C.c_size_t, C.POINTER(C.c_size_t)]
     _lib = lib
     return lib
 
@@ -344,6 +347,14 @@ class Engine:
         self._check(self.lib.ngsq_get_bai(self.h, buf.ctypes.data, n.value, C.byref(n)))
         return buf[: n.value].tobytes()
 
+    def find_record(self, data: np.ndarray, file_off: int = 0):
+        """Record anchor in whole BGZF blocks `data` (uint8 array) that start at file offset `file_off`: (virtual offset of
+        the first offset that starts a chain of plausible records to the end of the window, its reference id), or (0, -1)
+        when the window holds none.  Speculative: a range that ends there proves it (ngsq_find_record)."""
+        v, r = C.c_uint64(0), C.c_int32(-1)
+        self._check(self.lib.ngsq_find_record(self.h, data.ctypes.data, data.size, file_off, C.byref(v), C.byref(r)))
+        return v.value, r.value
+
     def stats(self) -> dict:
         st = Stats()
         self._check(self.lib.ngsq_get_stats(self.h, C.byref(st)))
@@ -384,6 +395,21 @@ class Engine:
     def resolve_split(self, is_root: bool):
         """After the split arrays were summed into the root's: resolve them there, zero them elsewhere."""
         self._check(self.lib.ngsq_resolve_split(self.h, int(bool(is_root))))
+
+
+def join_bai(parts) -> bytes:
+    """The .bai of a file from its NGSQ_F_INDEX_PART engines, in file order (ngsq_join_bai)."""
+    lib = load_library()
+    hs = (C.c_void_p * len(parts))(*[p.h.value for p in parts])
+    n = C.c_size_t(0)
+
+    def check(rc):
+        if rc:
+            raise NgsqError(rc, lib.ngsq_last_error(parts[0].h if parts else None).decode())
+    check(lib.ngsq_join_bai(hs, len(parts), None, 0, C.byref(n)))
+    buf = np.empty(max(n.value, 1), dtype=np.uint8)
+    check(lib.ngsq_join_bai(hs, len(parts), buf.ctypes.data, n.value, C.byref(n)))
+    return buf[: n.value].tobytes()
 
 
 def nccl_unique_id() -> bytes:

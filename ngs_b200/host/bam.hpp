@@ -12,6 +12,7 @@
 #include <cstdint>
 #include <cstring>
 #include <fstream>
+#include <functional>
 #include <stdexcept>
 #include <string>
 #include <vector>
@@ -210,7 +211,8 @@ inline std::vector<Shard> plan_shards(const BamHeader& h, const BaiIndex& bai, u
 struct ShardPlan {
   std::vector<Shard> shards;
   std::vector<uint32_t> split;  // split references, ascending
-  bool split_plan = false;      // plan_shards_split's plan (choose_shards)
+  bool split_plan = false;      // plan_shards_split's plan (choose_shards), or plan_shards_unindexed's
+  uint32_t dropped = 0;         // plan_shards_unindexed: cuts left out (no record found, or an anchor repeated)
 };
 
 // Record starts the planner may cut at, ascending and distinct: zeros, entries below their contig's first record and
@@ -316,6 +318,76 @@ inline ShardPlan choose_shards(const BamHeader& h, const BaiIndex& bai, uint32_t
   ShardPlan split = plan_shards_split(h, bai, n_shards, file_size);
   if (all_live && (double)split_reduce_bytes(h, split.split) > kSplitReduceShards * mean) return plan;
   return split;
+}
+
+// ---- cuts without an index (DESIGN 5): a freshly sorted BAM has no .bai, so the anchors come from the records themselves
+// BGZF header of a block that carries only the BC subfield: magic, CM = 8, FLG = FEXTRA, XLEN = 6, 'B' 'C', SLEN = 2
+inline bool bgzf_signature(const uint8_t* p) {
+  return p[0] == 0x1f && p[1] == 0x8b && p[2] == 8 && p[3] == 4 && p[10] == 6 && p[11] == 0 && p[12] == 'B' && p[13] == 'C' && p[14] == 2 && p[15] == 0;
+}
+
+// The first block start at or after `from`: a signature confirmed by a chain of whole blocks behind it (at least three, or
+// exactly to the end of the file), so that a signature inside a block's payload is skipped.  file_size when there is none.
+constexpr uint32_t kChainConfirm = 3;
+inline uint64_t next_block_start(const uint8_t* bam, uint64_t file_size, uint64_t from) {
+  for (uint64_t q = from; q + 18 <= file_size; ++q) {
+    if (!bgzf_signature(bam + q)) continue;
+    const uint64_t len = std::min<uint64_t>(file_size - q, (uint64_t)(kChainConfirm + 1) << 16);
+    uint32_t n = 0;
+    size_t used = 0;
+    if (ngsq_bgzf_walk(bam + q, len, q, nullptr, 0, &n, &used)) continue;
+    if (n >= kChainConfirm || q + used == file_size) return q;
+  }
+  return file_size;
+}
+
+// The record anchor finder (ngsq_find_record on an engine; a fake in the CPU tests): whole BGZF blocks `bgzf` at file
+// offset `file_off` -> the first record start in them as a virtual offset and its reference id, 0 when there is none.
+using FindRecord = std::function<void(const uint8_t* bgzf, size_t nbytes, uint64_t file_off, uint64_t* voffset, int32_t* ref_id)>;
+constexpr uint32_t kFindBlocks = 4;        // first window of the finder, in blocks
+constexpr uint32_t kFindBlocksMax = 4096;  // its largest window (256 MiB inflated): a read longer than that leaves the cut out
+
+// Cuts at targets first_record_coffset + (file_size - that) * k / n, each snapped to the next block start and moved to the
+// first record the finder sees from there (its window doubles until it sees one).  A cut is dropped when no record is found
+// or when its anchor does not lie strictly behind the previous one; its device gets an empty shard.  The anchors are
+// speculative until the range in front of each closes on it (run_parts in the driver).  Only the reference of the first
+// record behind a cut can have records on both sides of it (sorted input), so those references are the split set; the
+// driver declares them whether or not Coverage processes them, because Edits keeps per-position counters of every contig.
+inline ShardPlan plan_shards_unindexed(const BamHeader& h, const uint8_t* bam, uint64_t file_size, uint32_t n_shards, const FindRecord& find) {
+  ShardPlan plan;
+  plan.split_plan = true;
+  const uint64_t first = h.first_record_voffset, base = std::min<uint64_t>(first >> 16, file_size);
+  std::vector<uint64_t> bounds{first};
+  std::vector<uint32_t> split;
+  std::vector<ngsq_block> tmp(kFindBlocksMax);
+  for (uint32_t k = 1; k < n_shards; ++k) {
+    const uint64_t target = base + (uint64_t)((unsigned __int128)(file_size - base) * k / n_shards);
+    const uint64_t p = next_block_start(bam, file_size, target);
+    uint64_t anchor = 0;
+    int32_t ref = -1;
+    for (uint32_t nb = kFindBlocks; p < file_size && nb <= kFindBlocksMax; nb *= 2) {
+      uint32_t n = 0;
+      size_t used = 0;
+      const uint64_t len = std::min<uint64_t>(file_size - p, (uint64_t)nb << 16);
+      if (ngsq_bgzf_walk(bam + p, len, p, tmp.data(), nb, &n, &used) || !used) break;
+      find(bam + p, used, p, &anchor, &ref);
+      if (anchor || p + used == file_size) break;
+    }
+    if (!anchor || anchor <= bounds.back()) { ++plan.dropped; continue; }
+    bounds.push_back(anchor);
+    if (ref >= 0) split.push_back((uint32_t)ref);
+  }
+  for (size_t i = 0; i < bounds.size(); ++i) {
+    Shard s;
+    s.first_voffset = bounds[i];
+    s.end_voffset = i + 1 < bounds.size() ? bounds[i + 1] : 0;
+    plan.shards.push_back(s);
+  }
+  std::sort(split.begin(), split.end());
+  split.erase(std::unique(split.begin(), split.end()), split.end());
+  plan.split = split;
+  while (plan.shards.size() < n_shards) { Shard s; s.empty = true; plan.shards.push_back(s); }
+  return plan;
 }
 
 // Compressed byte range [lo, hi) a shard submits: through the block that holds end_voffset.

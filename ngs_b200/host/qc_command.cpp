@@ -4,9 +4,14 @@
 // app() (305-316 and 350-397) are replaced by one pass of the CUDA engine per GPU.  `index` builds the
 // BAI that `qc` needs (src/index/bam.rs:39-109) in one pass of the engine on one GPU.
 //
+// A BAM without an index is cut between GPUs at record anchors the engine finds (ngsq_find_record), each GPU indexes its part
+// (NGSQ_F_INDEX_PART) and the host joins the parts (ngsq_join_bai): `index --cuda-devices`, and `qc --cuda-build-index`,
+// which writes the missing .bai in the same pass as the results.
+//
 //   ngs-cuda-qc qc <BAM> <REFERENCE_GENOME> [-n N] [-o DIR] [-p PREFIX] [--only FACET]
-//               [--cuda-devices 0,1,..] [--cuda-gc-seed S] [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io] [--cuda-perf]
-//   ngs-cuda-qc index <BAM> [--cuda-device N] [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io]
+//               [--cuda-devices 0,1,..] [--cuda-build-index] [--cuda-gc-seed S] [--cuda-no-crc] [--cuda-chunk-mb M]
+//               [--cuda-buffered-io] [--cuda-perf]
+//   ngs-cuda-qc index <BAM> [--cuda-device N | --cuda-devices 0,1,..] [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io]
 #include <cerrno>
 #include <cstdio>
 #include <cstdlib>
@@ -41,6 +46,7 @@ struct QcArgs {
   size_t chunk_mb = 64;
   bool direct_io = true;
   bool perf = false;
+  bool build_index = false;  // a missing .bai is built in the same pass and written next to the BAM
 };
 
 void info(const std::string& s) { std::cerr << "INFO " << s << "\n"; }
@@ -164,7 +170,7 @@ class ChunkReader {
 };
 
 void run_shard(ngsq_engine* e, const std::string& path, const MappedFile& file, const Shard& shard, size_t chunk_bytes, bool direct, bool log_progress,
-               std::string* err) {
+               std::string* err, int* code) {
   try {
     if (shard.empty) { check(e, ngsq_set_range(e, 0, 0)); check(e, ngsq_finish(e)); return; }
     uint64_t lo, hi;
@@ -185,6 +191,7 @@ void run_shard(ngsq_engine* e, const std::string& path, const MappedFile& file, 
         check(e, ngsq_set_quality_positions(e, (uint32_t)st.max_read_len + 1));
         continue;
       }
+      if (code) *code = rc;
       check(e, rc);
       if (log_progress) progress.report(e);
       break;
@@ -194,13 +201,89 @@ void run_shard(ngsq_engine* e, const std::string& path, const MappedFile& file, 
   }
 }
 
+// The parts of a file cut without an index (plan_shards_unindexed), one thread per engine.  An anchor is proven when the
+// range in front of it closes on it; the first record after the header is proven, so the cuts are proven in file order: a
+// part whose start is proven and that fails with NGSQ_E_CHAIN or NGSQ_E_TRUNCATED, with a next part behind it, ends on a
+// false anchor.  That cut is dropped: the part is run again over both ranges, the next engine over an empty one.  Any other
+// failure is the file's and is reported.  On return every engine has finished; shards holds the ranges that ran.
+void run_parts(const std::vector<ngsq_engine*>& engines, std::vector<Shard>& shards, const std::string& path, const MappedFile& file,
+               size_t chunk_bytes, bool direct) {
+  const size_t n = engines.size();
+  std::vector<std::string> errs(n);
+  std::vector<int> codes(n, 0);
+  {
+    std::vector<std::thread> ts;
+    for (size_t i = 0; i < n; ++i)
+      ts.emplace_back(run_shard, engines[i], std::cref(path), std::cref(file), std::cref(shards[i]), chunk_bytes, direct, i == 0, &errs[i], &codes[i]);
+    for (auto& t : ts) t.join();
+  }
+  for (size_t k = 0; k < n; ++k) {
+    while (!errs[k].empty()) {
+      size_t j = k + 1;  // the next live part: its start is the cut in question
+      while (j < n && shards[j].empty) ++j;
+      if (j == n || (codes[k] != NGSQ_E_CHAIN && codes[k] != NGSQ_E_TRUNCATED)) throw std::runtime_error(errs[k]);
+      info("  [*] The record anchor at virtual offset " + std::to_string(shards[j].first_voffset) +
+           " is not a record start: dropping that cut and reading the range again.");
+      shards[k].end_voffset = shards[j].end_voffset;
+      shards[j] = Shard();
+      shards[j].empty = true;
+      for (size_t i : {k, j}) {
+        check(engines[i], ngsq_reset(engines[i]));
+        errs[i].clear();
+        codes[i] = 0;
+      }
+      run_shard(engines[j], path, file, shards[j], chunk_bytes, direct, false, &errs[j], &codes[j]);
+      if (!errs[j].empty()) throw std::runtime_error(errs[j]);
+      run_shard(engines[k], path, file, shards[k], chunk_bytes, direct, false, &errs[k], &codes[k]);
+    }
+  }
+}
+
+// The record anchor finder of plan_shards_unindexed on engine e (after ngsq_set_references)
+FindRecord engine_finder(ngsq_engine* e) {
+  return [e](const uint8_t* p, size_t n, uint64_t off, uint64_t* voff, int32_t* ref) { check(e, ngsq_find_record(e, p, n, off, voff, ref)); };
+}
+
+// The parts' .bai, in file order (engines with an empty range hold no part)
+std::vector<uint8_t> join_parts(const std::vector<ngsq_engine*>& engines, const std::vector<Shard>& shards) {
+  std::vector<ngsq_engine*> parts;
+  for (size_t i = 0; i < engines.size(); ++i)
+    if (!shards[i].empty) parts.push_back(engines[i]);
+  size_t n = 0;
+  check(parts[0], ngsq_join_bai(parts.data(), (uint32_t)parts.size(), nullptr, 0, &n));
+  std::vector<uint8_t> bai(n);
+  check(parts[0], ngsq_join_bai(parts.data(), (uint32_t)parts.size(), bai.data(), bai.size(), &n));
+  return bai;
+}
+
+// The .bai next to the BAM.  O_EXCL: an index that appeared while the file was read is not replaced either.
+void write_index(const std::string& dst, const std::vector<uint8_t>& bai) {
+  info("Writing index to " + dst + ".");
+  const int fd = open(dst.c_str(), O_WRONLY | O_CREAT | O_EXCL, 0644);
+  if (fd < 0) throw std::runtime_error("cannot create " + dst + (errno == EEXIST ? ": index file already exists" : ""));
+  size_t done = 0;
+  while (done < bai.size()) {
+    const ssize_t w = write(fd, bai.data() + done, bai.size() - done);
+    if (w <= 0) { close(fd); std::filesystem::remove(dst); throw std::runtime_error("write error on " + dst); }
+    done += (size_t)w;
+  }
+  if (close(fd)) { std::filesystem::remove(dst); throw std::runtime_error("write error on " + dst); }
+}
+
+void log_dropped_cuts(const ShardPlan& plan) {
+  if (plan.dropped) info("  [*] " + std::to_string(plan.dropped) + " cut(s) left out: no record start found behind the target, or the anchor repeats.");
+}
+
 // command.rs:226-421
 int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& output_prefix, const std::string& output_directory) {
   // open_and_parse(src, IndexCheck::Full): bam.rs:77-123
   if (args.src.size() < 4 || args.src.substr(args.src.size() - 4) != ".bam")
     throw std::runtime_error("could not open " + args.src + ": expected a .bam file");
   MappedFile file(args.src);
-  BaiIndex bai = read_bai(args.src + ".bai");  // pathbuf.rs:59-75: x.bam -> x.bam.bai
+  const std::string bai_path = args.src + ".bai";  // pathbuf.rs:59-75: x.bam -> x.bam.bai
+  // --cuda-build-index: an existing index is used as it is; a missing one is built by this pass
+  const bool build_index = args.build_index && !std::filesystem::exists(bai_path);
+  BaiIndex bai = build_index ? BaiIndex{} : read_bai(bai_path);
   const uint32_t n_dev = (uint32_t)args.devices.size();
 
   // facets first (cheap) so `--only` errors surface before any device work.  The two optional facets read their
@@ -221,6 +304,7 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   if (features) flags |= NGSQ_F_FEATURES;
   if (edits) flags |= NGSQ_F_EDITS;
   if (args.verify_crc) flags |= NGSQ_F_VERIFY_CRC;
+  if (build_index) flags |= n_dev > 1 ? NGSQ_F_INDEX_PART : NGSQ_F_INDEX;
   if (args.num_records && n_dev > 1) throw std::runtime_error("-n needs a single device (records are counted in file order)");
 
   std::vector<ngsq_engine*> engines(n_dev, nullptr);
@@ -250,15 +334,23 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
 
   // shards: contig-aligned file ranges from the BAI, or ranges cut inside contigs when those leave a device idle or
   // unbalanced (choose_shards); a contig cut between shards is declared on every engine and merged by ngsq_reduce
-  const ShardPlan plan = choose_shards(header, bai, n_dev, file.size());
-  const std::vector<Shard>& shards = plan.shards;
+  std::vector<uint32_t> ref_len;
+  for (auto& rs : header.reference_sequences) ref_len.push_back(rs.length);
+  ShardPlan plan;
+  if (build_index && n_dev > 1) {
+    // no index to cut at: anchors from the records (the finder needs the references; every engine sets them again below)
+    check(engines[0], ngsq_set_references(engines[0], (uint32_t)ref_len.size(), ref_len.data(), std::vector<uint8_t>(ref_len.size(), 0).data()));
+    plan = plan_shards_unindexed(header, file.data(), file.size(), n_dev, engine_finder(engines[0]));
+    log_dropped_cuts(plan);
+  } else {
+    plan = choose_shards(header, bai, n_dev, file.size());
+  }
+  std::vector<Shard> shards = plan.shards;
   if (plan.split_plan) {
     std::string names;
     for (uint32_t c : plan.split) names += (names.empty() ? "" : ", ") + header.reference_sequences[c].name;
     info("  [*] Sharding inside contigs: " + std::to_string(n_dev) + " shards" + (names.empty() ? std::string() : ", split: " + names) + ".");
   }
-  std::vector<uint32_t> ref_len;
-  for (auto& rs : header.reference_sequences) ref_len.push_back(rs.length);
   for (uint32_t i = 0; i < n_dev; ++i) {
     // the same mask on every engine: the packed result buffer (the NCCL payload) is laid out from it, and a
     // contig outside an engine's shard simply stays untouched there (ngsq_reduce rejects differing layouts)
@@ -285,11 +377,13 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   // the hot path: one thread per GPU
   info("Starting CUDA pass for QC stats.");
   const auto t_hot = std::chrono::steady_clock::now();
-  {
+  if (build_index && n_dev > 1) {
+    run_parts(engines, shards, args.src, file, args.chunk_mb << 20, args.direct_io);
+  } else {
     std::vector<std::thread> ts;
     std::vector<std::string> errs(n_dev);
     for (uint32_t i = 0; i < n_dev; ++i)
-      ts.emplace_back(run_shard, engines[i], std::cref(args.src), std::cref(file), std::cref(shards[i]), args.chunk_mb << 20, args.direct_io, i == 0, &errs[i]);
+      ts.emplace_back(run_shard, engines[i], std::cref(args.src), std::cref(file), std::cref(shards[i]), args.chunk_mb << 20, args.direct_io, i == 0, &errs[i], nullptr);
     for (auto& t : ts) t.join();
     for (auto& s : errs) if (!s.empty()) throw std::runtime_error(s);
   }
@@ -299,6 +393,15 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
     for (uint32_t i = 0; i < n_dev; ++i) ts.emplace_back([&, i] { if (ngsq_reduce(engines[i], 0)) errs[i] = ngsq_last_error(engines[i]); });
     for (auto& t : ts) t.join();
     for (auto& s : errs) if (!s.empty()) throw std::runtime_error("NCCL: " + s);
+  }
+  // the index of this pass: joined (and its order checked) before any output is written
+  std::vector<uint8_t> new_bai;
+  if (build_index && n_dev > 1) new_bai = join_parts(engines, shards);
+  else if (build_index) {
+    size_t n = 0;
+    check(engines[0], ngsq_get_bai(engines[0], nullptr, 0, &n));
+    new_bai.resize(n);
+    check(engines[0], ngsq_get_bai(engines[0], new_bai.data(), new_bai.size(), &n));
   }
   const double hot_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_hot).count();
   ngsq_engine* root = engines[0];
@@ -331,6 +434,7 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   for (auto& f : facets.sequence_based) f->aggregate(results);
   info("Writing output.");
   results.write(output_prefix, output_directory);
+  if (build_index) write_index(bai_path, new_bai);
 
   if (args.perf) {
     std::ofstream pf(output_directory + "/" + output_prefix + ".perf.json");
@@ -366,6 +470,7 @@ int qc(const QcArgs& args) {
 struct IndexArgs {
   std::string src;
   int device = 0;
+  std::vector<int> devices;  // --cuda-devices: several engines, one part of the file each
   bool verify_crc = true;
   size_t chunk_mb = 64;
   bool direct_io = true;
@@ -403,17 +508,39 @@ int index_bam(const IndexArgs& a) {
   check(e, ngsq_get_bai(e, nullptr, 0, &n));
   std::vector<uint8_t> bai(n);
   check(e, ngsq_get_bai(e, bai.data(), bai.size(), &n));
-  info("Writing index to " + dst + ".");
-  // O_EXCL: an index that appeared while the file was read is not replaced either
-  const int fd = open(dst.c_str(), O_WRONLY | O_CREAT | O_EXCL, 0644);
-  if (fd < 0) throw std::runtime_error("cannot create " + dst + (errno == EEXIST ? ": index file already exists" : ""));
-  size_t done = 0;
-  while (done < bai.size()) {
-    const ssize_t w = write(fd, bai.data() + done, bai.size() - done);
-    if (w <= 0) { close(fd); std::filesystem::remove(dst); throw std::runtime_error("write error on " + dst); }
-    done += (size_t)w;
+  write_index(dst, bai);
+  return 0;
+}
+
+// `index` on several devices: the file cut at record anchors, one NGSQ_F_INDEX_PART engine and one thread per part, the parts
+// joined on the host.  No collective is involved, so a device may repeat.
+int index_bam_parts(const IndexArgs& a) {
+  info("Starting index command...");
+  const std::string dst = a.src + ".bai";
+  if (std::filesystem::exists(dst)) throw std::runtime_error("index file already exists: " + dst);
+  MappedFile file(a.src);
+  const size_t n_dev = a.devices.size();
+  std::vector<ngsq_engine*> engines(n_dev, nullptr);
+  struct Cleanup { std::vector<ngsq_engine*>& v; ~Cleanup() { for (auto* e : v) if (e) ngsq_destroy(e); } } cleanup{engines};
+  for (size_t i = 0; i < n_dev; ++i) {
+    ngsq_config cfg{};
+    cfg.struct_size = sizeof cfg;
+    cfg.flags = NGSQ_F_INDEX_PART | (a.verify_crc ? NGSQ_F_VERIFY_CRC : 0u);
+    if (ngsq_create(a.devices[i], &cfg, &engines[i])) throw std::runtime_error(std::string("CUDA engine: ") + ngsq_last_error(nullptr));
   }
-  if (close(fd)) { std::filesystem::remove(dst); throw std::runtime_error("write error on " + dst); }
+  BamHeader header = read_bam_header(engines[0], file.data(), file.size());
+  std::vector<uint32_t> ref_len;
+  for (auto& rs : header.reference_sequences) ref_len.push_back(rs.length);
+  std::vector<uint8_t> no_coverage(ref_len.size(), 0);
+  for (auto* e : engines) check(e, ngsq_set_references(e, (uint32_t)ref_len.size(), ref_len.data(), no_coverage.data()));
+  ShardPlan plan = plan_shards_unindexed(header, file.data(), file.size(), (uint32_t)n_dev, engine_finder(engines[0]));
+  log_dropped_cuts(plan);
+  info("Indexing BAM file in " + std::to_string(n_dev - plan.dropped) + " parts.");
+  run_parts(engines, plan.shards, a.src, file, a.chunk_mb << 20, a.direct_io);
+  uint64_t records = 0;
+  for (auto* e : engines) { ngsq_stats st; check(e, ngsq_get_stats(e, &st)); records += st.records; }
+  info("Processed " + std::to_string(records) + " records.");
+  write_index(dst, join_parts(engines, plan.shards));
   return 0;
 }
 
@@ -424,6 +551,7 @@ int index_main(int argc, char** argv, int i) {
     std::string s = argv[i];
     auto val = [&]() -> std::string { if (i + 1 >= argc) throw std::runtime_error("missing value for " + s); return argv[++i]; };
     if (s == "--cuda-device") a.device = std::stoi(val());
+    else if (s == "--cuda-devices") { a.devices.clear(); std::stringstream ss(val()); std::string t; while (std::getline(ss, t, ',')) a.devices.push_back(std::stoi(t)); }
     else if (s == "--cuda-no-crc") a.verify_crc = false;
     else if (s == "--cuda-chunk-mb") a.chunk_mb = std::stoull(val());
     else if (s == "--cuda-buffered-io") a.direct_io = false;
@@ -432,14 +560,18 @@ int index_main(int argc, char** argv, int i) {
   }
   if (pos.size() != 1 || !a.chunk_mb) return -1;
   a.src = pos[0];
+  if (a.devices.size() > 1) return index_bam_parts(a);
+  if (a.devices.size() == 1) a.device = a.devices[0];
   return index_bam(a);
 }
 
 void usage() {
   std::cerr << "usage: ngs-cuda-qc qc <BAM> <REFERENCE_GENOME> [-n N] [-o DIR] [-p PREFIX] [--only FACET]\n"
-               "                  [--cuda-devices 0,1,..] [--cuda-gc-seed S] [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io] [--cuda-perf]\n"
-               "       ngs-cuda-qc index <BAM> [--cuda-device N] [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io]\n"
-               "                  (writes <BAM>.bai; an existing index is never overwritten)\n";
+               "                  [--cuda-devices 0,1,..] [--cuda-build-index] [--cuda-gc-seed S] [--cuda-no-crc] [--cuda-chunk-mb M]\n"
+               "                  [--cuda-buffered-io] [--cuda-perf]\n"
+               "                  (--cuda-build-index: without <BAM>.bai, build it in the same pass and write it once the run succeeded)\n"
+               "       ngs-cuda-qc index <BAM> [--cuda-device N | --cuda-devices 0,1,..] [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io]\n"
+               "                  (writes <BAM>.bai; an existing index is never overwritten; several devices index one part of the file each)\n";
 }
 
 }  // namespace
@@ -475,12 +607,14 @@ extern "C" int ngs_cuda_qc_main(int argc, char** argv) {
       else if (s == "--cuda-no-crc") a.verify_crc = false;
       else if (s == "--cuda-chunk-mb") a.chunk_mb = std::stoull(val());
       else if (s == "--cuda-perf") a.perf = true;
+      else if (s == "--cuda-build-index") a.build_index = true;
       else if (s == "--cuda-buffered-io") a.direct_io = false;
       else if (s == "-h" || s == "--help") { usage(); return 0; }
       else if (!s.empty() && s[0] == '-' && s != "-") throw std::runtime_error("unknown flag " + s);
       else pos.push_back(s);
     }
     if (pos.size() != 2 || a.devices.empty()) { usage(); return 2; }
+    if (a.build_index && a.num_records) throw std::runtime_error("--cuda-build-index cannot be combined with -n: an index covers every record of the file");
     a.src = pos[0];
     a.reference_genome = pos[1];
     return qc(a);

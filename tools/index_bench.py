@@ -10,7 +10,16 @@ synchronise and include the host's assembly of the .bai.  The result is compared
 the same file (tests/cpp/bai_oracle.c, a restatement of the reference's `ngs index` loop over zlib; its time is the CPU
 baseline) and with bamgen's (equal up to bamgen's clamped linear index).  Prints one JSON line; --out writes it too.
 
-  python tools/index_bench.py [--records N] [--steps K] [--warmup W] [--chunk-mb M] [--no-oracle] [--out FILE]
+--gpus N measures the index of a file without an index cut between N devices instead (NGSQ_F_INDEX_PART): cuts by the
+driver's rule (targets snapped to the next block start, anchors from ngsq_find_record), one engine and one host thread per
+device, each part's compressed bytes resident on its device (resident) or streamed from pinned host memory (end to end); the
+step is the slowest thread, and the host's ngsq_join_bai is timed on its own.  The joined .bai must equal one NGSQ_F_INDEX
+engine's and the oracle's byte for byte.
+
+--driver compares the host driver on a file: `qc --cuda-build-index` (one read) against `index` then `qc` (two reads), wall
+time per command sequence, alternated.  The driver reads with O_DIRECT, so the page cache does not serve the file.
+
+  python tools/index_bench.py [--records N] [--steps K] [--warmup W] [--chunk-mb M] [--no-oracle] [--gpus N | --driver] [--out FILE]
 """
 import argparse
 import ctypes as C
@@ -39,6 +48,8 @@ def main():
     p.add_argument("--warmup", type=int, default=2)
     p.add_argument("--chunk-mb", type=int, default=256)
     p.add_argument("--no-oracle", action="store_true", help="skip the single-thread oracle index (minutes on 100 M records)")
+    p.add_argument("--gpus", type=int, default=0, help="index parts on N devices (0: the one-engine measurements)")
+    p.add_argument("--driver", action="store_true", help="qc --cuda-build-index against index + qc, from a file")
     p.add_argument("--out", default=None)
     args = p.parse_args()
 
@@ -55,6 +66,8 @@ def main():
     n_rec, C_bytes, D_bytes = info["n_records"], int(bam.size), int(info["inflated_bytes"])
     print(f"generated {n_rec} records, {C_bytes} bytes in {gen_s:.1f} s", file=sys.stderr)
 
+    if args.driver:
+        return driver_bench(args, bam, bai_writer, n_rec)
     lib = ffi.load_library()
     pin = lib.ngsq_host_alloc(C_bytes)
     pinned = np.ctypeslib.as_array(C.cast(pin, C.POINTER(C.c_uint8)), shape=(C_bytes,))
@@ -73,6 +86,9 @@ def main():
             cuts.append(acc)
     if cuts[-1] != C_bytes:
         cuts.append(C_bytes)
+
+    if args.gpus:
+        return parts_bench(args, pinned, pin, blocks, n_blocks, n_rec, C_bytes, D_bytes, d_comp, lib)
 
     def engine(flags):
         e = ffi.Engine(flags=flags, gc_seed=bench.GC_SEED, reserve_compressed=C_bytes, reserve_inflated=D_bytes + 65536, reserve_blocks=n_blocks + 16)
@@ -165,6 +181,188 @@ def main():
     lib.ngsq_host_free(pin)
     if not out["equal_to_bamgen_up_to_its_linear_clamp"] or out.get("equal_to_oracle") is False:
         raise SystemExit("the GPU index differs from the reference indexes")
+
+
+def _emit(args, out):
+    line = json.dumps(out)
+    print(line)
+    if args.out:
+        with open(args.out, "w") as f:
+            f.write(line + "\n")
+
+
+def parts_bench(args, pinned, pin, blocks, n_blocks, n_rec, C_bytes, D_bytes, d_comp_0, lib):
+    import threading
+
+    import torch
+    from ngs_b200 import ffi, formats
+    from baiutil import oracle_bai
+    n = args.gpus
+    if torch.cuda.device_count() < n:
+        raise SystemExit(f"--gpus {n}: only {torch.cuda.device_count()} device(s) visible")
+    crc = ffi.NGSQ_F_VERIFY_CRC
+    starts = [blocks[i].coffset for i in range(n_blocks)]
+    whole = ffi.Engine(0, flags=ffi.NGSQ_F_INDEX | crc, reserve_compressed=C_bytes, reserve_inflated=D_bytes + 65536, reserve_blocks=n_blocks + 16)
+    hdr = formats.read_header(whole, pinned)
+    lens = [l for _, l in hdr.refs]
+    whole.set_references(lens, [0] * len(lens))
+    whole.set_range(hdr.first_voffset, 0)
+    whole.submit_device(d_comp_0.data_ptr(), C_bytes, blocks, n_blocks)
+    whole.finish()
+    one_bai = whole.bai()
+    whole.close()
+    # cuts by the driver's rule
+    t = time.perf_counter()
+    finder = ffi.Engine(0, flags=ffi.NGSQ_F_INDEX_PART)
+    finder.set_references(lens, [0] * len(lens))
+    base = hdr.first_voffset >> 16
+    bounds = [hdr.first_voffset]
+    for k in range(1, n):
+        target = base + (C_bytes - base) * k // n
+        i = int(np.searchsorted(np.asarray(starts, dtype=np.uint64), target))
+        nb = 4
+        v = 0
+        while i < n_blocks and nb <= 4096:
+            j = min(n_blocks, i + nb)
+            hi = blocks[j - 1].coffset + blocks[j - 1].csize
+            v, _ = finder.find_record(np.ascontiguousarray(pinned[starts[i]:hi]), starts[i])
+            if v or j == n_blocks:
+                break
+            nb *= 2
+        if v and v > bounds[-1]:
+            bounds.append(v)
+    finder.close()
+    plan_ms = (time.perf_counter() - t) * 1e3
+    ranges = []
+    for k, first in enumerate(bounds):
+        end = bounds[k + 1] if k + 1 < len(bounds) else 0
+        lo, hi = formats.shard_byte_range(formats.Shard(first, end, []), blocks, n_blocks, C_bytes)
+        ranges.append((first, end, lo, hi))
+    del d_comp_0
+    torch.cuda.empty_cache()
+    engines, dev = [], []
+    for k, (first, end, lo, hi) in enumerate(ranges):
+        b0 = int(np.searchsorted(np.asarray(starts, dtype=np.uint64), lo))
+        b1 = int(np.searchsorted(np.asarray(starts, dtype=np.uint64), hi)) if hi < C_bytes else n_blocks
+        with torch.cuda.device(k):
+            d = torch.empty(hi - lo + 512, dtype=torch.uint8, device=f"cuda:{k}")
+            d[: hi - lo].copy_(torch.from_numpy(pinned[lo:hi]))
+        sub = (ffi.Block * (b1 - b0))(*[blocks[i] for i in range(b0, b1)])
+        e = ffi.Engine(k, flags=ffi.NGSQ_F_INDEX_PART | crc, reserve_compressed=hi - lo, reserve_inflated=D_bytes // len(ranges) * 2 + 65536,
+                       reserve_blocks=b1 - b0 + 16)
+        e.set_references(lens, [0] * len(lens))
+        engines.append(e)
+        dev.append((d, sub, b1 - b0))
+    torch.cuda.synchronize()
+
+    def step(mode):
+        times = [None] * len(engines)
+
+        def run(k):
+            e, (first, end, lo, hi), (d, sub, nb) = engines[k], ranges[k], dev[k]
+            t0 = time.perf_counter()
+            e.reset()
+            e.set_range(first, end)
+            if mode == "resident":
+                e.submit_device(d.data_ptr(), hi - lo, sub, nb)
+            else:
+                a = lo
+                while a < hi:
+                    b = min(hi, a + (args.chunk_mb << 20))
+                    if b < hi:  # whole blocks per chunk
+                        b = int(starts_np[int(np.searchsorted(starts_np, b))])
+                    e.submit_ptr(pin + a, b - a, a)
+                    a = b
+            e.finish()
+            times[k] = ((time.perf_counter() - t0) * 1e3, e.stats()["ms_total"])
+        ts = [threading.Thread(target=run, args=(k,)) for k in range(len(engines))]
+        t0 = time.perf_counter()
+        for x in ts:
+            x.start()
+        for x in ts:
+            x.join()
+        wall = (time.perf_counter() - t0) * 1e3
+        t1 = time.perf_counter()
+        bai = ffi.join_bai(engines)
+        join_ms = (time.perf_counter() - t1) * 1e3
+        return wall, max(tt[1] for tt in times), join_ms, bai
+
+    starts_np = np.asarray(starts, dtype=np.int64)
+    for _ in range(args.warmup):
+        step("resident")
+    res = [step("resident") for _ in range(args.steps)]
+    for _ in range(max(1, args.warmup // 2)):
+        step("e2e")
+    ee = [step("e2e") for _ in range(args.steps)]
+    joined = res[-1][3]
+    assert all(r[3] == joined for r in res + ee)
+    med = lambda xs: float(np.median(xs))  # noqa: E731
+    out = {
+        "metric": "BAI build of a file without an index cut between devices (NGSQ_F_INDEX_PART + ngsq_join_bai)", "gpus": n,
+        "parts": len(ranges), "records": n_rec, "compressed_bytes": C_bytes, "steps": args.steps, "warmup": args.warmup, "gpu": gpu_name_and_power(),
+        "plan_ms_host": plan_ms,
+        "index_resident_ms_device_slowest_part": med([r[1] for r in res]), "index_resident_ms_wall_parts": med([r[0] for r in res]),
+        "index_e2e_ms_device_slowest_part": med([r[1] for r in ee]), "index_e2e_ms_wall_parts": med([r[0] for r in ee]), "e2e_chunk_mb": args.chunk_mb,
+        "join_ms_host": med([r[2] for r in res + ee]),
+        "index_resident_ms_wall_with_join": med([r[0] + r[2] for r in res]),
+        "index_e2e_ms_wall_with_join": med([r[0] + r[2] for r in ee]),
+        "equal_to_one_engine": joined == one_bai, "bai_bytes": len(joined),
+    }
+    if not args.no_oracle:
+        out["equal_to_oracle"] = oracle_bai(pinned) == joined
+    _emit(args, out)
+    for e in engines:
+        e.close()
+    lib.ngsq_host_free(pin)
+    if not out["equal_to_one_engine"] or out.get("equal_to_oracle") is False:
+        raise SystemExit("the joined index differs from one engine's or the oracle's")
+
+
+def driver_bench(args, bam, bai_writer, n_rec):
+    import shutil
+    import tempfile
+    from baiutil import oracle_bai  # noqa: F401
+    drv = os.path.join(ROOT, "ngs_b200", "ngs-cuda-qc")
+    d = tempfile.mkdtemp(prefix="index_bench_")
+    try:
+        src = os.path.join(d, "w.bam")
+        bam.tofile(src)
+        del bam
+
+        def run(cmd):
+            r = subprocess.run([drv] + cmd, capture_output=True, text=True)
+            if r.returncode:
+                raise SystemExit(r.stderr)
+
+        def two():
+            os.remove(src + ".bai") if os.path.exists(src + ".bai") else None
+            t = time.perf_counter()
+            run(["index", src])
+            run(["qc", src, "GRCh38_no_alt_AnalysisSet", "-o", d, "-p", "two"])
+            return (time.perf_counter() - t) * 1e3
+
+        def one():
+            os.remove(src + ".bai") if os.path.exists(src + ".bai") else None
+            t = time.perf_counter()
+            run(["qc", src, "GRCh38_no_alt_AnalysisSet", "-o", d, "-p", "one", "--cuda-build-index"])
+            return (time.perf_counter() - t) * 1e3
+
+        for _ in range(args.warmup):
+            two()
+            one()
+        a, b = [], []
+        for _ in range(args.steps):  # alternated
+            a.append(two())
+            b.append(one())
+        same = open(os.path.join(d, "one.results.json")).read() == open(os.path.join(d, "two.results.json")).read()
+        med = lambda xs: float(np.median(xs))  # noqa: E731
+        out = {"metric": "host driver wall time from a file, qc --cuda-build-index vs index + qc", "records": n_rec, "steps": args.steps,
+               "gpu": gpu_name_and_power(), "io": "O_DIRECT reads (the page cache does not serve the BAM)",
+               "index_then_qc_ms_wall": med(a), "qc_build_index_ms_wall": med(b), "all_index_then_qc_ms": a, "all_qc_build_index_ms": b,
+               "same_results_json": same}
+        _emit(args, out)
+    finally:
+        shutil.rmtree(d, ignore_errors=True)
 
 
 if __name__ == "__main__":
