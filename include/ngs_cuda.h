@@ -76,6 +76,10 @@ enum {
                                    allowed.  ngsq_finish keeps the part's index state on the host without assembling it, and does not
                                    check the order (it is checked across the parts by the join); ngsq_get_bai is refused: join the
                                    finished parts with ngsq_join_bai. */
+#define NGSQ_F_INDEX_CSI 256u  /* with NGSQ_F_INDEX or NGSQ_F_INDEX_PART: build a CSI instead of a BAI (alone: NGSQ_E_ARG).  Bins are
+                                   CSIv1's hts_reg2bin(beg, end, min_shift, depth) (ngsq_set_index_binning; default min_shift 14 and
+                                   samtools' depth rule), records may end at most at 2^(min_shift + 3 depth) and references may be at
+                                   most that long.  Read the bytes with ngsq_get_csi, join parts with ngsq_join_csi. */
 
 typedef struct ngsq_engine ngsq_engine;
 
@@ -240,6 +244,14 @@ int ngsq_get_stats(ngsq_engine* e, ngsq_stats* out);
  * n_no_coor) of the records submitted since ngsq_set_range.  After ngsq_finish.  *n_out = its size; out = NULL with cap = 0
  * asks for the size only.  DESIGN.md section 4 (K13) lists where its bytes may differ from samtools' index of the same file. */
 int ngsq_get_bai(ngsq_engine* e, uint8_t* out, size_t cap, size_t* n_out);
+/* NGSQ_F_INDEX_CSI: the binning of the CSI.  min_shift in [12, 24] (windows of 2^min_shift bases); depth in [1, 7], or 0 for
+ * the rule of `samtools index -c`: the smallest depth n with (longest reference + 256) <= 2^(min_shift + 3n).  Optional (default
+ * 14, 0); before ngsq_set_references, which resolves the depth; kept across ngsq_reset. */
+int ngsq_set_index_binning(ngsq_engine* e, uint32_t min_shift, uint32_t depth);
+/* NGSQ_F_INDEX | NGSQ_F_INDEX_CSI: the .csi payload, UNCOMPRESSED ("CSI\1", min_shift, depth, l_aux = 0, n_ref; per reference
+ * its bins with loffset and chunks and the pseudo-bin n_bins + 1; n_no_coor): the file on disk is this payload BGZF-compressed
+ * by the caller.  Conventions of ngsq_get_bai; each of the two refuses an engine of the other format. */
+int ngsq_get_csi(ngsq_engine* e, uint8_t* out, size_t cap, size_t* n_out);
 
 /* ---- a BAM without an index cut between engines (DESIGN.md sections 4 K13 and 5) ----
  * Record anchor finder: `bgzf` holds whole BGZF blocks starting at file offset `file_off`.  They are inflated on the device
@@ -257,6 +269,10 @@ int ngsq_find_record(ngsq_engine* e, const uint8_t* bgzf, size_t nbytes, uint64_
  * the size; out = NULL with cap = 0 asks for the size only.  The message of a failure is ngsq_last_error(parts[0]) (of NULL
  * when parts is NULL or n is 0). */
 int ngsq_join_bai(ngsq_engine* const* parts, uint32_t n, uint8_t* out, size_t cap, size_t* n_out);
+/* The same for NGSQ_F_INDEX_PART | NGSQ_F_INDEX_CSI parts: the uncompressed .csi one NGSQ_F_INDEX | NGSQ_F_INDEX_CSI engine
+ * gives.  Every part must also have the same binning (NGSQ_E_ARG otherwise); BAI parts are refused here, CSI parts by
+ * ngsq_join_bai. */
+int ngsq_join_csi(ngsq_engine* const* parts, uint32_t n, uint8_t* out, size_t cap, size_t* n_out);
 
 /* ---- multi-GPU merge: one sum-reduce of the packed u64 result buffer ---- */
 int ngsq_nccl_unique_id(char out[128]);

@@ -99,6 +99,8 @@ pub mod sys {
     pub const NGSQ_F_INDEX: u32 = 64;
     /// index one range of a file cut between engines (set instead of NGSQ_F_INDEX); join the parts with ngsq_join_bai
     pub const NGSQ_F_INDEX_PART: u32 = 128;
+    /// with NGSQ_F_INDEX / NGSQ_F_INDEX_PART: a CSI instead of a BAI (ngsq_get_csi, ngsq_join_csi)
+    pub const NGSQ_F_INDEX_CSI: u32 = 256;
     pub const NGSQ_E_UNSORTED: c_int = -14;
 
     /// Device arrays of a reference split between shards (`struct ngsq_split_arrays`); null pointers for facets that are off.
@@ -160,6 +162,9 @@ pub mod sys {
         pub fn ngsq_resolve_split(e: *mut NgsqEngine, is_root: c_int) -> c_int;
         pub fn ngsq_find_record(e: *mut NgsqEngine, bgzf: *const u8, nbytes: usize, file_off: u64, voffset: *mut u64, ref_id: *mut i32) -> c_int;
         pub fn ngsq_join_bai(parts: *const *mut NgsqEngine, n: u32, out: *mut u8, cap: usize, n_out: *mut usize) -> c_int;
+        pub fn ngsq_set_index_binning(e: *mut NgsqEngine, min_shift: u32, depth: u32) -> c_int;
+        pub fn ngsq_get_csi(e: *mut NgsqEngine, out: *mut u8, cap: usize, n_out: *mut usize) -> c_int;
+        pub fn ngsq_join_csi(parts: *const *mut NgsqEngine, n: u32, out: *mut u8, cap: usize, n_out: *mut usize) -> c_int;
     }
 }
 
@@ -343,6 +348,40 @@ impl Engine {
         Ok(out)
     }
 
+    /// An engine that builds the CSI of a whole coordinate-sorted BAM (NGSQ_F_INDEX | NGSQ_F_INDEX_CSI) at `min_shift`, the
+    /// depth by samtools' rule.
+    pub fn create_csi_indexer(device: i32, min_shift: u32) -> anyhow::Result<Self> {
+        let cfg = sys::NgsqConfig {
+            struct_size: std::mem::size_of::<sys::NgsqConfig>() as u32,
+            flags: sys::NGSQ_F_INDEX | sys::NGSQ_F_INDEX_CSI | sys::NGSQ_F_VERIFY_CRC,
+            ..Default::default()
+        };
+        let mut raw = std::ptr::null_mut();
+        let rc = unsafe { sys::ngsq_create(device as c_int, &cfg, &mut raw) };
+        if rc != 0 {
+            let msg = unsafe { CStr::from_ptr(sys::ngsq_last_error(std::ptr::null_mut())) }.to_string_lossy().into_owned();
+            bail!("ngs-cuda: {}", msg);
+        }
+        let mut e = Self { raw, submits: 0 };
+        e.check(unsafe { sys::ngsq_set_index_binning(e.raw, min_shift, 0) })?;
+        Ok(e)
+    }
+
+    /// The UNCOMPRESSED `.csi` payload of the BAM at `path` (an engine of `create_csi_indexer`); the file on disk is its BGZF
+    /// compression.  Arguments and refusals as `build_bai`, with the CSI's limit 2^(min_shift + 3 depth).
+    pub fn build_csi(&mut self, path: &Path, lengths: &[u32], first_record: u64, chunk_bytes: usize, on_progress: impl FnMut(u64)) -> anyhow::Result<Vec<u8>> {
+        self.set_references(lengths, &vec![false; lengths.len()])?;
+        self.set_range(first_record, 0)?;
+        let size = std::fs::metadata(path)?.len();
+        self.stream_file(path, first_record >> 16, size, chunk_bytes, on_progress)?;
+        self.finish()?;
+        let mut n = 0usize;
+        self.check(unsafe { sys::ngsq_get_csi(self.raw, std::ptr::null_mut(), 0, &mut n) })?;
+        let mut out = vec![0u8; n];
+        self.check(unsafe { sys::ngsq_get_csi(self.raw, out.as_mut_ptr(), out.len(), &mut n) })?;
+        Ok(out)
+    }
+
     /// An engine that indexes one range of a file cut between engines (NGSQ_F_INDEX_PART beside `flags`, e.g. the qc flags);
     /// its part is joined with the others by `join_bai` after `finish`.
     pub fn create_index_part(device: i32, flags: u32) -> anyhow::Result<Self> {
@@ -520,6 +559,20 @@ pub fn join_bai(parts: &[&Engine]) -> anyhow::Result<Vec<u8>> {
     parts[0].check(unsafe { sys::ngsq_join_bai(raws.as_ptr(), raws.len() as u32, std::ptr::null_mut(), 0, &mut n) })?;
     let mut out = vec![0u8; n];
     parts[0].check(unsafe { sys::ngsq_join_bai(raws.as_ptr(), raws.len() as u32, out.as_mut_ptr(), out.len(), &mut n) })?;
+    Ok(out)
+}
+
+/// The uncompressed `.csi` of a file from its finished NGSQ_F_INDEX_PART | NGSQ_F_INDEX_CSI engines, in file order
+/// (ngsq_join_csi; every part must have the same binning).
+pub fn join_csi(parts: &[&Engine]) -> anyhow::Result<Vec<u8>> {
+    if parts.is_empty() {
+        bail!("ngs-cuda: join_csi needs at least one part");
+    }
+    let raws: Vec<*mut sys::NgsqEngine> = parts.iter().map(|e| e.raw).collect();
+    let mut n = 0usize;
+    parts[0].check(unsafe { sys::ngsq_join_csi(raws.as_ptr(), raws.len() as u32, std::ptr::null_mut(), 0, &mut n) })?;
+    let mut out = vec![0u8; n];
+    parts[0].check(unsafe { sys::ngsq_join_csi(raws.as_ptr(), raws.len() as u32, out.as_mut_ptr(), out.len(), &mut n) })?;
     Ok(out)
 }
 

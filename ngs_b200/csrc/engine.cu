@@ -77,11 +77,12 @@ bool load_nccl(std::string& err) {
 }  // namespace
 
 // NGSQ_F_INDEX / NGSQ_F_INDEX_PART: an engine's index state on the host once its last wave is done.  Every part is linear or
-// order-free, so the state of parts cut from one file joins exactly (ngsq_join_bai): runs and overflow lists concatenate,
-// windows take the minimum, maxw the maximum, counts and n_no_coor add up.
+// order-free, so the state of parts cut from one file joins exactly (ngsq_join_bai / ngsq_join_csi): runs and overflow lists
+// concatenate, windows take the minimum, maxw the maximum, counts and n_no_coor add up.
 struct IxHost {
   IndexState S{};
-  std::vector<IndexRun> runs, ovf;  // runs in any order (assemble_bai sorts them)
+  std::vector<IndexRun> runs;       // in any order (ix_collect sorts them)
+  std::vector<IndexOvf> ovf;        // the overflow list, BAI entries unpacked
   std::vector<uint64_t> win, counts;
   std::vector<uint32_t> maxw;
   uint64_t last_order_key = 0;      // of the part's last record that constrains the order (0 = none)
@@ -207,7 +208,7 @@ struct ngsq_engine {
   IndexState* d_ix = nullptr;
   IndexRun* d_ix_runs[2] = {nullptr, nullptr};
   uint64_t ix_runs_cap = 0;
-  IndexRun* d_ix_ovf = nullptr;
+  void* d_ix_ovf = nullptr;          // IndexRun entries (BAI) or IndexOvf entries (CSI)
   uint64_t* d_ix_win_base = nullptr;
   uint32_t* d_ix_win_n = nullptr;
   unsigned long long* d_ix_win = nullptr;
@@ -221,8 +222,11 @@ struct ngsq_engine {
   std::vector<IxWave> ix_waves;
   std::vector<std::pair<const IndexRun*, uint64_t>> ix_drained;  // pinned copies of drained run tables
   uint64_t data_end_coff = 0;        // end of the last non-empty block submitted (the offset after the last record)
-  std::vector<uint8_t> bai;
-  IxHost ix;                         // NGSQ_F_INDEX_PART: the part's state for ngsq_join_bai
+  std::vector<uint8_t> ix_bytes;     // the .bai, or the uncompressed .csi (NGSQ_F_INDEX_CSI)
+  IxHost ix;                         // NGSQ_F_INDEX_PART: the part's state for ngsq_join_bai / ngsq_join_csi
+  // NGSQ_F_INDEX_CSI: the binning asked for (ngsq_set_index_binning; depth 0 = samtools' rule) and the one in use, resolved
+  // by ngsq_set_references from the longest reference; kept across ngsq_reset
+  uint32_t ix_min_shift = kIxWindowShift, ix_depth_req = 0, ix_depth = 5;
   bool ix_part_ok = false;           // ... valid: ngsq_finish succeeded
 
   // references split between shards (ngsq_split_reference): scattered as usual, resolved only by the merge
@@ -274,6 +278,8 @@ uint32_t wave_blocks(const ngsq_engine* e) { return (uint32_t)e->n_sm * kDecThre
 
 // the K13 index pass runs: a whole file (NGSQ_F_INDEX) or one part of it (NGSQ_F_INDEX_PART)
 bool ix_on(const ngsq_engine* e) { return e->cfg.flags & (NGSQ_F_INDEX | NGSQ_F_INDEX_PART); }
+// ... and builds a CSI instead of a BAI
+bool ix_csi(const ngsq_engine* e) { return e->cfg.flags & NGSQ_F_INDEX_CSI; }
 
 uint32_t launch_quantum(const ngsq_engine* e) {
   // One wave = one block per decoder lane: a launch takes about one block-decode latency whatever its size (every
@@ -790,9 +796,11 @@ int launch_wave(ngsq_engine* e, uint32_t b0, uint32_t b1, bool final_wave) {
     X.ovf = e->d_ix_ovf; X.ovf_cap = kIndexOverflowCap;
     X.win_base = e->d_ix_win_base; X.win_n = e->d_ix_win_n; X.win = e->d_ix_win; X.max_win = e->d_ix_maxw; X.counts = e->d_ix_counts;
     X.part = (e->cfg.flags & NGSQ_F_INDEX_PART) ? 1u : 0u;
+    X.min_shift = e->ix_min_shift; X.depth = e->ix_depth;
     const uint32_t per_cta = 31 * (kIndexThreads / 32);
     const uint32_t xgrid = (uint32_t)std::min<uint64_t>((bytes / 36 + 2 + per_cta - 1) / per_cta, (uint64_t)e->n_sm * 8);
-    index_kernel<<<xgrid, kIndexThreads, 0, st>>>(X);
+    if (ix_csi(e)) index_kernel<true><<<xgrid, kIndexThreads, 0, st>>>(X);
+    else index_kernel<false><<<xgrid, kIndexThreads, 0, st>>>(X);
     CU(cudaGetLastError());
     e->other_launches++;
     CU(cudaMemcpyAsync(e->h_ix_probe + par, &e->d_ix->n_runs[par], 8, cudaMemcpyDeviceToHost, st));
@@ -868,28 +876,31 @@ int acquire_comp(ngsq_engine* e, size_t nbytes, uint8_t** dst) {
   return NGSQ_OK;
 }
 
-// K13 on the host: runs -> chunks per (reference, bin), the linear index, the .bai bytes of the state H (one engine's, or the
-// join of several parts').  Sorts H.runs.
-void assemble_bai(IxHost& H, uint32_t nr, const std::vector<uint64_t>& win_base, const std::vector<uint32_t>& win_n, std::vector<uint8_t>& b) {
+// K13 on the host, the part a BAI and a CSI share: runs -> chunks per (reference, bin), merged where they touch, bins in order
+// of first use; the per-window minimum offsets, untouched windows filled with the previous window's value (0 before the
+// first touched one).  For the state H (one engine's, or the join of several parts').  Sorts H.runs.
+struct IxRef {
+  std::vector<std::pair<uint32_t, std::vector<std::pair<uint64_t, uint64_t>>>> bins;  // in order of first use
+  uint64_t beg = 0, end = 0;
+  bool any = false;
+  std::vector<uint64_t> win;  // windows 0 ..= the last touched one, filled
+};
+size_t ix_collect(IxHost& H, uint32_t nr, uint32_t n_bins, const std::vector<uint64_t>& win_base, const std::vector<uint32_t>& win_n,
+                  std::vector<IxRef>& refs) {
   std::vector<IndexRun>& runs = H.runs;
   // runs were ticketed in any order; each starts at a distinct record, and run r ends where run r + 1 starts
   std::sort(runs.begin(), runs.end(), [](const IndexRun& a, const IndexRun& b) { return a.voff < b.voff; });
-  struct Ref {
-    std::vector<std::pair<uint32_t, std::vector<std::pair<uint64_t, uint64_t>>>> bins;  // in order of first use
-    uint64_t beg = 0, end = 0;
-    bool any = false;
-  };
-  std::vector<Ref> refs(nr);
+  refs.assign(nr, IxRef{});
   const uint64_t data_end = H.data_end;
   // the runs of one reference are consecutive (sorted input): one bin -> slot table, cleared when the reference changes
-  std::vector<int32_t> slot_of(kIxMetaBin, -1);
+  std::vector<int32_t> slot_of(n_bins + 1, -1);
   uint32_t cur = kIxUnplacedRef;
   size_t chunks = 0;
   for (size_t i = 0; i < runs.size(); ++i) {
     const IndexRun& u = runs[i];
     if (u.ref == kIxUnplacedRef) continue;
     const uint64_t end = i + 1 < runs.size() ? runs[i + 1].voff : data_end;
-    Ref& R = refs[u.ref];
+    IxRef& R = refs[u.ref];
     if (u.ref != cur) {
       if (cur != kIxUnplacedRef) for (auto& bn : refs[cur].bins) slot_of[bn.first] = -1;
       cur = u.ref;
@@ -903,16 +914,39 @@ void assemble_bai(IxHost& H, uint32_t nr, const std::vector<uint64_t>& win_base,
     if (!ch.empty() && ch.back().second == u.voff) ch.back().second = end;
     else { ch.push_back({u.voff, end}); ++chunks; }
   }
-  const uint64_t win_total = H.win.size();
+  for (uint32_t c = 0; c < nr; ++c) {
+    IxRef& R = refs[c];
+    if (!R.any) continue;
+    const uint32_t n_intv = H.maxw[c] + 1;
+    std::vector<uint64_t>& lin = R.win;
+    lin.assign(n_intv, ~0ull);
+    const uint32_t in_table = std::min(n_intv, win_n[c]);
+    for (uint32_t w = 0; w < in_table; ++w) lin[w] = H.win[win_base[c] + w];
+    for (const IndexOvf& o : H.ovf)
+      if (o.ref == c)
+        for (uint32_t w = o.lo; w <= o.hi && w < n_intv; ++w) lin[w] = std::min(lin[w], o.voff);
+    uint64_t last = 0;
+    for (uint32_t w = 0; w < n_intv; ++w) {
+      if (lin[w] == ~0ull) lin[w] = last; else last = lin[w];
+    }
+  }
+  return chunks;
+}
+
+// The .bai bytes: per reference its bins and chunks, the pseudo-bin 37450 and the linear index; n_no_coor.
+void assemble_bai(IxHost& H, uint32_t nr, const std::vector<uint64_t>& win_base, const std::vector<uint32_t>& win_n, std::vector<uint8_t>& b) {
+  std::vector<IxRef> refs;
+  const size_t chunks = ix_collect(H, nr, kIxMetaBin - 1, win_base, win_n, refs);
+  size_t wins = 0;
+  for (const IxRef& R : refs) wins += R.win.size();
   b.clear();
-  b.reserve(16 + (size_t)nr * 64 + chunks * 16 + ((win_total + H.ovf.size()) * 8));
+  b.reserve(16 + (size_t)nr * 64 + chunks * 16 + wins * 8);
   auto p32 = [&](uint32_t v) { uint8_t t[4]; memcpy(t, &v, 4); b.insert(b.end(), t, t + 4); };
   auto p64 = [&](uint64_t v) { uint8_t t[8]; memcpy(t, &v, 8); b.insert(b.end(), t, t + 8); };
   b.insert(b.end(), {'B', 'A', 'I', 1});
   p32(nr);
-  std::vector<uint64_t> lin;
   for (uint32_t c = 0; c < nr; ++c) {
-    const Ref& R = refs[c];
+    const IxRef& R = refs[c];
     if (!R.any) { p32(0); p32(0); continue; }
     p32((uint32_t)R.bins.size() + 1);
     for (auto& bn : R.bins) {
@@ -921,22 +955,48 @@ void assemble_bai(IxHost& H, uint32_t nr, const std::vector<uint64_t>& win_base,
       for (auto& ck : bn.second) { p64(ck.first); p64(ck.second); }
     }
     p32(kIxMetaBin); p32(2); p64(R.beg); p64(R.end); p64(H.counts[2 * c]); p64(H.counts[2 * c + 1]);
-    // windows nobody touched take the previous window's value (0 before the first touched one)
-    const uint32_t n_intv = H.maxw[c] + 1;
-    lin.assign(n_intv, ~0ull);
-    const uint32_t in_table = std::min(n_intv, win_n[c]);
-    for (uint32_t w = 0; w < in_table; ++w) lin[w] = H.win[win_base[c] + w];
-    for (const IndexRun& o : H.ovf)
-      if (o.ref == c)
-        for (uint32_t w = o.bin & 0xFFFF; w <= (o.bin >> 16) && w < n_intv; ++w) lin[w] = std::min(lin[w], o.voff);
-    uint64_t last = 0;
-    for (uint32_t w = 0; w < n_intv; ++w) {
-      if (lin[w] == ~0ull) lin[w] = last; else last = lin[w];
-    }
-    p32(n_intv);
-    for (uint64_t v : lin) p64(v);
+    p32((uint32_t)R.win.size());
+    for (uint64_t v : R.win) p64(v);
   }
   p64(H.S.n_no_coor);
+}
+
+// The .csi payload (CSIv1, uncompressed): magic, min_shift, depth, l_aux = 0, n_ref; per reference its bins, each with its
+// loffset (the filled window minimum at the bin's first leaf window, 0 past the last touched window) and chunks, then the
+// pseudo-bin n_bins + 1 with loffset 0; n_no_coor.  No linear index.
+void assemble_csi(IxHost& H, uint32_t nr, uint32_t min_shift, uint32_t depth, const std::vector<uint64_t>& win_base,
+                  const std::vector<uint32_t>& win_n, std::vector<uint8_t>& b) {
+  std::vector<IxRef> refs;
+  const uint32_t n_bins = ix_csi_n_bins(depth);
+  const size_t chunks = ix_collect(H, nr, n_bins, win_base, win_n, refs);
+  size_t bins = 0;
+  for (const IxRef& R : refs) bins += R.bins.size();
+  b.clear();
+  b.reserve(24 + (size_t)nr * 64 + chunks * 16 + bins * 16);
+  auto p32 = [&](uint32_t v) { uint8_t t[4]; memcpy(t, &v, 4); b.insert(b.end(), t, t + 4); };
+  auto p64 = [&](uint64_t v) { uint8_t t[8]; memcpy(t, &v, 8); b.insert(b.end(), t, t + 8); };
+  b.insert(b.end(), {'C', 'S', 'I', 1});
+  p32(min_shift); p32(depth); p32(0); p32(nr);
+  for (uint32_t c = 0; c < nr; ++c) {
+    const IxRef& R = refs[c];
+    if (!R.any) { p32(0); continue; }
+    p32((uint32_t)R.bins.size() + 1);
+    for (auto& bn : R.bins) {
+      const uint64_t bot = ix_csi_bin_bot(bn.first, depth);
+      p32(bn.first);
+      p64(bot < R.win.size() ? R.win[bot] : 0);
+      p32((uint32_t)bn.second.size());
+      for (auto& ck : bn.second) { p64(ck.first); p64(ck.second); }
+    }
+    p32(n_bins + 1); p64(0); p32(2); p64(R.beg); p64(R.end); p64(H.counts[2 * c]); p64(H.counts[2 * c + 1]);
+  }
+  p64(H.S.n_no_coor);
+}
+
+// the index bytes of the state H in the engine's format
+void assemble_index(const ngsq_engine* e, IxHost& H, std::vector<uint8_t>& b) {
+  if (ix_csi(e)) assemble_csi(H, e->n_ref, e->ix_min_shift, e->ix_depth, e->ix_win_base, e->ix_win_n, b);
+  else assemble_bai(H, e->n_ref, e->ix_win_base, e->ix_win_n, b);
 }
 
 int fail_unsorted(ngsq_engine* e, uint64_t voff) {
@@ -958,6 +1018,9 @@ int finish_index(ngsq_engine* e) {
   IndexState& S = H.S;
   CU(cudaMemcpy(&S, e->d_ix, sizeof S, cudaMemcpyDeviceToHost));
   if (S.err & kIxBadRecord) return fail(e, NGSQ_E_BAD_RECORD, "malformed BAM record (field overrun, CIGAR op > 8 or reference id out of range)");
+  if ((S.err & kIxTooLong) && ix_csi(e))
+    return fail(e, NGSQ_E_BAD_RECORD, "a record ends beyond position 2^%u, which a CSI of min_shift %u and depth %u cannot address",
+                e->ix_min_shift + 3 * e->ix_depth, e->ix_min_shift, e->ix_depth);
   if (S.err & kIxTooLong) return fail(e, NGSQ_E_BAD_RECORD, "a record ends beyond position 2^29, which a BAI cannot address (CSI can)");
   if (S.err & kIxRunTable) return fail(e, NGSQ_E_CHAIN, "index run table overflow");
   if (S.err & kIxOverflowList)
@@ -973,13 +1036,19 @@ int finish_index(ngsq_engine* e) {
     CU(cudaMemcpy(H.counts.data(), e->d_ix_counts, (size_t)nr * 16, cudaMemcpyDeviceToHost));
     CU(cudaMemcpy(H.maxw.data(), e->d_ix_maxw, (size_t)nr * 4, cudaMemcpyDeviceToHost));
   }
-  H.ovf.resize(std::min<uint64_t>(S.n_ovf, kIndexOverflowCap));
-  if (!H.ovf.empty()) CU(cudaMemcpy(H.ovf.data(), e->d_ix_ovf, H.ovf.size() * sizeof(IndexRun), cudaMemcpyDeviceToHost));
+  const size_t n_ovf = std::min<uint64_t>(S.n_ovf, kIndexOverflowCap);
+  H.ovf.resize(n_ovf);
+  if (n_ovf && ix_csi(e)) CU(cudaMemcpy(H.ovf.data(), e->d_ix_ovf, n_ovf * sizeof(IndexOvf), cudaMemcpyDeviceToHost));
+  else if (n_ovf) {
+    std::vector<IndexRun> packed(n_ovf);
+    CU(cudaMemcpy(packed.data(), e->d_ix_ovf, n_ovf * sizeof(IndexRun), cudaMemcpyDeviceToHost));
+    for (size_t i = 0; i < n_ovf; ++i) H.ovf[i] = IndexOvf{packed[i].voff, packed[i].ref, packed[i].bin & 0xFFFF, packed[i].bin >> 16, 0};
+  }
   for (auto& d : e->ix_drained) H.runs.insert(H.runs.end(), d.first, d.first + d.second);
   H.last_order_key = S.carry[e->ix_waves.size() & 1].order_key;  // the carry the last indexed wave wrote
   H.data_end = e->data_end_coff << 16;
   if (part) { e->ix_part_ok = true; return NGSQ_OK; }
-  assemble_bai(H, nr, e->ix_win_base, e->ix_win_n, e->bai);
+  assemble_index(e, H, e->ix_bytes);
   H = IxHost{};
   return NGSQ_OK;
 }
@@ -1118,6 +1187,8 @@ int ngsq_create(int device, const ngsq_config* cfg, ngsq_engine** out) {
   if (device < 0 || device >= n_dev) return fail(e, NGSQ_E_ARG, "device %d out of range (%d devices)", device, n_dev);
   if (cfg && (cfg->flags & NGSQ_F_INDEX) && (cfg->flags & NGSQ_F_INDEX_PART))
     return fail(e, NGSQ_E_ARG, "NGSQ_F_INDEX_PART is set instead of NGSQ_F_INDEX, not with it");
+  if (cfg && (cfg->flags & NGSQ_F_INDEX_CSI) && !(cfg->flags & (NGSQ_F_INDEX | NGSQ_F_INDEX_PART)))
+    return fail(e, NGSQ_E_ARG, "NGSQ_F_INDEX_CSI selects the format of NGSQ_F_INDEX or NGSQ_F_INDEX_PART: set one of them with it");
   if (cfg && (cfg->flags & (NGSQ_F_INDEX | NGSQ_F_INDEX_PART)) && cfg->max_records)
     return fail(e, NGSQ_E_ARG, "NGSQ_F_INDEX cannot be combined with max_records: an index covers every record of the file");
   ngsq_engine* ne = new ngsq_engine();
@@ -1151,7 +1222,7 @@ int ngsq_create(int device, const ngsq_config* cfg, ngsq_engine** out) {
   CUC(cudaHostAlloc((void**)&e->h_prog, kProgSlots * 16, cudaHostAllocDefault));
   if (ix_on(e)) {
     CUC(cudaMalloc(&e->d_ix, sizeof(IndexState)));
-    CUC(cudaMalloc(&e->d_ix_ovf, kIndexOverflowCap * sizeof(IndexRun)));
+    CUC(cudaMalloc(&e->d_ix_ovf, kIndexOverflowCap * (ix_csi(e) ? sizeof(IndexOvf) : sizeof(IndexRun))));
     CUC(cudaHostAlloc((void**)&e->h_ix_probe, 16, cudaHostAllocDefault));
   }
   CUC(cudaMalloc(&e->d_crc_tables, sizeof(CrcTables)));
@@ -1242,7 +1313,7 @@ int ngsq_reset(ngsq_engine* e) {
   e->ix_waves.clear();
   e->ix_drained.clear();  // pinned memory of the pin slabs, released above
   e->data_end_coff = 0;
-  e->bai.clear();
+  e->ix_bytes.clear();
   e->ix = IxHost{};
   e->ix_part_ok = false;
   e->split_merged = false;  // the split set itself is kept
@@ -1253,7 +1324,16 @@ int ngsq_reset(ngsq_engine* e) {
 int ngsq_set_references(ngsq_engine* e, uint32_t n_ref, const uint32_t* ref_len, const uint8_t* coverage_enabled) {
   if (!e || (n_ref && (!ref_len || !coverage_enabled))) return fail(e, NGSQ_E_ARG, "bad references");
   if (e->run_started) return fail(e, NGSQ_E_ARG, "ngsq_set_references must precede the first submit");
-  if (ix_on(e))
+  if (ix_on(e) && ix_csi(e)) {
+    uint32_t max_len = 0;
+    for (uint32_t c = 0; c < n_ref; ++c) max_len = std::max(max_len, ref_len[c]);
+    const uint32_t depth = e->ix_depth_req ? e->ix_depth_req : ix_csi_default_depth(max_len, e->ix_min_shift);
+    for (uint32_t c = 0; c < n_ref; ++c)
+      if (ref_len[c] > ix_csi_max_end(e->ix_min_shift, depth))
+        return fail(e, NGSQ_E_ARG, "reference %u is %u bases long: a CSI of min_shift %u and depth %u addresses at most 2^%u bases", c,
+                    ref_len[c], e->ix_min_shift, depth, e->ix_min_shift + 3 * depth);
+    e->ix_depth = depth;
+  } else if (ix_on(e))
     for (uint32_t c = 0; c < n_ref; ++c)
       if (ref_len[c] >= kIxMaxEnd)
         return fail(e, NGSQ_E_ARG, "reference %u is %u bases long: a BAI addresses fewer than 2^29 bases (index this file as CSI)", c, ref_len[c]);
@@ -1347,13 +1427,14 @@ int ngsq_set_references(ngsq_engine* e, uint32_t n_ref, const uint32_t* ref_len,
     if (!e->d_ft_res) CU(cudaMalloc(&e->d_ft_res, F_WORDS * 8));
   }
   if (ix_on(e)) {
-    // linear-index table per reference: windows 0 ..= L >> 14 (reads overhanging the end go to the overflow list)
+    // window table per reference: windows 0 ..= L >> 14 (BAI) or L >> min_shift (CSI); reads overhanging the end go to the
+    // overflow list
     e->ix_win_base.assign(n_ref, 0);
     e->ix_win_n.assign(n_ref, 0);
     uint64_t total = 0;
     for (uint32_t c = 0; c < n_ref; ++c) {
       e->ix_win_base[c] = total;
-      e->ix_win_n[c] = (ref_len[c] >> kIxWindowShift) + 1;
+      e->ix_win_n[c] = (ref_len[c] >> (ix_csi(e) ? e->ix_min_shift : kIxWindowShift)) + 1;
       total += e->ix_win_n[c];
     }
     e->ix_win_total = total;
@@ -1732,16 +1813,38 @@ int ngsq_finish(ngsq_engine* e) {
   return NGSQ_OK;
 }
 
-int ngsq_get_bai(ngsq_engine* e, uint8_t* out, size_t cap, size_t* n_out) {
+namespace {
+// ngsq_get_bai (csi = false) and ngsq_get_csi: the index bytes of a finished NGSQ_F_INDEX engine of that format
+int get_index(ngsq_engine* e, bool csi, uint8_t* out, size_t cap, size_t* n_out) {
   if (!e) return NGSQ_E_ARG;
+  const char* fn = csi ? "ngsq_get_csi" : "ngsq_get_bai";
   if (e->cfg.flags & NGSQ_F_INDEX_PART)
-    return fail(e, NGSQ_E_ARG, "ngsq_get_bai: this engine indexed one part of a file (NGSQ_F_INDEX_PART); join the finished parts with ngsq_join_bai");
-  if (!(e->cfg.flags & NGSQ_F_INDEX)) return fail(e, NGSQ_E_ARG, "ngsq_get_bai: the engine was created without NGSQ_F_INDEX");
-  if (!e->finished || e->bai.empty()) return fail(e, NGSQ_E_ARG, "ngsq_get_bai: no index before a successful ngsq_finish");
-  if (n_out) *n_out = e->bai.size();
+    return fail(e, NGSQ_E_ARG, "%s: this engine indexed one part of a file (NGSQ_F_INDEX_PART); join the finished parts with %s", fn,
+                ix_csi(e) ? "ngsq_join_csi" : "ngsq_join_bai");
+  if (!(e->cfg.flags & NGSQ_F_INDEX)) return fail(e, NGSQ_E_ARG, "%s: the engine was created without NGSQ_F_INDEX", fn);
+  if (csi && !ix_csi(e)) return fail(e, NGSQ_E_ARG, "ngsq_get_csi: the engine builds a BAI (created without NGSQ_F_INDEX_CSI); read it with ngsq_get_bai");
+  if (!csi && ix_csi(e)) return fail(e, NGSQ_E_ARG, "ngsq_get_bai: the engine builds a CSI (NGSQ_F_INDEX_CSI); read it with ngsq_get_csi");
+  if (!e->finished || e->ix_bytes.empty()) return fail(e, NGSQ_E_ARG, "%s: no index before a successful ngsq_finish", fn);
+  if (n_out) *n_out = e->ix_bytes.size();
   if (!out && !cap) return NGSQ_OK;
-  if (!out || cap < e->bai.size()) return fail(e, NGSQ_E_ARG, "ngsq_get_bai: buffer holds %zu bytes, %zu needed", cap, e->bai.size());
-  memcpy(out, e->bai.data(), e->bai.size());
+  if (!out || cap < e->ix_bytes.size()) return fail(e, NGSQ_E_ARG, "%s: buffer holds %zu bytes, %zu needed", fn, cap, e->ix_bytes.size());
+  memcpy(out, e->ix_bytes.data(), e->ix_bytes.size());
+  return NGSQ_OK;
+}
+}  // namespace
+
+int ngsq_get_bai(ngsq_engine* e, uint8_t* out, size_t cap, size_t* n_out) { return get_index(e, false, out, cap, n_out); }
+int ngsq_get_csi(ngsq_engine* e, uint8_t* out, size_t cap, size_t* n_out) { return get_index(e, true, out, cap, n_out); }
+
+int ngsq_set_index_binning(ngsq_engine* e, uint32_t min_shift, uint32_t depth) {
+  if (!e) return NGSQ_E_ARG;
+  if (!ix_on(e) || !ix_csi(e)) return fail(e, NGSQ_E_ARG, "ngsq_set_index_binning: the engine was created without NGSQ_F_INDEX_CSI");
+  if (e->d_ref_len) return fail(e, NGSQ_E_ARG, "ngsq_set_index_binning must precede ngsq_set_references (the window tables depend on it)");
+  if (min_shift < kCsiMinShiftLo || min_shift > kCsiMinShiftHi)
+    return fail(e, NGSQ_E_ARG, "ngsq_set_index_binning: min_shift %u is outside [%u, %u]", min_shift, kCsiMinShiftLo, kCsiMinShiftHi);
+  if (depth > kCsiDepthHi) return fail(e, NGSQ_E_ARG, "ngsq_set_index_binning: depth %u is outside [1, %u] (0 = the default rule)", depth, kCsiDepthHi);
+  e->ix_min_shift = min_shift;
+  e->ix_depth_req = depth;
   return NGSQ_OK;
 }
 
@@ -2141,20 +2244,28 @@ int ngsq_find_record(ngsq_engine* e, const uint8_t* bgzf, size_t nbytes, uint64_
   return NGSQ_OK;
 }
 
-int ngsq_join_bai(ngsq_engine* const* parts, uint32_t n, uint8_t* out, size_t cap, size_t* n_out) {
-  if (!parts || !n) return fail(nullptr, NGSQ_E_ARG, "ngsq_join_bai: no parts");
+namespace {
+// ngsq_join_bai (csi = false) and ngsq_join_csi
+int join_index(ngsq_engine* const* parts, uint32_t n, uint8_t* out, size_t cap, size_t* n_out, bool csi) {
+  const char* fn = csi ? "ngsq_join_csi" : "ngsq_join_bai";
+  if (!parts || !n) return fail(nullptr, NGSQ_E_ARG, "%s: no parts", fn);
   ngsq_engine* e = parts[0];  // carries the message
   for (uint32_t k = 0; k < n; ++k) {
     const ngsq_engine* p = parts[k];
-    if (!p) return fail(e, NGSQ_E_ARG, "ngsq_join_bai: part %u is NULL", k);
-    if (!(p->cfg.flags & NGSQ_F_INDEX_PART)) return fail(e, NGSQ_E_ARG, "ngsq_join_bai: part %u was created without NGSQ_F_INDEX_PART", k);
-    if (!p->finished || !p->ix_part_ok) return fail(e, NGSQ_E_ARG, "ngsq_join_bai: part %u has no index (it did not finish without error)", k);
-    if (p->ref_len != parts[0]->ref_len) return fail(e, NGSQ_E_ARG, "ngsq_join_bai: part %u has other references than part 0", k);
+    if (!p) return fail(e, NGSQ_E_ARG, "%s: part %u is NULL", fn, k);
+    if (!(p->cfg.flags & NGSQ_F_INDEX_PART)) return fail(e, NGSQ_E_ARG, "%s: part %u was created without NGSQ_F_INDEX_PART", fn, k);
+    if (!p->finished || !p->ix_part_ok) return fail(e, NGSQ_E_ARG, "%s: part %u has no index (it did not finish without error)", fn, k);
+    if (p->ref_len != parts[0]->ref_len) return fail(e, NGSQ_E_ARG, "%s: part %u has other references than part 0", fn, k);
+    if (ix_csi(p) != csi)
+      return fail(e, NGSQ_E_ARG, "%s: part %u builds a %s (join it with %s)", fn, k, csi ? "BAI" : "CSI", csi ? "ngsq_join_bai" : "ngsq_join_csi");
+    if (csi && (p->ix_min_shift != parts[0]->ix_min_shift || p->ix_depth != parts[0]->ix_depth))
+      return fail(e, NGSQ_E_ARG, "%s: part %u has min_shift %u and depth %u, part 0 has %u and %u: the parts must share one binning", fn, k,
+                  p->ix_min_shift, p->ix_depth, parts[0]->ix_min_shift, parts[0]->ix_depth);
     if (k + 1 < n && p->end_voff != parts[k + 1]->first_voff)
-      return fail(e, NGSQ_E_ARG, "ngsq_join_bai: part %u ends at virtual offset %llu, part %u starts at %llu: the parts must be contiguous, in file order", k,
+      return fail(e, NGSQ_E_ARG, "%s: part %u ends at virtual offset %llu, part %u starts at %llu: the parts must be contiguous, in file order", fn, k,
                   (unsigned long long)p->end_voff, k + 1, (unsigned long long)parts[k + 1]->first_voff);
   }
-  if (parts[n - 1]->end_voff) return fail(e, NGSQ_E_ARG, "ngsq_join_bai: the last part must run to the end of the data (end offset 0)");
+  if (parts[n - 1]->end_voff) return fail(e, NGSQ_E_ARG, "%s: the last part must run to the end of the data (end offset 0)", fn);
   // the order across every cut: a part's first placed record against the last record before the part that constrains the
   // order (an unplaced one: ~0); every other record was checked inside its part
   uint64_t unsorted = ~0ull, last = 0;
@@ -2181,12 +2292,16 @@ int ngsq_join_bai(ngsq_engine* const* parts, uint32_t n, uint8_t* out, size_t ca
   }
   U.data_end = parts[n - 1]->ix.data_end;
   std::vector<uint8_t> b;
-  assemble_bai(U, p0->n_ref, p0->ix_win_base, p0->ix_win_n, b);
+  assemble_index(p0, U, b);
   if (n_out) *n_out = b.size();
   if (!out && !cap) return NGSQ_OK;
-  if (!out || cap < b.size()) return fail(e, NGSQ_E_ARG, "ngsq_join_bai: buffer holds %zu bytes, %zu needed", cap, b.size());
+  if (!out || cap < b.size()) return fail(e, NGSQ_E_ARG, "%s: buffer holds %zu bytes, %zu needed", fn, cap, b.size());
   memcpy(out, b.data(), b.size());
   return NGSQ_OK;
 }
+}  // namespace
+
+int ngsq_join_bai(ngsq_engine* const* parts, uint32_t n, uint8_t* out, size_t cap, size_t* n_out) { return join_index(parts, n, out, cap, n_out, false); }
+int ngsq_join_csi(ngsq_engine* const* parts, uint32_t n, uint8_t* out, size_t cap, size_t* n_out) { return join_index(parts, n, out, cap, n_out, true); }
 
 }  // extern "C"

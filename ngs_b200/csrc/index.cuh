@@ -1,10 +1,12 @@
-// K13 — BAI index build (`ngs index`, reference src/index/bam.rs:39-109 over noodles' BAI indexer): per record, its
-// (reference, bin, [beg, end)) key and start offset; per wave, the runs of records that share a (reference, bin), the
-// order check, the per-reference counters and the 16 kb linear index.  The host (engine.cu, finish_index) turns the runs
-// into chunks and writes the .bai bytes at ngsq_finish.  The contract is DESIGN.md section 4, "K13 index".
+// K13 — BAI and CSI index build (`ngs index`, reference src/index/bam.rs:39-109 over noodles' BAI indexer; `samtools index
+// -c` for CSI): per record, its (reference, bin, [beg, end)) key and start offset; per wave, the runs of records that share a
+// (reference, bin), the order check, the per-reference counters and the per-window minimum offsets (16 kb windows for a BAI,
+// 2^min_shift for a CSI).  The host (engine.cu, finish_index) turns the runs into chunks and writes the .bai or .csi bytes
+// at ngsq_finish.  The contract is DESIGN.md section 4, "K13 index" and "K13 CSI".
 //
-// The per-record functions are NGSQ_HD: tools/index_model.cpp runs them on the CPU against the oracle
-// (tests/cpp/bai_oracle.c, oracle_build_bai; tests/test_index_model.py).  GPU parity: tests/test_gpu_index.py.
+// The per-record functions are NGSQ_HD: tools/index_model.cpp runs them on the CPU against the oracles
+// (tests/cpp/bai_oracle.c, oracle_build_bai; tests/cpp/csi_oracle.c, oracle_build_csi; tests/test_index_model.py,
+// test_index_model_csi.py).  GPU parity: tests/test_gpu_index.py, test_gpu_index_csi.py.
 #pragma once
 #include <stdint.h>
 
@@ -29,9 +31,13 @@ constexpr uint64_t kIxUnplacedRun = ~0ull;         // run key of records that ar
 constexpr uint64_t kIxNoRun = ~1ull;               // run key "before the first record"
 constexpr uint32_t kIxUnplacedRef = 0xFFFFFFFFu;   // IndexRun::ref of a run of unplaced records
 
+// CSI binning (NGSQ_F_INDEX_CSI): windows of 2^min_shift bases, `depth` levels of bins below bin 0.  The bounds keep bin ids
+// below 2^24 and a reference's window table (L >> min_shift) + 1 below 2^20 entries for any 32-bit length.
+constexpr uint32_t kCsiMinShiftLo = 12, kCsiMinShiftHi = 24, kCsiDepthHi = 7;
+
 enum : uint32_t {
   kIxBadRecord = 1,  // field overrun, CIGAR op > 8, reference id out of range
-  kIxTooLong = 2,    // end > 2^29: not addressable by a BAI
+  kIxTooLong = 2,    // end > 2^29 (BAI) or 2^(min_shift + 3 depth) (CSI): not addressable
   kIxRunTable = 4,   // more runs than the wave's run table holds (sized by records: cannot happen)
   kIxOverflowList = 8,  // more records reach past their reference's window table than the overflow list holds
 };
@@ -58,6 +64,30 @@ NGSQ_HD uint32_t ix_reg2bin(uint64_t beg, uint64_t end) {
   if (beg >> 23 == end >> 23) return (uint32_t)(((1u << 6) - 1) / 7 + (beg >> 23));
   if (beg >> 26 == end >> 26) return (uint32_t)(((1u << 3) - 1) / 7 + (beg >> 26));
   return 0;
+}
+
+// CSIv1: hts_reg2bin, the generalised form of SAM 5.3 (at min_shift 14, depth 5 it is ix_reg2bin)
+NGSQ_HD uint32_t ix_csi_reg2bin(uint64_t beg, uint64_t end, uint32_t min_shift, uint32_t depth) {
+  --end;
+  uint32_t s = min_shift, t = ((1u << 3 * depth) - 1) / 7;
+  for (uint32_t l = depth; l > 0; --l, s += 3, t -= 1u << 3 * l)
+    if (beg >> s == end >> s) return t + (uint32_t)(beg >> s);
+  return 0;
+}
+// bins of a CSI: ids 0 .. n_bins - 1; the per-reference pseudo-bin is n_bins + 1 (37450 at depth 5, as in the BAI)
+NGSQ_HD uint32_t ix_csi_n_bins(uint32_t depth) { return ((1u << 3 * (depth + 1)) - 1) / 7; }
+NGSQ_HD uint64_t ix_csi_max_end(uint32_t min_shift, uint32_t depth) { return 1ull << (min_shift + 3 * depth); }
+// first leaf window of a bin (htslib hts_bin_bot): the window whose filled minimum is the bin's loffset
+NGSQ_HD uint64_t ix_csi_bin_bot(uint32_t bin, uint32_t depth) {
+  uint32_t l = 0;
+  for (uint32_t b = bin; b; b = (b - 1) >> 3) ++l;
+  return (uint64_t)(bin - ((1u << 3 * l) - 1) / 7) << 3 * (depth - l);
+}
+// samtools index -c: the smallest depth n with max_len + 256 <= 2^(min_shift + 3n)
+NGSQ_HD uint32_t ix_csi_default_depth(uint64_t max_len, uint32_t min_shift) {
+  uint32_t n = 0;
+  for (uint64_t s = 1ull << min_shift; max_len + 256 > s; s <<= 3) ++n;
+  return n;
 }
 
 // Header of the record at `rec` (its block_size first): fills ref / pos / unmapped and the CIGAR's place; 0 or kIxBadRecord.
@@ -103,21 +133,33 @@ NGSQ_HD uint32_t index_finish_key(IndexKey* k, uint64_t span) {
   return 0;
 }
 
+// The same for a CSI of the given binning.  0 or kIxTooLong (end > 2^(min_shift + 3 depth)).
+NGSQ_HD uint32_t index_finish_key_csi(IndexKey* k, uint64_t span, uint32_t min_shift, uint32_t depth) {
+  if (k->ref < 0 || k->pos < 0) return 0;
+  k->placed = 1;
+  k->beg = (uint64_t)k->pos;
+  k->end = k->beg + (span ? span : 1);
+  if (k->end > ix_csi_max_end(min_shift, depth)) { k->placed = 0; return kIxTooLong; }
+  k->bin = ix_csi_reg2bin(k->beg, k->end, min_shift, depth);
+  return 0;
+}
+
 // The whole key of one record, serially (the host model; the kernel splits the CIGAR walk over a warp for long CIGARs).
-NGSQ_HD uint32_t index_record(const uint8_t* rec, int32_t n_ref, IndexKey* k) {
+// csi = 0: the BAI key; otherwise the CSI key at (min_shift, depth).
+NGSQ_HD uint32_t index_record(const uint8_t* rec, int32_t n_ref, IndexKey* k, bool csi = false, uint32_t min_shift = 0, uint32_t depth = 0) {
   uint32_t ncig;
   const uint8_t* cig;
   uint32_t bad = index_header(rec, n_ref, k, &ncig, &cig);
   if (bad) return bad;
   uint64_t span;
   if ((bad = index_cigar_span(cig, 0, ncig, 1, &span))) return bad;
-  return index_finish_key(k, span);
+  return csi ? index_finish_key_csi(k, span, min_shift, depth) : index_finish_key(k, span);
 }
 
-// Linear-index windows [lo, hi] a placed record touches.
-NGSQ_HD void index_windows(const IndexKey& k, uint32_t* lo, uint32_t* hi) {
-  *lo = (uint32_t)(k.beg >> kIxWindowShift);
-  *hi = (uint32_t)((k.end - 1) >> kIxWindowShift);
+// Windows [lo, hi] a placed record touches, of 2^shift bases (kIxWindowShift: the BAI's linear index).
+NGSQ_HD void index_windows(const IndexKey& k, uint32_t* lo, uint32_t* hi, uint32_t shift = kIxWindowShift) {
+  *lo = (uint32_t)(k.beg >> shift);
+  *hi = (uint32_t)((k.end - 1) >> shift);
 }
 
 // Runs: consecutive records with equal keys share a chunk.  Unplaced records share one key: they end a chunk, join none.
@@ -127,11 +169,17 @@ NGSQ_HD uint64_t index_run_key(const IndexKey& k) { return k.placed ? ((uint64_t
 NGSQ_HD bool index_constrains(const IndexKey& k) { return k.placed || k.ref < 0; }
 NGSQ_HD uint64_t index_order_key(const IndexKey& k) { return k.ref < 0 ? ~0ull : ((uint64_t)(uint32_t)k.ref << 32) | (uint32_t)k.pos; }
 
-// One entry of the run table (and of the overflow list, whose `bin` holds window lo | hi << 16).
+// One entry of the run table (and of the BAI's overflow list, whose `bin` holds window lo | hi << 16).
 struct IndexRun {
   uint64_t voff;  // virtual offset of the run's first record; the run ends where the next one starts
   uint32_t ref;   // kIxUnplacedRef for unplaced records
   uint32_t bin;
+};
+// One entry of the CSI's overflow list: windows [lo, hi] of a record past its reference's table (a CSI reference may have
+// more than 2^16 windows)
+struct IndexOvf {
+  uint64_t voff;
+  uint32_t ref, lo, hi, pad;
 };
 
 #if defined(__CUDACC__)
@@ -168,14 +216,16 @@ struct IndexParams {
   IndexState* S;
   IndexRun* runs;           // this wave's run table
   uint64_t runs_cap;
-  IndexRun* ovf;            // whole run: records whose windows reach past their reference's table
+  void* ovf;                // whole run: records whose windows reach past their reference's table (IndexRun for a BAI,
+                            // IndexOvf for a CSI)
   uint64_t ovf_cap;
   const uint64_t* win_base; // per reference: first entry in win
-  const uint32_t* win_n;    // per reference: windows in the table ((L >> 14) + 1)
-  unsigned long long* win;  // linear index: smallest start offset per window (~0 = untouched)
+  const uint32_t* win_n;    // per reference: windows in the table ((L >> shift) + 1)
+  unsigned long long* win;  // smallest start offset per window (~0 = untouched)
   unsigned int* max_win;    // per reference: largest window touched
   unsigned long long* counts;  // per reference: mapped, unmapped
   uint32_t part;            // NGSQ_F_INDEX_PART: also record the first placed record (IndexState::first_key / first_voff)
+  uint32_t min_shift, depth;  // CSI binning (index_kernel<true>)
 };
 
 // 128-bit minimum of (voff, key) into S->first_key / first_voff.  A torn read of the current value only costs a failed CAS:
@@ -205,6 +255,9 @@ __device__ __forceinline__ uint64_t index_voff(const IndexParams& P, uint64_t rv
 
 // Warp steps of 31 records: lane l holds record r0 - 1 + l, so every lane but 0 finds its predecessor's key in lane l - 1;
 // lane 0 holds the previous step's last record (or, for record 0 of the wave, the carry of the previous wave).
+// kCsi = false: the BAI (bins of SAM 5.3, 16 kb windows, ends up to 2^29); true: the CSI binning of P.min_shift / P.depth.
+// The two differ only in constexpr branches, so the BAI instance is the kernel it was before CSI existed.
+template <bool kCsi>
 __global__ void __launch_bounds__(kIndexThreads) index_kernel(IndexParams P) {
   const uint32_t lane = threadIdx.x & 31;
   const uint64_t n = P.st->fatal ? 0 : P.st->wave_rec;
@@ -245,7 +298,10 @@ __global__ void __launch_bounds__(kIndexThreads) index_kernel(IndexParams P) {
       const bool any_bad = __any_sync(0xFFFFFFFFu, b);
       if ((int)lane == j) { span = sp; if (any_bad) bad = kIxBadRecord; }
     }
-    if (have && !bad) bad = index_finish_key(&k, span);
+    if (have && !bad) {
+      if constexpr (kCsi) bad = index_finish_key_csi(&k, span, P.min_shift, P.depth);
+      else bad = index_finish_key(&k, span);
+    }
     if (bad) { k.ref = -1; k.pos = -1; k.placed = 0; if (own) err |= bad; }
 
     // ---- runs: a record starts one when its key differs from its predecessor's
@@ -295,7 +351,8 @@ __global__ void __launch_bounds__(kIndexThreads) index_kernel(IndexParams P) {
     if (P.part && pm && (int)lane == __ffs(pm) - 1) index_first_min(P.S, voff, index_order_key(k));  // the warp's first in file order
     uint32_t w_lo = 0, w_hi = 0, nw = 0;
     if (pl) {
-      index_windows(k, &w_lo, &w_hi);
+      if constexpr (kCsi) index_windows(k, &w_lo, &w_hi, P.min_shift);
+      else index_windows(k, &w_lo, &w_hi);
       nw = P.win_n[k.ref];
       const uint32_t cslot = 2u * (uint32_t)k.ref + k.unmapped;
       const uint32_t peers = __match_any_sync(pm, cslot);
@@ -330,8 +387,10 @@ __global__ void __launch_bounds__(kIndexThreads) index_kernel(IndexParams P) {
       if (over) {
         const uint64_t idx = base + __popc(om & ((1u << lane) - 1));
         const uint32_t lo = w_lo > nw ? w_lo : nw;
-        if (idx < P.ovf_cap) P.ovf[idx] = IndexRun{voff, (uint32_t)k.ref, lo | (w_hi << 16)};
-        else err |= kIxOverflowList;
+        if (idx < P.ovf_cap) {
+          if constexpr (kCsi) static_cast<IndexOvf*>(P.ovf)[idx] = IndexOvf{voff, (uint32_t)k.ref, lo, w_hi, 0u};
+          else static_cast<IndexRun*>(P.ovf)[idx] = IndexRun{voff, (uint32_t)k.ref, lo | (w_hi << 16)};
+        } else err |= kIxOverflowList;
       }
     }
   }

@@ -24,6 +24,7 @@ NGSQ_F_FEATURES = 16
 NGSQ_F_SERIAL_STAGES = 32  # measurement aid: no overlap between the stages of consecutive waves
 NGSQ_F_INDEX = 64  # build the file's BAI in the same pass (Engine.bai())
 NGSQ_F_INDEX_PART = 128  # index one range of a file cut between engines (join the parts with join_bai())
+NGSQ_F_INDEX_CSI = 256  # with NGSQ_F_INDEX / NGSQ_F_INDEX_PART: a CSI instead of a BAI (Engine.csi(), join_csi())
 
 ERROR_NAMES = {
     0: "NGSQ_OK", -1: "NGSQ_E_ARG", -2: "NGSQ_E_CUDA", -3: "NGSQ_E_TRUNCATED", -4: "NGSQ_E_BAD_BLOCK",
@@ -42,6 +43,7 @@ EXPORTED = [
     "ngsq_set_reference_bases", "ngsq_get_edits", "ngsq_get_edit_positions", "ngsq_set_feature_model", "ngsq_set_features", "ngsq_get_features",
     "ngsq_wait_copied", "ngsq_host_register", "ngsq_host_unregister", "ngsq_flush", "ngsq_progress",
     "ngsq_get_bai", "ngsq_split_reference", "ngsq_split_arrays", "ngsq_resolve_split", "ngsq_find_record", "ngsq_join_bai",
+    "ngsq_set_index_binning", "ngsq_get_csi", "ngsq_join_csi",
 ]
 
 
@@ -150,6 +152,9 @@ def load_library() -> C.CDLL:
     lib.ngsq_resolve_split.argtypes = [P, C.c_int]
     lib.ngsq_find_record.argtypes = [P, P, C.c_size_t, C.c_uint64, u64p, C.POINTER(C.c_int32)]
     lib.ngsq_join_bai.argtypes = [C.POINTER(P), C.c_uint32, P, C.c_size_t, C.POINTER(C.c_size_t)]
+    lib.ngsq_set_index_binning.argtypes = [P, C.c_uint32, C.c_uint32]
+    lib.ngsq_get_csi.argtypes = [P, P, C.c_size_t, C.POINTER(C.c_size_t)]
+    lib.ngsq_join_csi.argtypes = [C.POINTER(P), C.c_uint32, P, C.c_size_t, C.POINTER(C.c_size_t)]
     _lib = lib
     return lib
 
@@ -341,10 +346,22 @@ class Engine:
     # ---- BAI (NGSQ_F_INDEX) ----
     def bai(self) -> bytes:
         """The .bai file of the records submitted since set_range (after finish)."""
+        return self._index_bytes(self.lib.ngsq_get_bai)
+
+    # ---- CSI (NGSQ_F_INDEX | NGSQ_F_INDEX_CSI) ----
+    def set_index_binning(self, min_shift: int = 14, depth: int = 0):
+        """The CSI's binning (depth 0: samtools' rule from the longest reference); before set_references."""
+        self._check(self.lib.ngsq_set_index_binning(self.h, min_shift, depth))
+
+    def csi(self) -> bytes:
+        """The uncompressed .csi payload of the records submitted since set_range (after finish); the file is its BGZF."""
+        return self._index_bytes(self.lib.ngsq_get_csi)
+
+    def _index_bytes(self, getter) -> bytes:
         n = C.c_size_t(0)
-        self._check(self.lib.ngsq_get_bai(self.h, None, 0, C.byref(n)))
+        self._check(getter(self.h, None, 0, C.byref(n)))
         buf = np.empty(max(n.value, 1), dtype=np.uint8)
-        self._check(self.lib.ngsq_get_bai(self.h, buf.ctypes.data, n.value, C.byref(n)))
+        self._check(getter(self.h, buf.ctypes.data, n.value, C.byref(n)))
         return buf[: n.value].tobytes()
 
     def find_record(self, data: np.ndarray, file_off: int = 0):
@@ -399,6 +416,15 @@ class Engine:
 
 def join_bai(parts) -> bytes:
     """The .bai of a file from its NGSQ_F_INDEX_PART engines, in file order (ngsq_join_bai)."""
+    return _join(load_library().ngsq_join_bai, parts)
+
+
+def join_csi(parts) -> bytes:
+    """The uncompressed .csi of a file from its NGSQ_F_INDEX_PART | NGSQ_F_INDEX_CSI engines, in file order (ngsq_join_csi)."""
+    return _join(load_library().ngsq_join_csi, parts)
+
+
+def _join(fn, parts) -> bytes:
     lib = load_library()
     hs = (C.c_void_p * len(parts))(*[p.h.value for p in parts])
     n = C.c_size_t(0)
@@ -406,9 +432,9 @@ def join_bai(parts) -> bytes:
     def check(rc):
         if rc:
             raise NgsqError(rc, lib.ngsq_last_error(parts[0].h if parts else None).decode())
-    check(lib.ngsq_join_bai(hs, len(parts), None, 0, C.byref(n)))
+    check(fn(hs, len(parts), None, 0, C.byref(n)))
     buf = np.empty(max(n.value, 1), dtype=np.uint8)
-    check(lib.ngsq_join_bai(hs, len(parts), buf.ctypes.data, n.value, C.byref(n)))
+    check(fn(hs, len(parts), buf.ctypes.data, n.value, C.byref(n)))
     return buf[: n.value].tobytes()
 
 

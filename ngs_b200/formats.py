@@ -164,6 +164,56 @@ def parse_bai(buf: bytes) -> Bai:
 
 
 @dataclass
+class CsiRef:
+    bins: dict = field(default_factory=dict)     # bin -> [(beg, end)]
+    loffset: dict = field(default_factory=dict)  # bin -> loffset
+    ref_beg: int | None = None                   # pseudo-bin n_bins + 1
+    ref_end: int | None = None
+    n_mapped: int = 0
+    n_unmapped: int = 0
+
+
+@dataclass
+class Csi:
+    min_shift: int
+    depth: int
+    aux: bytes
+    refs: list
+    n_no_coor: int | None
+
+
+def parse_csi(buf: bytes) -> Csi:
+    """An uncompressed CSIv1 payload (a .csi file after gzip.decompress)."""
+    if buf[:4] != b"CSI\x01":
+        raise ValueError("bad CSI magic")
+    min_shift, depth, l_aux = struct.unpack_from("<iii", buf, 4)
+    aux = bytes(buf[16:16 + l_aux])
+    o = 16 + l_aux
+    n_ref = struct.unpack_from("<i", buf, o)[0]
+    o += 4
+    meta = ((1 << 3 * (depth + 1)) - 1) // 7 + 1
+    refs = []
+    for _ in range(n_ref):
+        r = CsiRef()
+        n_bin = struct.unpack_from("<i", buf, o)[0]
+        o += 4
+        for _ in range(n_bin):
+            b, loff, n_chunk = struct.unpack_from("<IQi", buf, o)
+            o += 16
+            chunks = [struct.unpack_from("<QQ", buf, o + 16 * k) for k in range(n_chunk)]
+            o += 16 * n_chunk
+            if b == meta and n_chunk == 2:
+                r.ref_beg, r.ref_end = chunks[0]
+                r.n_mapped, r.n_unmapped = chunks[1]
+            else:
+                r.bins[b] = chunks
+                r.loffset[b] = loff
+        refs.append(r)
+    n_no_coor = struct.unpack_from("<Q", buf, o)[0] if o + 8 <= len(buf) else None
+    return Csi(min_shift, depth, aux, refs, n_no_coor)
+
+
+@dataclass
 class Shard:
     first_voffset: int   # first record owned
     end_voffset: int     # first record not owned (0 = to EOF)

@@ -11,7 +11,8 @@
 //   ngs-cuda-qc qc <BAM> <REFERENCE_GENOME> [-n N] [-o DIR] [-p PREFIX] [--only FACET]
 //               [--cuda-devices 0,1,..] [--cuda-build-index] [--cuda-gc-seed S] [--cuda-no-crc] [--cuda-chunk-mb M]
 //               [--cuda-buffered-io] [--cuda-perf]
-//   ngs-cuda-qc index <BAM> [--cuda-device N | --cuda-devices 0,1,..] [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io]
+//   ngs-cuda-qc index <BAM> [--csi [-m|--min-shift N]] [--cuda-device N | --cuda-devices 0,1,..] [--cuda-no-crc] [--cuda-chunk-mb M]
+//                     [--cuda-buffered-io]
 #include <cerrno>
 #include <cstdio>
 #include <cstdlib>
@@ -244,16 +245,48 @@ FindRecord engine_finder(ngsq_engine* e) {
   return [e](const uint8_t* p, size_t n, uint64_t off, uint64_t* voff, int32_t* ref) { check(e, ngsq_find_record(e, p, n, off, voff, ref)); };
 }
 
-// The parts' .bai, in file order (engines with an empty range hold no part)
-std::vector<uint8_t> join_parts(const std::vector<ngsq_engine*>& engines, const std::vector<Shard>& shards) {
+// The parts' .bai (or uncompressed .csi), in file order (engines with an empty range hold no part)
+std::vector<uint8_t> join_parts(const std::vector<ngsq_engine*>& engines, const std::vector<Shard>& shards, bool csi = false) {
   std::vector<ngsq_engine*> parts;
   for (size_t i = 0; i < engines.size(); ++i)
     if (!shards[i].empty) parts.push_back(engines[i]);
+  auto join = csi ? ngsq_join_csi : ngsq_join_bai;
   size_t n = 0;
-  check(parts[0], ngsq_join_bai(parts.data(), (uint32_t)parts.size(), nullptr, 0, &n));
+  check(parts[0], join(parts.data(), (uint32_t)parts.size(), nullptr, 0, &n));
   std::vector<uint8_t> bai(n);
-  check(parts[0], ngsq_join_bai(parts.data(), (uint32_t)parts.size(), bai.data(), bai.size(), &n));
+  check(parts[0], join(parts.data(), (uint32_t)parts.size(), bai.data(), bai.size(), &n));
   return bai;
+}
+
+// A .csi file is BGZF: the payload in blocks of at most 0xFF00 bytes, each deflated at level 6 (as htslib writes them), then
+// the 28-byte EOF block.
+std::vector<uint8_t> bgzf_compress(const std::vector<uint8_t>& data) {
+  static const uint8_t kEof[28] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+  std::vector<uint8_t> out;
+  uint8_t blk[65536];
+  for (size_t o = 0; o < data.size(); o += 0xFF00) {
+    const uInt n = (uInt)std::min<size_t>(0xFF00, data.size() - o);
+    z_stream zs{};
+    if (deflateInit2(&zs, 6, Z_DEFLATED, -15, 8, Z_DEFAULT_STRATEGY) != Z_OK) throw std::runtime_error("deflateInit2 failed");
+    zs.next_in = const_cast<uint8_t*>(data.data() + o);
+    zs.avail_in = n;
+    zs.next_out = blk + 18;
+    zs.avail_out = sizeof blk - 26;
+    const int rc = deflate(&zs, Z_FINISH);
+    const size_t clen = zs.total_out;
+    deflateEnd(&zs);
+    if (rc != Z_STREAM_END || 26 + clen > sizeof blk) throw std::runtime_error("BGZF block does not fit in 64 KiB");
+    static const uint8_t kHdr[16] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0};
+    memcpy(blk, kHdr, 16);
+    const uint16_t bsize = (uint16_t)(26 + clen - 1);
+    const uint32_t crc = (uint32_t)crc32(crc32(0, nullptr, 0), data.data() + o, n), isize = n;
+    memcpy(blk + 16, &bsize, 2);
+    memcpy(blk + 18 + clen, &crc, 4);
+    memcpy(blk + 22 + clen, &isize, 4);
+    out.insert(out.end(), blk, blk + 26 + clen);
+  }
+  out.insert(out.end(), kEof, kEof + 28);
+  return out;
 }
 
 // The .bai next to the BAM.  O_EXCL: an index that appeared while the file was read is not replaced either.
@@ -469,6 +502,8 @@ int qc(const QcArgs& args) {
 // overwrites an existing index.
 struct IndexArgs {
   std::string src;
+  bool csi = false;          // --csi: <BAM>.csi (BGZF) instead of <BAM>.bai
+  uint32_t min_shift = 14;   // -m / --min-shift (CSI); the depth follows samtools' rule
   int device = 0;
   std::vector<int> devices;  // --cuda-devices: several engines, one part of the file each
   bool verify_crc = true;
@@ -476,14 +511,19 @@ struct IndexArgs {
   bool direct_io = true;
 };
 
+// the index file of the engine(s): the .bai as it is, the .csi payload BGZF-compressed
+void write_index_file(const IndexArgs& a, const std::string& dst, const std::vector<uint8_t>& payload) {
+  write_index(dst, a.csi ? bgzf_compress(payload) : payload);
+}
+
 int index_bam(const IndexArgs& a) {
   info("Starting index command...");
-  const std::string dst = a.src + ".bai";
+  const std::string dst = a.src + (a.csi ? ".csi" : ".bai");
   if (std::filesystem::exists(dst)) throw std::runtime_error("index file already exists: " + dst);
   MappedFile file(a.src);
   ngsq_config cfg{};
   cfg.struct_size = sizeof cfg;
-  cfg.flags = NGSQ_F_INDEX | (a.verify_crc ? NGSQ_F_VERIFY_CRC : 0u);
+  cfg.flags = NGSQ_F_INDEX | (a.verify_crc ? NGSQ_F_VERIFY_CRC : 0u) | (a.csi ? NGSQ_F_INDEX_CSI : 0u);
   ngsq_engine* e = nullptr;
   if (ngsq_create(a.device, &cfg, &e)) throw std::runtime_error(std::string("CUDA engine: ") + ngsq_last_error(nullptr));
   struct Cleanup { ngsq_engine* e; ~Cleanup() { ngsq_destroy(e); } } cleanup{e};
@@ -491,6 +531,7 @@ int index_bam(const IndexArgs& a) {
   std::vector<uint32_t> ref_len;
   for (auto& rs : header.reference_sequences) ref_len.push_back(rs.length);
   std::vector<uint8_t> no_coverage(ref_len.size(), 0);
+  if (a.csi) check(e, ngsq_set_index_binning(e, a.min_shift, 0));
   check(e, ngsq_set_references(e, (uint32_t)ref_len.size(), ref_len.data(), no_coverage.data()));
   check(e, ngsq_set_range(e, header.first_record_voffset, 0));
   info("Indexing BAM file.");
@@ -504,11 +545,12 @@ int index_bam(const IndexArgs& a) {
   ngsq_stats st;
   check(e, ngsq_get_stats(e, &st));
   info("Processed " + std::to_string(st.records) + " records.");
+  auto get = a.csi ? ngsq_get_csi : ngsq_get_bai;
   size_t n = 0;
-  check(e, ngsq_get_bai(e, nullptr, 0, &n));
+  check(e, get(e, nullptr, 0, &n));
   std::vector<uint8_t> bai(n);
-  check(e, ngsq_get_bai(e, bai.data(), bai.size(), &n));
-  write_index(dst, bai);
+  check(e, get(e, bai.data(), bai.size(), &n));
+  write_index_file(a, dst, bai);
   return 0;
 }
 
@@ -516,7 +558,7 @@ int index_bam(const IndexArgs& a) {
 // joined on the host.  No collective is involved, so a device may repeat.
 int index_bam_parts(const IndexArgs& a) {
   info("Starting index command...");
-  const std::string dst = a.src + ".bai";
+  const std::string dst = a.src + (a.csi ? ".csi" : ".bai");
   if (std::filesystem::exists(dst)) throw std::runtime_error("index file already exists: " + dst);
   MappedFile file(a.src);
   const size_t n_dev = a.devices.size();
@@ -525,14 +567,17 @@ int index_bam_parts(const IndexArgs& a) {
   for (size_t i = 0; i < n_dev; ++i) {
     ngsq_config cfg{};
     cfg.struct_size = sizeof cfg;
-    cfg.flags = NGSQ_F_INDEX_PART | (a.verify_crc ? NGSQ_F_VERIFY_CRC : 0u);
+    cfg.flags = NGSQ_F_INDEX_PART | (a.verify_crc ? NGSQ_F_VERIFY_CRC : 0u) | (a.csi ? NGSQ_F_INDEX_CSI : 0u);
     if (ngsq_create(a.devices[i], &cfg, &engines[i])) throw std::runtime_error(std::string("CUDA engine: ") + ngsq_last_error(nullptr));
   }
   BamHeader header = read_bam_header(engines[0], file.data(), file.size());
   std::vector<uint32_t> ref_len;
   for (auto& rs : header.reference_sequences) ref_len.push_back(rs.length);
   std::vector<uint8_t> no_coverage(ref_len.size(), 0);
-  for (auto* e : engines) check(e, ngsq_set_references(e, (uint32_t)ref_len.size(), ref_len.data(), no_coverage.data()));
+  for (auto* e : engines) {
+    if (a.csi) check(e, ngsq_set_index_binning(e, a.min_shift, 0));
+    check(e, ngsq_set_references(e, (uint32_t)ref_len.size(), ref_len.data(), no_coverage.data()));
+  }
   ShardPlan plan = plan_shards_unindexed(header, file.data(), file.size(), (uint32_t)n_dev, engine_finder(engines[0]));
   log_dropped_cuts(plan);
   info("Indexing BAM file in " + std::to_string(n_dev - plan.dropped) + " parts.");
@@ -540,12 +585,13 @@ int index_bam_parts(const IndexArgs& a) {
   uint64_t records = 0;
   for (auto* e : engines) { ngsq_stats st; check(e, ngsq_get_stats(e, &st)); records += st.records; }
   info("Processed " + std::to_string(records) + " records.");
-  write_index(dst, join_parts(engines, plan.shards));
+  write_index_file(a, dst, join_parts(engines, plan.shards, a.csi));
   return 0;
 }
 
 int index_main(int argc, char** argv, int i) {
   IndexArgs a;
+  bool min_shift_set = false;
   std::vector<std::string> pos;
   for (; i < argc; ++i) {
     std::string s = argv[i];
@@ -555,9 +601,12 @@ int index_main(int argc, char** argv, int i) {
     else if (s == "--cuda-no-crc") a.verify_crc = false;
     else if (s == "--cuda-chunk-mb") a.chunk_mb = std::stoull(val());
     else if (s == "--cuda-buffered-io") a.direct_io = false;
+    else if (s == "--csi") a.csi = true;
+    else if (s == "-m" || s == "--min-shift") { a.min_shift = (uint32_t)std::stoul(val()); min_shift_set = true; }
     else if (!s.empty() && s[0] == '-' && s != "-") throw std::runtime_error("unknown flag " + s);
     else pos.push_back(s);
   }
+  if (min_shift_set && !a.csi) throw std::runtime_error("--min-shift sets the binning of a CSI: use it with --csi");
   if (pos.size() != 1 || !a.chunk_mb) return -1;
   a.src = pos[0];
   if (a.devices.size() > 1) return index_bam_parts(a);
@@ -570,8 +619,10 @@ void usage() {
                "                  [--cuda-devices 0,1,..] [--cuda-build-index] [--cuda-gc-seed S] [--cuda-no-crc] [--cuda-chunk-mb M]\n"
                "                  [--cuda-buffered-io] [--cuda-perf]\n"
                "                  (--cuda-build-index: without <BAM>.bai, build it in the same pass and write it once the run succeeded)\n"
-               "       ngs-cuda-qc index <BAM> [--cuda-device N | --cuda-devices 0,1,..] [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io]\n"
-               "                  (writes <BAM>.bai; an existing index is never overwritten; several devices index one part of the file each)\n";
+               "       ngs-cuda-qc index <BAM> [--csi [-m|--min-shift N]] [--cuda-device N | --cuda-devices 0,1,..] [--cuda-no-crc] [--cuda-chunk-mb M]\n"
+               "                  [--cuda-buffered-io]\n"
+               "                  (writes <BAM>.bai, or with --csi <BAM>.csi (min_shift N, default 14); an existing index is never overwritten;\n"
+               "                  several devices index one part of the file each)\n";
 }
 
 }  // namespace

@@ -15,7 +15,9 @@
 //
 // Shapes (BASELINE.json configs): 0 = C1 3-contig 2x150, 1 = WGS 25-contig
 // 2x150 (C2/C3), 2 = long reads 10-50 kb on chr1-5 (C4), 3 = spliced 2x100
-// RNA-seq (C5).
+// RNA-seq (C5), 4 = references past 2^29 and 2^30 bases (a CSI's inputs:
+// a 1.9 Gbp, a 0.8 Gbp and a 1 Mbp reference) with short, 10-50 kb and spliced
+// reads, some of them across 2^29; no BAI can address it, so none is written.
 //
 // Exposed both as a C API (libngs_synth.so, used by tests/bench via ctypes)
 // and as a CLI (`bamgen <shape> <n_records> <out.bam> [seed] [level] [threads]`).
@@ -43,6 +45,7 @@ struct Contig {
 };
 
 const Contig kC1[] = {{"chr1", 20000000}, {"chr2", 10000000}, {"chrM", 16569}};
+const Contig kBig[] = {{"chrA", 1900000000}, {"chrB", 800000000}, {"chrS", 1000000}};
 const Contig kWGS[] = {
     {"chr1", 248956422},  {"chr2", 242193529},  {"chr3", 198295559},  {"chr4", 190214555},
     {"chr5", 181538259},  {"chr6", 170805979},  {"chr7", 159345973},  {"chr8", 145138636},
@@ -115,6 +118,7 @@ struct Meta {
   uint32_t cigar[8];      // short-read shapes: at most 8 ops
   uint32_t size;          // bytes incl. the 4-byte block_size prefix
   bool missing_qual;
+  bool long_read;         // the CIGAR is a LongCigar (shape 2, and shape 4's long reads)
   uint64_t rng_state;     // state handed to the payload generator
 };
 
@@ -191,12 +195,14 @@ void make_meta(const Shape& sh, uint64_t i, Meta& m) {
   uint64_t j;
   locate(sh, i, c, j);
   m.missing_qual = false;
+  m.long_read = sh.kind == 2;
   m.n_cigar = 0;
   m.span = 0;
   uint32_t R = sh.read_len;
   if (sh.kind == 2) R = 10000 + rng.below(40001);
+  if (sh.kind == 4 && rng.permille() < 10) { m.long_read = true; R = 10000 + rng.below(40001); }
   uint32_t pm = rng.permille();
-  if (sh.kind != 2) {
+  if (sh.kind != 2 && !m.long_read) {
     if (pm < 20) R = 30 + rng.below(R - 30);        // trimmed (<100 exercises GC too-short)
     else if (pm < 23) R = 100 + (pm & 1);           // exactly 100 / 101
   }
@@ -277,7 +283,7 @@ void make_meta(const Shape& sh, uint64_t i, Meta& m) {
   bool mapped = c >= 0 && !self_unmapped;
   uint32_t cig_bytes = 0;
   if (mapped && R > 0) {
-    if (sh.kind == 2) {
+    if (m.long_read) {
       LongCigar lc(m.rng_state, R);
       uint32_t n = 0, span = 0;
       while (uint32_t o = lc.next()) {
@@ -292,9 +298,11 @@ void make_meta(const Shape& sh, uint64_t i, Meta& m) {
       uint32_t k = rng.permille();
       uint32_t* cg = m.cigar;
       uint32_t n = 0;
-      if (rna && k < 600 && R >= 40) {
+      if ((rna || sh.kind == 4) && k < (rna ? 600u : 300u) && R >= 40) {
         uint32_t a = 10 + rng.below(R - 20);
-        uint32_t skip = 100 + rng.below(199901);
+        // shape 4: introns up to 8 record spacings (at most 2^26), so that some spliced reads cross 2^29 at any record count
+        const uint32_t spacing = sh.kind == 4 ? (uint32_t)(sh.contigs[c].len / (sh.cum[c + 1] - sh.cum[c])) : 0;
+        uint32_t skip = 100 + rng.below(sh.kind == 4 ? std::min<uint32_t>(std::max<uint32_t>(199901, 8 * spacing), 1u << 26) : 199901);
         cg[n++] = op(a, 0); cg[n++] = op(skip, 3); cg[n++] = op(R - a, 0);
         if (k < 60 && R - a > 20) {  // second junction
           uint32_t b = 5 + rng.below(R - a - 10);
@@ -337,6 +345,7 @@ void make_meta(const Shape& sh, uint64_t i, Meta& m) {
   if (c >= 0) {
     int64_t end = (int64_t)m.pos + (m.span ? m.span : 1);
     m.bin = (uint16_t)reg2bin(m.pos, end);
+    if (end > (1 << 29)) m.bin = 4680;  // shape 4: past what the bin field addresses (reg2bin(-1, 0), as for no position)
   }
   if (R > 0 && rng.permille() < 2) m.missing_qual = true;
   m.size = 4 + 32 + kNameLen + cig_bytes + (R + 1) / 2 + R + kAuxLen;
@@ -357,7 +366,7 @@ void make_record(const Shape& sh, uint64_t i, const Meta& m, uint8_t* out) {
   char name[32];
   snprintf(name, sizeof name, "syn:%015llu", (unsigned long long)i);
   memcpy(p, name, kNameLen); p += kNameLen;
-  if (sh.kind == 2) {
+  if (m.long_read) {
     if (m.n_cigar) {
       LongCigar lc(m.rng_state, m.l_seq);
       while (uint32_t o = lc.next()) { put32(p, o); p += 4; }
@@ -443,6 +452,7 @@ void setup_shape(Shape& sh, int kind, uint64_t n, uint64_t seed) {
   sh.read_len = kind == 3 ? 100 : 150;
   if (kind == 0) sh.contigs.assign(kC1, kC1 + 3);
   else if (kind == 2) sh.contigs.assign(kWGS, kWGS + 5);
+  else if (kind == 4) sh.contigs.assign(kBig, kBig + 3);
   else sh.contigs.assign(kWGS, kWGS + 25);
   size_t n_ref = sh.contigs.size();
   sh.n_unmapped_tail = n / 100;
@@ -590,7 +600,8 @@ void build(const Shape& sh, int level, int threads, Built& out) {
   out.header_inflated = hdr.size();
   out.n_blocks = (uint32_t)(n_hdr_blocks + n_rec_blocks + 1);
 
-  // pass 3: BAI, one task per contig
+  // pass 3: BAI, one task per contig (none for shape 4: a BAI cannot address its references)
+  if (sh.kind == 4) return;
   size_t n_ref = sh.contigs.size();
   std::vector<BaiRef> refs(n_ref);
   auto voff_of = [&](uint64_t stream_byte) -> uint64_t {
@@ -680,7 +691,7 @@ struct synth_info {
 // Generates a BAM+BAI pair in memory. Buffers are malloc'd; release with synth_free.
 int synth_bam(int shape, uint64_t n_records, uint64_t seed, int level, int threads, uint8_t** bam,
               uint8_t** bai, synth_info* info) {
-  if (shape < 0 || shape > 3 || !bam || !bai) return -1;
+  if (shape < 0 || shape > 4 || !bam || !bai) return -1;
   if (threads <= 0) threads = (int)std::thread::hardware_concurrency();
   if (threads <= 0) threads = 1;
   Shape sh;
@@ -709,7 +720,7 @@ int synth_bam(int shape, uint64_t n_records, uint64_t seed, int level, int threa
 // corresponding records of the full file (records are pure functions of their global index).
 int synth_bam_subset(int shape, uint64_t n_records, uint64_t seed, int level, int threads, uint64_t contig_mask,
                      int with_tail, uint8_t** bam, uint8_t** bai, synth_info* info) {
-  if (shape < 0 || shape > 3 || !bam || !bai) return -1;
+  if (shape < 0 || shape > 4 || !bam || !bai) return -1;
   if (threads <= 0) threads = (int)std::thread::hardware_concurrency();
   if (threads <= 0) threads = 1;
   Shape sh;
@@ -763,7 +774,7 @@ void synth_free(void* p) { free(p); }
 #ifdef BAMGEN_MAIN
 int main(int argc, char** argv) {
   if (argc < 4) {
-    fprintf(stderr, "usage: bamgen <shape 0..3> <n_records> <out.bam> [seed] [zlib level] [threads]\n");
+    fprintf(stderr, "usage: bamgen <shape 0..4> <n_records> <out.bam> [seed] [zlib level] [threads]\n");
     return 2;
   }
   int shape = atoi(argv[1]);

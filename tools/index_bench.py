@@ -19,7 +19,14 @@ engine's and the oracle's byte for byte.
 --driver compares the host driver on a file: `qc --cuda-build-index` (one read) against `index` then `qc` (two reads), wall
 time per command sequence, alternated.  The driver reads with O_DIRECT, so the page cache does not serve the file.
 
-  python tools/index_bench.py [--records N] [--steps K] [--warmup W] [--chunk-mb M] [--no-oracle] [--gpus N | --driver] [--out FILE]
+--csi compares the CSI build (NGSQ_F_INDEX_CSI, min_shift 14, depth 5 on this workload) with the BAI build on the same
+file: index-only device time resident and end to end, the two engines alternated; the host assembly of each format, timed
+as the join of one part (ngsq_join_bai / ngsq_join_csi over a single NGSQ_F_INDEX_PART engine: the run sort, the chunks,
+the windows and the serialiser); then the CSI of bamgen shape 4 (references of 1.9 and 0.8 Gbp) at --shape4-records.  Both
+payloads must equal the oracle's (unless --no-oracle).
+
+  python tools/index_bench.py [--records N] [--steps K] [--warmup W] [--chunk-mb M] [--no-oracle] [--gpus N | --driver | --csi]
+                              [--shape4-records N] [--out FILE]
 """
 import argparse
 import ctypes as C
@@ -50,6 +57,8 @@ def main():
     p.add_argument("--no-oracle", action="store_true", help="skip the single-thread oracle index (minutes on 100 M records)")
     p.add_argument("--gpus", type=int, default=0, help="index parts on N devices (0: the one-engine measurements)")
     p.add_argument("--driver", action="store_true", help="qc --cuda-build-index against index + qc, from a file")
+    p.add_argument("--csi", action="store_true", help="CSI against BAI on the workload, then CSI on bamgen shape 4")
+    p.add_argument("--shape4-records", type=int, default=20_000_000)
     p.add_argument("--out", default=None)
     args = p.parse_args()
 
@@ -89,6 +98,8 @@ def main():
 
     if args.gpus:
         return parts_bench(args, pinned, pin, blocks, n_blocks, n_rec, C_bytes, D_bytes, d_comp, lib)
+    if args.csi:
+        return csi_bench(args, pinned, pin, blocks, n_blocks, n_rec, C_bytes, D_bytes, d_comp, cuts, wl, lib)
 
     def engine(flags):
         e = ffi.Engine(flags=flags, gc_seed=bench.GC_SEED, reserve_compressed=C_bytes, reserve_inflated=D_bytes + 65536, reserve_blocks=n_blocks + 16)
@@ -181,6 +192,122 @@ def main():
     lib.ngsq_host_free(pin)
     if not out["equal_to_bamgen_up_to_its_linear_clamp"] or out.get("equal_to_oracle") is False:
         raise SystemExit("the GPU index differs from the reference indexes")
+
+
+def _index_run(eng_factory, flags, pinned, d_comp, C_bytes, blocks, n_blocks, pin=None, cuts=None):
+    """One index-only run of a fresh engine: resident (d_comp) or streamed from pinned memory (cuts); (wall ms, device ms,
+    engine)."""
+    e = eng_factory(flags)
+    t = time.perf_counter()
+    if cuts is None:
+        e.submit_device(d_comp.data_ptr(), C_bytes, blocks, n_blocks)
+    else:
+        for a, b in zip(cuts[:-1], cuts[1:]):
+            if b == C_bytes:
+                e.flush()
+            e.submit_ptr(pin + a, b - a, a)
+    e.finish()
+    return (time.perf_counter() - t) * 1e3, e.stats()["ms_total"], e
+
+
+def csi_bench(args, pinned, pin, blocks, n_blocks, n_rec, C_bytes, D_bytes, d_comp, cuts, wl, lib):
+    import torch
+    from ngs_b200 import ffi, formats
+    from baiutil import oracle_bai
+    from csiutil import oracle_csi
+    med = lambda xs: float(np.median(xs))  # noqa: E731
+    crc = ffi.NGSQ_F_VERIFY_CRC
+
+    def factory(data, c_bytes, d_bytes, nb):
+        def make(flags):
+            e = ffi.Engine(flags=flags, reserve_compressed=c_bytes, reserve_inflated=d_bytes + 65536, reserve_blocks=nb + 16)
+            hdr = formats.read_header(e, data)
+            e.set_references([l for _, l in hdr.refs], [0] * len(hdr.refs))
+            e.set_range(hdr.first_voffset, 0)
+            return e
+        return make
+
+    make = factory(pinned, C_bytes, D_bytes, n_blocks)
+    fmt = {"bai": ffi.NGSQ_F_INDEX | crc, "csi": ffi.NGSQ_F_INDEX | ffi.NGSQ_F_INDEX_CSI | crc}
+    get = {"bai": lambda e: e.bai(), "csi": lambda e: e.csi()}
+    res, ee, payload = {"bai": [], "csi": []}, {"bai": [], "csi": []}, {}
+    for step in range(args.warmup + args.steps):
+        for f in ("bai", "csi"):  # alternated
+            w, d, e = _index_run(make, fmt[f], pinned, d_comp, C_bytes, blocks, n_blocks)
+            payload.setdefault(f, get[f](e))
+            assert get[f](e) == payload[f]
+            e.close()
+            if step >= args.warmup:
+                res[f].append((w, d))
+    for step in range(1 + args.steps):
+        for f in ("bai", "csi"):
+            w, d, e = _index_run(make, fmt[f], pinned, d_comp, C_bytes, blocks, n_blocks, pin=pin, cuts=cuts)
+            assert get[f](e) == payload[f]
+            e.close()
+            if step:
+                ee[f].append((w, d))
+    # host assembly: the join of one part engine (the whole file) per format
+    join = {"bai": ffi.join_bai, "csi": ffi.join_csi}
+    assembly = {}
+    for f in ("bai", "csi"):
+        _, _, p = _index_run(make, (fmt[f] & ~ffi.NGSQ_F_INDEX) | ffi.NGSQ_F_INDEX_PART, pinned, d_comp, C_bytes, blocks, n_blocks)
+        ts = []
+        for _ in range(args.steps):
+            t = time.perf_counter()
+            assert join[f]([p]) == payload[f]
+            ts.append((time.perf_counter() - t) * 1e3)
+        assembly[f] = med(ts)
+        p.close()
+    csi = formats.parse_csi(payload["csi"])
+    out = {
+        "metric": "CSI (min_shift 14) against BAI build, index only", "records": n_rec, "compressed_bytes": C_bytes,
+        "inflated_bytes": D_bytes, "zlib_level": wl["level"], "steps": args.steps, "warmup": args.warmup, "gpu": gpu_name_and_power(),
+        "gpu_count": torch.cuda.device_count(), "csi_min_shift": csi.min_shift, "csi_depth": csi.depth,
+    }
+    for f in ("bai", "csi"):
+        out[f"{f}_resident_ms_device"] = med([r[1] for r in res[f]])
+        out[f"{f}_resident_ms_wall"] = med([r[0] for r in res[f]])
+        out[f"{f}_e2e_ms_device"] = med([r[1] for r in ee[f]])
+        out[f"{f}_e2e_ms_wall"] = med([r[0] for r in ee[f]])
+        out[f"{f}_host_assembly_ms"] = assembly[f]
+        out[f"{f}_bytes"] = len(payload[f])
+    if not args.no_oracle:
+        out["bai_equal_to_oracle"] = oracle_bai(pinned) == payload["bai"]
+        out["csi_equal_to_oracle"] = oracle_csi(pinned) == payload["csi"]
+    del d_comp
+    torch.cuda.synchronize()
+    lib.ngsq_host_free(pin)
+
+    # shape 4: references past 2^29 and 2^30
+    t0 = time.perf_counter()
+    bam4, _, info4 = ffi.synth_bam(4, args.shape4_records, level=wl["level"])
+    gen_s = time.perf_counter() - t0
+    C4, D4 = int(bam4.size), int(info4["inflated_bytes"])
+    b4, nb4, _ = ffi.bgzf_walk(bam4)
+    d4 = torch.empty(C4 + 512, dtype=torch.uint8, device="cuda")
+    d4[:C4].copy_(torch.from_numpy(np.asarray(bam4)))
+    torch.cuda.synchronize()
+    make4 = factory(bam4, C4, D4, nb4)
+    r4, first = [], None
+    for step in range(args.warmup + args.steps):
+        w, d, e = _index_run(make4, fmt["csi"], bam4, d4, C4, b4, nb4)
+        first = first or e.csi()
+        assert e.csi() == first
+        e.close()
+        if step >= args.warmup:
+            r4.append((w, d))
+    _, _, p = _index_run(make4, ffi.NGSQ_F_INDEX_PART | ffi.NGSQ_F_INDEX_CSI | crc, bam4, d4, C4, b4, nb4)
+    t = time.perf_counter()
+    assert ffi.join_csi([p]) == first
+    out["shape4"] = {"records": int(info4["n_records"]), "compressed_bytes": C4, "inflated_bytes": D4, "generate_s": gen_s,
+                     "csi_depth": formats.parse_csi(first).depth, "csi_resident_ms_device": med([r[1] for r in r4]),
+                     "csi_resident_ms_wall": med([r[0] for r in r4]), "csi_host_assembly_ms": (time.perf_counter() - t) * 1e3,
+                     "csi_bytes": len(first)}
+    if not args.no_oracle:
+        out["shape4"]["csi_equal_to_oracle"] = oracle_csi(bam4) == first
+    _emit(args, out)
+    if out.get("csi_equal_to_oracle") is False or out.get("bai_equal_to_oracle") is False or out["shape4"].get("csi_equal_to_oracle") is False:
+        raise SystemExit("the GPU index differs from the oracle's")
 
 
 def _emit(args, out):

@@ -1,8 +1,9 @@
-// CPU model of the BAI index kernel (test tooling; NOT part of the product library): runs the per-record functions the
+// CPU model of the BAI / CSI index kernel (test tooling; NOT part of the product library): runs the per-record functions the
 // CUDA kernel calls (ngs_b200/csrc/index.cuh: index_record, index_windows) over every
 // record of a BAM, with the virtual offsets the engine gives them.
 //   g++ -O2 -std=c++17 -o /tmp/index_model tools/index_model.cpp -lz
 //   /tmp/index_model file.bam   -> per record "ref pos bin beg end placed unmapped voff w_lo w_hi", or a last line "error <kind>"
+//   /tmp/index_model file.bam --csi MIN_SHIFT DEPTH   -> the same with the CSI key and windows of 2^MIN_SHIFT bases
 #include <zlib.h>
 
 #include <cstdio>
@@ -27,7 +28,9 @@ static std::vector<uint8_t> slurp(const char* path) {
 }
 
 int main(int argc, char** argv) {
-  if (argc < 2) { fprintf(stderr, "usage: %s file.bam\n", argv[0]); return 2; }
+  const bool csi = argc == 5 && !strcmp(argv[2], "--csi");
+  if (argc != 2 && !csi) { fprintf(stderr, "usage: %s file.bam [--csi MIN_SHIFT DEPTH]\n", argv[0]); return 2; }
+  const uint32_t min_shift = csi ? (uint32_t)atoi(argv[3]) : kIxWindowShift, depth = csi ? (uint32_t)atoi(argv[4]) : 5;
   std::vector<uint8_t> bam = slurp(argv[1]);
   // inflated stream + file offset of the block that holds each of its bytes (non-empty blocks only, like the engine)
   std::vector<uint8_t> s;
@@ -69,10 +72,10 @@ int main(int argc, char** argv) {
     uint32_t bs;
     memcpy(&bs, &s[p], 4);
     IndexKey k;
-    const uint32_t err = index_record(&s[p], (int32_t)n_ref, &k);
+    const uint32_t err = index_record(&s[p], (int32_t)n_ref, &k, csi, min_shift, depth);
     if (err) { printf("error %u\n", err); return 0; }
     uint32_t w_lo = 0, w_hi = 0;
-    if (k.placed) index_windows(k, &w_lo, &w_hi);
+    if (k.placed) index_windows(k, &w_lo, &w_hi, min_shift);
     printf("%d %d %u %llu %llu %u %u %llu %u %u\n", k.ref, k.pos, k.bin, (unsigned long long)k.beg, (unsigned long long)k.end, k.placed,
            k.unmapped, (unsigned long long)voff(p), w_lo, w_hi);
     p += 4 + (size_t)bs;
