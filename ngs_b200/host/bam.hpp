@@ -157,6 +157,79 @@ inline BaiIndex read_bai(const std::string& path) {
   return idx;
 }
 
+// CSIv1 (the CSI spec; `samtools index -c`, `ngs-cuda-qc index --csi`), UNCOMPRESSED, read into the planner's input: each
+// reference's extent and counts from its pseudo-bin ((1 << 3(depth + 1)) - 1) / 7 + 1 (BAI bin 37450's fields), and as its
+// ioffset the loffsets of its other bins, sorted.  A bin's loffset is the virtual offset of the first record overlapping its first
+// window (htslib forward-fills empty windows, may store 0 or all ones, and folds small bins into a parent holding the minimum):
+// a record start or a value bai_anchors drops.  The aux bytes (tabix meta) are skipped.  `path` names the file in errors.
+inline BaiIndex parse_csi(const uint8_t* p, size_t n, const std::string& path, size_t n_ref_header) {
+  size_t o = 0;
+  auto fail = [&](const std::string& what) { throw std::runtime_error("reading CSI index " + path + ": " + what); };
+  auto need = [&](uint64_t k, const char* field) { if (k > n - o) fail(std::string("truncated in ") + field); };
+  auto i32 = [&](size_t at) { int32_t v; memcpy(&v, p + at, 4); return v; };
+  need(16, "the header");
+  if (memcmp(p, "CSI\1", 4)) fail("bad magic");
+  const int32_t min_shift = i32(4), depth = i32(8), l_aux = i32(12);
+  // bins are u32: the pseudo-bin's 1 << 3(depth + 1) fits 32 bits up to depth 9; coordinates are 64-bit
+  if (depth < 0 || depth > 9 || min_shift < 0 || (int64_t)min_shift + 3 * depth > 63)
+    fail("min_shift " + std::to_string(min_shift) + " with depth " + std::to_string(depth) + " overflows the bin arithmetic");
+  if (l_aux < 0) fail("negative l_aux");
+  o = 16;
+  if ((uint64_t)l_aux > n - o) fail("l_aux " + std::to_string(l_aux) + " runs past the end");
+  o += (size_t)l_aux;
+  need(4, "n_ref");
+  const int32_t n_ref = i32(o);
+  o += 4;
+  if (n_ref < 0 || (size_t)n_ref != n_ref_header)
+    fail(std::to_string(n_ref) + " references, the BAM header has " + std::to_string(n_ref_header));
+  const uint32_t meta = ((1u << (3 * (depth + 1))) - 1) / 7 + 1;
+  BaiIndex idx;
+  for (int32_t r = 0; r < n_ref; ++r) {
+    BaiReference R;
+    need(4, "n_bin");
+    const int32_t n_bin = i32(o);
+    o += 4;
+    if (n_bin < 0) fail("negative n_bin");
+    R.n_bins = (uint32_t)n_bin;
+    for (int32_t k = 0; k < n_bin; ++k) {
+      need(16, "a bin");
+      uint32_t bin;
+      uint64_t loffset;
+      memcpy(&bin, p + o, 4);
+      memcpy(&loffset, p + o + 4, 8);
+      const int32_t n_chunk = i32(o + 12);
+      o += 16;
+      if (n_chunk < 0 || 16ull * (uint32_t)n_chunk > n - o) fail("n_chunk " + std::to_string(n_chunk) + " runs past the end");
+      if (bin == meta && n_chunk == 2) {
+        memcpy(&R.ref_beg, p + o, 8); memcpy(&R.ref_end, p + o + 8, 8);
+        memcpy(&R.n_mapped, p + o + 16, 8); memcpy(&R.n_unmapped, p + o + 24, 8);
+        R.has_extent = R.ref_end > R.ref_beg;
+      } else {
+        R.ioffset.push_back(loffset);
+      }
+      o += 16ull * (uint32_t)n_chunk;
+    }
+    std::sort(R.ioffset.begin(), R.ioffset.end());
+    R.n_intv = (uint32_t)R.ioffset.size();
+    idx.refs.push_back(std::move(R));
+  }
+  if (o + 8 <= n) { idx.has_n_no_coor = true; memcpy(&idx.n_no_coor, p + o, 8); }
+  return idx;
+}
+
+// <BAM>.csi: BGZF framed on the host and inflated on the GPU (ngsq_inflate_to_host), like the BAM header, then parse_csi.
+inline BaiIndex read_csi(ngsq_engine* e, const std::string& path, size_t n_ref_header) {
+  MappedFile f(path);
+  uint32_t nb = 0;
+  size_t used = 0;
+  if (f.size() && (ngsq_bgzf_walk(f.data(), f.size(), 0, nullptr, 0, &nb, &used) || used != f.size()))
+    throw std::runtime_error("reading CSI index " + path + ": malformed BGZF framing");
+  std::vector<uint8_t> payload((size_t)nb * 65536 + 16);
+  size_t got = 0;
+  if (used) check(e, ngsq_inflate_to_host(e, f.data(), used, payload.data(), payload.size(), &got));
+  return parse_csi(payload.data(), got, path, n_ref_header);
+}
+
 // One contiguous range of the file owned by a shard.
 struct Shard {
   uint64_t first_voffset = 0, end_voffset = 0;  // end 0 = to EOF

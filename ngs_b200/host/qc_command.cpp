@@ -6,11 +6,12 @@
 //
 // A BAM without an index is cut between GPUs at record anchors the engine finds (ngsq_find_record), each GPU indexes its part
 // (NGSQ_F_INDEX_PART) and the host joins the parts (ngsq_join_bai): `index --cuda-devices`, and `qc --cuda-build-index`,
-// which writes the missing .bai in the same pass as the results.
+// which writes the missing index (.bai, or .csi with --cuda-csi) in the same pass as the results.  `qc` plans its shards from
+// <BAM>.bai, or from <BAM>.csi when there is no .bai (the reference needs the .bai).
 //
 //   ngs-cuda-qc qc <BAM> <REFERENCE_GENOME> [-n N] [-o DIR] [-p PREFIX] [--only FACET]
-//               [--cuda-devices 0,1,..] [--cuda-build-index] [--cuda-gc-seed S] [--cuda-no-crc] [--cuda-chunk-mb M]
-//               [--cuda-buffered-io] [--cuda-perf]
+//               [--cuda-devices 0,1,..] [--cuda-build-index [--cuda-csi [--cuda-min-shift N]]] [--cuda-gc-seed S]
+//               [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io] [--cuda-perf]
 //   ngs-cuda-qc index <BAM> [--csi [-m|--min-shift N]] [--cuda-device N | --cuda-devices 0,1,..] [--cuda-no-crc] [--cuda-chunk-mb M]
 //                     [--cuda-buffered-io]
 #include <cerrno>
@@ -47,7 +48,9 @@ struct QcArgs {
   size_t chunk_mb = 64;
   bool direct_io = true;
   bool perf = false;
-  bool build_index = false;  // a missing .bai is built in the same pass and written next to the BAM
+  bool build_index = false;  // a missing index is built in the same pass and written next to the BAM
+  bool csi = false;          // --cuda-csi: that index is <BAM>.csi instead of <BAM>.bai
+  uint32_t min_shift = 14;   // --cuda-min-shift (CSI); the depth follows samtools' rule
 };
 
 void info(const std::string& s) { std::cerr << "INFO " << s << "\n"; }
@@ -314,9 +317,13 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
     throw std::runtime_error("could not open " + args.src + ": expected a .bam file");
   MappedFile file(args.src);
   const std::string bai_path = args.src + ".bai";  // pathbuf.rs:59-75: x.bam -> x.bam.bai
-  // --cuda-build-index: an existing index is used as it is; a missing one is built by this pass
-  const bool build_index = args.build_index && !std::filesystem::exists(bai_path);
-  BaiIndex bai = build_index ? BaiIndex{} : read_bai(bai_path);
+  const std::string csi_path = args.src + ".csi";  // x.bam -> x.bam.csi: planned from when there is no .bai
+  const bool have_bai = std::filesystem::exists(bai_path), have_csi = !have_bai && std::filesystem::exists(csi_path);
+  // --cuda-build-index: an existing index (.bai, else .csi) is used as it is; a missing one is built by this pass
+  const bool build_index = args.build_index && !have_bai && !have_csi;
+  const bool build_csi = build_index && args.csi;
+  // the .csi is BGZF: it is read once an engine can inflate it (below); without any index read_bai reports the missing .bai
+  BaiIndex bai = build_index || have_csi ? BaiIndex{} : read_bai(bai_path);
   const uint32_t n_dev = (uint32_t)args.devices.size();
 
   // facets first (cheap) so `--only` errors surface before any device work.  The two optional facets read their
@@ -337,7 +344,7 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   if (features) flags |= NGSQ_F_FEATURES;
   if (edits) flags |= NGSQ_F_EDITS;
   if (args.verify_crc) flags |= NGSQ_F_VERIFY_CRC;
-  if (build_index) flags |= n_dev > 1 ? NGSQ_F_INDEX_PART : NGSQ_F_INDEX;
+  if (build_index) flags |= (n_dev > 1 ? NGSQ_F_INDEX_PART : NGSQ_F_INDEX) | (build_csi ? NGSQ_F_INDEX_CSI : 0u);
   if (args.num_records && n_dev > 1) throw std::runtime_error("-n needs a single device (records are counted in file order)");
 
   std::vector<ngsq_engine*> engines(n_dev, nullptr);
@@ -349,8 +356,10 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
     cfg.gc_seed = args.gc_seed;
     cfg.max_records = args.num_records.value_or(0);
     if (ngsq_create(args.devices[i], &cfg, &engines[i])) throw std::runtime_error(std::string("CUDA engine: ") + ngsq_last_error(nullptr));
+    if (build_csi) check(engines[i], ngsq_set_index_binning(engines[i], args.min_shift, 0));  // before any ngsq_set_references
   }
   BamHeader header = read_bam_header(engines[0], file.data(), file.size());
+  if (have_csi) bai = read_csi(engines[0], csi_path, header.reference_sequences.size());
 
   if (!std::filesystem::exists(output_directory)) std::filesystem::create_directories(output_directory);
 
@@ -365,7 +374,7 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   for (auto& f : facets.record_based) info(std::string("  [*] ") + f->name() + ", " + to_string(f->computational_load()));
   for (auto& f : facets.sequence_based) info(std::string("  [*] ") + f->name() + ", " + to_string(f->computational_load()));
 
-  // shards: contig-aligned file ranges from the BAI, or ranges cut inside contigs when those leave a device idle or
+  // shards: contig-aligned file ranges from the index (BAI or CSI), or ranges cut inside contigs when those leave a device idle or
   // unbalanced (choose_shards); a contig cut between shards is declared on every engine and merged by ngsq_reduce
   std::vector<uint32_t> ref_len;
   for (auto& rs : header.reference_sequences) ref_len.push_back(rs.length);
@@ -428,13 +437,14 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
     for (auto& s : errs) if (!s.empty()) throw std::runtime_error("NCCL: " + s);
   }
   // the index of this pass: joined (and its order checked) before any output is written
-  std::vector<uint8_t> new_bai;
-  if (build_index && n_dev > 1) new_bai = join_parts(engines, shards);
+  std::vector<uint8_t> new_index;
+  if (build_index && n_dev > 1) new_index = join_parts(engines, shards, build_csi);
   else if (build_index) {
+    auto get = build_csi ? ngsq_get_csi : ngsq_get_bai;
     size_t n = 0;
-    check(engines[0], ngsq_get_bai(engines[0], nullptr, 0, &n));
-    new_bai.resize(n);
-    check(engines[0], ngsq_get_bai(engines[0], new_bai.data(), new_bai.size(), &n));
+    check(engines[0], get(engines[0], nullptr, 0, &n));
+    new_index.resize(n);
+    check(engines[0], get(engines[0], new_index.data(), new_index.size(), &n));
   }
   const double hot_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_hot).count();
   ngsq_engine* root = engines[0];
@@ -467,7 +477,7 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   for (auto& f : facets.sequence_based) f->aggregate(results);
   info("Writing output.");
   results.write(output_prefix, output_directory);
-  if (build_index) write_index(bai_path, new_bai);
+  if (build_index) write_index(build_csi ? csi_path : bai_path, build_csi ? bgzf_compress(new_index) : new_index);
 
   if (args.perf) {
     std::ofstream pf(output_directory + "/" + output_prefix + ".perf.json");
@@ -616,9 +626,11 @@ int index_main(int argc, char** argv, int i) {
 
 void usage() {
   std::cerr << "usage: ngs-cuda-qc qc <BAM> <REFERENCE_GENOME> [-n N] [-o DIR] [-p PREFIX] [--only FACET]\n"
-               "                  [--cuda-devices 0,1,..] [--cuda-build-index] [--cuda-gc-seed S] [--cuda-no-crc] [--cuda-chunk-mb M]\n"
-               "                  [--cuda-buffered-io] [--cuda-perf]\n"
-               "                  (--cuda-build-index: without <BAM>.bai, build it in the same pass and write it once the run succeeded)\n"
+               "                  [--cuda-devices 0,1,..] [--cuda-build-index [--cuda-csi [--cuda-min-shift N]]] [--cuda-gc-seed S]\n"
+               "                  [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io] [--cuda-perf]\n"
+               "                  (the index is <BAM>.bai, or <BAM>.csi when there is no .bai; --cuda-build-index: without either,\n"
+               "                  build <BAM>.bai, or with --cuda-csi <BAM>.csi (min_shift N, default 14), in the same pass and write it\n"
+               "                  once the run succeeded)\n"
                "       ngs-cuda-qc index <BAM> [--csi [-m|--min-shift N]] [--cuda-device N | --cuda-devices 0,1,..] [--cuda-no-crc] [--cuda-chunk-mb M]\n"
                "                  [--cuda-buffered-io]\n"
                "                  (writes <BAM>.bai, or with --csi <BAM>.csi (min_shift N, default 14); an existing index is never overwritten;\n"
@@ -630,6 +642,7 @@ void usage() {
 extern "C" int ngs_cuda_qc_main(int argc, char** argv) {
   try {
     QcArgs a;
+    bool min_shift_set = false;
     std::vector<std::string> pos;
     int i = 1;
     if (i < argc && std::string(argv[i]) == "index") {
@@ -659,6 +672,8 @@ extern "C" int ngs_cuda_qc_main(int argc, char** argv) {
       else if (s == "--cuda-chunk-mb") a.chunk_mb = std::stoull(val());
       else if (s == "--cuda-perf") a.perf = true;
       else if (s == "--cuda-build-index") a.build_index = true;
+      else if (s == "--cuda-csi") a.csi = true;
+      else if (s == "--cuda-min-shift") { a.min_shift = (uint32_t)std::stoul(val()); min_shift_set = true; }
       else if (s == "--cuda-buffered-io") a.direct_io = false;
       else if (s == "-h" || s == "--help") { usage(); return 0; }
       else if (!s.empty() && s[0] == '-' && s != "-") throw std::runtime_error("unknown flag " + s);
@@ -666,6 +681,8 @@ extern "C" int ngs_cuda_qc_main(int argc, char** argv) {
     }
     if (pos.size() != 2 || a.devices.empty()) { usage(); return 2; }
     if (a.build_index && a.num_records) throw std::runtime_error("--cuda-build-index cannot be combined with -n: an index covers every record of the file");
+    if (a.csi && !a.build_index) throw std::runtime_error("--cuda-csi sets the format of the index --cuda-build-index writes: use it with --cuda-build-index");
+    if (min_shift_set && !a.csi) throw std::runtime_error("--cuda-min-shift sets the binning of a CSI: use it with --cuda-csi");
     a.src = pos[0];
     a.reference_genome = pos[1];
     return qc(a);
