@@ -524,7 +524,9 @@ impl Engine {
 
     // ---- shards cut inside a contig (DESIGN.md section 5) ----
     /// Declares reference `r` split between shards: the same set on every engine, after `set_references`, before the first
-    /// submit.  Its coverage and VAF counters are resolved by `reduce` (or `resolve_split`), not by `finish`.
+    /// submit.  Its coverage and VAF counters are resolved by `reduce` (or `resolve_split`), not by `finish`.  With records in
+    /// any order (`--cuda-any-order` on several devices) every reference of the header is declared: any contig can have
+    /// records on both sides of any cut.
     pub fn split_reference(&mut self, r: u32) -> anyhow::Result<()> {
         self.check(unsafe { sys::ngsq_split_reference(self.raw, r) })
     }

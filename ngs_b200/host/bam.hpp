@@ -463,6 +463,23 @@ inline ShardPlan plan_shards_unindexed(const BamHeader& h, const uint8_t* bam, u
   return plan;
 }
 
+// Records in any order (`qc --cuda-any-order`, DESIGN 5): one shard from the first record to EOF, or on several devices the
+// cuts of plan_shards_unindexed.  Any reference can then have records on both sides of any cut, so the anchors' references
+// are no complete split set: every reference of the header is split (Coverage's and, for Edits, the ones Coverage skips).
+inline ShardPlan plan_shards_any_order(const BamHeader& h, const uint8_t* bam, uint64_t file_size, uint32_t n_shards, const FindRecord& find) {
+  ShardPlan plan;
+  if (n_shards <= 1) {
+    Shard s;
+    s.first_voffset = h.first_record_voffset;
+    plan.shards.push_back(s);
+    return plan;
+  }
+  plan = plan_shards_unindexed(h, bam, file_size, n_shards, find);
+  plan.split.clear();
+  for (uint32_t c = 0; c < h.reference_sequences.size(); ++c) plan.split.push_back(c);
+  return plan;
+}
+
 // Compressed byte range [lo, hi) a shard submits: through the block that holds end_voffset.
 inline void shard_bytes(const Shard& s, const uint8_t* bam, uint64_t file_size, uint64_t* lo, uint64_t* hi) {
   *lo = s.first_voffset >> 16;

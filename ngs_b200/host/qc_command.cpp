@@ -7,10 +7,12 @@
 // A BAM without an index is cut between GPUs at record anchors the engine finds (ngsq_find_record), each GPU indexes its part
 // (NGSQ_F_INDEX_PART) and the host joins the parts (ngsq_join_bai): `index --cuda-devices`, and `qc --cuda-build-index`,
 // which writes the missing index (.bai, or .csi with --cuda-csi) in the same pass as the results.  `qc` plans its shards from
-// <BAM>.bai, or from <BAM>.csi when there is no .bai (the reference needs the .bai).
+// <BAM>.bai, or from <BAM>.csi when there is no .bai (the reference needs the .bai).  `qc --cuda-any-order` reads no index and
+// takes records in any order (unsorted, queryname-sorted or collated files): one shard, or cuts at record anchors with every
+// reference split between the devices.
 //
 //   ngs-cuda-qc qc <BAM> <REFERENCE_GENOME> [-n N] [-o DIR] [-p PREFIX] [--only FACET]
-//               [--cuda-devices 0,1,..] [--cuda-build-index [--cuda-csi [--cuda-min-shift N]]] [--cuda-gc-seed S]
+//               [--cuda-devices 0,1,..] [--cuda-build-index [--cuda-csi [--cuda-min-shift N]] | --cuda-any-order] [--cuda-gc-seed S]
 //               [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io] [--cuda-perf]
 //   ngs-cuda-qc index <BAM> [--csi [-m|--min-shift N]] [--cuda-device N | --cuda-devices 0,1,..] [--cuda-no-crc] [--cuda-chunk-mb M]
 //                     [--cuda-buffered-io]
@@ -51,6 +53,7 @@ struct QcArgs {
   bool build_index = false;  // a missing index is built in the same pass and written next to the BAM
   bool csi = false;          // --cuda-csi: that index is <BAM>.csi instead of <BAM>.bai
   uint32_t min_shift = 14;   // --cuda-min-shift (CSI); the depth follows samtools' rule
+  bool any_order = false;    // --cuda-any-order: no index is read, the records may come in any order
 };
 
 void info(const std::string& s) { std::cerr << "INFO " << s << "\n"; }
@@ -318,12 +321,13 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   MappedFile file(args.src);
   const std::string bai_path = args.src + ".bai";  // pathbuf.rs:59-75: x.bam -> x.bam.bai
   const std::string csi_path = args.src + ".csi";  // x.bam -> x.bam.csi: planned from when there is no .bai
-  const bool have_bai = std::filesystem::exists(bai_path), have_csi = !have_bai && std::filesystem::exists(csi_path);
+  // --cuda-any-order: neither index is read, even when one exists (it may belong to another order of the same records)
+  const bool have_bai = !args.any_order && std::filesystem::exists(bai_path), have_csi = !args.any_order && !have_bai && std::filesystem::exists(csi_path);
   // --cuda-build-index: an existing index (.bai, else .csi) is used as it is; a missing one is built by this pass
   const bool build_index = args.build_index && !have_bai && !have_csi;
   const bool build_csi = build_index && args.csi;
   // the .csi is BGZF: it is read once an engine can inflate it (below); without any index read_bai reports the missing .bai
-  BaiIndex bai = build_index || have_csi ? BaiIndex{} : read_bai(bai_path);
+  BaiIndex bai = build_index || have_csi || args.any_order ? BaiIndex{} : read_bai(bai_path);
   const uint32_t n_dev = (uint32_t)args.devices.size();
 
   // facets first (cheap) so `--only` errors surface before any device work.  The two optional facets read their
@@ -379,16 +383,23 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   std::vector<uint32_t> ref_len;
   for (auto& rs : header.reference_sequences) ref_len.push_back(rs.length);
   ShardPlan plan;
-  if (build_index && n_dev > 1) {
+  const bool cut_at_anchors = (build_index || args.any_order) && n_dev > 1;
+  if (cut_at_anchors) {
     // no index to cut at: anchors from the records (the finder needs the references; every engine sets them again below)
     check(engines[0], ngsq_set_references(engines[0], (uint32_t)ref_len.size(), ref_len.data(), std::vector<uint8_t>(ref_len.size(), 0).data()));
-    plan = plan_shards_unindexed(header, file.data(), file.size(), n_dev, engine_finder(engines[0]));
+    const FindRecord find = engine_finder(engines[0]);
+    plan = args.any_order ? plan_shards_any_order(header, file.data(), file.size(), n_dev, find)
+                          : plan_shards_unindexed(header, file.data(), file.size(), n_dev, find);
     log_dropped_cuts(plan);
+  } else if (args.any_order) {
+    plan = plan_shards_any_order(header, file.data(), file.size(), 1, nullptr);
   } else {
     plan = choose_shards(header, bai, n_dev, file.size());
   }
   std::vector<Shard> shards = plan.shards;
-  if (plan.split_plan) {
+  if (args.any_order && n_dev > 1) {
+    info("  [*] Records in any order: " + std::to_string(n_dev - plan.dropped) + " shards, every reference split.");
+  } else if (plan.split_plan) {
     std::string names;
     for (uint32_t c : plan.split) names += (names.empty() ? "" : ", ") + header.reference_sequences[c].name;
     info("  [*] Sharding inside contigs: " + std::to_string(n_dev) + " shards" + (names.empty() ? std::string() : ", split: " + names) + ".");
@@ -419,7 +430,7 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   // the hot path: one thread per GPU
   info("Starting CUDA pass for QC stats.");
   const auto t_hot = std::chrono::steady_clock::now();
-  if (build_index && n_dev > 1) {
+  if (cut_at_anchors) {
     run_parts(engines, shards, args.src, file, args.chunk_mb << 20, args.direct_io);
   } else {
     std::vector<std::thread> ts;
@@ -626,11 +637,12 @@ int index_main(int argc, char** argv, int i) {
 
 void usage() {
   std::cerr << "usage: ngs-cuda-qc qc <BAM> <REFERENCE_GENOME> [-n N] [-o DIR] [-p PREFIX] [--only FACET]\n"
-               "                  [--cuda-devices 0,1,..] [--cuda-build-index [--cuda-csi [--cuda-min-shift N]]] [--cuda-gc-seed S]\n"
-               "                  [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io] [--cuda-perf]\n"
+               "                  [--cuda-devices 0,1,..] [--cuda-build-index [--cuda-csi [--cuda-min-shift N]] | --cuda-any-order]\n"
+               "                  [--cuda-gc-seed S] [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io] [--cuda-perf]\n"
                "                  (the index is <BAM>.bai, or <BAM>.csi when there is no .bai; --cuda-build-index: without either,\n"
                "                  build <BAM>.bai, or with --cuda-csi <BAM>.csi (min_shift N, default 14), in the same pass and write it\n"
-               "                  once the run succeeded)\n"
+               "                  once the run succeeded; --cuda-any-order: read no index and take the records in any order, not\n"
+               "                  with -n, --cuda-build-index or --cuda-csi)\n"
                "       ngs-cuda-qc index <BAM> [--csi [-m|--min-shift N]] [--cuda-device N | --cuda-devices 0,1,..] [--cuda-no-crc] [--cuda-chunk-mb M]\n"
                "                  [--cuda-buffered-io]\n"
                "                  (writes <BAM>.bai, or with --csi <BAM>.csi (min_shift N, default 14); an existing index is never overwritten;\n"
@@ -673,6 +685,7 @@ extern "C" int ngs_cuda_qc_main(int argc, char** argv) {
       else if (s == "--cuda-perf") a.perf = true;
       else if (s == "--cuda-build-index") a.build_index = true;
       else if (s == "--cuda-csi") a.csi = true;
+      else if (s == "--cuda-any-order") a.any_order = true;
       else if (s == "--cuda-min-shift") { a.min_shift = (uint32_t)std::stoul(val()); min_shift_set = true; }
       else if (s == "--cuda-buffered-io") a.direct_io = false;
       else if (s == "-h" || s == "--help") { usage(); return 0; }
@@ -680,6 +693,11 @@ extern "C" int ngs_cuda_qc_main(int argc, char** argv) {
       else pos.push_back(s);
     }
     if (pos.size() != 2 || a.devices.empty()) { usage(); return 2; }
+    if (a.any_order && a.num_records)
+      throw std::runtime_error("--cuda-any-order cannot be combined with -n: the first N records are counted in the order of the per-contig "
+                               "queries, which records in any order do not have");
+    if (a.any_order && a.build_index) throw std::runtime_error("--cuda-any-order cannot be combined with --cuda-build-index: an index needs coordinate-sorted records");
+    if (a.any_order && a.csi) throw std::runtime_error("--cuda-any-order cannot be combined with --cuda-csi: an index needs coordinate-sorted records");
     if (a.build_index && a.num_records) throw std::runtime_error("--cuda-build-index cannot be combined with -n: an index covers every record of the file");
     if (a.csi && !a.build_index) throw std::runtime_error("--cuda-csi sets the format of the index --cuda-build-index writes: use it with --cuda-build-index");
     if (min_shift_set && !a.csi) throw std::runtime_error("--cuda-min-shift sets the binning of a CSI: use it with --cuda-csi");
