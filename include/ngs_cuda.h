@@ -188,6 +188,17 @@ int ngsq_submit(ngsq_engine* e, const uint8_t* bgzf, size_t nbytes, uint64_t fil
 /* Enqueues a wave for every block submitted so far instead of waiting for a full one.  A caller that knows its last
  * chunk calls this just before submitting it: what remains after the last copied byte is then one small wave. */
 int ngsq_flush(ngsq_engine* e);
+/* Several files in one run (`qc --cuda-also`, DESIGN.md section 5, "Several files"): the chunks submitted since the last
+ * ngsq_set_range form one whole file.  This call enqueues that file's last wave as ngsq_flush does, so that no wave holds
+ * blocks of two files, and a record still open at its end fails the run with NGSQ_E_TRUNCATED at ngsq_finish.  It drops the
+ * open-record carry and the end-of-range state, so no record chain links two files, and leaves every accumulator as it is:
+ * the facet histograms, Coverage's difference arrays and touched words, the Edits and Genomic Features state, the quality
+ * table and the stats (ngsq_get_stats sums over the files of the run).  The caller then calls ngsq_set_range for the next
+ * file and submits its chunks at that file's own offsets; ngsq_finish (and ngsq_reduce) run once, after the last file.  A
+ * file may contribute nothing: ngsq_set_range, no submit, ngsq_next_file.  NGSQ_E_ARG after ngsq_finish, with NGSQ_F_INDEX or
+ * NGSQ_F_INDEX_PART (an index describes one file), with max_records != 0 (`-n` counts in one file's order), and before the
+ * file's ngsq_set_range.  The GC window of a record is keyed by its virtual offset in its own file. */
+int ngsq_next_file(ngsq_engine* e);
 /* Records whose wave has been scanned so far (never blocks; lags the submits by about one wave): the caller's
  * RecordCounter log line, src/utils/display.rs:43-52. */
 int ngsq_progress(ngsq_engine* e, uint64_t* records);

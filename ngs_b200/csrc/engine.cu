@@ -179,6 +179,10 @@ struct ngsq_engine {
   uint64_t first_voff = 0, end_voff = 0;
   bool range_set = false, start_resolved = false, end_resolved = false;
   uint32_t start_block = 0, start_uo = 0, end_block = 0, end_uo = 0;
+  // several files in one run (ngsq_next_file): the current file's blocks are [file_b0, ..); between ngsq_next_file and the
+  // next ngsq_set_range no chunk may be submitted
+  uint32_t file_b0 = 0;
+  bool awaiting_range = false;
 
   ngsq_stats stats{};
   uint32_t other_launches = 0;
@@ -385,7 +389,7 @@ int append_blocks(ngsq_engine* e, const ngsq_block* blk, uint32_t n, uint64_t de
     const ngsq_block& b = blk[i];
     if (b.csize < b.hdr_len + 8 || b.isize > 65536) return fail(e, NGSQ_E_BAD_BLOCK, "malformed BGZF block at file offset %llu", (unsigned long long)b.coffset);
     if (b.isize == 0) continue;  // empty blocks (incl. the EOF marker) carry nothing
-    if (!e->h_blocks.empty() && b.coffset <= e->h_blocks.back().coff) return fail(e, NGSQ_E_ARG, "chunks must be submitted in file order (block at file offset %llu)", (unsigned long long)b.coffset);
+    if (e->h_blocks.size() > e->file_b0 && b.coffset <= e->h_blocks.back().coff) return fail(e, NGSQ_E_ARG, "chunks must be submitted in file order (block at file offset %llu)", (unsigned long long)b.coffset);
     BlockDesc d;
     d.in_off = dev_base_addr + (b.coffset - first_coffset) + b.hdr_len;
     d.out_off = e->out_used;
@@ -445,9 +449,9 @@ int upload_descriptors(ngsq_engine* e, uint32_t first, uint32_t end) {
   return NGSQ_OK;
 }
 
-// first block with file offset >= co among blocks [0, n)
+// first block with file offset >= co among the current file's blocks [file_b0, n)
 uint32_t block_lower_bound(const ngsq_engine* e, uint32_t n, uint64_t co) {
-  uint32_t lo = 0, hi = n;
+  uint32_t lo = e->file_b0, hi = n;
   while (lo < hi) {
     const uint32_t mid = lo + (hi - lo) / 2;
     if (e->h_blocks[mid].coff < co) lo = mid + 1; else hi = mid;
@@ -1301,6 +1305,7 @@ int ngsq_reset(ngsq_engine* e) {
   for (auto& ps : e->pin_slabs) ps.used = 0;
   e->out_used = 0; e->comp_bytes_total = 0; e->other_launches = 0;
   e->start_resolved = e->end_resolved = false;
+  e->file_b0 = 0; e->awaiting_range = false;
   e->prog_seen = 0; e->prog_records = 0;
   e->host_ms.clear();
   // rows of the quality table the next run has to clear; a run that never reached ngsq_finish may have touched any
@@ -1529,9 +1534,13 @@ int ngsq_set_reference_bases(ngsq_engine* e, uint32_t ref, const uint8_t* letter
 
 int ngsq_set_range(ngsq_engine* e, uint64_t first_rec_voffset, uint64_t end_voffset) {
   if (!e) return NGSQ_E_ARG;
-  if (e->launched) return fail(e, NGSQ_E_ARG, "ngsq_set_range must precede the first submit of a run");
+  if (e->launched && !e->awaiting_range) return fail(e, NGSQ_E_ARG, "ngsq_set_range must precede the first submit of a run");
   if ((e->cfg.flags & NGSQ_F_INDEX) && end_voffset)
     return fail(e, NGSQ_E_ARG, "NGSQ_F_INDEX needs end_voffset 0: an index covers the whole file from its first record");
+  if (e->awaiting_range) {  // the next file of the run: its blocks start behind the last one's
+    e->file_b0 = (uint32_t)e->h_blocks.size();
+    e->awaiting_range = false;
+  }
   e->first_voff = first_rec_voffset;
   e->end_voff = end_voffset;
   e->range_set = true;
@@ -1580,6 +1589,7 @@ int ngsq_submit(ngsq_engine* e, const uint8_t* bgzf, size_t nbytes, uint64_t fil
   if (!e || !bgzf) return fail(e, NGSQ_E_ARG, "bad submit arguments");
   if (e->finished) return fail(e, NGSQ_E_ARG, "submit after finish; call ngsq_reset");
   if (!e->range_set) return fail(e, NGSQ_E_ARG, "ngsq_set_range must precede the first submit");
+  if (e->awaiting_range) return fail(e, NGSQ_E_ARG, "ngsq_set_range must follow ngsq_next_file before the next file's first submit");
   CU(cudaSetDevice(e->device));
   uint32_t n = 0;
   size_t used = 0;
@@ -1622,6 +1632,35 @@ int ngsq_flush(ngsq_engine* e) {
   return launch_pending(e, (uint32_t)e->h_blocks.size(), false);
 }
 
+int ngsq_next_file(ngsq_engine* e) {
+  if (!e) return NGSQ_E_ARG;
+  if (e->finished) return fail(e, NGSQ_E_ARG, "ngsq_next_file after finish; call ngsq_reset");
+  if (ix_on(e)) return fail(e, NGSQ_E_ARG, "ngsq_next_file: an index (NGSQ_F_INDEX, NGSQ_F_INDEX_PART) describes one file");
+  if (e->cfg.max_records) return fail(e, NGSQ_E_ARG, "ngsq_next_file: max_records counts the records of one file in its order");
+  if (!e->range_set || e->awaiting_range) return fail(e, NGSQ_E_ARG, "ngsq_next_file: call ngsq_set_range for the file first");
+  CU(cudaSetDevice(e->device));
+  int rc = start_run(e);
+  if (rc) return rc;
+  // the file's last wave: a record that runs past its end is a truncation, and no later wave holds blocks of this file
+  const uint32_t nb = (uint32_t)e->h_blocks.size();
+  if ((rc = launch_pending(e, nb, true))) return rc;
+  if (nb > e->file_b0) {
+    if (!e->start_resolved && (e->first_voff & 0xFFFF)) return fail(e, NGSQ_E_ARG, "virtual offset %llu is beyond the submitted data", (unsigned long long)e->first_voff);
+    if (e->end_voff && !e->end_resolved && (e->end_voff & 0xFFFF)) return fail(e, NGSQ_E_ARG, "virtual offset %llu is beyond the submitted data", (unsigned long long)e->end_voff);
+  }
+  if (!e->waves.empty()) {
+    // behind the last wave on the stream of its record kernels, ahead of the next file's first wave_begin_kernel; its
+    // facets_end is recorded again so that ngsq_finish waits for this kernel too
+    cudaStream_t st = (e->cfg.flags & NGSQ_F_SERIAL_STAGES) ? e->s_comp : e->s_scan;
+    file_end_kernel<<<1, 1, 0, st>>>(e->d_state);
+    CU(cudaGetLastError());
+    e->other_launches++;
+    CU(cudaEventRecord(e->waves.back().facets_end, st));
+  }
+  e->awaiting_range = true;
+  return NGSQ_OK;
+}
+
 int ngsq_progress(ngsq_engine* e, uint64_t* records) {
   if (!e || !records) return NGSQ_E_ARG;
   // waves complete in order: consume the probes of those whose scan has finished (never blocks)
@@ -1651,6 +1690,7 @@ int ngsq_submit_device(ngsq_engine* e, const void* dev_bgzf, size_t nbytes, cons
   if (!e || !dev_bgzf || (!blocks && n_blocks)) return fail(e, NGSQ_E_ARG, "bad submit arguments");
   if (e->finished) return fail(e, NGSQ_E_ARG, "submit after finish; call ngsq_reset");
   if (!e->range_set) return fail(e, NGSQ_E_ARG, "ngsq_set_range must precede the first submit");
+  if (e->awaiting_range) return fail(e, NGSQ_E_ARG, "ngsq_set_range must follow ngsq_next_file before the next file's first submit");
   CU(cudaSetDevice(e->device));
   int rc = start_run(e);
   if (rc) return rc;
@@ -1681,7 +1721,7 @@ int ngsq_finish(ngsq_engine* e) {
   if (nb && !e->range_set) return fail(e, NGSQ_E_ARG, "ngsq_set_range was not called");
   rc = launch_pending(e, nb, true);
   if (rc) return rc;
-  if (nb) {
+  if (nb > e->file_b0) {
     // a virtual offset behind the last block can only mean "end of data"
     if (!e->start_resolved && (e->first_voff & 0xFFFF)) return fail(e, NGSQ_E_ARG, "virtual offset %llu is beyond the submitted data", (unsigned long long)e->first_voff);
     if (e->end_voff && !e->end_resolved && (e->end_voff & 0xFFFF)) return fail(e, NGSQ_E_ARG, "virtual offset %llu is beyond the submitted data", (unsigned long long)e->end_voff);

@@ -167,6 +167,15 @@ __global__ void __launch_bounds__(1024) wave_begin_kernel(RunState* st, uint8_t*
   }
 }
 
+// ngsq_next_file (one thread, behind the file's last wave): a record still open at the end of a file is a truncation, as
+// ngsq_finish finds it at the end of a run; then the carry and the end-of-range state are dropped so that no record chain
+// links two files.  Every accumulator stays.
+__global__ void file_end_kernel(RunState* st) {
+  if (!st->fatal && st->cn_len && !st->end_pending && !st->end_reached) st->fatal |= kFatalTruncated;
+  st->cn_len = 0;
+  st->end_pending = st->end_reached = 0;
+}
+
 // Waves outside the shard's range are inflated (and CRC-checked) like the rest; only their verdicts are folded.
 __global__ void status_fold_kernel(const uint32_t* __restrict__ status, uint32_t n_blocks, uint32_t first_global, RunState* st) {
   const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;

@@ -43,7 +43,7 @@ EXPORTED = [
     "ngsq_set_reference_bases", "ngsq_get_edits", "ngsq_get_edit_positions", "ngsq_set_feature_model", "ngsq_set_features", "ngsq_get_features",
     "ngsq_wait_copied", "ngsq_host_register", "ngsq_host_unregister", "ngsq_flush", "ngsq_progress",
     "ngsq_get_bai", "ngsq_split_reference", "ngsq_split_arrays", "ngsq_resolve_split", "ngsq_find_record", "ngsq_join_bai",
-    "ngsq_set_index_binning", "ngsq_get_csi", "ngsq_join_csi",
+    "ngsq_set_index_binning", "ngsq_get_csi", "ngsq_join_csi", "ngsq_next_file",
 ]
 
 
@@ -143,6 +143,7 @@ def load_library() -> C.CDLL:
     lib.ngsq_get_features.argtypes = [P, u64p]
     lib.ngsq_wait_copied.argtypes = [P, C.c_uint32]
     lib.ngsq_flush.argtypes = [P]
+    lib.ngsq_next_file.argtypes = [P]
     lib.ngsq_progress.argtypes = [P, u64p]
     lib.ngsq_host_register.argtypes = [P, C.c_size_t]
     lib.ngsq_host_unregister.argtypes = [P]
@@ -239,6 +240,10 @@ class Engine:
 
     def flush(self):
         self._check(self.lib.ngsq_flush(self.h))
+
+    def next_file(self):
+        """The chunks since the last set_range were one whole file; the next set_range starts another of the same run."""
+        self._check(self.lib.ngsq_next_file(self.h))
 
     def progress(self) -> int:
         v = C.c_uint64(0)

@@ -480,6 +480,89 @@ inline ShardPlan plan_shards_any_order(const BamHeader& h, const uint8_t* bam, u
   return plan;
 }
 
+// ---- several files of one sample (`qc --cuda-also`, DESIGN 5): the files' records are checked together, so every file must
+// describe the same references.  The dictionary of `path` against the positional file's: the same count, names, lengths and
+// order, or an error naming the file and the first reference that differs.
+inline void check_same_dictionary(const std::string& first_path, const std::vector<ReferenceSequence>& first, const std::string& path,
+                                  const std::vector<ReferenceSequence>& refs) {
+  const size_t n = std::min(first.size(), refs.size());
+  size_t i = 0;
+  while (i < n && first[i].name == refs[i].name && first[i].length == refs[i].length) ++i;
+  if (i == n && first.size() == refs.size()) return;
+  auto at = [i](const std::vector<ReferenceSequence>& v) {
+    return i < v.size() ? "\"" + v[i].name + "\" of length " + std::to_string(v[i].length) : std::string("missing");
+  };
+  throw std::runtime_error("the reference sequences of " + path + " differ from those of " + first_path + " (" + std::to_string(refs.size()) + " and " +
+                           std::to_string(first.size()) + " references): reference " + std::to_string(i) + " is " + at(refs) + " in " + path +
+                           " and " + at(first) + " in " + first_path);
+}
+
+// F >= D: whole files, largest first, each to the device with the fewest compressed bytes so far (ties: the lower index).
+// Returns every device's files in the order it runs them.
+inline std::vector<std::vector<uint32_t>> assign_files(const std::vector<uint64_t>& bytes, uint32_t n_dev) {
+  std::vector<uint32_t> order(bytes.size());
+  for (uint32_t f = 0; f < order.size(); ++f) order[f] = f;
+  std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return bytes[a] > bytes[b]; });
+  std::vector<std::vector<uint32_t>> queues(n_dev);
+  std::vector<uint64_t> load(n_dev, 0);
+  for (uint32_t f : order) {
+    const uint32_t d = (uint32_t)(std::min_element(load.begin(), load.end()) - load.begin());  // the first of the least loaded
+    queues[d].push_back(f);
+    load[d] += bytes[f];
+  }
+  return queues;
+}
+
+// F < D: how many devices cut each file, in proportion to its compressed bytes, at least one each and n_dev in all.  Each
+// further device goes to the file with the most bytes per device so far (ties: the lower index).
+inline std::vector<uint32_t> devices_per_file(const std::vector<uint64_t>& bytes, uint32_t n_dev) {
+  std::vector<uint32_t> n(bytes.size(), 1);
+  for (uint32_t left = n_dev - (uint32_t)bytes.size(); left; --left) {
+    uint32_t best = 0;
+    for (uint32_t f = 1; f < n.size(); ++f)
+      if ((unsigned __int128)bytes[f] * n[best] > (unsigned __int128)bytes[best] * n[f]) best = f;
+    ++n[best];
+  }
+  return n;
+}
+
+struct FilePart { uint32_t file = 0; Shard shard; };
+struct FilePlan {
+  std::vector<std::vector<FilePart>> queues;  // per device, in the order it runs them
+  bool cut = false;                           // F < D: one part of one file per device, the devices of a file in file order
+  uint32_t dropped = 0;                       // cuts left out (plan_shards_unindexed)
+};
+
+// The plan of F files on D devices.  F >= D: assign_files, each file from its first record to EOF.  F < D: each file cut by
+// plan_shards_any_order into devices_per_file parts, the devices of file 0 first.  Every reference is split between the
+// devices either way (the caller declares them when D > 1): each device holds records of any reference.
+inline FilePlan plan_files(const std::vector<BamHeader>& headers, const std::vector<const uint8_t*>& data, const std::vector<uint64_t>& sizes,
+                           uint32_t n_dev, const FindRecord& find) {
+  const uint32_t n_files = (uint32_t)headers.size();
+  std::vector<uint64_t> bytes(n_files);
+  std::vector<Shard> whole(n_files);
+  for (uint32_t f = 0; f < n_files; ++f) {
+    whole[f].first_voffset = headers[f].first_record_voffset;
+    bytes[f] = shard_compressed_bytes(whole[f], sizes[f]);
+  }
+  FilePlan plan;
+  if (n_files >= n_dev) {
+    for (const auto& files : assign_files(bytes, n_dev)) {
+      plan.queues.emplace_back();
+      for (uint32_t f : files) plan.queues.back().push_back({f, whole[f]});
+    }
+    return plan;
+  }
+  plan.cut = true;
+  const std::vector<uint32_t> n = devices_per_file(bytes, n_dev);
+  for (uint32_t f = 0; f < n_files; ++f) {
+    const ShardPlan p = plan_shards_any_order(headers[f], data[f], sizes[f], n[f], find);
+    plan.dropped += p.dropped;
+    for (const Shard& s : p.shards) plan.queues.push_back({{f, s}});
+  }
+  return plan;
+}
+
 // Compressed byte range [lo, hi) a shard submits: through the block that holds end_voffset.
 inline void shard_bytes(const Shard& s, const uint8_t* bam, uint64_t file_size, uint64_t* lo, uint64_t* hi) {
   *lo = s.first_voffset >> 16;

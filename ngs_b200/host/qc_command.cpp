@@ -9,11 +9,12 @@
 // which writes the missing index (.bai, or .csi with --cuda-csi) in the same pass as the results.  `qc` plans its shards from
 // <BAM>.bai, or from <BAM>.csi when there is no .bai (the reference needs the .bai).  `qc --cuda-any-order` reads no index and
 // takes records in any order (unsorted, queryname-sorted or collated files): one shard, or cuts at record anchors with every
-// reference split between the devices.
+// reference split between the devices.  `qc --cuda-also <BAM>` adds files of the same sample under the same rules: whole files
+// queued on each device (ngsq_next_file between them), or with fewer files than devices each file cut between its devices.
 //
 //   ngs-cuda-qc qc <BAM> <REFERENCE_GENOME> [-n N] [-o DIR] [-p PREFIX] [--only FACET]
 //               [--cuda-devices 0,1,..] [--cuda-build-index [--cuda-csi [--cuda-min-shift N]] | --cuda-any-order] [--cuda-gc-seed S]
-//               [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io] [--cuda-perf]
+//               [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io] [--cuda-perf] [--cuda-also <BAM> ..]
 //   ngs-cuda-qc index <BAM> [--csi [-m|--min-shift N]] [--cuda-device N | --cuda-devices 0,1,..] [--cuda-no-crc] [--cuda-chunk-mb M]
 //                     [--cuda-buffered-io]
 #include <cerrno>
@@ -54,6 +55,7 @@ struct QcArgs {
   bool csi = false;          // --cuda-csi: that index is <BAM>.csi instead of <BAM>.bai
   uint32_t min_shift = 14;   // --cuda-min-shift (CSI); the depth follows samtools' rule
   bool any_order = false;    // --cuda-any-order: no index is read, the records may come in any order
+  std::vector<std::string> also;  // --cuda-also: more files of the sample, checked with src as one (implies any_order)
 };
 
 void info(const std::string& s) { std::cerr << "INFO " << s << "\n"; }
@@ -86,17 +88,23 @@ class ChunkReader {
  public:
   static constexpr size_t kLead = 1 << 17;  // room in front of every buffer for the previous chunk's partial block
   ChunkReader(const std::string& path, size_t chunk_bytes, bool direct) : chunk_((chunk_bytes + 4095) & ~size_t(4095)) {
+    reopen(path, direct);
+    for (auto& b : buf_) {
+      b = (uint8_t*)ngsq_host_alloc(kLead + chunk_ + 4096);
+      if (!b) throw std::runtime_error("cannot allocate pinned staging buffers");
+    }
+  }
+  // reads another file through the same pinned buffers (`--cuda-also`)
+  void reopen(const std::string& path, bool direct) {
+    if (fd_ >= 0) close(fd_);
     fd_ = -1;
+    direct_ = false;
 #ifdef O_DIRECT
     if (direct) fd_ = open(path.c_str(), O_RDONLY | O_DIRECT);
     direct_ = fd_ >= 0;
 #endif
     if (fd_ < 0) fd_ = open(path.c_str(), O_RDONLY);
     if (fd_ < 0) throw std::runtime_error("cannot open " + path);
-    for (auto& b : buf_) {
-      b = (uint8_t*)ngsq_host_alloc(kLead + chunk_ + 4096);
-      if (!b) throw std::runtime_error("cannot allocate pinned staging buffers");
-    }
   }
   ~ChunkReader() {
     for (auto& b : buf_) if (b) ngsq_host_free(b);
@@ -104,15 +112,19 @@ class ChunkReader {
   }
   bool direct() const { return direct_; }
 
-  // streams file bytes [lo, hi) (lo on a block boundary) into e
-  void run(ngsq_engine* e, uint64_t lo, uint64_t hi, Progress* progress) {
+  // streams file bytes [lo, hi) (lo on a block boundary) into e.  same_run: e's run already holds the submits of the previous
+  // call (an earlier file, before ngsq_next_file), whose copies may still read the buffers.
+  void run(ngsq_engine* e, uint64_t lo, uint64_t hi, Progress* progress, bool same_run = false) {
     uint64_t pos = lo & ~uint64_t(4095);  // aligned file position of the next read
     size_t skip = (size_t)(lo - pos);     // bytes of the first read that precede the shard
     size_t carry = 0;                     // bytes of a partial block kept from the previous chunk
     const uint8_t* carry_src = nullptr;
-    uint32_t submits = 0;
-    int32_t used_by[kBufs];
-    for (auto& u : used_by) u = -1;
+    uint32_t& submits = submits_;         // ngsq_submit calls of e's run so far (ngsq_wait_copied counts them)
+    int32_t* used_by = used_by_;          // the submit that last read each buffer
+    if (!same_run) {
+      submits = 0;
+      for (int b = 0; b < kBufs; ++b) used_by[b] = -1;
+    }
     uint64_t file_off = lo;               // file offset of the next byte to submit
     for (uint32_t k = 0; pos < hi; ++k) {
       const uint32_t bi = k % kBufs;
@@ -174,6 +186,8 @@ class ChunkReader {
   bool direct_ = false;
   size_t chunk_;
   uint8_t* buf_[kBufs] = {nullptr, nullptr, nullptr};
+  uint32_t submits_ = 0;
+  int32_t used_by_[kBufs] = {-1, -1, -1};
 };
 
 void run_shard(ngsq_engine* e, const std::string& path, const MappedFile& file, const Shard& shard, size_t chunk_bytes, bool direct, bool log_progress,
@@ -199,6 +213,42 @@ void run_shard(ngsq_engine* e, const std::string& path, const MappedFile& file, 
         continue;
       }
       if (code) *code = rc;
+      check(e, rc);
+      if (log_progress) progress.report(e);
+      break;
+    }
+  } catch (const std::exception& ex) {
+    *err = ex.what();
+  }
+}
+
+// `--cuda-also`: a device's queue of whole files through one engine, ngsq_next_file behind each, then one ngsq_finish.  A read
+// longer than the quality table in any of them enlarges the table and runs the whole queue again, as run_shard does for one file.
+void run_queue(ngsq_engine* e, const std::vector<FilePart>& queue, const std::vector<std::string>& paths, const std::vector<const MappedFile*>& files,
+               size_t chunk_bytes, bool direct, bool log_progress, std::string* err) {
+  try {
+    std::unique_ptr<ChunkReader> reader;
+    for (int attempt = 0;; ++attempt) {
+      Progress progress;
+      for (size_t k = 0; k < queue.size(); ++k) {
+        const FilePart& q = queue[k];
+        uint64_t lo, hi;
+        shard_bytes(q.shard, files[q.file]->data(), files[q.file]->size(), &lo, &hi);
+        if (!reader) reader = std::make_unique<ChunkReader>(paths[q.file], chunk_bytes, direct);
+        else reader->reopen(paths[q.file], direct);
+        check(e, ngsq_set_range(e, q.shard.first_voffset, 0));
+        reader->run(e, lo, hi, log_progress ? &progress : nullptr, k > 0);
+        check(e, ngsq_next_file(e));
+      }
+      const int rc = ngsq_finish(e);
+      if (rc == NGSQ_E_QUAL_CAP && attempt == 0) {
+        ngsq_stats st;
+        check(e, ngsq_get_stats(e, &st));
+        info("  [*] Reads of up to " + std::to_string(st.max_read_len) + " bases: enlarging the quality table and reading the files again.");
+        check(e, ngsq_reset(e));
+        check(e, ngsq_set_quality_positions(e, (uint32_t)st.max_read_len + 1));
+        continue;
+      }
       check(e, rc);
       if (log_progress) progress.report(e);
       break;
@@ -244,6 +294,38 @@ void run_parts(const std::vector<ngsq_engine*>& engines, std::vector<Shard>& sha
       run_shard(engines[k], path, file, shards[k], chunk_bytes, direct, false, &errs[k], &codes[k]);
     }
   }
+}
+
+// `--cuda-also`: the plan's queues, one thread per engine (run_queue), or with fewer files than engines each file's parts through
+// run_parts on that file's engines, the files side by side.  On return every engine has finished; a cut file's queue entries
+// hold the ranges that ran.
+void run_files(const std::vector<ngsq_engine*>& engines, FilePlan& plan, const std::vector<std::string>& paths, const std::vector<const MappedFile*>& files,
+               size_t chunk_bytes, bool direct) {
+  const size_t n = engines.size();
+  std::vector<std::string> errs(n);
+  std::vector<std::thread> ts;
+  for (size_t i = 0, j; i < n; i = j) {
+    j = i + 1;
+    if (!plan.cut) {
+      ts.emplace_back(run_queue, engines[i], std::cref(plan.queues[i]), std::cref(paths), std::cref(files), chunk_bytes, direct, i == 0, &errs[i]);
+      continue;
+    }
+    const uint32_t f = plan.queues[i][0].file;
+    while (j < n && plan.queues[j][0].file == f) ++j;
+    ts.emplace_back([&, i, j, f] {
+      std::vector<ngsq_engine*> group(engines.begin() + i, engines.begin() + j);
+      std::vector<Shard> shards;
+      for (size_t k = i; k < j; ++k) shards.push_back(plan.queues[k][0].shard);
+      try {
+        run_parts(group, shards, paths[f], *files[f], chunk_bytes, direct);
+      } catch (const std::exception& ex) {
+        errs[i] = ex.what();
+      }
+      for (size_t k = i; k < j; ++k) plan.queues[k][0].shard = shards[k - i];
+    });
+  }
+  for (auto& t : ts) t.join();
+  for (auto& s : errs) if (!s.empty()) throw std::runtime_error(s);
 }
 
 // The record anchor finder of plan_shards_unindexed on engine e (after ngsq_set_references)
@@ -315,10 +397,14 @@ void log_dropped_cuts(const ShardPlan& plan) {
 
 // command.rs:226-421
 int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& output_prefix, const std::string& output_directory) {
-  // open_and_parse(src, IndexCheck::Full): bam.rs:77-123
-  if (args.src.size() < 4 || args.src.substr(args.src.size() - 4) != ".bam")
-    throw std::runtime_error("could not open " + args.src + ": expected a .bam file");
+  // open_and_parse(src, IndexCheck::Full): bam.rs:77-123, for every file of the sample
+  std::vector<std::string> paths{args.src};
+  paths.insert(paths.end(), args.also.begin(), args.also.end());
+  for (const std::string& p : paths)
+    if (p.size() < 4 || p.substr(p.size() - 4) != ".bam") throw std::runtime_error("could not open " + p + ": expected a .bam file");
   MappedFile file(args.src);
+  std::vector<std::unique_ptr<MappedFile>> also_files;
+  for (const std::string& p : args.also) also_files.push_back(std::make_unique<MappedFile>(p));
   const std::string bai_path = args.src + ".bai";  // pathbuf.rs:59-75: x.bam -> x.bam.bai
   const std::string csi_path = args.src + ".csi";  // x.bam -> x.bam.csi: planned from when there is no .bai
   // --cuda-any-order: neither index is read, even when one exists (it may belong to another order of the same records)
@@ -364,6 +450,18 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   }
   BamHeader header = read_bam_header(engines[0], file.data(), file.size());
   if (have_csi) bai = read_csi(engines[0], csi_path, header.reference_sequences.size());
+  // --cuda-also: one dictionary for the sample, checked before the qc pass (the genome check below then covers every file)
+  std::vector<BamHeader> headers{header};
+  std::vector<const MappedFile*> files{&file};
+  std::vector<uint64_t> sizes{file.size()};
+  std::vector<const uint8_t*> data{file.data()};
+  for (size_t k = 0; k < args.also.size(); ++k) {
+    headers.push_back(read_bam_header(engines[0], also_files[k]->data(), also_files[k]->size()));
+    check_same_dictionary(args.src, header.reference_sequences, args.also[k], headers.back().reference_sequences);
+    files.push_back(also_files[k].get());
+    sizes.push_back(also_files[k]->size());
+    data.push_back(also_files[k]->data());
+  }
 
   if (!std::filesystem::exists(output_directory)) std::filesystem::create_directories(output_directory);
 
@@ -383,8 +481,18 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   std::vector<uint32_t> ref_len;
   for (auto& rs : header.reference_sequences) ref_len.push_back(rs.length);
   ShardPlan plan;
-  const bool cut_at_anchors = (build_index || args.any_order) && n_dev > 1;
-  if (cut_at_anchors) {
+  const bool several_files = !args.also.empty();
+  const bool cut_at_anchors = !several_files && (build_index || args.any_order) && n_dev > 1;
+  FilePlan file_plan;
+  if (several_files) {
+    // whole files queued on the devices, or each file cut between its devices; every reference split on several devices
+    if (n_dev > 1) check(engines[0], ngsq_set_references(engines[0], (uint32_t)ref_len.size(), ref_len.data(), std::vector<uint8_t>(ref_len.size(), 0).data()));
+    file_plan = plan_files(headers, data, sizes, n_dev, n_dev > 1 ? engine_finder(engines[0]) : FindRecord());
+    plan.dropped = file_plan.dropped;
+    log_dropped_cuts(plan);
+    if (n_dev > 1)
+      for (uint32_t c = 0; c < ref_len.size(); ++c) plan.split.push_back(c);
+  } else if (cut_at_anchors) {
     // no index to cut at: anchors from the records (the finder needs the references; every engine sets them again below)
     check(engines[0], ngsq_set_references(engines[0], (uint32_t)ref_len.size(), ref_len.data(), std::vector<uint8_t>(ref_len.size(), 0).data()));
     const FindRecord find = engine_finder(engines[0]);
@@ -397,7 +505,11 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
     plan = choose_shards(header, bai, n_dev, file.size());
   }
   std::vector<Shard> shards = plan.shards;
-  if (args.any_order && n_dev > 1) {
+  if (several_files) {
+    info("  [*] " + std::to_string(paths.size()) + " files of one sample" +
+         (n_dev == 1 ? std::string(" on one device.")
+                     : std::string(file_plan.cut ? ", each cut between its devices" : ", whole files queued on the devices") + ", every reference split."));
+  } else if (args.any_order && n_dev > 1) {
     info("  [*] Records in any order: " + std::to_string(n_dev - plan.dropped) + " shards, every reference split.");
   } else if (plan.split_plan) {
     std::string names;
@@ -430,7 +542,9 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   // the hot path: one thread per GPU
   info("Starting CUDA pass for QC stats.");
   const auto t_hot = std::chrono::steady_clock::now();
-  if (cut_at_anchors) {
+  if (several_files) {
+    run_files(engines, file_plan, paths, files, args.chunk_mb << 20, args.direct_io);
+  } else if (cut_at_anchors) {
     run_parts(engines, shards, args.src, file, args.chunk_mb << 20, args.direct_io);
   } else {
     std::vector<std::thread> ts;
@@ -499,7 +613,13 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
       pf << (i ? "," : "") << "{\"device\":" << args.devices[i] << ",\"records\":" << st.records << ",\"blocks\":" << st.blocks
          << ",\"compressed_bytes\":" << st.compressed_bytes << ",\"inflated_bytes\":" << st.inflated_bytes << ",\"ms_inflate\":" << st.ms_inflate
          << ",\"ms_crc\":" << st.ms_crc << ",\"ms_scan\":" << st.ms_scan << ",\"ms_facets\":" << st.ms_facets << ",\"ms_coverage\":" << st.ms_coverage
-         << ",\"ms_total\":" << st.ms_total << ",\"ms_tail\":" << st.ms_tail << ",\"waves\":" << st.waves << ",\"wall_ms_file_to_results\":" << hot_ms << "}";
+         << ",\"ms_total\":" << st.ms_total << ",\"ms_tail\":" << st.ms_tail << ",\"waves\":" << st.waves << ",\"wall_ms_file_to_results\":" << hot_ms;
+      if (several_files) {
+        uint32_t n_files = 0;
+        for (const FilePart& q : file_plan.queues[i]) n_files += q.shard.empty ? 0 : 1;
+        pf << ",\"files\":" << n_files;
+      }
+      pf << "}";
     }
     pf << "]\n";
   }
@@ -643,6 +763,9 @@ void usage() {
                "                  build <BAM>.bai, or with --cuda-csi <BAM>.csi (min_shift N, default 14), in the same pass and write it\n"
                "                  once the run succeeded; --cuda-any-order: read no index and take the records in any order, not\n"
                "                  with -n, --cuda-build-index or --cuda-csi)\n"
+               "       ngs-cuda-qc qc <BAM> <REFERENCE_GENOME> --cuda-also <BAM> [--cuda-also <BAM> ..] [the options above]\n"
+               "                  (the records of every file are checked as one sample: the files must have the same reference\n"
+               "                  sequences; the rules of --cuda-any-order apply; the output prefix is the first <BAM>'s name)\n"
                "       ngs-cuda-qc index <BAM> [--csi [-m|--min-shift N]] [--cuda-device N | --cuda-devices 0,1,..] [--cuda-no-crc] [--cuda-chunk-mb M]\n"
                "                  [--cuda-buffered-io]\n"
                "                  (writes <BAM>.bai, or with --csi <BAM>.csi (min_shift N, default 14); an existing index is never overwritten;\n"
@@ -686,6 +809,7 @@ extern "C" int ngs_cuda_qc_main(int argc, char** argv) {
       else if (s == "--cuda-build-index") a.build_index = true;
       else if (s == "--cuda-csi") a.csi = true;
       else if (s == "--cuda-any-order") a.any_order = true;
+      else if (s == "--cuda-also") a.also.push_back(val());
       else if (s == "--cuda-min-shift") { a.min_shift = (uint32_t)std::stoul(val()); min_shift_set = true; }
       else if (s == "--cuda-buffered-io") a.direct_io = false;
       else if (s == "-h" || s == "--help") { usage(); return 0; }
@@ -693,6 +817,13 @@ extern "C" int ngs_cuda_qc_main(int argc, char** argv) {
       else pos.push_back(s);
     }
     if (pos.size() != 2 || a.devices.empty()) { usage(); return 2; }
+    if (!a.also.empty()) {
+      if (a.num_records)
+        throw std::runtime_error("--cuda-also cannot be combined with -n: the first N records are counted in the order of one file");
+      if (a.build_index) throw std::runtime_error("--cuda-also cannot be combined with --cuda-build-index: an index describes one file");
+      if (a.csi) throw std::runtime_error("--cuda-also cannot be combined with --cuda-csi: an index describes one file");
+      a.any_order = true;  // a file boundary is one more cut: records of several files come in no common order
+    }
     if (a.any_order && a.num_records)
       throw std::runtime_error("--cuda-any-order cannot be combined with -n: the first N records are counted in the order of the per-contig "
                                "queries, which records in any order do not have");

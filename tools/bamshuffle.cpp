@@ -1,7 +1,9 @@
 // bamshuffle — writes the records of a BAM again in a seeded random order (the header as it is), for measuring
-// `qc --cuda-any-order` on a file of realistic size (tools/any_order_bench.py).  Blocks are inflated and deflated on all
-// threads; the records are packed into BGZF blocks of 0xFF00 bytes, so they straddle block boundaries.
-//   bamshuffle <in.bam> <out.bam> [seed] [zlib level] [threads]
+// `qc --cuda-any-order` on a file of realistic size (tools/any_order_bench.py).  Seed 0 keeps the file's order; with parts > 1
+// the records go to that many files <out>.<k>.bam of consecutive records, each with the header, for measuring `qc --cuda-also`
+// (tools/multi_file_bench.py).  Blocks are inflated and deflated on all threads; the records are packed into BGZF blocks of
+// 0xFF00 bytes, so they straddle block boundaries.
+//   bamshuffle <in.bam> <out.bam> [seed] [zlib level] [threads] [parts]
 #include <zlib.h>
 
 #include <algorithm>
@@ -65,10 +67,11 @@ std::vector<uint8_t> deflate_block(const uint8_t* p, size_t n, int level) {
 }  // namespace
 
 int main(int argc, char** argv) {
-  if (argc < 3) { fprintf(stderr, "usage: bamshuffle <in.bam> <out.bam> [seed] [zlib level] [threads]\n"); return 2; }
+  if (argc < 3) { fprintf(stderr, "usage: bamshuffle <in.bam> <out.bam> [seed] [zlib level] [threads] [parts]\n"); return 2; }
   const uint64_t seed = argc > 3 ? strtoull(argv[3], nullptr, 0) : 1;
   const int level = argc > 4 ? atoi(argv[4]) : 1;
   const int threads = argc > 5 ? atoi(argv[5]) : (int)std::max(1u, std::thread::hardware_concurrency());
+  const size_t parts = argc > 6 ? std::max(1, atoi(argv[6])) : 1;
   const std::vector<uint8_t> in = slurp(argv[1]);
   // blocks, then their inflated bytes side by side
   std::vector<size_t> coff, uoff{0};
@@ -99,31 +102,41 @@ int main(int argc, char** argv) {
   for (uint32_t c = 0; c < n_ref; ++c) h += 4 + rd32(&data[h]) + 4;
   std::vector<size_t> rec;
   for (size_t o = h; o + 4 <= data.size(); o += 4 + rd32(&data[o])) rec.push_back(o);
-  std::mt19937_64 rng(seed);
-  for (size_t i = rec.size(); i > 1; --i) std::swap(rec[i - 1], rec[std::uniform_int_distribution<size_t>(0, i - 1)(rng)]);
-  std::vector<uint8_t> stream(data.size() - h);
-  size_t w = 0;
-  for (size_t o : rec) {
-    const size_t n = 4 + rd32(&data[o]);
-    memcpy(stream.data() + w, &data[o], n);
-    w += n;
+  if (seed) {
+    std::mt19937_64 rng(seed);
+    for (size_t i = rec.size(); i > 1; --i) std::swap(rec[i - 1], rec[std::uniform_int_distribution<size_t>(0, i - 1)(rng)]);
   }
   // the header in blocks of its own, as bamgen and samtools write it
-  std::vector<std::vector<uint8_t>> blocks;
-  for (size_t o = 0; o < h; o += 0xFF00) blocks.push_back(deflate_block(data.data() + o, std::min<size_t>(0xFF00, h - o), level));
-  std::vector<uint8_t>().swap(data);
-  const size_t n_hdr = blocks.size(), n_out = (stream.size() + 0xFF00 - 1) / 0xFF00;
-  blocks.resize(n_hdr + n_out);
-  parallel_for(n_out, threads, [&](size_t k) {
-    blocks[n_hdr + k] = deflate_block(stream.data() + k * 0xFF00, std::min<size_t>(0xFF00, stream.size() - k * 0xFF00), level);
-  });
-  FILE* f = fopen(argv[2], "wb");
-  if (!f) { fprintf(stderr, "cannot create %s\n", argv[2]); return 1; }
+  std::vector<std::vector<uint8_t>> hdr_blocks;
+  for (size_t o = 0; o < h; o += 0xFF00) hdr_blocks.push_back(deflate_block(data.data() + o, std::min<size_t>(0xFF00, h - o), level));
   static const uint8_t kEof[28] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-  bool ok = true;
-  for (const auto& b : blocks) ok = ok && fwrite(b.data(), 1, b.size(), f) == b.size();
-  ok = ok && fwrite(kEof, 1, 28, f) == 28;
-  if (fclose(f) || !ok) { fprintf(stderr, "write error on %s\n", argv[2]); return 1; }
-  fprintf(stderr, "%zu records, %zu blocks\n", rec.size(), n_out);
+  size_t n_blocks = 0;
+  for (size_t k = 0; k < parts; ++k) {
+    const size_t r0 = rec.size() * k / parts, r1 = rec.size() * (k + 1) / parts;
+    size_t bytes = 0;
+    for (size_t i = r0; i < r1; ++i) bytes += 4 + rd32(&data[rec[i]]);
+    std::vector<uint8_t> stream(bytes);
+    size_t w = 0;
+    for (size_t i = r0; i < r1; ++i) {
+      const size_t n = 4 + rd32(&data[rec[i]]);
+      memcpy(stream.data() + w, &data[rec[i]], n);
+      w += n;
+    }
+    const size_t n_out = (stream.size() + 0xFF00 - 1) / 0xFF00;
+    std::vector<std::vector<uint8_t>> blocks(n_out);
+    parallel_for(n_out, threads, [&](size_t j) {
+      blocks[j] = deflate_block(stream.data() + j * 0xFF00, std::min<size_t>(0xFF00, stream.size() - j * 0xFF00), level);
+    });
+    const std::string path = parts == 1 ? std::string(argv[2]) : std::string(argv[2]) + "." + std::to_string(k) + ".bam";
+    FILE* f = fopen(path.c_str(), "wb");
+    if (!f) { fprintf(stderr, "cannot create %s\n", path.c_str()); return 1; }
+    bool ok = true;
+    for (const auto& b : hdr_blocks) ok = ok && fwrite(b.data(), 1, b.size(), f) == b.size();
+    for (const auto& b : blocks) ok = ok && fwrite(b.data(), 1, b.size(), f) == b.size();
+    ok = ok && fwrite(kEof, 1, 28, f) == 28;
+    if (fclose(f) || !ok) { fprintf(stderr, "write error on %s\n", path.c_str()); return 1; }
+    n_blocks += n_out;
+  }
+  fprintf(stderr, "%zu records, %zu blocks, %zu file(s)\n", rec.size(), n_blocks, parts);
   return 0;
 }
