@@ -80,6 +80,8 @@ enum {
                                    CSIv1's hts_reg2bin(beg, end, min_shift, depth) (ngsq_set_index_binning; default min_shift 14 and
                                    samtools' depth rule), records may end at most at 2^(min_shift + 3 depth) and references may be at
                                    most that long.  Read the bytes with ngsq_get_csi, join parts with ngsq_join_csi. */
+#define NGSQ_F_READ_GROUPS 512u  /* with NGSQ_F_RECORD_FACETS (alone: NGSQ_E_ARG): the four record facets once more per read group
+                                    (ngsq_set_read_groups, ngsq_select_read_group); the sample's results are unchanged */
 
 typedef struct ngsq_engine ngsq_engine;
 
@@ -123,7 +125,7 @@ typedef struct ngsq_stats {
   float ms_crc;
   float ms_scan;             /* record-boundary discovery + offset table */
   float ms_facets;           /* fused record-facet + coverage-scatter kernel, and the other per-wave record kernels (Edits,
-                                Genomic Features, the NGSQ_F_INDEX key / run kernel) */
+                                Genomic Features, the NGSQ_F_INDEX key / run kernel, the NGSQ_F_READ_GROUPS kernels) */
   float ms_coverage;         /* difference-array resolve */
   float ms_total;            /* first submit -> end of finish on the engine's stream */
   uint32_t inflate_launches, other_launches;
@@ -199,6 +201,28 @@ int ngsq_flush(ngsq_engine* e);
  * NGSQ_F_INDEX_PART (an index describes one file), with max_records != 0 (`-n` counts in one file's order), and before the
  * file's ngsq_set_range.  The GC window of a record is keyed by its virtual offset in its own file. */
 int ngsq_next_file(ngsq_engine* e);
+/* Read groups (`qc --cuda-by-read-group`, DESIGN.md section 5, "Read groups"), with NGSQ_F_READ_GROUPS: the @RG IDs of the
+ * header(s), `ids` = n NUL-terminated IDs back to back in ids_bytes bytes.  Group g < n is the records whose FIRST aux field
+ * tagged RG (htslib's bam_aux_get) is of type Z and equals ID g byte for byte; group n ("ungrouped") is every other record:
+ * no RG field, an RG field of another type, or a value no ID matches.  Records outside max_records belong to no group.  With
+ * the flag, the aux fields in front of a record's first RG field are read, and a malformed one (unknown type, no NUL, a field
+ * that runs past the record) fails the run with NGSQ_E_BAD_RECORD; without it aux bytes are never read.  Each of the n + 1
+ * groups holds the integers of the four record facets: the 34 of ngsq_get_general, the TLEN histogram and its two counters,
+ * the GC histogram with its nucleobase and record counters, and a quality length and table with as many rows as the sample's
+ * (ngsq_set_quality_positions resizes both): (n + 1) x (1169 + 94 x rows) x 8 bytes of device memory in one buffer apart from
+ * the packed result buffer (about 99 MB per group at the default 131072 rows).  A group's reads are never longer than the
+ * sample's, so NGSQ_E_QUAL_CAP covers the group tables too.  After ngsq_set_references, before the first submit; kept across
+ * ngsq_reset and ngsq_next_file accumulates like every other result.  NGSQ_E_ARG without the flag, for n > 65534, an empty or
+ * repeated ID or ids_bytes that does not hold exactly n IDs; NGSQ_E_NOMEM (naming n and the rows) when the tables do not fit.
+ * ngsq_reduce merges the groups too: the quality lengths with max, the rest with sum; the ranks must agree on n, the IDs and
+ * the rows (NGSQ_E_ARG before any group data moves). */
+int ngsq_set_read_groups(ngsq_engine* e, uint32_t n, const char* ids, size_t ids_bytes);
+/* After ngsq_finish (and ngsq_reduce): which results the getters return.  -1 (the default, and again after ngsq_reset) is the
+ * sample; 0..n a group (n = ungrouped).  While a group is selected, ngsq_get_general, ngsq_get_tlen, ngsq_get_gc and
+ * ngsq_get_quality return that group's integers in the sample's layout, and the Coverage, Edits, Genomic Features and
+ * edit-position getters fail with NGSQ_E_ARG (those facets are the sample's only).  NGSQ_E_ARG before ngsq_finish, without
+ * NGSQ_F_READ_GROUPS, or for g outside [-1, n]. */
+int ngsq_select_read_group(ngsq_engine* e, int32_t g);
 /* Records whose wave has been scanned so far (never blocks; lags the submits by about one wave): the caller's
  * RecordCounter log line, src/utils/display.rs:43-52. */
 int ngsq_progress(ngsq_engine* e, uint64_t* records);

@@ -32,6 +32,7 @@
 #include "features.cuh"
 #include "index.cuh"
 #include "inflate2.cuh"
+#include "read_groups.cuh"
 #include "recscan.cuh"
 
 using namespace ngsq;
@@ -238,6 +239,25 @@ struct ngsq_engine {
   uint32_t n_split = 0;
   bool split_merged = false;         // the split references of this run have been merged (reduce / resolve_split)
 
+  // read groups (NGSQ_F_READ_GROUPS): the IDs, their device hash table, the group buffer
+  // [sums (rg_n + 1) x kGroupSums | quality lengths (rg_n + 1) | quality tables (rg_n + 1) x grp_rows x 94], the per-wave
+  // bucketing arrays, and the host copies ngsq_select_read_group serves
+  bool rg_set = false;
+  uint32_t rg_n = 0, rg_mask = 0;
+  uint64_t rg_sig = 0;               // hash of the IDs and their number (part of ngsq_reduce's layout agreement)
+  uint8_t* d_rg_ids = nullptr;
+  uint32_t *d_rg_id_off = nullptr, *d_rg_table = nullptr;
+  uint64_t* d_grp = nullptr;
+  uint32_t grp_rows = 0, grp_dirty = 0;  // rows of each group table; rows an earlier run may have written
+  uint16_t* d_rg_of = nullptr;
+  uint32_t *d_rg_order = nullptr, *d_rg_count = nullptr, *d_rg_cursor = nullptr, *d_rg_total = nullptr;
+  uint64_t rg_cap = 0;               // records the bucketing arrays hold
+  size_t rg_smem = 0;
+  int rg_occ = 1;
+  std::vector<uint64_t> h_grp_sums, h_grp_qlen;
+  std::vector<std::vector<uint64_t>> h_grp_qual;
+  int32_t rg_sel = -1;
+
   // nccl
   void* comm = nullptr;
   int n_ranks = 1, rank = 0;
@@ -318,6 +338,35 @@ int layout_results(ngsq_engine* e, uint32_t qpos) {
   return NGSQ_OK;
 }
 
+bool rg_on(const ngsq_engine* e) { return e->cfg.flags & NGSQ_F_READ_GROUPS; }
+
+// The group buffer for `rows` quality rows per group (layout: see ngsq_engine::d_grp).  keep: the counters and the quality
+// rows a finished run wrote move into the new buffer.  Only between runs.
+int alloc_groups(ngsq_engine* e, uint32_t rows, bool keep) {
+  const uint64_t ng = (uint64_t)e->rg_n + 1, head = ng * (kGroupSums + 1), words = head + ng * rows * 94;
+  uint64_t* np = nullptr;
+  cudaError_t rc = cudaMalloc(&np, words * 8);
+  if (rc != cudaSuccess) {
+    cudaGetLastError();
+    return fail(e, NGSQ_E_NOMEM, "read-group tables: %llu groups (%u read groups + ungrouped) with %u quality rows each need %.1f GB of device memory "
+                "(ngsq_set_read_groups sets the groups, ngsq_set_quality_positions the rows): %s",
+                (unsigned long long)ng, e->rg_n, rows, words * 8 / 1e9, cudaGetErrorString(rc));
+  }
+  CU(cudaMemsetAsync(np, 0, words * 8, e->s_comp));
+  if (keep && e->d_grp) {
+    const uint32_t old = e->grp_rows, copy = std::min(old, rows);
+    CU(cudaMemcpyAsync(np, e->d_grp, head * 8, cudaMemcpyDeviceToDevice, e->s_comp));
+    if (copy) CU(cudaMemcpy2DAsync(np + head, (size_t)rows * 94 * 8, e->d_grp + head, (size_t)old * 94 * 8, (size_t)copy * 94 * 8, ng,
+                                   cudaMemcpyDeviceToDevice, e->s_comp));
+  }
+  CU(cudaStreamSynchronize(e->s_comp));
+  if (e->d_grp) cudaFree(e->d_grp);
+  e->d_grp = np;
+  e->grp_rows = rows;
+  e->grp_dirty = keep ? e->grp_dirty : 0;
+  return NGSQ_OK;
+}
+
 // Result buffer with room for `qpos` quality rows.  Only between runs (or after ngsq_finish): nothing is in flight.
 int ensure_res(ngsq_engine* e, uint32_t qpos, bool keep) {
   if (qpos < 256) qpos = 256;
@@ -339,6 +388,7 @@ int ensure_res(ngsq_engine* e, uint32_t qpos, bool keep) {
   }
   if (e->d_cov_slot) CU(cudaMemcpyAsync(e->d_cov_slot, e->cov_slot.data(), e->n_ref * 4, cudaMemcpyHostToDevice, e->s_comp));
   CU(cudaStreamSynchronize(e->s_comp));
+  if (e->rg_set && e->grp_rows != e->qpos_cap) return alloc_groups(e, e->qpos_cap, keep);  // a group table has the sample's rows
   return NGSQ_OK;
 }
 
@@ -358,6 +408,16 @@ int start_run(ngsq_engine* e) {
   e->h_state->next_carry = kNoCarry;
   CU(cudaMemcpyAsync(e->d_state, e->h_state, sizeof(RunState), cudaMemcpyHostToDevice, e->s_comp));
   if ((e->cfg.flags & NGSQ_F_FEATURES) && e->d_ft_res) CU(cudaMemsetAsync(e->d_ft_res, 0, F_WORDS * 8, e->s_comp));
+  if (rg_on(e)) {
+    if (!e->rg_set) return fail(e, NGSQ_E_ARG, "NGSQ_F_READ_GROUPS needs ngsq_set_read_groups before the first submit");
+    // the counters, the lengths, and every quality row an earlier run may have touched
+    const uint64_t ng = (uint64_t)e->rg_n + 1, head = ng * (kGroupSums + 1);
+    CU(cudaMemsetAsync(e->d_grp, 0, head * 8, e->s_comp));
+    const uint32_t dirty = std::min(e->grp_dirty, e->grp_rows);
+    if (dirty) CU(cudaMemset2DAsync(e->d_grp + head, (size_t)e->grp_rows * 94 * 8, 0, (size_t)dirty * 94 * 8, ng, e->s_comp));
+    e->grp_dirty = e->grp_rows;  // until ngsq_finish knows better
+    CU(cudaMemsetAsync(e->d_rg_count, 0, ng * 4, e->s_comp));
+  }
   if (ix_on(e)) {
     if (!e->d_ix) return fail(e, NGSQ_E_ARG, "NGSQ_F_INDEX needs ngsq_set_references before the first submit");
     IndexState z{};
@@ -589,6 +649,12 @@ int ensure_wave_buffers(ngsq_engine* e, int s, uint32_t n, uint64_t bytes) {
     if ((rc = fresh(e, e->d_long, need_long, "long-read list"))) return rc;
     e->long_cap = need_long;
   }
+  if (rg_on(e) && need_rec > e->rg_cap) {
+    if ((rc = quiesce())) return rc;
+    if ((rc = fresh(e, e->d_rg_of, need_rec, "read-group tags"))) return rc;
+    if ((rc = fresh(e, e->d_rg_order, need_rec + 32ull * (e->rg_n + 1), "read-group buckets"))) return rc;
+    e->rg_cap = need_rec;
+  }
   if ((e->cfg.flags & (NGSQ_F_COVERAGE | NGSQ_F_EDITS)) && e->cfg.max_records && need_rec > e->mark_cap) {
     if ((rc = quiesce())) return rc;
     if ((rc = fresh(e, e->d_mark, need_rec, "record marks"))) return rc;
@@ -751,6 +817,24 @@ int launch_wave(ngsq_engine* e, uint32_t b0, uint32_t b1, bool final_wave) {
       qual_verdict_kernel<<<e->n_sm, 256, 0, st>>>(T);
       CU(cudaGetLastError());
       e->other_launches += 2;
+    }
+    if (rg_on(e)) {
+      // the four record facets per read group: tag, bucket, tally (read_groups.cuh)
+      ReadGroupParams G{};
+      G.d = slot; G.rec = e->d_rec; G.st = e->d_state; G.blocks = wblocks; G.headroom = e->headroom; G.out0 = out0;
+      G.max_records = e->cfg.max_records; G.gc_seed = e->cfg.gc_seed; G.n_ref = (int32_t)e->n_ref;
+      G.n_groups = e->rg_n; G.ids = e->d_rg_ids; G.id_off = e->d_rg_id_off; G.table = e->d_rg_table; G.mask = e->rg_mask;
+      G.grp = e->d_rg_of; G.count = e->d_rg_count; G.cursor = e->d_rg_cursor; G.order = e->d_rg_order; G.total = e->d_rg_total;
+      const uint64_t ng = (uint64_t)e->rg_n + 1;
+      G.sums = e->d_grp; G.qlen = e->d_grp + ng * kGroupSums; G.qual = e->d_grp + ng * (kGroupSums + 1); G.rows = e->grp_rows;
+      G.res = e->d_res;
+      const uint32_t tgrid = (uint32_t)std::min<uint64_t>((bytes / 36 + 2 + kRgThreads - 1) / kRgThreads, (uint64_t)e->n_sm * 8);
+      rg_tag_kernel<<<tgrid, kRgThreads, 0, st>>>(G);
+      rg_scan_kernel<<<1, kRgScanThreads, 0, st>>>(G);
+      rg_scatter_kernel<<<tgrid, kRgThreads, 0, st>>>(G);
+      rg_facets_kernel<<<(uint32_t)e->n_sm * e->rg_occ, kFacetThreads, e->rg_smem, st>>>(G);
+      CU(cudaGetLastError());
+      e->other_launches += 4;
     }
   }
   // `-n`: which records the second pass processes (one counter over all sequences) — Coverage and Edits share the marks
@@ -1176,6 +1260,27 @@ int inflate_run(ngsq_engine* e, const uint8_t* bgzf, DevInflated& D) {
 
 extern "C" {
 
+namespace {
+// Host copies of the group buffer after ngsq_finish / ngsq_reduce: the counters and lengths, then each group's quality rows
+int fetch_groups(ngsq_engine* e, cudaStream_t s) {
+  const uint64_t ng = (uint64_t)e->rg_n + 1, head = ng * (kGroupSums + 1);
+  e->h_grp_sums.assign(ng * kGroupSums, 0);
+  e->h_grp_qlen.assign(ng, 0);
+  CU(cudaMemcpyAsync(e->h_grp_sums.data(), e->d_grp, ng * kGroupSums * 8, cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(e->h_grp_qlen.data(), e->d_grp + ng * kGroupSums, ng * 8, cudaMemcpyDeviceToHost, s));
+  CU(cudaStreamSynchronize(s));
+  e->h_grp_qual.assign(ng, {});
+  for (uint64_t g = 0; g < ng; ++g) {
+    e->h_grp_qlen[g] = std::min<uint64_t>(e->h_grp_qlen[g], e->grp_rows);
+    e->h_grp_qual[g].resize(e->h_grp_qlen[g] * 94);
+    if (e->h_grp_qlen[g])
+      CU(cudaMemcpyAsync(e->h_grp_qual[g].data(), e->d_grp + head + g * e->grp_rows * 94, e->h_grp_qlen[g] * 94 * 8, cudaMemcpyDeviceToHost, s));
+  }
+  CU(cudaStreamSynchronize(s));
+  return NGSQ_OK;
+}
+}  // namespace
+
 int ngsq_version(void) { return NGSQ_VERSION; }
 
 const char* ngsq_last_error(ngsq_engine* e) { return e ? e->err.c_str() : g_create_err.c_str(); }
@@ -1195,6 +1300,8 @@ int ngsq_create(int device, const ngsq_config* cfg, ngsq_engine** out) {
     return fail(e, NGSQ_E_ARG, "NGSQ_F_INDEX_CSI selects the format of NGSQ_F_INDEX or NGSQ_F_INDEX_PART: set one of them with it");
   if (cfg && (cfg->flags & (NGSQ_F_INDEX | NGSQ_F_INDEX_PART)) && cfg->max_records)
     return fail(e, NGSQ_E_ARG, "NGSQ_F_INDEX cannot be combined with max_records: an index covers every record of the file");
+  if (cfg && (cfg->flags & NGSQ_F_READ_GROUPS) && !(cfg->flags & NGSQ_F_RECORD_FACETS))
+    return fail(e, NGSQ_E_ARG, "NGSQ_F_READ_GROUPS splits the record facets by read group: set NGSQ_F_RECORD_FACETS with it");
   ngsq_engine* ne = new ngsq_engine();
   ne->device = device;
   if (cfg) memcpy(&ne->cfg, cfg, std::min<size_t>(cfg->struct_size ? cfg->struct_size : sizeof(ngsq_config), sizeof(ngsq_config)));
@@ -1239,6 +1346,13 @@ int ngsq_create(int device, const ngsq_config* cfg, ngsq_engine** out) {
   CUC(cudaFuncSetAttribute(qual_tiles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTileSmem));
   CUC(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&e->facet_occ, facets_kernel, kFacetThreads, e->facet_smem));
   if (e->facet_occ < 1) e->facet_occ = 1;
+  if (rg_on(e)) {
+    e->rg_smem = rg_facets_smem(kFacetThreads / 32);
+    CUC(cudaFuncSetAttribute(rg_facets_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)e->rg_smem));
+    CUC(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&e->rg_occ, rg_facets_kernel, kFacetThreads, e->rg_smem));
+    if (e->rg_occ < 1) e->rg_occ = 1;
+    CUC(cudaMalloc(&e->d_rg_total, 4));
+  }
   {
     CrcTables t;
     crc_make_tables(t);
@@ -1276,6 +1390,8 @@ void ngsq_destroy(ngsq_engine* e) {
   for (void* p : {(void*)e->d_ed_contigs, (void*)e->d_ed_refs, (void*)e->d_ed_alts, (void*)e->d_ed_res}) if (p) cudaFree(p);
   for (void* p : e->ft_allocs) cudaFree(p);
   for (void* p : {(void*)e->d_ft_contigs, (void*)e->d_ft_res}) if (p) cudaFree(p);
+  for (void* p : {(void*)e->d_rg_ids, (void*)e->d_rg_id_off, (void*)e->d_rg_table, (void*)e->d_grp, (void*)e->d_rg_of, (void*)e->d_rg_order,
+                  (void*)e->d_rg_count, (void*)e->d_rg_cursor, (void*)e->d_rg_total}) if (p) cudaFree(p);
   for (auto& w : e->ix_waves) cudaEventDestroy(w.done);
   for (void* p : {(void*)e->d_ix, (void*)e->d_ix_runs[0], (void*)e->d_ix_runs[1], (void*)e->d_ix_ovf, (void*)e->d_ix_win_base, (void*)e->d_ix_win_n,
                   (void*)e->d_ix_win, (void*)e->d_ix_maxw, (void*)e->d_ix_counts}) if (p) cudaFree(p);
@@ -1314,6 +1430,8 @@ int ngsq_reset(ngsq_engine* e) {
   e->h_res.clear(); e->h_qpos = 0;
   e->h_ed_res.clear();
   e->h_ft_res.clear();
+  e->h_grp_sums.clear(); e->h_grp_qlen.clear(); e->h_grp_qual.clear();
+  e->rg_sel = -1;  // the IDs, the table and the group buffer are kept
   for (auto& w : e->ix_waves) cudaEventDestroy(w.done);
   e->ix_waves.clear();
   e->ix_drained.clear();  // pinned memory of the pin slabs, released above
@@ -1661,6 +1779,72 @@ int ngsq_next_file(ngsq_engine* e) {
   return NGSQ_OK;
 }
 
+int ngsq_set_read_groups(ngsq_engine* e, uint32_t n, const char* ids, size_t ids_bytes) {
+  if (!e) return NGSQ_E_ARG;
+  if (!rg_on(e)) return fail(e, NGSQ_E_ARG, "ngsq_set_read_groups: the engine was created without NGSQ_F_READ_GROUPS");
+  if (e->run_started) return fail(e, NGSQ_E_ARG, "ngsq_set_read_groups must precede the first submit");
+  if (!e->d_res) return fail(e, NGSQ_E_ARG, "ngsq_set_read_groups: call ngsq_set_references first");
+  if (n > 65534) return fail(e, NGSQ_E_ARG, "ngsq_set_read_groups: %u read groups, at most 65534", n);
+  if (n && !ids) return fail(e, NGSQ_E_ARG, "ngsq_set_read_groups: ids is NULL");
+  std::vector<uint32_t> off(n + 1, 0);
+  std::vector<std::string> seen;
+  size_t o = 0;
+  for (uint32_t g = 0; g < n; ++g) {
+    const void* z = o < ids_bytes ? memchr(ids + o, 0, ids_bytes - o) : nullptr;
+    if (!z) return fail(e, NGSQ_E_ARG, "ngsq_set_read_groups: ids holds fewer than %u NUL-terminated IDs", n);
+    const size_t len = (size_t)((const char*)z - (ids + o));
+    if (!len) return fail(e, NGSQ_E_ARG, "ngsq_set_read_groups: read group %u has an empty ID", g);
+    seen.emplace_back(ids + o, len);
+    off[g] = (uint32_t)o;
+    o += len + 1;
+  }
+  off[n] = (uint32_t)o;
+  if (o != ids_bytes) return fail(e, NGSQ_E_ARG, "ngsq_set_read_groups: ids holds %zu bytes after its %u IDs", ids_bytes - o, n);
+  std::vector<std::string> sorted = seen;
+  std::sort(sorted.begin(), sorted.end());
+  for (size_t i = 1; i < sorted.size(); ++i)
+    if (sorted[i] == sorted[i - 1]) return fail(e, NGSQ_E_ARG, "ngsq_set_read_groups: the ID \"%s\" is given twice", sorted[i].c_str());
+  // open addressing by FNV-1a, at most half full
+  uint32_t slots = 2;
+  while (slots < 2 * n) slots <<= 1;
+  std::vector<uint32_t> table(slots, kRgEmpty);
+  uint64_t sig = 0xcbf29ce484222325ull ^ n;
+  for (uint32_t g = 0; g < n; ++g) {
+    uint32_t s = rg_hash((const uint8_t*)ids + off[g], (uint32_t)seen[g].size()) & (slots - 1);
+    while (table[s] != kRgEmpty) s = (s + 1) & (slots - 1);
+    table[s] = g + 1;
+  }
+  for (size_t i = 0; i < ids_bytes; ++i) sig = (sig ^ (uint8_t)ids[i]) * 0x100000001b3ull;
+  CU(cudaSetDevice(e->device));
+  e->rg_set = false;
+  e->rg_n = n;
+  int rc;
+  if ((rc = alloc_groups(e, e->qpos_cap, false))) return rc;
+  if ((rc = fresh(e, e->d_rg_ids, std::max<size_t>(ids_bytes, 1), "read-group IDs"))) return rc;
+  if ((rc = fresh(e, e->d_rg_id_off, (size_t)n + 1, "read-group IDs"))) return rc;
+  if ((rc = fresh(e, e->d_rg_table, slots, "read-group table"))) return rc;
+  if ((rc = fresh(e, e->d_rg_count, (size_t)n + 1, "read-group counts"))) return rc;
+  if ((rc = fresh(e, e->d_rg_cursor, (size_t)n + 1, "read-group counts"))) return rc;
+  if (ids_bytes) CU(cudaMemcpy(e->d_rg_ids, ids, ids_bytes, cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(e->d_rg_id_off, off.data(), off.size() * 4, cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(e->d_rg_table, table.data(), table.size() * 4, cudaMemcpyHostToDevice));
+  e->rg_mask = slots - 1;
+  e->rg_sig = sig;
+  e->rg_cap = 0;  // the buckets hold 32 slots of padding per group: sized again by the first wave
+  e->rg_set = true;
+  e->layout_agreed = false;
+  return NGSQ_OK;
+}
+
+int ngsq_select_read_group(ngsq_engine* e, int32_t g) {
+  if (!e) return NGSQ_E_ARG;
+  if (!rg_on(e)) return fail(e, NGSQ_E_ARG, "ngsq_select_read_group: the engine was created without NGSQ_F_READ_GROUPS");
+  if (!e->finished || e->h_grp_sums.empty()) return fail(e, NGSQ_E_ARG, "ngsq_select_read_group before ngsq_finish");
+  if (g < -1 || g > (int32_t)e->rg_n) return fail(e, NGSQ_E_ARG, "ngsq_select_read_group: group %d outside [-1, %u]", g, e->rg_n);
+  e->rg_sel = g;
+  return NGSQ_OK;
+}
+
 int ngsq_progress(ngsq_engine* e, uint64_t* records) {
   if (!e || !records) return NGSQ_E_ARG;
   // waves complete in order: consume the probes of those whose scan has finished (never blocks)
@@ -1777,9 +1961,14 @@ int ngsq_finish(ngsq_engine* e) {
   const uint32_t qpos = (uint32_t)std::min<uint64_t>(e->h_res[R_QUAL_POSITIONS], e->qpos_cap);
   e->h_res.resize((size_t)e->qual_off + (size_t)qpos * 94);
   if (qpos) CU(cudaMemcpyAsync(e->h_res.data() + e->qual_off, e->d_res + e->qual_off, (size_t)qpos * 94 * 8, cudaMemcpyDeviceToHost, s));
+  if (rg_on(e)) {
+    int grc = fetch_groups(e, s);
+    if (grc) return grc;
+  }
   CU(cudaEventRecord(e->ev_f, s));
   CU(cudaStreamSynchronize(s));
   e->finished = true;
+  if (rg_on(e)) e->grp_dirty = std::min(e->grp_rows, std::max<uint32_t>(e->h_state->max_lseq, 256));
   e->h_qpos = qpos;
   e->qpos_dirty = std::max(e->qpos_dirty, std::min<uint32_t>(std::max<uint32_t>(e->h_state->max_lseq, qpos), e->qpos_cap));
   // stats
@@ -1813,6 +2002,7 @@ int ngsq_finish(ngsq_engine* e) {
               i < e->host_ms.size() ? e->host_ms[i] : -1.0, at(w.begin), at(w.decoded_from), at(w.decoded), at(w.resolved), at(w.scan_begin), at(w.scan_end), at(w.facets_end), at(w.crc_begin), at(w.crc_end));
     }
     fprintf(stderr, "[ngsq trace] coverage %.1f..%.1f end %.1f\n", at(e->ev_d), at(e->ev_e), at(e->ev_f));
+    if (rg_on(e)) fprintf(stderr, "[ngsq trace] rg_facets_kernel: %d CTAs per SM, %zu bytes of shared memory each\n", e->rg_occ, e->rg_smem);
   }
   // verdicts, in the order the reference would meet them: a block that does not inflate, a block whose CRC32 is wrong
   // (its garbage bytes break the record chain too: CRC first), then the record chain, then the records
@@ -1888,8 +2078,14 @@ int ngsq_set_index_binning(ngsq_engine* e, uint32_t min_shift, uint32_t depth) {
   return NGSQ_OK;
 }
 
+// the sample's counters, or those of the selected read group (same offsets)
+#define RESULT_WORDS() (e->rg_sel >= 0 ? &e->h_grp_sums[(size_t)e->rg_sel * kGroupSums] : e->h_res.data())
+#define SAMPLE_ONLY(what)                                                                \
+  if (e && e->rg_sel >= 0) return fail(e, NGSQ_E_ARG, "%s: read group %d is selected, and this facet is the sample's only (ngsq_select_read_group(e, -1))", what, e->rg_sel)
+
 int ngsq_get_features(ngsq_engine* e, uint64_t counts[9]) {
   if (!e || !counts) return NGSQ_E_ARG;
+  SAMPLE_ONLY("ngsq_get_features");
   if (!e->finished || e->h_ft_res.size() != F_WORDS) return fail(e, NGSQ_E_ARG, "Genomic Features results requested before ngsq_finish or without NGSQ_F_FEATURES");
   if (e->h_ft_res[F_ERR]) return fail(e, NGSQ_E_FEATURES, "the Genomic Features facet failed; no results");
   memcpy(counts, e->h_ft_res.data(), 9 * 8);
@@ -1898,6 +2094,7 @@ int ngsq_get_features(ngsq_engine* e, uint64_t counts[9]) {
 
 int ngsq_get_edits(ngsq_engine* e, uint64_t read_one[513], uint64_t read_two[513], uint64_t vaf[101], uint64_t* records) {
   if (!e) return NGSQ_E_ARG;
+  SAMPLE_ONLY("ngsq_get_edits");
   if (!e->finished || e->h_ed_res.size() != E_WORDS) return fail(e, NGSQ_E_ARG, "Edits results requested before ngsq_finish or without NGSQ_F_EDITS");
   if (e->h_ed_res[E_ERR]) return fail(e, NGSQ_E_EDITS, "the Edits facet failed; no results");
   if (e->n_split && !e->split_merged)
@@ -1913,6 +2110,7 @@ int ngsq_get_edits(ngsq_engine* e, uint64_t read_one[513], uint64_t read_two[513
 // 1-based like alignment_start + reference_ptr (edits.rs:279-281), entry 0 is never written.
 int ngsq_get_edit_positions(ngsq_engine* e, uint32_t ref, uint32_t* refs, uint32_t* alts, uint64_t n) {
   if (!e) return NGSQ_E_ARG;
+  SAMPLE_ONLY("ngsq_get_edit_positions");
   if (!e->finished || e->h_ed_res.size() != E_WORDS) return fail(e, NGSQ_E_ARG, "Edits results requested before ngsq_finish or without NGSQ_F_EDITS");
   if (e->h_ed_res[E_ERR]) return fail(e, NGSQ_E_EDITS, "the Edits facet failed; no results");
   if (ref >= e->n_ref || ref >= e->ed_contigs.size() || !refs || !alts) return fail(e, NGSQ_E_ARG, "ngsq_get_edit_positions: bad reference id or null output");
@@ -1932,38 +2130,42 @@ int ngsq_get_edit_positions(ngsq_engine* e, uint32_t ref, uint32_t* refs, uint32
 
 int ngsq_get_general(ngsq_engine* e, uint64_t out[34]) {
   NEED_RESULTS();
-  memcpy(out, &e->h_res[R_GENERAL], 34 * 8);
+  memcpy(out, RESULT_WORDS() + R_GENERAL, 34 * 8);
   return NGSQ_OK;
 }
 
 int ngsq_get_tlen(ngsq_engine* e, uint64_t hist[1025], uint64_t* processed, uint64_t* ignored) {
   NEED_RESULTS();
-  memcpy(hist, &e->h_res[R_TLEN_HIST], 1025 * 8);
-  *processed = e->h_res[R_TLEN_PROCESSED];
-  *ignored = e->h_res[R_TLEN_IGNORED];
+  const uint64_t* w = RESULT_WORDS();
+  memcpy(hist, w + R_TLEN_HIST, 1025 * 8);
+  *processed = w[R_TLEN_PROCESSED];
+  *ignored = w[R_TLEN_IGNORED];
   return NGSQ_OK;
 }
 
 int ngsq_get_gc(ngsq_engine* e, uint64_t hist[101], uint64_t nuc[3], uint64_t rec[3]) {
   NEED_RESULTS();
-  memcpy(hist, &e->h_res[R_GC_HIST], 101 * 8);
-  memcpy(nuc, &e->h_res[R_GC_NUC], 24);
-  memcpy(rec, &e->h_res[R_GC_REC], 24);
+  const uint64_t* w = RESULT_WORDS();
+  memcpy(hist, w + R_GC_HIST, 101 * 8);
+  memcpy(nuc, w + R_GC_NUC, 24);
+  memcpy(rec, w + R_GC_REC, 24);
   return NGSQ_OK;
 }
 
 int ngsq_get_quality(ngsq_engine* e, uint64_t* out, size_t cap_positions, uint32_t* n_positions) {
   NEED_RESULTS();
-  uint32_t n = e->h_qpos;
+  const bool grp = e->rg_sel >= 0;
+  uint32_t n = grp ? (uint32_t)e->h_grp_qlen[e->rg_sel] : e->h_qpos;
   if (n_positions) *n_positions = n;
   if (!out) return NGSQ_OK;
   if (cap_positions < n) return fail(e, NGSQ_E_ARG, "quality buffer holds %zu positions, %u needed", cap_positions, n);
-  memcpy(out, &e->h_res[e->qual_off], (size_t)n * 94 * 8);
+  memcpy(out, grp ? e->h_grp_qual[e->rg_sel].data() : &e->h_res[e->qual_off], (size_t)n * 94 * 8);
   return NGSQ_OK;
 }
 
 int ngsq_get_coverage_contig(ngsq_engine* e, uint32_t ref, ngsq_cov_ints* out, uint64_t* bin_sums, size_t cap) {
   NEED_RESULTS();
+  SAMPLE_ONLY("ngsq_get_coverage_contig");
   if (ref >= e->n_ref || !out) return fail(e, NGSQ_E_ARG, "bad reference index");
   if (is_split(e, ref) && !e->split_merged)
     return fail(e, NGSQ_E_ARG, "reference %u is split between shards and not merged yet (ngsq_reduce or ngsq_resolve_split)", ref);
@@ -1984,6 +2186,7 @@ int ngsq_get_coverage_contig(ngsq_engine* e, uint32_t ref, ngsq_cov_ints* out, u
 
 int ngsq_get_coverage_global(ngsq_engine* e, uint64_t* nonsensical_records) {
   NEED_RESULTS();
+  SAMPLE_ONLY("ngsq_get_coverage_global");
   *nonsensical_records = e->h_res[R_NONSENSICAL];
   return NGSQ_OK;
 }
@@ -2068,7 +2271,8 @@ int ngsq_reduce(ngsq_engine* e, int root) {
   const int ncclInt32 = 2, ncclUint32 = 3, ncclUint64 = 5, ncclSum = 0, ncclMax = 2;
   auto nccl_err = [&](const char* what, int rc) { return fail(e, NGSQ_E_NCCL, "%s: %s", what, g_nccl.GetErrorString ? g_nccl.GetErrorString(rc) : "?"); };
   // the split set is part of the agreed layout: ranks that disagree on it would issue different collectives below
-  const uint64_t layout = ((uint64_t)e->qual_off | ((uint64_t)e->qpos_cap << 32)) ^ split_signature(e);
+  const uint64_t layout = ((uint64_t)e->qual_off | ((uint64_t)e->qpos_cap << 32)) ^ split_signature(e) ^
+                          (rg_on(e) ? e->rg_sig * 31 + e->grp_rows : 0);
   int rc;
   if (!e->layout_agreed) {
     uint64_t agree[2] = {layout, ~layout};
@@ -2149,6 +2353,26 @@ int ngsq_reduce(ngsq_engine* e, int root) {
     CU(cudaMemcpyAsync(e->h_ft_res.data(), e->d_ft_res, F_WORDS * 8, cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
     e->other_launches += 1;
+  }
+  if (rg_on(e) && e->rg_set) {
+    // the groups: lengths with max (every rank then issues the same quality reduces), counters with sum, the tables' rows
+    // up to each group's length onto the root
+    const uint64_t ng = (uint64_t)e->rg_n + 1, head = ng * (kGroupSums + 1);
+    uint64_t* qlen = e->d_grp + ng * kGroupSums;
+    if ((rc = g_nccl.AllReduce(qlen, qlen, ng, ncclUint64, ncclMax, e->comm, s))) return nccl_err("ncclAllReduce (read-group lengths)", rc);
+    if ((rc = g_nccl.AllReduce(e->d_grp, e->d_grp, ng * kGroupSums, ncclUint64, ncclSum, e->comm, s))) return nccl_err("ncclAllReduce (read groups)", rc);
+    std::vector<uint64_t> len(ng);
+    CU(cudaMemcpyAsync(len.data(), qlen, ng * 8, cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    e->other_launches += 2;
+    for (uint64_t g = 0; g < ng; ++g) {
+      const uint64_t rows = std::min<uint64_t>(len[g], e->grp_rows);
+      if (!rows) continue;
+      uint64_t* t = e->d_grp + head + g * e->grp_rows * 94;
+      if ((rc = g_nccl.Reduce(t, t, rows * 94, ncclUint64, ncclSum, root, e->comm, s))) return nccl_err("ncclReduce (read-group quality)", rc);
+      e->other_launches += 1;
+    }
+    if ((rc = fetch_groups(e, s))) return rc;
   }
   rc = ngsq_refresh_results(e);
   if (rc) return rc;

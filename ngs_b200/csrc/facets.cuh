@@ -181,6 +181,83 @@ __device__ __forceinline__ void gc_window_counts(const uint8_t* seq, uint32_t gj
   *at_out = at;
 }
 
+// ---- per-record rules, shared by facets_kernel and the per-read-group pass (read_groups.cuh) ----
+// The fixed 36 header bytes of the record at p (its block_size word) at any alignment: ten aligned words, nine funnel shifts.
+// Returns false when the fields overrun block_size or a reference id is out of range (the run fails with NGSQ_E_BAD_RECORD).
+struct RecHeader {
+  uint32_t bs, lseq, f, ncig, lname, mapq;
+  int32_t ref, pos, nref, tlen;
+};
+__device__ __forceinline__ bool load_record_header(const uint8_t* p, int32_t n_ref, RecHeader& h) {
+  const uint32_t* w = reinterpret_cast<const uint32_t*>(reinterpret_cast<uintptr_t>(p) & ~uintptr_t(3));
+  const uint32_t sh = (uint32_t)(reinterpret_cast<uintptr_t>(p) & 3) * 8;
+  const uint32_t a0 = w[0], a1 = w[1], a2 = w[2], a3 = w[3], a4 = w[4], a5 = w[5], a6 = w[6], a7 = w[7], a8 = w[8], a9 = w[9];
+  h.bs = __funnelshift_r(a0, a1, sh);
+  h.ref = (int32_t)__funnelshift_r(a1, a2, sh);
+  h.pos = (int32_t)__funnelshift_r(a2, a3, sh);
+  const uint32_t w3 = __funnelshift_r(a3, a4, sh);
+  const uint32_t w4 = __funnelshift_r(a4, a5, sh);
+  h.lseq = __funnelshift_r(a5, a6, sh);
+  h.nref = (int32_t)__funnelshift_r(a6, a7, sh);
+  h.tlen = (int32_t)__funnelshift_r(a8, a9, sh);
+  h.lname = w3 & 255; h.mapq = (w3 >> 8) & 255; h.ncig = w4 & 0xFFFF; h.f = w4 >> 16;
+  const uint64_t need = 32ull + h.lname + 4ull * h.ncig + (h.lseq + 1ull) / 2 + h.lseq;
+  return !(need > h.bs || h.ref < -1 || h.ref >= n_ref || h.nref < -1 || h.nref >= n_ref);
+}
+
+// General counters (general.rs:31-101): bit k set <=> counter k of ngsq_get_general counts the record.  A mapped pair
+// without reference ids sets err_rec (the reference panics there, general.rs:81-83).
+__device__ __forceinline__ uint32_t general_bits(uint32_t f, int32_t ref, int32_t nref, uint32_t mapq, uint32_t& err_rec) {
+  uint32_t bits = 1u;
+  if (f & 0x4) bits |= 1u << 1;
+  if (f & 0x400) bits |= 1u << 2;
+  if (f & 0x100) bits |= 1u << 4;
+  else if (f & 0x800) bits |= 1u << 5;
+  else {
+    bits |= 1u << 3;
+    if (!(f & 0x4)) bits |= 1u << 6;
+    if (f & 0x400) bits |= 1u << 7;
+    if (f & 0x1) {
+      bits |= 1u << 8;
+      if (f & 0x40) bits |= 1u << 9;
+      if (f & 0x80) bits |= 1u << 10;
+      if (!(f & 0x4)) {
+        if (f & 0x2) bits |= 1u << 11;
+        if (f & 0x8) bits |= 1u << 12;
+        else {
+          bits |= 1u << 13;
+          if (ref < 0 || nref < 0) err_rec = 1;  // the reference panics here (general.rs:81-83)
+          else if (ref != nref) {
+            bits |= 1u << 14;
+            if (mapq >= 5) bits |= 1u << 15;     // missing (255) counts (general.rs:88-95)
+          }
+        }
+      }
+    }
+  }
+  return bits;
+}
+
+// Template length (template_length.rs:79-87, `tlen as usize`, bins 0..=1024): bit 16 processed (bin = tlen), bit 17 ignored
+__device__ __forceinline__ uint32_t tlen_bits(int32_t tlen) { return (tlen >= 0 && tlen <= 1024) ? 1u << 16 : 1u << 17; }
+
+// GC content eligibility (gc_content.rs:38-75): bit 18 processed, 19 ignored (flags), 20 ignored (too short)
+__device__ __forceinline__ uint32_t gc_bits(uint32_t f, uint32_t lseq) {
+  if (f & (0x400 | 0x100)) return 1u << 19;
+  if (lseq < 100) return 1u << 20;
+  return 1u << 18;
+}
+
+// Window offset of a GC-processed read with l_seq > 100 (gc_content.rs:69-74, see ngsq_get_gc): keyed by the record's BGZF
+// virtual offset, i.e. its block's file offset and its offset in that block (the record carried into the wave: carry_voff)
+__device__ __forceinline__ uint32_t gc_window_offset(uint64_t rv, const BlockDesc* blocks, uint64_t carry_voff, uint32_t headroom,
+                                                     uint64_t out0, uint64_t gc_seed, uint32_t lseq) {
+  const uint32_t t = (uint32_t)(rv >> 40);
+  uint64_t voff = carry_voff;
+  if (t) { const BlockDesc& bd = blocks[t - 1]; voff = (bd.coff << 16) | ((rv & kRecOffMask) - headroom - (bd.out_off - out0)); }
+  return (uint32_t)(((splitmix64_dev(gc_seed ^ voff) >> 32) * (uint64_t)(lseq - 100)) >> 32);
+}
+
 __global__ void __launch_bounds__(kFacetThreads) facets_kernel(FacetParams P) {
   extern __shared__ uint32_t sm[];
   const uint32_t warps_in_cta = blockDim.x >> 5;
@@ -217,21 +294,10 @@ __global__ void __launch_bounds__(kFacetThreads) facets_kernel(FacetParams P) {
     if (valid) {
       rv = P.rec[r];
       p = P.d + (rv & kRecOffMask);
-      // 36 header bytes at any alignment: ten aligned words, nine funnel shifts
-      const uint32_t* w = reinterpret_cast<const uint32_t*>(reinterpret_cast<uintptr_t>(p) & ~uintptr_t(3));
-      const uint32_t sh = (uint32_t)(reinterpret_cast<uintptr_t>(p) & 3) * 8;
-      const uint32_t a0 = w[0], a1 = w[1], a2 = w[2], a3 = w[3], a4 = w[4], a5 = w[5], a6 = w[6], a7 = w[7], a8 = w[8], a9 = w[9];
-      const uint32_t bs = __funnelshift_r(a0, a1, sh);
-      ref = (int32_t)__funnelshift_r(a1, a2, sh);
-      pos = (int32_t)__funnelshift_r(a2, a3, sh);
-      const uint32_t w3 = __funnelshift_r(a3, a4, sh);
-      const uint32_t w4 = __funnelshift_r(a4, a5, sh);
-      lseq = __funnelshift_r(a5, a6, sh);
-      nref = (int32_t)__funnelshift_r(a6, a7, sh);
-      tlen = (int32_t)__funnelshift_r(a8, a9, sh);
-      lname = w3 & 255; mapq = (w3 >> 8) & 255; ncig = w4 & 0xFFFF; f = w4 >> 16;
-      const uint64_t need = 32ull + lname + 4ull * ncig + (lseq + 1ull) / 2 + lseq;
-      if (need > bs || ref < -1 || ref >= P.n_ref || nref < -1 || nref >= P.n_ref) { err_rec = 1; valid = false; }
+      RecHeader h;
+      if (!load_record_header(p, P.n_ref, h)) { err_rec = 1; valid = false; }
+      ref = h.ref; pos = h.pos; lseq = h.lseq; nref = h.nref; tlen = h.tlen;
+      lname = h.lname; mapq = h.mapq; ncig = h.ncig; f = h.f;
     }
     const uint8_t* cig = p + 36 + lname;
     const uint8_t* seq = cig + 4 * (size_t)ncig;
@@ -328,51 +394,13 @@ __global__ void __launch_bounds__(kFacetThreads) facets_kernel(FacetParams P) {
     bool gc_on = false;
     uint32_t gc_off = 0;
     if (rec_on) {
-      bits = 1u;
-      if (f & 0x4) bits |= 1u << 1;
-      if (f & 0x400) bits |= 1u << 2;
-      if (f & 0x100) bits |= 1u << 4;
-      else if (f & 0x800) bits |= 1u << 5;
-      else {
-        bits |= 1u << 3;
-        if (!(f & 0x4)) bits |= 1u << 6;
-        if (f & 0x400) bits |= 1u << 7;
-        if (f & 0x1) {
-          bits |= 1u << 8;
-          if (f & 0x40) bits |= 1u << 9;
-          if (f & 0x80) bits |= 1u << 10;
-          if (!(f & 0x4)) {
-            if (f & 0x2) bits |= 1u << 11;
-            if (f & 0x8) bits |= 1u << 12;
-            else {
-              bits |= 1u << 13;
-              if (ref < 0 || nref < 0) err_rec = 1;  // the reference panics here (general.rs:81-83)
-              else if (ref != nref) {
-                bits |= 1u << 14;
-                if (mapq >= 5) bits |= 1u << 15;     // missing (255) counts (general.rs:88-95)
-              }
-            }
-          }
-        }
-      }
-      // ---- Template length (template_length.rs:79-87): `tlen as usize`, bins 0..=1024
-      if (tlen >= 0 && tlen <= 1024) {
-        bits |= 1u << 16;
-        atomicAdd(&s_tlen[tlen], 1u);
-      } else bits |= 1u << 17;
-      // ---- GC content eligibility (gc_content.rs:38-75)
-      if (f & (0x400 | 0x100)) bits |= 1u << 19;
-      else if (lseq < 100) bits |= 1u << 20;
-      else {
-        bits |= 1u << 18;
+      bits = general_bits(f, ref, nref, mapq, err_rec);
+      bits |= tlen_bits(tlen);
+      if (bits & (1u << 16)) atomicAdd(&s_tlen[tlen], 1u);
+      bits |= gc_bits(f, lseq);
+      if (bits & (1u << 18)) {
         gc_on = true;
-        if (lseq > 100) {
-          // the record's BGZF virtual offset: its block's file offset and its offset in that block
-          const uint32_t t = (uint32_t)(rv >> 40);
-          uint64_t voff = P.st->carry_voff;
-          if (t) { const BlockDesc& bd = P.blocks[t - 1]; voff = (bd.coff << 16) | ((rv & kRecOffMask) - P.headroom - (bd.out_off - P.out0)); }
-          gc_off = (uint32_t)(((splitmix64_dev(P.gc_seed ^ voff) >> 32) * (uint64_t)(lseq - 100)) >> 32);
-        }
+        if (lseq > 100) gc_off = gc_window_offset(rv, P.blocks, P.st->carry_voff, P.headroom, P.out0, P.gc_seed, lseq);
       }
     }
 #pragma unroll

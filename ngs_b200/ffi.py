@@ -25,6 +25,7 @@ NGSQ_F_SERIAL_STAGES = 32  # measurement aid: no overlap between the stages of c
 NGSQ_F_INDEX = 64  # build the file's BAI in the same pass (Engine.bai())
 NGSQ_F_INDEX_PART = 128  # index one range of a file cut between engines (join the parts with join_bai())
 NGSQ_F_INDEX_CSI = 256  # with NGSQ_F_INDEX / NGSQ_F_INDEX_PART: a CSI instead of a BAI (Engine.csi(), join_csi())
+NGSQ_F_READ_GROUPS = 512  # with NGSQ_F_RECORD_FACETS: the record facets per read group (Engine.set_read_groups / select_read_group)
 
 ERROR_NAMES = {
     0: "NGSQ_OK", -1: "NGSQ_E_ARG", -2: "NGSQ_E_CUDA", -3: "NGSQ_E_TRUNCATED", -4: "NGSQ_E_BAD_BLOCK",
@@ -43,7 +44,8 @@ EXPORTED = [
     "ngsq_set_reference_bases", "ngsq_get_edits", "ngsq_get_edit_positions", "ngsq_set_feature_model", "ngsq_set_features", "ngsq_get_features",
     "ngsq_wait_copied", "ngsq_host_register", "ngsq_host_unregister", "ngsq_flush", "ngsq_progress",
     "ngsq_get_bai", "ngsq_split_reference", "ngsq_split_arrays", "ngsq_resolve_split", "ngsq_find_record", "ngsq_join_bai",
-    "ngsq_set_index_binning", "ngsq_get_csi", "ngsq_join_csi", "ngsq_next_file",
+    "ngsq_set_index_binning", "ngsq_get_csi", "ngsq_join_csi", "ngsq_next_file", "ngsq_set_read_groups",
+    "ngsq_select_read_group",
 ]
 
 
@@ -156,6 +158,8 @@ def load_library() -> C.CDLL:
     lib.ngsq_set_index_binning.argtypes = [P, C.c_uint32, C.c_uint32]
     lib.ngsq_get_csi.argtypes = [P, P, C.c_size_t, C.POINTER(C.c_size_t)]
     lib.ngsq_join_csi.argtypes = [C.POINTER(P), C.c_uint32, P, C.c_size_t, C.POINTER(C.c_size_t)]
+    lib.ngsq_set_read_groups.argtypes = [P, C.c_uint32, C.c_char_p, C.c_size_t]
+    lib.ngsq_select_read_group.argtypes = [P, C.c_int32]
     _lib = lib
     return lib
 
@@ -244,6 +248,16 @@ class Engine:
     def next_file(self):
         """The chunks since the last set_range were one whole file; the next set_range starts another of the same run."""
         self._check(self.lib.ngsq_next_file(self.h))
+
+    def set_read_groups(self, ids):
+        """The @RG IDs (str or bytes), in order: group g = ids[g], group len(ids) = ungrouped (NGSQ_F_READ_GROUPS)."""
+        raw = [i.encode() if isinstance(i, str) else bytes(i) for i in ids]
+        blob = b"".join(i + b"\0" for i in raw)
+        self._check(self.lib.ngsq_set_read_groups(self.h, len(raw), blob, len(blob)))
+
+    def select_read_group(self, g: int):
+        """After finish: -1 = the sample, 0..n = a read group; the record-facet getters then return its integers."""
+        self._check(self.lib.ngsq_select_read_group(self.h, g))
 
     def progress(self) -> int:
         v = C.c_uint64(0)
@@ -480,6 +494,8 @@ def _load_synth():
                                      C.POINTER(C.c_void_p), C.POINTER(SynthInfo)]
         _synth.synth_bam_subset.argtypes = [C.c_int, C.c_uint64, C.c_uint64, C.c_int, C.c_int, C.c_uint64, C.c_int,
                                             C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(SynthInfo)]
+        _synth.synth_bam_rg.argtypes = [C.c_int, C.c_uint64, C.c_uint64, C.c_int, C.c_int, C.c_uint32, C.POINTER(C.c_void_p),
+                                        C.POINTER(C.c_void_p), C.POINTER(SynthInfo)]
         _synth.synth_layout.argtypes = [C.c_int, C.c_uint64, C.POINTER(C.c_uint64), C.c_uint32, C.POINTER(C.c_uint32),
                                         C.POINTER(C.c_uint64)]
         _synth.synth_free.argtypes = [C.c_void_p]
@@ -487,15 +503,21 @@ def _load_synth():
 
 
 def synth_bam(shape: int, n_records: int, seed: int | None = None, level: int = 6, threads: int = 0,
-              contig_mask: int | None = None, with_tail: bool = True):
+              contig_mask: int | None = None, with_tail: bool = True, read_groups: int = 1):
     """Deterministic synthetic BAM + BAI (tools/bamgen.cpp).  Returns (bam u8 array, bai u8 array, info dict).
-    With contig_mask, only those contigs (and the tail if with_tail) of the logical n_records file are written."""
+    With contig_mask, only those contigs (and the tail if with_tail) of the logical n_records file are written.
+    read_groups = K in 1..10: the header declares rg0..rg{K-1} and every record carries one of them (K = 1: rg0, the
+    bytes of the generator without the option); not with contig_mask."""
     global _synth
     _load_synth()
     if seed is None:
         seed = 0x5EED0001 + shape
     bam, bai, info = C.c_void_p(), C.c_void_p(), SynthInfo()
-    if contig_mask is None:
+    if read_groups != 1:
+        if contig_mask is not None:
+            raise ValueError("synth_bam: read_groups is not available with contig_mask")
+        rc = _synth.synth_bam_rg(shape, n_records, seed, level, threads, read_groups, C.byref(bam), C.byref(bai), C.byref(info))
+    elif contig_mask is None:
         rc = _synth.synth_bam(shape, n_records, seed, level, threads, C.byref(bam), C.byref(bai), C.byref(info))
     else:
         rc = _synth.synth_bam_subset(shape, n_records, seed, level, threads, contig_mask, int(with_tail), C.byref(bam),

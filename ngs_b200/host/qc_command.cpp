@@ -11,10 +11,11 @@
 // takes records in any order (unsorted, queryname-sorted or collated files): one shard, or cuts at record anchors with every
 // reference split between the devices.  `qc --cuda-also <BAM>` adds files of the same sample under the same rules: whole files
 // queued on each device (ngsq_next_file between them), or with fewer files than devices each file cut between its devices.
+// `qc --cuda-by-read-group` also writes the record facets of every @RG read group, tallied in the same pass (NGSQ_F_READ_GROUPS).
 //
 //   ngs-cuda-qc qc <BAM> <REFERENCE_GENOME> [-n N] [-o DIR] [-p PREFIX] [--only FACET]
 //               [--cuda-devices 0,1,..] [--cuda-build-index [--cuda-csi [--cuda-min-shift N]] | --cuda-any-order] [--cuda-gc-seed S]
-//               [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io] [--cuda-perf] [--cuda-also <BAM> ..]
+//               [--cuda-no-crc] [--cuda-chunk-mb M] [--cuda-buffered-io] [--cuda-perf] [--cuda-also <BAM> ..] [--cuda-by-read-group]
 //   ngs-cuda-qc index <BAM> [--csi [-m|--min-shift N]] [--cuda-device N | --cuda-devices 0,1,..] [--cuda-no-crc] [--cuda-chunk-mb M]
 //                     [--cuda-buffered-io]
 #include <cerrno>
@@ -32,6 +33,7 @@
 
 #include "bam.hpp"
 #include "facets.hpp"
+#include "read_groups.hpp"
 
 using namespace ngs;
 
@@ -56,6 +58,7 @@ struct QcArgs {
   uint32_t min_shift = 14;   // --cuda-min-shift (CSI); the depth follows samtools' rule
   bool any_order = false;    // --cuda-any-order: no index is read, the records may come in any order
   std::vector<std::string> also;  // --cuda-also: more files of the sample, checked with src as one (implies any_order)
+  bool by_read_group = false;     // --cuda-by-read-group: one more results JSON per @RG read group
 };
 
 void info(const std::string& s) { std::cerr << "INFO " << s << "\n"; }
@@ -433,9 +436,21 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   if (coverage) flags |= NGSQ_F_COVERAGE;
   if (features) flags |= NGSQ_F_FEATURES;
   if (edits) flags |= NGSQ_F_EDITS;
+  if (args.by_read_group) flags |= NGSQ_F_READ_GROUPS;  // --only leaves a record facet here (check_read_group_facet)
   if (args.verify_crc) flags |= NGSQ_F_VERIFY_CRC;
   if (build_index) flags |= (n_dev > 1 ? NGSQ_F_INDEX_PART : NGSQ_F_INDEX) | (build_csi ? NGSQ_F_INDEX_CSI : 0u);
   if (args.num_records && n_dev > 1) throw std::runtime_error("-n needs a single device (records are counted in file order)");
+  // --cuda-by-read-group: the groups are the union of the files' @RG IDs, checked before any device work
+  std::vector<std::string> rg_ids;
+  if (args.by_read_group) {
+    std::vector<std::vector<std::string>> per_file{read_group_ids(bam_header_text(file.data(), file.size(), args.src), args.src)};
+    for (size_t k = 0; k < args.also.size(); ++k)
+      per_file.push_back(read_group_ids(bam_header_text(also_files[k]->data(), also_files[k]->size(), args.also[k]), args.also[k]));
+    rg_ids = union_read_group_ids(per_file);
+    info("  [*] " + std::to_string(rg_ids.size()) + " read group" + (rg_ids.size() == 1 ? "" : "s") + ": one more results file each.");
+  }
+  std::string rg_blob;
+  for (const std::string& id : rg_ids) { rg_blob += id; rg_blob += '\0'; }
 
   std::vector<ngsq_engine*> engines(n_dev, nullptr);
   struct Cleanup { std::vector<ngsq_engine*>& v; ~Cleanup() { for (auto* e : v) if (e) ngsq_destroy(e); } } cleanup{engines};
@@ -527,6 +542,7 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
     if (features) features->upload(engines[i], header.reference_sequences);
     if (edits) edits->upload(engines[i], header.reference_sequences);
     for (uint32_t c : plan.split) check(engines[i], ngsq_split_reference(engines[i], c));
+    if (args.by_read_group) check(engines[i], ngsq_set_read_groups(engines[i], (uint32_t)rg_ids.size(), rg_blob.data(), rg_blob.size()));
   }
   if (n_dev > 1) {
     char id[128];
@@ -602,6 +618,12 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   for (auto& f : facets.sequence_based) f->aggregate(results);
   info("Writing output.");
   results.write(output_prefix, output_directory);
+  if (args.by_read_group) {
+    const uint64_t ungrouped = write_read_group_results(root, rg_ids, genome, args.only_facet, output_prefix, output_directory);
+    if (ungrouped)
+      std::cerr << "WARN " << ungrouped << " record(s) carry no RG tag, or one that no @RG line declares: written to "
+                << no_read_group_prefix(output_prefix) << ".results.json\n";
+  }
   if (build_index) write_index(build_csi ? csi_path : bai_path, build_csi ? bgzf_compress(new_index) : new_index);
 
   if (args.perf) {
@@ -766,6 +788,11 @@ void usage() {
                "       ngs-cuda-qc qc <BAM> <REFERENCE_GENOME> --cuda-also <BAM> [--cuda-also <BAM> ..] [the options above]\n"
                "                  (the records of every file are checked as one sample: the files must have the same reference\n"
                "                  sequences; the rules of --cuda-any-order apply; the output prefix is the first <BAM>'s name)\n"
+               "       ngs-cuda-qc qc <BAM> <REFERENCE_GENOME> --cuda-by-read-group [the options above]\n"
+               "                  (also writes <PREFIX>.read_group.<ID>.results.json for every @RG line, with General, Template Length,\n"
+               "                  GC Content and Quality Score of that group's records, and <PREFIX>.no_read_group.results.json for\n"
+               "                  records of no declared group; <ID> with bytes outside [A-Za-z0-9._-] and '%' as %XX; not with\n"
+               "                  --only Coverage, Edits or \"Genomic Features\")\n"
                "       ngs-cuda-qc index <BAM> [--csi [-m|--min-shift N]] [--cuda-device N | --cuda-devices 0,1,..] [--cuda-no-crc] [--cuda-chunk-mb M]\n"
                "                  [--cuda-buffered-io]\n"
                "                  (writes <BAM>.bai, or with --csi <BAM>.csi (min_shift N, default 14); an existing index is never overwritten;\n"
@@ -810,6 +837,7 @@ extern "C" int ngs_cuda_qc_main(int argc, char** argv) {
       else if (s == "--cuda-csi") a.csi = true;
       else if (s == "--cuda-any-order") a.any_order = true;
       else if (s == "--cuda-also") a.also.push_back(val());
+      else if (s == "--cuda-by-read-group") a.by_read_group = true;
       else if (s == "--cuda-min-shift") { a.min_shift = (uint32_t)std::stoul(val()); min_shift_set = true; }
       else if (s == "--cuda-buffered-io") a.direct_io = false;
       else if (s == "-h" || s == "--help") { usage(); return 0; }
@@ -832,6 +860,7 @@ extern "C" int ngs_cuda_qc_main(int argc, char** argv) {
     if (a.build_index && a.num_records) throw std::runtime_error("--cuda-build-index cannot be combined with -n: an index covers every record of the file");
     if (a.csi && !a.build_index) throw std::runtime_error("--cuda-csi sets the format of the index --cuda-build-index writes: use it with --cuda-build-index");
     if (min_shift_set && !a.csi) throw std::runtime_error("--cuda-min-shift sets the binning of a CSI: use it with --cuda-csi");
+    if (a.by_read_group) check_read_group_facet(a.only_facet);
     a.src = pos[0];
     a.reference_genome = pos[1];
     return qc(a);

@@ -93,6 +93,7 @@ struct Shape {
   std::vector<uint64_t> cum;  // cum[c] = first record index of contig c; cum[n_ref] = first tail record
   uint64_t seed = 0;
   uint32_t read_len = 150;
+  uint32_t read_groups = 1;  // @RG rg0..rg{K-1}; K = 1 writes the bytes of a generator without read groups
   uint64_t hot_lo = 0, hot_n = 0;  // hotspot in contig 0: records [hot_lo, hot_lo+hot_n) share one pos
   // subset generation (one shard of the logical file): global record-index ranges, ascending
   std::vector<std::pair<uint64_t, uint64_t>> ranges;
@@ -416,6 +417,7 @@ void make_record(const Shape& sh, uint64_t i, const Meta& m, uint8_t* out) {
   p[0] = 'N'; p[1] = 'M'; p[2] = 'C'; p[3] = (uint8_t)(r % 6);
   p[4] = 'A'; p[5] = 'S'; p[6] = 'C'; p[7] = (uint8_t)(100 + (r >> 8) % 51);
   memcpy(p + 8, "RGZrg0", 7);  // includes NUL
+  if (sh.read_groups > 1) p[13] = (uint8_t)('0' + (r >> 32) % sh.read_groups);  // the high half of the NM / AS draw
 }
 
 struct Built {
@@ -478,7 +480,7 @@ void setup_shape(Shape& sh, int kind, uint64_t n, uint64_t seed) {
 std::vector<uint8_t> make_header(const Shape& sh) {
   std::string text = "@HD\tVN:1.6\tSO:coordinate\n";
   for (auto& c : sh.contigs) text += std::string("@SQ\tSN:") + c.name + "\tLN:" + std::to_string(c.len) + "\n";
-  text += "@RG\tID:rg0\tSM:synthetic\n";
+  for (uint32_t k = 0; k < sh.read_groups; ++k) text += "@RG\tID:rg" + std::to_string(k) + "\tSM:synthetic\n";
   text += "@PG\tID:bamgen\tPN:bamgen\n";
   std::vector<uint8_t> h;
   auto p32 = [&](uint32_t v) { uint8_t b[4]; put32(b, v); h.insert(h.end(), b, b + 4); };
@@ -752,6 +754,35 @@ int synth_bam_subset(int shape, uint64_t n_records, uint64_t seed, int level, in
     info->bai_bytes = b.bai.size();
     info->n_blocks = b.n_blocks;
     info->n_ref = (uint32_t)n_ref;
+  }
+  return 0;
+}
+
+// synth_bam with K read groups (1..10): the header declares rg0..rg{K-1} and each record's RG:Z takes its group from bits of
+// the random draw its NM and AS values come from, so records keep their length; K = 1 is synth_bam.
+int synth_bam_rg(int shape, uint64_t n_records, uint64_t seed, int level, int threads, uint32_t read_groups, uint8_t** bam,
+                 uint8_t** bai, synth_info* info) {
+  if (shape < 0 || shape > 4 || !bam || !bai || read_groups < 1 || read_groups > 10) return -1;
+  if (threads <= 0) threads = (int)std::thread::hardware_concurrency();
+  if (threads <= 0) threads = 1;
+  Shape sh;
+  setup_shape(sh, shape, n_records, seed);
+  sh.read_groups = read_groups;
+  Built b;
+  build(sh, level, threads, b);
+  *bam = (uint8_t*)malloc(b.bam.size() ? b.bam.size() : 1);
+  *bai = (uint8_t*)malloc(b.bai.size() ? b.bai.size() : 1);
+  if (!*bam || !*bai) return -2;
+  memcpy(*bam, b.bam.data(), b.bam.size());
+  memcpy(*bai, b.bai.data(), b.bai.size());
+  if (info) {
+    info->n_records = b.n_records;
+    info->inflated_bytes = b.inflated;
+    info->header_bytes = b.header_inflated;
+    info->bam_bytes = b.bam.size();
+    info->bai_bytes = b.bai.size();
+    info->n_blocks = b.n_blocks;
+    info->n_ref = (uint32_t)sh.contigs.size();
   }
   return 0;
 }
