@@ -423,7 +423,7 @@ constexpr uint32_t kFindBlocksMax = 4096;  // its largest window (256 MiB inflat
 // Cuts at targets first_record_coffset + (file_size - that) * k / n, each snapped to the next block start and moved to the
 // first record the finder sees from there (its window doubles until it sees one).  A cut is dropped when no record is found
 // or when its anchor does not lie strictly behind the previous one; its device gets an empty shard.  The anchors are
-// speculative until the range in front of each closes on it (run_parts in the driver).  Only the reference of the first
+// speculative until the range in front of each closes on it (run_plan in the driver).  Only the reference of the first
 // record behind a cut can have records on both sides of it (sorted input), so those references are the split set; the
 // driver declares them whether or not Coverage processes them, because Edits keeps per-position counters of every contig.
 inline ShardPlan plan_shards_unindexed(const BamHeader& h, const uint8_t* bam, uint64_t file_size, uint32_t n_shards, const FindRecord& find) {
@@ -529,13 +529,16 @@ inline std::vector<uint32_t> devices_per_file(const std::vector<uint64_t>& bytes
 struct FilePart { uint32_t file = 0; Shard shard; };
 struct FilePlan {
   std::vector<std::vector<FilePart>> queues;  // per device, in the order it runs them
-  bool cut = false;                           // F < D: one part of one file per device, the devices of a file in file order
+  std::vector<uint32_t> split;                // split references, ascending: declared on every engine
+  // one part of one file per device, the devices of a file in file order; the parts after a file's first start at record
+  // anchors, which are speculative until the run proves them (the range in front of each closes on it)
+  bool cut = false;
   uint32_t dropped = 0;                       // cuts left out (plan_shards_unindexed)
 };
 
 // The plan of F files on D devices.  F >= D: assign_files, each file from its first record to EOF.  F < D: each file cut by
 // plan_shards_any_order into devices_per_file parts, the devices of file 0 first.  Every reference is split between the
-// devices either way (the caller declares them when D > 1): each device holds records of any reference.
+// devices either way when D > 1: each device holds records of any reference.
 inline FilePlan plan_files(const std::vector<BamHeader>& headers, const std::vector<const uint8_t*>& data, const std::vector<uint64_t>& sizes,
                            uint32_t n_dev, const FindRecord& find) {
   const uint32_t n_files = (uint32_t)headers.size();
@@ -546,6 +549,8 @@ inline FilePlan plan_files(const std::vector<BamHeader>& headers, const std::vec
     bytes[f] = shard_compressed_bytes(whole[f], sizes[f]);
   }
   FilePlan plan;
+  if (n_dev > 1)
+    for (uint32_t c = 0; c < headers[0].reference_sequences.size(); ++c) plan.split.push_back(c);
   if (n_files >= n_dev) {
     for (const auto& files : assign_files(bytes, n_dev)) {
       plan.queues.emplace_back();

@@ -2,12 +2,14 @@
 // (src/qc/command.rs): QcArgs (36-102), qc() (109-218), app() (226-421).  Same positional
 // arguments and flags, same checks in the same order, same output file; the two hot loops of
 // app() (305-316 and 350-397) are replaced by one pass of the CUDA engine per GPU.  `index` builds the
-// BAI that `qc` needs (src/index/bam.rs:39-109) in one pass of the engine on one GPU.
+// BAI that `qc` needs (src/index/bam.rs:39-109) in one pass of the engine.
 //
-// A BAM without an index is cut between GPUs at record anchors the engine finds (ngsq_find_record), each GPU indexes its part
-// (NGSQ_F_INDEX_PART) and the host joins the parts (ngsq_join_bai): `index --cuda-devices`, and `qc --cuda-build-index`,
-// which writes the missing index (.bai, or .csi with --cuda-csi) in the same pass as the results.  `qc` plans its shards from
-// <BAM>.bai, or from <BAM>.csi when there is no .bai (the reference needs the .bai).  `qc --cuda-any-order` reads no index and
+// Every run is a FilePlan: each GPU runs a queue of (file, shard) entries through one engine (stream_queue), and cuts at record
+// anchors are proven by the run (run_plan).  A BAM without an index is cut between GPUs at record anchors the engine finds
+// (ngsq_find_record), each GPU indexes its part (NGSQ_F_INDEX_PART; one GPU indexes the whole file as one part) and the host
+// joins the parts (ngsq_join_bai): `index`, and `qc --cuda-build-index`, which writes the missing index (.bai, or .csi with
+// --cuda-csi) in the same pass as the results.  `qc` plans its shards from <BAM>.bai, or from <BAM>.csi when there is no .bai
+// (the reference needs the .bai).  `qc --cuda-any-order` reads no index and
 // takes records in any order (unsorted, queryname-sorted or collated files): one shard, or cuts at record anchors with every
 // reference split between the devices.  `qc --cuda-also <BAM>` adds files of the same sample under the same rules: whole files
 // queued on each device (ngsq_next_file between them), or with fewer files than devices each file cut between its devices.
@@ -193,142 +195,114 @@ class ChunkReader {
   int32_t used_by_[kBufs] = {-1, -1, -1};
 };
 
-void run_shard(ngsq_engine* e, const std::string& path, const MappedFile& file, const Shard& shard, size_t chunk_bytes, bool direct, bool log_progress,
-               std::string* err, int* code) {
-  try {
-    if (shard.empty) { check(e, ngsq_set_range(e, 0, 0)); check(e, ngsq_finish(e)); return; }
-    uint64_t lo, hi;
-    shard_bytes(shard, file.data(), file.size(), &lo, &hi);
-    ChunkReader reader(path, chunk_bytes, direct);
-    for (int attempt = 0;; ++attempt) {
-      check(e, ngsq_set_range(e, shard.first_voffset, shard.end_voffset));
-      Progress progress;
-      reader.run(e, lo, hi, log_progress ? &progress : nullptr);
-      const int rc = ngsq_finish(e);
-      if (rc == NGSQ_E_QUAL_CAP && attempt == 0) {
-        // a read longer than the quality-by-position table (131072 positions by default): size the table for the
-        // longest read the scan met and stream the shard again — the engine keeps nothing of a file it has streamed
-        ngsq_stats st;
-        check(e, ngsq_get_stats(e, &st));
-        info("  [*] Reads of up to " + std::to_string(st.max_read_len) + " bases: enlarging the quality table and reading the file again.");
-        check(e, ngsq_reset(e));
-        check(e, ngsq_set_quality_positions(e, (uint32_t)st.max_read_len + 1));
-        continue;
+// f(i) for every i < n, each in a thread of its own; once all have returned, the first error (the lowest i) is thrown again.
+template <class F>
+void on_each(size_t n, const F& f) {
+  std::vector<std::string> errs(n);
+  std::vector<std::thread> ts;
+  for (size_t i = 0; i < n; ++i)
+    ts.emplace_back([&, i] {
+      try {
+        f(i);
+      } catch (const std::exception& ex) {
+        errs[i] = ex.what();
       }
-      if (code) *code = rc;
-      check(e, rc);
-      if (log_progress) progress.report(e);
-      break;
+    });
+  for (auto& t : ts) t.join();
+  for (auto& s : errs) if (!s.empty()) throw std::runtime_error(s);
+}
+
+// One engine over its queue of (file, shard) entries: each entry's range and bytes, ngsq_next_file between two entries, one
+// ngsq_finish behind the last.  An empty entry sets the range (0, 0) and streams nothing.  A read longer than the
+// quality-by-position table (131072 positions by default) sizes the table for the longest read the scan met and runs the
+// queue again: the engine keeps nothing of a file it has streamed.  Returns ngsq_finish's code; any other failure throws.
+int stream_queue(ngsq_engine* e, const std::vector<FilePart>& queue, const std::vector<std::string>& paths, const std::vector<const MappedFile*>& files,
+              size_t chunk_bytes, bool direct, bool log_progress) {
+  std::unique_ptr<ChunkReader> reader;  // made at the first live entry: a queue without one allocates no pinned buffers
+  for (int attempt = 0;; ++attempt) {
+    Progress progress;
+    bool same_run = false;  // an earlier entry of this attempt has submitted to e
+    for (size_t k = 0; k < queue.size(); ++k) {
+      const FilePart& q = queue[k];
+      if (k) check(e, ngsq_next_file(e));
+      check(e, ngsq_set_range(e, q.shard.first_voffset, q.shard.end_voffset));
+      if (q.shard.empty) continue;
+      uint64_t lo, hi;
+      shard_bytes(q.shard, files[q.file]->data(), files[q.file]->size(), &lo, &hi);
+      if (!reader) reader = std::make_unique<ChunkReader>(paths[q.file], chunk_bytes, direct);
+      else reader->reopen(paths[q.file], direct);
+      reader->run(e, lo, hi, log_progress ? &progress : nullptr, same_run);
+      same_run = true;
     }
-  } catch (const std::exception& ex) {
-    *err = ex.what();
+    const int rc = ngsq_finish(e);
+    if (rc == NGSQ_E_QUAL_CAP && attempt == 0) {
+      ngsq_stats st;
+      check(e, ngsq_get_stats(e, &st));
+      info("  [*] Reads of up to " + std::to_string(st.max_read_len) + " bases: enlarging the quality table and reading the " +
+           (queue.size() > 1 ? "files" : "file") + " again.");
+      check(e, ngsq_reset(e));
+      check(e, ngsq_set_quality_positions(e, (uint32_t)st.max_read_len + 1));
+      continue;
+    }
+    if (!rc && log_progress) progress.report(e);
+    return rc;
   }
 }
 
-// `--cuda-also`: a device's queue of whole files through one engine, ngsq_next_file behind each, then one ngsq_finish.  A read
-// longer than the quality table in any of them enlarges the table and runs the whole queue again, as run_shard does for one file.
-void run_queue(ngsq_engine* e, const std::vector<FilePart>& queue, const std::vector<std::string>& paths, const std::vector<const MappedFile*>& files,
-               size_t chunk_bytes, bool direct, bool log_progress, std::string* err) {
-  try {
-    std::unique_ptr<ChunkReader> reader;
-    for (int attempt = 0;; ++attempt) {
-      Progress progress;
-      for (size_t k = 0; k < queue.size(); ++k) {
-        const FilePart& q = queue[k];
-        uint64_t lo, hi;
-        shard_bytes(q.shard, files[q.file]->data(), files[q.file]->size(), &lo, &hi);
-        if (!reader) reader = std::make_unique<ChunkReader>(paths[q.file], chunk_bytes, direct);
-        else reader->reopen(paths[q.file], direct);
-        check(e, ngsq_set_range(e, q.shard.first_voffset, 0));
-        reader->run(e, lo, hi, log_progress ? &progress : nullptr, k > 0);
-        check(e, ngsq_next_file(e));
-      }
-      const int rc = ngsq_finish(e);
-      if (rc == NGSQ_E_QUAL_CAP && attempt == 0) {
-        ngsq_stats st;
-        check(e, ngsq_get_stats(e, &st));
-        info("  [*] Reads of up to " + std::to_string(st.max_read_len) + " bases: enlarging the quality table and reading the files again.");
-        check(e, ngsq_reset(e));
-        check(e, ngsq_set_quality_positions(e, (uint32_t)st.max_read_len + 1));
-        continue;
-      }
-      check(e, rc);
-      if (log_progress) progress.report(e);
-      break;
-    }
-  } catch (const std::exception& ex) {
-    *err = ex.what();
-  }
-}
-
-// The parts of a file cut without an index (plan_shards_unindexed), one thread per engine.  An anchor is proven when the
-// range in front of it closes on it; the first record after the header is proven, so the cuts are proven in file order: a
-// part whose start is proven and that fails with NGSQ_E_CHAIN or NGSQ_E_TRUNCATED, with a next part behind it, ends on a
-// false anchor.  That cut is dropped: the part is run again over both ranges, the next engine over an empty one.  Any other
-// failure is the file's and is reported.  On return every engine has finished; shards holds the ranges that ran.
-void run_parts(const std::vector<ngsq_engine*>& engines, std::vector<Shard>& shards, const std::string& path, const MappedFile& file,
-               size_t chunk_bytes, bool direct) {
+// Every engine over its queue, one thread each; only engine 0 logs progress.  When the plan is cut, the shards of a file start
+// at record anchors that are speculative until the run proves them.  An anchor is proven when the range in front of it closes
+// on it; a file's first record after the header is proven, so the cuts are proven in file order: a part whose start is proven
+// and that fails with NGSQ_E_CHAIN or NGSQ_E_TRUNCATED, with a next part of the same file behind it, ends on a false anchor.
+// That cut is dropped: the part is run again over both ranges, the next engine over an empty one.  Any other failure is the
+// file's and is reported.  On return every engine has finished and the plan holds the ranges that ran.
+void run_plan(const std::vector<ngsq_engine*>& engines, FilePlan& plan, const std::vector<std::string>& paths, const std::vector<const MappedFile*>& files,
+              size_t chunk_bytes, bool direct) {
   const size_t n = engines.size();
   std::vector<std::string> errs(n);
   std::vector<int> codes(n, 0);
-  {
-    std::vector<std::thread> ts;
-    for (size_t i = 0; i < n; ++i)
-      ts.emplace_back(run_shard, engines[i], std::cref(path), std::cref(file), std::cref(shards[i]), chunk_bytes, direct, i == 0, &errs[i], &codes[i]);
-    for (auto& t : ts) t.join();
-  }
+  auto run = [&](size_t i, bool log_progress) {
+    try {
+      codes[i] = stream_queue(engines[i], plan.queues[i], paths, files, chunk_bytes, direct, log_progress);
+      check(engines[i], codes[i]);
+    } catch (const std::exception& ex) {
+      errs[i] = ex.what();
+    }
+  };
+  on_each(n, [&](size_t i) { run(i, i == 0); });
   for (size_t k = 0; k < n; ++k) {
     while (!errs[k].empty()) {
-      size_t j = k + 1;  // the next live part: its start is the cut in question
-      while (j < n && shards[j].empty) ++j;
-      if (j == n || (codes[k] != NGSQ_E_CHAIN && codes[k] != NGSQ_E_TRUNCATED)) throw std::runtime_error(errs[k]);
-      info("  [*] The record anchor at virtual offset " + std::to_string(shards[j].first_voffset) +
+      if (!plan.cut) throw std::runtime_error(errs[k]);
+      const uint32_t f = plan.queues[k][0].file;
+      size_t j = k + 1;  // the next live part of the file: its start is the cut in question
+      while (j < n && plan.queues[j][0].file == f && plan.queues[j][0].shard.empty) ++j;
+      if (j == n || plan.queues[j][0].file != f || (codes[k] != NGSQ_E_CHAIN && codes[k] != NGSQ_E_TRUNCATED)) throw std::runtime_error(errs[k]);
+      Shard& part = plan.queues[k][0].shard;
+      Shard& next = plan.queues[j][0].shard;
+      info("  [*] The record anchor at virtual offset " + std::to_string(next.first_voffset) +
            " is not a record start: dropping that cut and reading the range again.");
-      shards[k].end_voffset = shards[j].end_voffset;
-      shards[j] = Shard();
-      shards[j].empty = true;
+      part.end_voffset = next.end_voffset;
+      next = Shard();
+      next.empty = true;
       for (size_t i : {k, j}) {
         check(engines[i], ngsq_reset(engines[i]));
         errs[i].clear();
         codes[i] = 0;
       }
-      run_shard(engines[j], path, file, shards[j], chunk_bytes, direct, false, &errs[j], &codes[j]);
-      if (!errs[j].empty()) throw std::runtime_error(errs[j]);
-      run_shard(engines[k], path, file, shards[k], chunk_bytes, direct, false, &errs[k], &codes[k]);
+      check(engines[j], stream_queue(engines[j], plan.queues[j], paths, files, chunk_bytes, direct, false));
+      run(k, false);
     }
   }
 }
 
-// `--cuda-also`: the plan's queues, one thread per engine (run_queue), or with fewer files than engines each file's parts through
-// run_parts on that file's engines, the files side by side.  On return every engine has finished; a cut file's queue entries
-// hold the ranges that ran.
-void run_files(const std::vector<ngsq_engine*>& engines, FilePlan& plan, const std::vector<std::string>& paths, const std::vector<const MappedFile*>& files,
-               size_t chunk_bytes, bool direct) {
-  const size_t n = engines.size();
-  std::vector<std::string> errs(n);
-  std::vector<std::thread> ts;
-  for (size_t i = 0, j; i < n; i = j) {
-    j = i + 1;
-    if (!plan.cut) {
-      ts.emplace_back(run_queue, engines[i], std::cref(plan.queues[i]), std::cref(paths), std::cref(files), chunk_bytes, direct, i == 0, &errs[i]);
-      continue;
-    }
-    const uint32_t f = plan.queues[i][0].file;
-    while (j < n && plan.queues[j][0].file == f) ++j;
-    ts.emplace_back([&, i, j, f] {
-      std::vector<ngsq_engine*> group(engines.begin() + i, engines.begin() + j);
-      std::vector<Shard> shards;
-      for (size_t k = i; k < j; ++k) shards.push_back(plan.queues[k][0].shard);
-      try {
-        run_parts(group, shards, paths[f], *files[f], chunk_bytes, direct);
-      } catch (const std::exception& ex) {
-        errs[i] = ex.what();
-      }
-      for (size_t k = i; k < j; ++k) plan.queues[k][0].shard = shards[k - i];
-    });
-  }
-  for (auto& t : ts) t.join();
-  for (auto& s : errs) if (!s.empty()) throw std::runtime_error(s);
+// A one-file ShardPlan as a FilePlan: one entry per device.  cut: the shards start at record anchors found in the file
+// (plan_shards_unindexed), which the run proves.
+FilePlan file_plan_of(const ShardPlan& p, bool cut) {
+  FilePlan plan;
+  for (const Shard& s : p.shards) plan.queues.push_back({{0, s}});
+  plan.split = p.split;
+  plan.cut = cut;
+  plan.dropped = p.dropped;
+  return plan;
 }
 
 // The record anchor finder of plan_shards_unindexed on engine e (after ngsq_set_references)
@@ -336,11 +310,11 @@ FindRecord engine_finder(ngsq_engine* e) {
   return [e](const uint8_t* p, size_t n, uint64_t off, uint64_t* voff, int32_t* ref) { check(e, ngsq_find_record(e, p, n, off, voff, ref)); };
 }
 
-// The parts' .bai (or uncompressed .csi), in file order (engines with an empty range hold no part)
-std::vector<uint8_t> join_parts(const std::vector<ngsq_engine*>& engines, const std::vector<Shard>& shards, bool csi = false) {
+// The parts' .bai (or uncompressed .csi) of a one-file plan that has run, in file order (engines with an empty range hold no part)
+std::vector<uint8_t> join_parts(const std::vector<ngsq_engine*>& engines, const FilePlan& plan, bool csi) {
   std::vector<ngsq_engine*> parts;
   for (size_t i = 0; i < engines.size(); ++i)
-    if (!shards[i].empty) parts.push_back(engines[i]);
+    if (!plan.queues[i][0].shard.empty) parts.push_back(engines[i]);
   auto join = csi ? ngsq_join_csi : ngsq_join_bai;
   size_t n = 0;
   check(parts[0], join(parts.data(), (uint32_t)parts.size(), nullptr, 0, &n));
@@ -394,8 +368,8 @@ void write_index(const std::string& dst, const std::vector<uint8_t>& bai) {
   if (close(fd)) { std::filesystem::remove(dst); throw std::runtime_error("write error on " + dst); }
 }
 
-void log_dropped_cuts(const ShardPlan& plan) {
-  if (plan.dropped) info("  [*] " + std::to_string(plan.dropped) + " cut(s) left out: no record start found behind the target, or the anchor repeats.");
+void log_dropped_cuts(uint32_t dropped) {
+  if (dropped) info("  [*] " + std::to_string(dropped) + " cut(s) left out: no record start found behind the target, or the anchor repeats.");
 }
 
 // command.rs:226-421
@@ -438,7 +412,7 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   if (edits) flags |= NGSQ_F_EDITS;
   if (args.by_read_group) flags |= NGSQ_F_READ_GROUPS;  // --only leaves a record facet here (check_read_group_facet)
   if (args.verify_crc) flags |= NGSQ_F_VERIFY_CRC;
-  if (build_index) flags |= (n_dev > 1 ? NGSQ_F_INDEX_PART : NGSQ_F_INDEX) | (build_csi ? NGSQ_F_INDEX_CSI : 0u);
+  if (build_index) flags |= NGSQ_F_INDEX_PART | (build_csi ? NGSQ_F_INDEX_CSI : 0u);
   if (args.num_records && n_dev > 1) throw std::runtime_error("-n needs a single device (records are counted in file order)");
   // --cuda-by-read-group: the groups are the union of the files' @RG IDs, checked before any device work
   std::vector<std::string> rg_ids;
@@ -491,45 +465,39 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   for (auto& f : facets.record_based) info(std::string("  [*] ") + f->name() + ", " + to_string(f->computational_load()));
   for (auto& f : facets.sequence_based) info(std::string("  [*] ") + f->name() + ", " + to_string(f->computational_load()));
 
-  // shards: contig-aligned file ranges from the index (BAI or CSI), or ranges cut inside contigs when those leave a device idle or
-  // unbalanced (choose_shards); a contig cut between shards is declared on every engine and merged by ngsq_reduce
+  // every device's queue of (file, shard) entries.  Records in any order (and several files): whole files queued on the devices,
+  // or each file cut at record anchors between its devices, every reference split on several devices (plan_files).  Without an
+  // index on several devices: the file cut at record anchors (plan_shards_unindexed).  Otherwise contig-aligned file ranges from
+  // the index (BAI or CSI), or ranges cut inside contigs when those leave a device idle or unbalanced (choose_shards).  A
+  // contig cut between shards is declared on every engine and merged by ngsq_reduce.
   std::vector<uint32_t> ref_len;
   for (auto& rs : header.reference_sequences) ref_len.push_back(rs.length);
-  ShardPlan plan;
   const bool several_files = !args.also.empty();
-  const bool cut_at_anchors = !several_files && (build_index || args.any_order) && n_dev > 1;
-  FilePlan file_plan;
-  if (several_files) {
-    // whole files queued on the devices, or each file cut between its devices; every reference split on several devices
-    if (n_dev > 1) check(engines[0], ngsq_set_references(engines[0], (uint32_t)ref_len.size(), ref_len.data(), std::vector<uint8_t>(ref_len.size(), 0).data()));
-    file_plan = plan_files(headers, data, sizes, n_dev, n_dev > 1 ? engine_finder(engines[0]) : FindRecord());
-    plan.dropped = file_plan.dropped;
-    log_dropped_cuts(plan);
-    if (n_dev > 1)
-      for (uint32_t c = 0; c < ref_len.size(); ++c) plan.split.push_back(c);
-  } else if (cut_at_anchors) {
-    // no index to cut at: anchors from the records (the finder needs the references; every engine sets them again below)
+  FindRecord find;  // the anchor finder needs the references (every engine sets them again below)
+  if (n_dev > 1 && (args.any_order || build_index)) {
     check(engines[0], ngsq_set_references(engines[0], (uint32_t)ref_len.size(), ref_len.data(), std::vector<uint8_t>(ref_len.size(), 0).data()));
-    const FindRecord find = engine_finder(engines[0]);
-    plan = args.any_order ? plan_shards_any_order(header, file.data(), file.size(), n_dev, find)
-                          : plan_shards_unindexed(header, file.data(), file.size(), n_dev, find);
-    log_dropped_cuts(plan);
-  } else if (args.any_order) {
-    plan = plan_shards_any_order(header, file.data(), file.size(), 1, nullptr);
-  } else {
-    plan = choose_shards(header, bai, n_dev, file.size());
+    find = engine_finder(engines[0]);
   }
-  std::vector<Shard> shards = plan.shards;
-  if (several_files) {
-    info("  [*] " + std::to_string(paths.size()) + " files of one sample" +
-         (n_dev == 1 ? std::string(" on one device.")
-                     : std::string(file_plan.cut ? ", each cut between its devices" : ", whole files queued on the devices") + ", every reference split."));
-  } else if (args.any_order && n_dev > 1) {
-    info("  [*] Records in any order: " + std::to_string(n_dev - plan.dropped) + " shards, every reference split.");
-  } else if (plan.split_plan) {
-    std::string names;
-    for (uint32_t c : plan.split) names += (names.empty() ? "" : ", ") + header.reference_sequences[c].name;
-    info("  [*] Sharding inside contigs: " + std::to_string(n_dev) + " shards" + (names.empty() ? std::string() : ", split: " + names) + ".");
+  FilePlan plan;
+  if (args.any_order) {
+    plan = plan_files(headers, data, sizes, n_dev, find);
+    log_dropped_cuts(plan.dropped);
+    if (several_files)
+      info("  [*] " + std::to_string(paths.size()) + " files of one sample" +
+           (n_dev == 1 ? std::string(" on one device.")
+                       : std::string(plan.cut ? ", each cut between its devices" : ", whole files queued on the devices") + ", every reference split."));
+    else if (n_dev > 1)
+      info("  [*] Records in any order: " + std::to_string(n_dev - plan.dropped) + " shards, every reference split.");
+  } else {
+    const bool cut = build_index && n_dev > 1;
+    const ShardPlan p = cut ? plan_shards_unindexed(header, file.data(), file.size(), n_dev, find) : choose_shards(header, bai, n_dev, file.size());
+    log_dropped_cuts(p.dropped);
+    if (p.split_plan) {
+      std::string names;
+      for (uint32_t c : p.split) names += (names.empty() ? "" : ", ") + header.reference_sequences[c].name;
+      info("  [*] Sharding inside contigs: " + std::to_string(n_dev) + " shards" + (names.empty() ? std::string() : ", split: " + names) + ".");
+    }
+    plan = file_plan_of(p, cut);
   }
   for (uint32_t i = 0; i < n_dev; ++i) {
     // the same mask on every engine: the packed result buffer (the NCCL payload) is laid out from it, and a
@@ -547,46 +515,20 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
   if (n_dev > 1) {
     char id[128];
     if (ngsq_nccl_unique_id(id)) throw std::runtime_error(std::string("NCCL: ") + ngsq_last_error(nullptr));
-    std::vector<std::thread> ts;
-    std::vector<std::string> errs(n_dev);
-    for (uint32_t i = 0; i < n_dev; ++i)
-      ts.emplace_back([&, i] { if (ngsq_comm_init(engines[i], (int)n_dev, (int)i, id)) errs[i] = ngsq_last_error(engines[i]); });
-    for (auto& t : ts) t.join();
-    for (auto& s : errs) if (!s.empty()) throw std::runtime_error("NCCL: " + s);
+    on_each(n_dev, [&](size_t i) {
+      if (ngsq_comm_init(engines[i], (int)n_dev, (int)i, id)) throw std::runtime_error(std::string("NCCL: ") + ngsq_last_error(engines[i]));
+    });
   }
 
   // the hot path: one thread per GPU
   info("Starting CUDA pass for QC stats.");
   const auto t_hot = std::chrono::steady_clock::now();
-  if (several_files) {
-    run_files(engines, file_plan, paths, files, args.chunk_mb << 20, args.direct_io);
-  } else if (cut_at_anchors) {
-    run_parts(engines, shards, args.src, file, args.chunk_mb << 20, args.direct_io);
-  } else {
-    std::vector<std::thread> ts;
-    std::vector<std::string> errs(n_dev);
-    for (uint32_t i = 0; i < n_dev; ++i)
-      ts.emplace_back(run_shard, engines[i], std::cref(args.src), std::cref(file), std::cref(shards[i]), args.chunk_mb << 20, args.direct_io, i == 0, &errs[i], nullptr);
-    for (auto& t : ts) t.join();
-    for (auto& s : errs) if (!s.empty()) throw std::runtime_error(s);
-  }
-  if (n_dev > 1) {
-    std::vector<std::thread> ts;
-    std::vector<std::string> errs(n_dev);
-    for (uint32_t i = 0; i < n_dev; ++i) ts.emplace_back([&, i] { if (ngsq_reduce(engines[i], 0)) errs[i] = ngsq_last_error(engines[i]); });
-    for (auto& t : ts) t.join();
-    for (auto& s : errs) if (!s.empty()) throw std::runtime_error("NCCL: " + s);
-  }
+  run_plan(engines, plan, paths, files, args.chunk_mb << 20, args.direct_io);
+  if (n_dev > 1)
+    on_each(n_dev, [&](size_t i) { if (ngsq_reduce(engines[i], 0)) throw std::runtime_error(std::string("NCCL: ") + ngsq_last_error(engines[i])); });
   // the index of this pass: joined (and its order checked) before any output is written
   std::vector<uint8_t> new_index;
-  if (build_index && n_dev > 1) new_index = join_parts(engines, shards, build_csi);
-  else if (build_index) {
-    auto get = build_csi ? ngsq_get_csi : ngsq_get_bai;
-    size_t n = 0;
-    check(engines[0], get(engines[0], nullptr, 0, &n));
-    new_index.resize(n);
-    check(engines[0], get(engines[0], new_index.data(), new_index.size(), &n));
-  }
+  if (build_index) new_index = join_parts(engines, plan, build_csi);
   const double hot_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_hot).count();
   ngsq_engine* root = engines[0];
   uint64_t n_records = 0;
@@ -638,7 +580,7 @@ int app(const QcArgs& args, const ReferenceGenome& genome, const std::string& ou
          << ",\"ms_total\":" << st.ms_total << ",\"ms_tail\":" << st.ms_tail << ",\"waves\":" << st.waves << ",\"wall_ms_file_to_results\":" << hot_ms;
       if (several_files) {
         uint32_t n_files = 0;
-        for (const FilePart& q : file_plan.queues[i]) n_files += q.shard.empty ? 0 : 1;
+        for (const FilePart& q : plan.queues[i]) n_files += q.shard.empty ? 0 : 1;
         pf << ",\"files\":" << n_files;
       }
       pf << "}";
@@ -660,66 +602,23 @@ int qc(const QcArgs& args) {
   return app(args, *genome, prefix, outdir);
 }
 
-// `ngs index` for a BAM (src/index/bam.rs:39-109): the header, then every record through the engine's NGSQ_F_INDEX pass, and
-// the .bai next to the file (utils/pathbuf.rs:59-75: x.bam -> x.bam.bai).  Like the reference (bam.rs:52-58) it never
-// overwrites an existing index.
+// `ngs index` for a BAM (src/index/bam.rs:39-109): the header, then every record through the engines' NGSQ_F_INDEX_PART pass,
+// and the .bai next to the file (utils/pathbuf.rs:59-75: x.bam -> x.bam.bai).  Like the reference (bam.rs:52-58) it never
+// overwrites an existing index.  On several devices the file is cut at record anchors, one engine and one thread per part,
+// and the parts are joined on the host; one device indexes one part from the first record to EOF.  No collective is involved,
+// so a device may repeat.
 struct IndexArgs {
   std::string src;
   bool csi = false;          // --csi: <BAM>.csi (BGZF) instead of <BAM>.bai
   uint32_t min_shift = 14;   // -m / --min-shift (CSI); the depth follows samtools' rule
-  int device = 0;
+  int device = 0;            // --cuda-device: the one device when --cuda-devices names none
   std::vector<int> devices;  // --cuda-devices: several engines, one part of the file each
   bool verify_crc = true;
   size_t chunk_mb = 64;
   bool direct_io = true;
 };
 
-// the index file of the engine(s): the .bai as it is, the .csi payload BGZF-compressed
-void write_index_file(const IndexArgs& a, const std::string& dst, const std::vector<uint8_t>& payload) {
-  write_index(dst, a.csi ? bgzf_compress(payload) : payload);
-}
-
-int index_bam(const IndexArgs& a) {
-  info("Starting index command...");
-  const std::string dst = a.src + (a.csi ? ".csi" : ".bai");
-  if (std::filesystem::exists(dst)) throw std::runtime_error("index file already exists: " + dst);
-  MappedFile file(a.src);
-  ngsq_config cfg{};
-  cfg.struct_size = sizeof cfg;
-  cfg.flags = NGSQ_F_INDEX | (a.verify_crc ? NGSQ_F_VERIFY_CRC : 0u) | (a.csi ? NGSQ_F_INDEX_CSI : 0u);
-  ngsq_engine* e = nullptr;
-  if (ngsq_create(a.device, &cfg, &e)) throw std::runtime_error(std::string("CUDA engine: ") + ngsq_last_error(nullptr));
-  struct Cleanup { ngsq_engine* e; ~Cleanup() { ngsq_destroy(e); } } cleanup{e};
-  BamHeader header = read_bam_header(e, file.data(), file.size());
-  std::vector<uint32_t> ref_len;
-  for (auto& rs : header.reference_sequences) ref_len.push_back(rs.length);
-  std::vector<uint8_t> no_coverage(ref_len.size(), 0);
-  if (a.csi) check(e, ngsq_set_index_binning(e, a.min_shift, 0));
-  check(e, ngsq_set_references(e, (uint32_t)ref_len.size(), ref_len.data(), no_coverage.data()));
-  check(e, ngsq_set_range(e, header.first_record_voffset, 0));
-  info("Indexing BAM file.");
-  {
-    ChunkReader reader(a.src, a.chunk_mb << 20, a.direct_io);
-    Progress progress;
-    reader.run(e, std::min<uint64_t>(header.first_record_voffset >> 16, file.size()), file.size(), &progress);
-    check(e, ngsq_finish(e));
-    progress.report(e);
-  }
-  ngsq_stats st;
-  check(e, ngsq_get_stats(e, &st));
-  info("Processed " + std::to_string(st.records) + " records.");
-  auto get = a.csi ? ngsq_get_csi : ngsq_get_bai;
-  size_t n = 0;
-  check(e, get(e, nullptr, 0, &n));
-  std::vector<uint8_t> bai(n);
-  check(e, get(e, bai.data(), bai.size(), &n));
-  write_index_file(a, dst, bai);
-  return 0;
-}
-
-// `index` on several devices: the file cut at record anchors, one NGSQ_F_INDEX_PART engine and one thread per part, the parts
-// joined on the host.  No collective is involved, so a device may repeat.
-int index_bam_parts(const IndexArgs& a) {
+int index_command(const IndexArgs& a) {
   info("Starting index command...");
   const std::string dst = a.src + (a.csi ? ".csi" : ".bai");
   if (std::filesystem::exists(dst)) throw std::runtime_error("index file already exists: " + dst);
@@ -741,14 +640,16 @@ int index_bam_parts(const IndexArgs& a) {
     if (a.csi) check(e, ngsq_set_index_binning(e, a.min_shift, 0));
     check(e, ngsq_set_references(e, (uint32_t)ref_len.size(), ref_len.data(), no_coverage.data()));
   }
-  ShardPlan plan = plan_shards_unindexed(header, file.data(), file.size(), (uint32_t)n_dev, engine_finder(engines[0]));
-  log_dropped_cuts(plan);
-  info("Indexing BAM file in " + std::to_string(n_dev - plan.dropped) + " parts.");
-  run_parts(engines, plan.shards, a.src, file, a.chunk_mb << 20, a.direct_io);
+  const ShardPlan p = plan_shards_unindexed(header, file.data(), file.size(), (uint32_t)n_dev, engine_finder(engines[0]));
+  log_dropped_cuts(p.dropped);
+  info(n_dev == 1 ? std::string("Indexing BAM file.") : "Indexing BAM file in " + std::to_string(n_dev - p.dropped) + " parts.");
+  FilePlan plan = file_plan_of(p, true);
+  run_plan(engines, plan, {a.src}, {&file}, a.chunk_mb << 20, a.direct_io);
   uint64_t records = 0;
   for (auto* e : engines) { ngsq_stats st; check(e, ngsq_get_stats(e, &st)); records += st.records; }
   info("Processed " + std::to_string(records) + " records.");
-  write_index_file(a, dst, join_parts(engines, plan.shards, a.csi));
+  const std::vector<uint8_t> payload = join_parts(engines, plan, a.csi);
+  write_index(dst, a.csi ? bgzf_compress(payload) : payload);  // the .csi is BGZF
   return 0;
 }
 
@@ -772,9 +673,8 @@ int index_main(int argc, char** argv, int i) {
   if (min_shift_set && !a.csi) throw std::runtime_error("--min-shift sets the binning of a CSI: use it with --csi");
   if (pos.size() != 1 || !a.chunk_mb) return -1;
   a.src = pos[0];
-  if (a.devices.size() > 1) return index_bam_parts(a);
-  if (a.devices.size() == 1) a.device = a.devices[0];
-  return index_bam(a);
+  if (a.devices.empty()) a.devices = {a.device};
+  return index_command(a);
 }
 
 void usage() {
